@@ -19,6 +19,7 @@ refinement; `--pairs` pairs per GPU per step (default 10 000 = the config's batc
 
 Launch: python bench.py --gpus N --steps K --warmup W   (N>1 under torchrun, one rank per GPU)
         python bench.py --impl reference …              (the reference arm: CPU path only)
+        python bench.py … --dump-outputs DIR            (also writes the last timed step's results, see dump_outputs)
 """
 import argparse
 import json
@@ -46,7 +47,14 @@ def parse_args():
     ap.add_argument("--pairs", type=int, default=10000, help="image pairs per GPU per step")
     ap.add_argument("--cpu-sample", type=int, default=0, help="pairs in the CPU baseline sample (0 = auto)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (rank 0's pairs when --gpus > 1)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the GPU arm (--impl ours)")
+    return args
 
 
 def bench_config(cfg_name, c, pairs, world):
@@ -197,6 +205,32 @@ def _emit(line):
         os.write(_REAL_STDOUT, data)
 
 
+DUMP_BYTES = 64_000_000   # --dump-outputs writes at most this much, .npy headers included
+
+
+def dump_outputs(out_dir, offsets, models, stats, masks):
+    """What one estimate call returned, as float arrays two builds can be compared by:
+      models.npy      [P,12] f64  q (4), t (3), scale, shift1, shift2, f1, f2
+      stats.npy       [P,5]  f64  refinements, iterations, num_inliers, inlier_ratio, model_score
+      masks.npy       [M]    f32  inlier masks of the pairs in mask_pairs.npy, concatenated
+      mask_pairs.npy  [K]    f64  those pairs: all of them, or a fixed seeded sample when all masks (one value per match)
+                                  would not fit in DUMP_BYTES"""
+    from mdrp_b200 import _native as nv
+    st = stats.view(nv.STATS_DTYPE).reshape(-1)
+    out = {"models": np.ascontiguousarray(models, dtype=np.float64),
+           "stats": np.stack([st[f].astype(np.float64) for f in nv.STATS_DTYPE.names], axis=1)}
+    P = len(offsets) - 1
+    lens = np.diff(offsets)
+    budget = DUMP_BYTES - sum(a.nbytes for a in out.values()) - 8 * P - 4 * 1024
+    order = np.random.default_rng(0).permutation(P)
+    pairs = np.sort(order[:int(np.searchsorted(np.cumsum(4 * lens[order]), budget, side="right"))])
+    out["masks"] = np.concatenate([masks[offsets[i]:offsets[i + 1]] for i in pairs] or [masks[:0]]).astype(np.float32)
+    out["mask_pairs"] = pairs.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     args = parse_args()
     _claim_stdout()
@@ -293,6 +327,8 @@ def main():
     elapsed = e0.elapsed_time(e1) / 1000.0
     launches = ctx.launch_count - launches0
     clk = clocks.stop(t_timed)
+    # the last timed step's results, read back after the timed region; the legs below write other buffers
+    last_outputs = (d_models.cpu().numpy(), d_stats.cpu().numpy(), d_masks[:N].cpu().numpy()) if args.dump_outputs else None
     t = torch.tensor([elapsed], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -341,6 +377,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, offs, *last_outputs)
 
     # ---- rooflines ---------------------------------------------------------------------------------------------
     # Every kernel that holds > 10 % of the step gets an entry: its algorithmic work (stated in DESIGN.md §5, counted by
