@@ -140,6 +140,22 @@ RP_API int rp_estimate_batch_dev(rp_ctx *ctx, int variant, int64_t n_pairs, cons
                                  const double *cams, const rp_options *opt, rp_model *models,
                                  rp_stats *stats, uint8_t *masks, void *stream);
 
+/* The same two estimators for float32 keypoints and depths, the type matchers and depth networks produce: x1, x2, d1, d2
+ * are `const float *` with the layout above; cams, offsets, options and outputs are as above, and so are the argument
+ * checks and error codes.  The inputs are widened to FP64 on the device (float -> double is exact) and everything after
+ * that is the FP64 path, so the outputs are byte for byte those of rp_estimate_batch_host / _dev on the same values
+ * converted to double.  _host uploads 24 B per correspondence instead of 48 (double-buffered float staging, widened on
+ * the copy stream); _dev reads the caller's float arrays and needs 48 B per correspondence of the current chunk for the
+ * widened copy instead of an FP64 copy of the whole batch.  rp_last_timing slot [13] reports the widening time. */
+RP_API int rp_estimate_batch_host_f32(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets,
+                                      const float *x1, const float *x2, const float *d1, const float *d2,
+                                      const double *cams, const rp_options *opt, rp_model *models,
+                                      rp_stats *stats, uint8_t *masks);
+RP_API int rp_estimate_batch_dev_f32(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets,
+                                     const float *x1, const float *x2, const float *d1, const float *d2,
+                                     const double *cams, const rp_options *opt, rp_model *models,
+                                     rp_stats *stats, uint8_t *masks, void *stream);
+
 /* ---- stage entry points (parity tests; all pointers HOST memory) -----------------
  * Each mirrors one exported stage of the reference binary (SURVEY.md §8a). */
 
@@ -195,6 +211,16 @@ RP_API int rp_gather_depths_batch_dev(rp_ctx *ctx, int64_t n_pairs, const int64_
                                       const float *kp1, const float *kp2, double *x1, double *x2, double *d1, double *d2,
                                       int64_t *out_offsets, void *stream);
 
+/* The two gathers with float32 outputs x1, x2, d1, d2 (otherwise identical): what rp_estimate_batch_dev_f32 takes, so
+ * that the chain matcher -> gather -> estimate never holds an FP64 copy of its inputs. */
+RP_API int rp_gather_depths_dev_f32(rp_ctx *ctx, const float *depth1, int h1, int w1, const float *depth2, int h2, int w2,
+                                    const float *kp1, const float *kp2, int64_t n, float *x1, float *x2, float *d1,
+                                    float *d2, int64_t *n_out, void *stream);
+RP_API int rp_gather_depths_batch_dev_f32(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_offsets, const float *depth_maps,
+                                          int n_frames, int h, int w, const int32_t *frame1, const int32_t *frame2,
+                                          const float *kp1, const float *kp2, float *x1, float *x2, float *d1, float *d2,
+                                          int64_t *out_offsets, void *stream);
+
 /* ---- measurement helpers ---------------------------------------------------------
  * Pipe micro-benchmarks for the roofline denominators SURVEY.md §8d asks for (the driver's
  * MEASURED_PEAKS.json has only HBM and bf16): sustained FP64 and FP32 FMA throughput of
@@ -216,7 +242,10 @@ RP_API int rp_pair_status(const rp_ctx *ctx, int64_t n_pairs, int32_t *status);
 /* per-stage device time of the last rp_estimate_batch_* call on ctx, milliseconds (summed over chunks):
  * [0] prepare, [1] sample, [2] solve, [3] score(minimal: exact head + bound + prune + exact survivors),
  * [4] scan, [5] LO refine, [6] LO score+merge+final LO, [7] final refine, [8] total device, [9] H2D,
- * [10] D2H, [11] FP32 bound kernel alone, [12] tensor-core count tier alone, [13..15] reserved.
+ * [10] D2H, [11] FP32 bound kernel alone, [12] tensor-core count tier alone, [13] widening of float32 inputs to FP64
+ * (rp_estimate_batch_*_f32; 0 otherwise).  On the host path the widening runs on the copy stream after the H2D of [9],
+ * and for every chunk but the first it overlaps the previous chunk's kernels, so [13] there also counts the time the
+ * widening waits for SMs those kernels hold; the device path's [13] is the widening alone.  [14..15] reserved.
  * counters: [0] minimal models generated, [1] point-scores the FP32 bound kernel resolved (models x correspondences),
  * [2] LM problems, [3] LM iterations, [4] chunks (= launches of each pipeline kernel), [5] minimal models
  * that needed the exact scorer, [6] point-scores the FP32 bound kernel actually evaluated (before abandoning),

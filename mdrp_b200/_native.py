@@ -21,6 +21,7 @@ EXPORTS = [
     "rp_create", "rp_destroy", "rp_last_error", "rp_default_options", "rp_launch_count",
     "rp_estimate_batch_host", "rp_estimate_batch_dev", "rp_sample_batch", "rp_sample_batch_prosac", "rp_solve_batch",
     "rp_score_batch", "rp_refine_batch", "rp_measure_pipes", "rp_last_timing", "rp_gather_depths_dev", "rp_tc_count_batch", "rp_pair_status", "rp_gather_depths_batch_dev",
+    "rp_estimate_batch_host_f32", "rp_estimate_batch_dev_f32", "rp_gather_depths_dev_f32", "rp_gather_depths_batch_dev_f32",
 ]
 
 
@@ -99,6 +100,10 @@ def load():
     L.rp_estimate_batch_host.argtypes = est_args
     L.rp_estimate_batch_dev.restype = C.c_int
     L.rp_estimate_batch_dev.argtypes = est_args + [VP]
+    L.rp_estimate_batch_host_f32.restype = C.c_int
+    L.rp_estimate_batch_host_f32.argtypes = est_args
+    L.rp_estimate_batch_dev_f32.restype = C.c_int
+    L.rp_estimate_batch_dev_f32.argtypes = est_args + [VP]
     L.rp_sample_batch.restype = C.c_int
     L.rp_sample_batch.argtypes = [VP, C.c_int64, C.c_uint64, C.c_int64, VP]
     L.rp_sample_batch_prosac.restype = C.c_int
@@ -117,6 +122,10 @@ def load():
                                        C.POINTER(C.c_int64), VP]
     L.rp_gather_depths_batch_dev.restype = C.c_int
     L.rp_gather_depths_batch_dev.argtypes = [VP, C.c_int64, VP, VP, C.c_int, C.c_int, C.c_int, VP, VP, VP, VP, VP, VP, VP, VP, VP, VP]
+    for f in (L.rp_gather_depths_dev_f32, L.rp_gather_depths_batch_dev_f32):
+        f.restype = C.c_int
+    L.rp_gather_depths_dev_f32.argtypes = L.rp_gather_depths_dev.argtypes
+    L.rp_gather_depths_batch_dev_f32.argtypes = L.rp_gather_depths_batch_dev.argtypes
     L.rp_measure_pipes.restype = C.c_int
     L.rp_measure_pipes.argtypes = [VP, DP, DP]
     L.rp_pair_status.restype = C.c_int
@@ -137,12 +146,16 @@ def _f64(a):
     return np.ascontiguousarray(a, dtype=np.float64)
 
 
+def _f32(a):
+    return np.ascontiguousarray(a, dtype=np.float32)
+
+
 def _ptr(a):
     return a.ctypes.data if a is not None else None
 
 
 TIMING_KEYS = ["prepare", "sample", "solve", "score_minimal", "scan", "lo_refine", "lo_score_merge",
-               "final_refine", "device_total", "h2d", "d2h", "bound_kernel", "tc_kernel", "r13", "r14", "r15"]
+               "final_refine", "device_total", "h2d", "d2h", "bound_kernel", "tc_kernel", "widen", "r14", "r15"]
 COUNTER_KEYS = ["hypotheses", "point_scores", "lm_problems", "lm_iterations", "chunks", "exact_models",
                 "bound_evaluated", "head_models", "tc_evaluated", "tc_selected", "lm_flops", "c11", "c12", "c13", "c14", "c15"]
 
@@ -208,9 +221,17 @@ class Context:
     # ---- hot path -------------------------------------------------------------------------
     def estimate_batch_host(self, variant, offsets, x1, x2, d1, d2, cams, opt: Options):
         """Packed host arrays in, (models, stats, masks) numpy structured arrays out."""
+        return self._estimate_host(self._lib.rp_estimate_batch_host, _f64, variant, offsets, x1, x2, d1, d2, cams, opt)
+
+    def estimate_batch_host_f32(self, variant, offsets, x1, x2, d1, d2, cams, opt: Options):
+        """`estimate_batch_host` for float32 points and depths (rp_estimate_batch_host_f32): half the upload, the same
+        bytes out as `estimate_batch_host` on the values converted to float64."""
+        return self._estimate_host(self._lib.rp_estimate_batch_host_f32, _f32, variant, offsets, x1, x2, d1, d2, cams, opt)
+
+    def _estimate_host(self, fn, conv, variant, offsets, x1, x2, d1, d2, cams, opt):
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         n_pairs = len(offsets) - 1
-        x1, x2, d1, d2 = _f64(x1), _f64(x2), _f64(d1), _f64(d2)
+        x1, x2, d1, d2 = conv(x1), conv(x2), conv(d1), conv(d2)
         ntot = int(offsets[-1]) if n_pairs >= 0 else 0
         if x1.shape != (ntot, 2) or x2.shape != (ntot, 2) or d1.shape != (ntot,) or d2.shape != (ntot,):
             raise ValueError("x1/x2 must be [N,2] and d1/d2 [N] with N = offsets[-1]")
@@ -220,7 +241,7 @@ class Context:
         models = np.zeros(n_pairs, dtype=MODEL_DTYPE)
         stats = np.zeros(n_pairs, dtype=STATS_DTYPE)
         masks = np.zeros(max(ntot, 1), dtype=np.uint8)
-        self._call(self._lib.rp_estimate_batch_host,
+        self._call(fn,
             self._h, int(variant), n_pairs, _ptr(offsets), _ptr(x1), _ptr(x2), _ptr(d1), _ptr(d2),
             _ptr(cams), C.byref(opt), _ptr(models), _ptr(stats), _ptr(masks))
         return models, stats, masks[:ntot]
@@ -228,8 +249,19 @@ class Context:
     def estimate_batch_dev(self, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr, opt: Options,
                            models_ptr, stats_ptr, masks_ptr, stream=0):
         """Raw device pointers (e.g. torch tensor .data_ptr()); offsets is a host int64 array."""
+        self._estimate_dev(self._lib.rp_estimate_batch_dev, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr, opt,
+                           models_ptr, stats_ptr, masks_ptr, stream)
+
+    def estimate_batch_dev_f32(self, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr, opt: Options,
+                               models_ptr, stats_ptr, masks_ptr, stream=0):
+        """`estimate_batch_dev` with x1, x2, d1, d2 pointing at float32 device arrays (rp_estimate_batch_dev_f32)."""
+        self._estimate_dev(self._lib.rp_estimate_batch_dev_f32, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr,
+                           opt, models_ptr, stats_ptr, masks_ptr, stream)
+
+    def _estimate_dev(self, fn, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr, opt, models_ptr, stats_ptr,
+                      masks_ptr, stream):
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
-        self._call(self._lib.rp_estimate_batch_dev,
+        self._call(fn,
             self._h, int(variant), len(offsets) - 1, _ptr(offsets), x1_ptr, x2_ptr, d1_ptr, d2_ptr,
             cams_ptr, C.byref(opt), models_ptr, stats_ptr, masks_ptr, stream or None)
 

@@ -199,6 +199,41 @@ def _pack(list_x1, list_x2, list_d1, list_d2):
     return offsets, x1, x2, d1, d2
 
 
+def _all_float32(*lists):
+    """True when every point and depth array of the batch is float32 (and there is at least one pair): those batches take
+    the float32 entry points, which widen on the device and return the same bytes with half the upload."""
+    arrays = [a for xs in lists for a in xs]
+    return len(arrays) > 0 and all(getattr(a, "dtype", None) == np.float32 for a in arrays)
+
+
+def _pack_f32(list_x1, list_x2, list_d1, list_d2):
+    """`_pack` for a batch whose arrays are all float32 (`_all_float32`): the same checks and offsets, float32 packed
+    arrays, so no FP64 copy of the batch is made on the host."""
+    for a, b, c, d in zip(list_x1, list_x2, list_d1, list_d2):
+        if a.ndim != 2 or a.shape[1] != 2 or b.shape != a.shape:
+            raise TypeError("points must be [N, 2] arrays")
+        if not (len(a) == len(c) == len(d)):
+            raise ValueError("points and depths must have the same length")
+    offsets = np.zeros(len(list_d1) + 1, dtype=np.int64)
+    offsets[1:] = np.cumsum([len(d) for d in list_d1])
+    cat = lambda xs, shape: np.concatenate([np.asarray(x).reshape(shape) for x in xs])
+    return offsets, cat(list_x1, (-1, 2)), cat(list_x2, (-1, 2)), cat(list_d1, (-1,)), cat(list_d2, (-1,))
+
+
+def _pack_auto(list_x1, list_x2, list_d1, list_d2):
+    """`_pack_f32` when every array is float32, else `_pack` (float64)."""
+    if _all_float32(list_x1, list_x2, list_d1, list_d2):
+        return _pack_f32(list_x1, list_x2, list_d1, list_d2)
+    return _pack(list_x1, list_x2, list_d1, list_d2)
+
+
+def _estimate_host(ctx, variant, offsets, x1, x2, d1, d2, cams, opt):
+    """Packed host arrays through the float32 entry point when they are float32, else the FP64 one."""
+    if x1.dtype == np.float32 and x2.dtype == np.float32 and d1.dtype == np.float32 and d2.dtype == np.float32:
+        return ctx.estimate_batch_host_f32(variant, offsets, x1, x2, d1, d2, cams, opt)
+    return ctx.estimate_batch_host(variant, offsets, x1, x2, d1, d2, cams, opt)
+
+
 def _info(stats_row, mask):
     return {"refinements": int(stats_row["refinements"]), "iterations": int(stats_row["iterations"]),
             "num_inliers": int(stats_row["num_inliers"]), "inlier_ratio": float(stats_row["inlier_ratio"]),
@@ -212,20 +247,21 @@ def _geometry(m):
 # ---- batched entry points (the unit of GPU work) -----------------------------------------------------
 def estimate_monodepth_relative_pose_batch(points2D_1, points2D_2, depth_1, depth_2, cameras1, cameras2,
                                            ransac_opt=None, bundle_opt=None, device=0):
-    """Lists (one entry per image pair) in, list of (MonoDepthTwoViewGeometry, info) out."""
-    offsets, x1, x2, d1, d2 = _pack(points2D_1, points2D_2, depth_1, depth_2)
+    """Lists (one entry per image pair) in, list of (MonoDepthTwoViewGeometry, info) out.  When every point and depth
+    array is float32 the batch goes through the float32 entry point (same results, half the upload)."""
+    offsets, x1, x2, d1, d2 = _pack_auto(points2D_1, points2D_2, depth_1, depth_2)
     cams = np.array([Camera.from_any(a).fxfycxcy() + Camera.from_any(b).fxfycxcy()
                      for a, b in zip(cameras1, cameras2)], dtype=np.float64).reshape(-1, 8)
     opt = make_options(ransac_opt, bundle_opt, focal_variant=False)
     variant = nv.CALIB_SHIFT if opt.estimate_shift else nv.CALIB
-    models, stats, masks = context(device).estimate_batch_host(variant, offsets, x1, x2, d1, d2, cams, opt)
+    models, stats, masks = _estimate_host(context(device), variant, offsets, x1, x2, d1, d2, cams, opt)
     return [(_geometry(models[i]), _info(stats[i], masks[offsets[i]:offsets[i + 1]])) for i in range(len(models))]
 
 
 def _focal_batch(variant, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, bundle_opt, device):
-    offsets, x1, x2, d1, d2 = _pack(points2D_1, points2D_2, depth_1, depth_2)
+    offsets, x1, x2, d1, d2 = _pack_auto(points2D_1, points2D_2, depth_1, depth_2)
     opt = make_options(ransac_opt, bundle_opt, focal_variant=True)
-    models, stats, masks = context(device).estimate_batch_host(variant, offsets, x1, x2, d1, d2, None, opt)
+    models, stats, masks = _estimate_host(context(device), variant, offsets, x1, x2, d1, d2, None, opt)
     out = []
     for i, m in enumerate(models):
         pair = MonoDepthImagePair(_geometry(m), Camera("SIMPLE_PINHOLE", [m["f1"], 0.0, 0.0]),

@@ -10,6 +10,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "rp_kernels.cuh"
@@ -53,7 +54,9 @@ enum { B_OFFS, B_PAIRS, B_PTS64, B_PTS32, B_BEAR, B_SAMPLES, B_MODELS, B_HYPITER
        B_FEAT, B_TCOUT, B_TCLIST, B_TCLISTCNT, B_TCLISTPFX, B_PAIRCNT, B_TCPFX, B_TCSPLIT,
        // per-pair flags; re-run sub-batches (event-list overflow, early termination that needs more iterations)
        B_PAIRFLAGS, B_SUB_IDX, B_SUB_SRC, B_SUB_DST, B_SUB_X1, B_SUB_X2, B_SUB_D1, B_SUB_D2, B_SUB_CAMS, B_SUB_MODELS,
-       B_SUB_STATS, B_SUB_MASK, B_NBUF };
+       B_SUB_STATS, B_SUB_MASK,
+       // float32 inputs, host path: the chunk as uploaded (double-buffered), before it is widened into B_IN_*
+       B_F32_X1, B_F32_X2, B_F32_D1, B_F32_D2, B_F32_X1_B, B_F32_X2_B, B_F32_D1_B, B_F32_D2_B, B_NBUF };
 
 // device scalars living in B_SCALARS
 struct Scalars {
@@ -65,7 +68,7 @@ struct Scalars {
     unsigned long long tc_evaluated, tc_selected, lm_flops;
 };
 
-constexpr int N_EVENTS = 26;
+constexpr int N_EVENTS = 27;
 
 }  // namespace
 
@@ -690,13 +693,23 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
     return RP_OK;
 }
 
-size_t bytes_per_pair(int iters, long long avg_points, int ev_cap = EV) {
+size_t bytes_per_pair(int iters, long long avg_points, int ev_cap = EV, size_t input_bytes = 0) {
     const int nseg = std::max(1, cdiv(iters, SEG));
     const size_t slots_pp = (size_t)nseg * 4 * SEG;
     // per slot: model, hyp_iter, score, count, ub, lb, survivor list, tensor-core count + list; per correspondence:
-    // FP64 / FP32 / interleaved copies, bearings, mask, 128-byte feature row
+    // FP64 / FP32 / interleaved copies, bearings, mask, 128-byte feature row, `input_bytes` of input staging
     return slots_pp * (sizeof(Model) + 4 + 8 + 4 + 12 + 8) + (size_t)iters * 12 + (size_t)ev_cap * (sizeof(Model) + 24) +
-           (size_t)avg_points * (sizeof(Pt64) + 32 + sizeof(Bear) + 1 + 128) + 1024;
+           (size_t)avg_points * (sizeof(Pt64) + 32 + sizeof(Bear) + 1 + 128 + input_bytes) + 1024;
+}
+
+// widens a float32 chunk into the FP64 input arrays (no-op for an empty chunk)
+int launch_widen(rp_ctx *ctx, long long n, const float *x1, const float *x2, const float *d1, const float *d2, double *wx1,
+                 double *wx2, double *wd1, double *wd2, cudaStream_t st) {
+    if (n <= 0) return RP_OK;
+    const int grid = std::min<long long>(cdiv(2 * n, 256), 16LL * ctx->sms);
+    widen_inputs_kernel<<<grid, 256, 0, st>>>(n, x1, x2, d1, d2, wx1, wx2, wd1, wd2);
+    LAUNCHED();
+    return RP_OK;
 }
 
 int check_common(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const rp_options *opt) {
@@ -819,9 +832,14 @@ int rerun_flagged(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO
     return RP_OK;
 }
 
-int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const double *x1,
-                  const double *x2, const double *d1, const double *d2, const double *cams, const rp_options *opt_in,
+// In = double: the FP64 entry points.  In = float: rp_estimate_batch_*_f32 — the host path uploads the float chunk
+// (24 B per correspondence instead of 48) and widens it on the copy stream, the device path widens the caller's
+// chunk on the compute stream; either way every kernel after that reads the same FP64 chunk arrays as with In = double.
+template <class In>
+int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const In *x1,
+                  const In *x2, const In *d1, const In *d2, const double *cams, const rp_options *opt_in,
                   rp_model *models, rp_stats *stats, uint8_t *masks, bool host_io, cudaStream_t st) {
+    constexpr bool f32 = std::is_same<In, float>::value;
     int rc = check_common(ctx, variant, n_pairs, offsets, opt_in);
     if (rc) return rc;
     CK(cudaSetDevice(ctx->device));
@@ -842,14 +860,15 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
     const int iters0 = opt.min_iterations < opt.max_iterations
                            ? (int)std::min<int64_t>(opt.max_iterations, opt.min_iterations + 1)
                            : (int)opt.max_iterations;
-    const size_t bpp = bytes_per_pair(iters0, Ntot / n_pairs + 1, ctx->ev_cap0);
+    // float32 inputs: two 24-byte staging sets (host path) or the 48-byte widened copy (device path) per correspondence
+    const size_t bpp = bytes_per_pair(iters0, Ntot / n_pairs + 1, ctx->ev_cap0, f32 ? 48 : 0);
     int64_t chunk = (int64_t)std::max<size_t>(1, ctx->workspace_budget / bpp);
     chunk = std::min<int64_t>(chunk, 32768);
     std::vector<long long> rel;
     DevBuf *B = ctx->buf;
     // Chunk boundaries.  The remainder is split evenly (no tiny last chunk); on the host path a small first
     // chunk goes ahead so that the kernels start early and every later upload hides behind the previous
-    // chunk's kernels.  With U = upload time and C = kernel time of the whole batch, the exposed time
+    // chunk's kernels.  With U = upload time (+ widening, float32 inputs) and C = kernel time of the whole batch, the exposed time
     // f U + max(0, (1-f) U - f C) is smallest at f = U / (U + C); U / C is taken from the previous host call on
     // this context (1/8 of the batch before there is one).  Only timing depends on it, never results.
     std::vector<int64_t> bounds(1, 0);
@@ -872,9 +891,14 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
     static const int IN_X1[2] = {B_IN_X1, B_IN_X1_B}, IN_X2[2] = {B_IN_X2, B_IN_X2_B}, IN_D1[2] = {B_IN_D1, B_IN_D1_B},
                      IN_D2[2] = {B_IN_D2, B_IN_D2_B}, IN_CAMS[2] = {B_IN_CAMS, B_IN_CAMS_B}, OUT_M[2] = {B_TMP0, B_TMP0_B},
                      OUT_S[2] = {B_TMP1, B_TMP1_B}, OUT_K[2] = {B_MASK, B_MASK_B};
+    static const int F32_X1[2] = {B_F32_X1, B_F32_X1_B}, F32_X2[2] = {B_F32_X2, B_F32_X2_B}, F32_D1[2] = {B_F32_D1, B_F32_D1_B},
+                     F32_D2[2] = {B_F32_D2, B_F32_D2_B};
     cudaStream_t cs = ctx->copy_stream;
     cudaEvent_t *in_ready = &ctx->ev[12], *h2d_begin = &ctx->ev[14], *comp_done = &ctx->ev[16], *d2h_begin = &ctx->ev[18];
+    cudaEvent_t *h2d_end = &ctx->ev[23];  // float32 inputs: end of the upload, start of the widening (host path)
+    cudaEvent_t widen_begin = ctx->ev[25], widen_end = ctx->ev[26];  // float32 inputs, device path
     cudaEvent_t d2h_end = ctx->ev[11];
+    double widen_per_point0 = 0.0;  // float32 inputs, host path: widening time of chunk 0 per correspondence (ms)
     auto upload = [&](int64_t c) -> int {
         const int64_t p0 = bounds[c], p1 = bounds[c + 1];
         const int P = (int)(p1 - p0), par = (int)(c & 1);
@@ -886,11 +910,26 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
         CK(B[OUT_M[par]].reserve(sizeof(Model) * P)); CK(B[OUT_S[par]].reserve(sizeof(rp_stats) * P));
         CK(B[OUT_K[par]].reserve(nn));
         CK(cudaEventRecord(h2d_begin[par], cs));
-        CK(cudaMemcpyAsync(B[IN_X1[par]].p, x1 + 2 * o0, 16 * (size_t)N, cudaMemcpyHostToDevice, cs));
-        CK(cudaMemcpyAsync(B[IN_X2[par]].p, x2 + 2 * o0, 16 * (size_t)N, cudaMemcpyHostToDevice, cs));
-        CK(cudaMemcpyAsync(B[IN_D1[par]].p, d1 + o0, 8 * (size_t)N, cudaMemcpyHostToDevice, cs));
-        CK(cudaMemcpyAsync(B[IN_D2[par]].p, d2 + o0, 8 * (size_t)N, cudaMemcpyHostToDevice, cs));
-        if (pose) CK(cudaMemcpyAsync(B[IN_CAMS[par]].p, cams + 8 * p0, 64 * (size_t)P, cudaMemcpyHostToDevice, cs));
+        if constexpr (f32) {
+            CK(B[F32_X1[par]].reserve(8 * nn)); CK(B[F32_X2[par]].reserve(8 * nn));
+            CK(B[F32_D1[par]].reserve(4 * nn)); CK(B[F32_D2[par]].reserve(4 * nn));
+            CK(cudaMemcpyAsync(B[F32_X1[par]].p, x1 + 2 * o0, 8 * (size_t)N, cudaMemcpyHostToDevice, cs));
+            CK(cudaMemcpyAsync(B[F32_X2[par]].p, x2 + 2 * o0, 8 * (size_t)N, cudaMemcpyHostToDevice, cs));
+            CK(cudaMemcpyAsync(B[F32_D1[par]].p, d1 + o0, 4 * (size_t)N, cudaMemcpyHostToDevice, cs));
+            CK(cudaMemcpyAsync(B[F32_D2[par]].p, d2 + o0, 4 * (size_t)N, cudaMemcpyHostToDevice, cs));
+            if (pose) CK(cudaMemcpyAsync(B[IN_CAMS[par]].p, cams + 8 * p0, 64 * (size_t)P, cudaMemcpyHostToDevice, cs));
+            CK(cudaEventRecord(h2d_end[par], cs));
+            int rc2 = launch_widen(ctx, N, B[F32_X1[par]].as<float>(), B[F32_X2[par]].as<float>(), B[F32_D1[par]].as<float>(),
+                                   B[F32_D2[par]].as<float>(), B[IN_X1[par]].as<double>(), B[IN_X2[par]].as<double>(),
+                                   B[IN_D1[par]].as<double>(), B[IN_D2[par]].as<double>(), cs);
+            if (rc2) return rc2;
+        } else {
+            CK(cudaMemcpyAsync(B[IN_X1[par]].p, x1 + 2 * o0, 16 * (size_t)N, cudaMemcpyHostToDevice, cs));
+            CK(cudaMemcpyAsync(B[IN_X2[par]].p, x2 + 2 * o0, 16 * (size_t)N, cudaMemcpyHostToDevice, cs));
+            CK(cudaMemcpyAsync(B[IN_D1[par]].p, d1 + o0, 8 * (size_t)N, cudaMemcpyHostToDevice, cs));
+            CK(cudaMemcpyAsync(B[IN_D2[par]].p, d2 + o0, 8 * (size_t)N, cudaMemcpyHostToDevice, cs));
+            if (pose) CK(cudaMemcpyAsync(B[IN_CAMS[par]].p, cams + 8 * p0, 64 * (size_t)P, cudaMemcpyHostToDevice, cs));
+        }
         CK(cudaEventRecord(in_ready[par], cs));
         return RP_OK;
     };
@@ -920,7 +959,21 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
             io.models_out = B[OUT_M[par]].as<Model>(); io.stats_out = B[OUT_S[par]].as<rp_stats>();
             io.masks_out = B[OUT_K[par]].as<unsigned char>();
         } else {
-            io.x1 = x1 + 2 * o0; io.x2 = x2 + 2 * o0; io.d1 = d1 + o0; io.d2 = d2 + o0;
+            if constexpr (f32) {
+                // the chunk widened on the compute stream, ahead of its kernels (B_IN_* are free: run_chunk synchronises)
+                const size_t nn = (size_t)std::max<long long>(N, 1);
+                CK(B[B_IN_X1].reserve(16 * nn)); CK(B[B_IN_X2].reserve(16 * nn));
+                CK(B[B_IN_D1].reserve(8 * nn)); CK(B[B_IN_D2].reserve(8 * nn));
+                CK(cudaEventRecord(widen_begin, st));
+                rc = launch_widen(ctx, N, x1 + 2 * o0, x2 + 2 * o0, d1 + o0, d2 + o0, B[B_IN_X1].as<double>(), B[B_IN_X2].as<double>(),
+                                  B[B_IN_D1].as<double>(), B[B_IN_D2].as<double>(), st);
+                if (rc) return rc;
+                CK(cudaEventRecord(widen_end, st));
+                io.x1 = B[B_IN_X1].as<double>(); io.x2 = B[B_IN_X2].as<double>();
+                io.d1 = B[B_IN_D1].as<double>(); io.d2 = B[B_IN_D2].as<double>();
+            } else {
+                io.x1 = x1 + 2 * o0; io.x2 = x2 + 2 * o0; io.d1 = d1 + o0; io.d2 = d2 + o0;
+            }
             io.cams = pose ? cams + 8 * p0 : nullptr;
             io.models_out = (Model *)models + p0; io.stats_out = stats + p0; io.masks_out = masks + o0;
         }
@@ -930,10 +983,24 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
         for (int i = 0; i < P; ++i) ctx->pair_status[(size_t)(p0 + i)] = rel[i + 1] - rel[i] < 3 ? RP_PAIR_DEGENERATE : RP_PAIR_OK;
         rc = rerun_flagged(ctx, variant, opt, io, rel, flags, iters0, p0, st);
         if (rc) return rc;
+        if (f32 && !host_io) {
+            float ms = 0.f;
+            if (cudaEventElapsedTime(&ms, widen_begin, widen_end) == cudaSuccess) ctx->last_ms[13] += ms;
+        }
         if (host_io) {
             // run_chunk returned after synchronising the compute stream: results are complete
             float ms = 0.f;
-            if (cudaEventElapsedTime(&ms, h2d_begin[par], in_ready[par]) == cudaSuccess) ctx->last_ms[9] += ms;
+            if (f32) {
+                if (cudaEventElapsedTime(&ms, h2d_begin[par], h2d_end[par]) == cudaSuccess) ctx->last_ms[9] += ms;
+                // widening of chunks c >= 1 runs while chunk c-1's kernels hold the SMs, so its interval includes waiting
+                // for them; chunk 0's is the widening alone (nothing of this call runs yet) and sizes the next lead chunk
+                if (cudaEventElapsedTime(&ms, h2d_end[par], in_ready[par]) == cudaSuccess) {
+                    ctx->last_ms[13] += ms;
+                    if (c == 0 && N > 0) widen_per_point0 = ms / (double)N;
+                }
+            } else if (cudaEventElapsedTime(&ms, h2d_begin[par], in_ready[par]) == cudaSuccess) {
+                ctx->last_ms[9] += ms;
+            }
             CK(cudaEventRecord(d2h_begin[par], cs));
             CK(cudaMemcpyAsync(models + p0, io.models_out, sizeof(Model) * P, cudaMemcpyDeviceToHost, cs));
             CK(cudaMemcpyAsync(stats + p0, io.stats_out, sizeof(rp_stats) * P, cudaMemcpyDeviceToHost, cs));
@@ -944,7 +1011,7 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
     if (host_io) {
         CK(cudaEventRecord(d2h_end, cs));
         CK(cudaStreamSynchronize(cs));
-        ctx->prev_h2d_ms = ctx->last_ms[9];
+        ctx->prev_h2d_ms = ctx->last_ms[9] + widen_per_point0 * (double)Ntot;   // + widening of the batch, 0 with FP64 inputs
         ctx->prev_dev_ms = ctx->last_ms[8];
         for (int par = 0; par < 2 && par < n_chunks; ++par) {
             float ms = 0.f;
@@ -1069,6 +1136,25 @@ int rp_estimate_batch_host(rp_ctx *ctx, int variant, int64_t n_pairs, const int6
 int rp_estimate_batch_dev(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const double *x1,
                           const double *x2, const double *d1, const double *d2, const double *cams,
                           const rp_options *opt, rp_model *models, rp_stats *stats, uint8_t *masks, void *stream) {
+    if (!ctx) return RP_ERR_INVALID;
+    if (n_pairs > 0 && (!x1 || !x2 || !d1 || !d2 || !models || !stats || !masks))
+        return fail(ctx, RP_ERR_INVALID, "null data pointer");
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, cams, opt, models, stats, masks, false,
+                         stream ? (cudaStream_t)stream : ctx->stream);
+}
+
+int rp_estimate_batch_host_f32(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const float *x1,
+                               const float *x2, const float *d1, const float *d2, const double *cams,
+                               const rp_options *opt, rp_model *models, rp_stats *stats, uint8_t *masks) {
+    if (!ctx) return RP_ERR_INVALID;
+    if (n_pairs > 0 && (!x1 || !x2 || !d1 || !d2 || !models || !stats || !masks))
+        return fail(ctx, RP_ERR_INVALID, "null data pointer");
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, cams, opt, models, stats, masks, true, ctx->stream);
+}
+
+int rp_estimate_batch_dev_f32(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const float *x1,
+                              const float *x2, const float *d1, const float *d2, const double *cams,
+                              const rp_options *opt, rp_model *models, rp_stats *stats, uint8_t *masks, void *stream) {
     if (!ctx) return RP_ERR_INVALID;
     if (n_pairs > 0 && (!x1 || !x2 || !d1 || !d2 || !models || !stats || !masks))
         return fail(ctx, RP_ERR_INVALID, "null data pointer");
@@ -1303,9 +1389,15 @@ int rp_refine_batch(rp_ctx *ctx, int variant, int64_t n_models, rp_model *models
     return RP_OK;
 }
 
-int rp_gather_depths_dev(rp_ctx *ctx, const float *depth1, int h1, int w1, const float *depth2, int h2, int w2,
-                         const float *kp1, const float *kp2, int64_t n, double *x1, double *x2, double *d1, double *d2,
-                         int64_t *n_out, void *stream) {
+}  // extern "C"
+
+namespace {
+
+// rp_gather_depths_dev[_f32]: T is the output type
+template <class T>
+int gather_depths_impl(rp_ctx *ctx, const float *depth1, int h1, int w1, const float *depth2, int h2, int w2,
+                       const float *kp1, const float *kp2, int64_t n, T *x1, T *x2, T *d1, T *d2, int64_t *n_out,
+                       void *stream) {
     if (!ctx || n < 0 || !n_out || h1 <= 0 || w1 <= 0 || h2 <= 0 || w2 <= 0 ||
         (n > 0 && (!depth1 || !depth2 || !kp1 || !kp2 || !x1 || !x2 || !d1 || !d2)))
         return fail(ctx, RP_ERR_INVALID, "bad argument");
@@ -1315,7 +1407,7 @@ int rp_gather_depths_dev(rp_ctx *ctx, const float *depth1, int h1, int w1, const
     cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
     CK(ctx->buf[B_SCALARS].reserve(sizeof(Scalars)));
     long long *d_n = (long long *)ctx->buf[B_SCALARS].p;
-    gather_depths_kernel<<<1, 1024, 0, st>>>(depth1, h1, w1, depth2, h2, w2, kp1, kp2, (long long)n, x1, x2, d1, d2, d_n);
+    gather_depths_kernel<T><<<1, 1024, 0, st>>>(depth1, h1, w1, depth2, h2, w2, kp1, kp2, (long long)n, x1, x2, d1, d2, d_n);
     LAUNCHED();
     long long h_n = 0;
     CK(cudaMemcpyAsync(&h_n, d_n, sizeof h_n, cudaMemcpyDeviceToHost, st));
@@ -1324,9 +1416,11 @@ int rp_gather_depths_dev(rp_ctx *ctx, const float *depth1, int h1, int w1, const
     return RP_OK;
 }
 
-int rp_gather_depths_batch_dev(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_offsets, const float *depth_maps, int n_frames,
-                               int h, int w, const int32_t *frame1, const int32_t *frame2, const float *kp1, const float *kp2,
-                               double *x1, double *x2, double *d1, double *d2, int64_t *out_offsets, void *stream) {
+// rp_gather_depths_batch_dev[_f32]: T is the output type
+template <class T>
+int gather_depths_batch_impl(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_offsets, const float *depth_maps, int n_frames,
+                             int h, int w, const int32_t *frame1, const int32_t *frame2, const float *kp1, const float *kp2,
+                             T *x1, T *x2, T *d1, T *d2, int64_t *out_offsets, void *stream) {
     if (!ctx || n_pairs < 0 || !in_offsets || !out_offsets || h <= 0 || w <= 0 || n_frames <= 0 ||
         (n_pairs > 0 && (!depth_maps || !frame1 || !frame2)))
         return fail(ctx, RP_ERR_INVALID, "bad argument");
@@ -1351,13 +1445,13 @@ int rp_gather_depths_batch_dev(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_o
     CK(cudaMemcpyAsync(B[B_SUB_SRC].p, rel.data(), 8 * ((size_t)n_pairs + 1), cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(d_f1, frame1, sizeof(int) * (size_t)n_pairs, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(d_f2, frame2, sizeof(int) * (size_t)n_pairs, cudaMemcpyHostToDevice, st));
-    GatherBatchArgs g;
+    GatherBatchArgs<T> g;
     g.n_pairs = (int)n_pairs; g.h = h; g.w = w; g.depth = depth_maps; g.frame1 = d_f1; g.frame2 = d_f2;
     g.in_off = B[B_SUB_SRC].as<long long>(); g.out_off = B[B_SUB_DST].as<long long>();
     g.kp1 = kp1; g.kp2 = kp2;
-    g.tx1 = B[B_SUB_X1].as<double>(); g.tx2 = B[B_SUB_X2].as<double>(); g.td1 = B[B_SUB_D1].as<double>(); g.td2 = B[B_SUB_D2].as<double>();
+    g.tx1 = B[B_SUB_X1].as<T>(); g.tx2 = B[B_SUB_X2].as<T>(); g.td1 = B[B_SUB_D1].as<T>(); g.td2 = B[B_SUB_D2].as<T>();
     g.x1 = x1; g.x2 = x2; g.d1 = d1; g.d2 = d2; g.count = d_cnt;
-    gather_depths_batch_kernel<<<(unsigned)n_pairs, 256, 0, st>>>(g);
+    gather_depths_batch_kernel<T><<<(unsigned)n_pairs, 256, 0, st>>>(g);
     LAUNCHED();
     std::vector<int> cnt((size_t)n_pairs);
     CK(cudaMemcpyAsync(cnt.data(), d_cnt, sizeof(int) * (size_t)n_pairs, cudaMemcpyDeviceToHost, st));
@@ -1366,10 +1460,41 @@ int rp_gather_depths_batch_dev(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_o
     for (int64_t p = 0; p < n_pairs; ++p) out[(size_t)p + 1] = out[(size_t)p] + cnt[(size_t)p];
     for (int64_t p = 0; p <= n_pairs; ++p) out_offsets[p] = out[(size_t)p];
     CK(cudaMemcpyAsync(B[B_SUB_DST].p, out.data(), 8 * ((size_t)n_pairs + 1), cudaMemcpyHostToDevice, st));
-    gather_depths_pack_kernel<<<(unsigned)n_pairs, 256, 0, st>>>(g);
+    gather_depths_pack_kernel<T><<<(unsigned)n_pairs, 256, 0, st>>>(g);
     LAUNCHED();
     CK(cudaStreamSynchronize(st));   // `out` is a stack-lifetime host buffer
     return RP_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int rp_gather_depths_dev(rp_ctx *ctx, const float *depth1, int h1, int w1, const float *depth2, int h2, int w2,
+                         const float *kp1, const float *kp2, int64_t n, double *x1, double *x2, double *d1, double *d2,
+                         int64_t *n_out, void *stream) {
+    return gather_depths_impl(ctx, depth1, h1, w1, depth2, h2, w2, kp1, kp2, n, x1, x2, d1, d2, n_out, stream);
+}
+
+int rp_gather_depths_dev_f32(rp_ctx *ctx, const float *depth1, int h1, int w1, const float *depth2, int h2, int w2,
+                             const float *kp1, const float *kp2, int64_t n, float *x1, float *x2, float *d1, float *d2,
+                             int64_t *n_out, void *stream) {
+    return gather_depths_impl(ctx, depth1, h1, w1, depth2, h2, w2, kp1, kp2, n, x1, x2, d1, d2, n_out, stream);
+}
+
+int rp_gather_depths_batch_dev(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_offsets, const float *depth_maps, int n_frames,
+                               int h, int w, const int32_t *frame1, const int32_t *frame2, const float *kp1, const float *kp2,
+                               double *x1, double *x2, double *d1, double *d2, int64_t *out_offsets, void *stream) {
+    return gather_depths_batch_impl(ctx, n_pairs, in_offsets, depth_maps, n_frames, h, w, frame1, frame2, kp1, kp2, x1, x2, d1,
+                                    d2, out_offsets, stream);
+}
+
+int rp_gather_depths_batch_dev_f32(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_offsets, const float *depth_maps,
+                                   int n_frames, int h, int w, const int32_t *frame1, const int32_t *frame2, const float *kp1,
+                                   const float *kp2, float *x1, float *x2, float *d1, float *d2, int64_t *out_offsets,
+                                   void *stream) {
+    return gather_depths_batch_impl(ctx, n_pairs, in_offsets, depth_maps, n_frames, h, w, frame1, frame2, kp1, kp2, x1, x2, d1,
+                                    d2, out_offsets, stream);
 }
 
 int rp_measure_pipes(rp_ctx *ctx, double *fp64_tflops, double *fp32_tflops) {

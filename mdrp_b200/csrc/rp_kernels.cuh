@@ -1609,11 +1609,13 @@ __global__ void fill_int_kernel(int *p, int n, int v) {
 // front end (SURVEY.md §8f item 2): the reference's callers look the monocular depth up at the matched
 // keypoints, depth_map[(int)y, (int)x], and drop the rows whose two depths are both infinite
 // (/root/reference/make_pair.py:97-106) on the host after a .cpu().numpy() round trip.  This kernel does
-// the lookup, the mask and the stable compaction on the device, straight into the packed FP64 layout
-// the estimator takes.  One block; rows keep their order.
+// the lookup, the mask and the stable compaction on the device, straight into the packed layout the
+// estimator takes: T = double for rp_estimate_batch_*, T = float for rp_estimate_batch_*_f32 (the float
+// inputs unchanged).  One block; rows keep their order.
+template <class T>
 __global__ void gather_depths_kernel(const float *depth1, int h1, int w1, const float *depth2, int h2, int w2,
-                                     const float *kp1, const float *kp2, long long n, double *x1, double *x2,
-                                     double *d1, double *d2, long long *n_out) {
+                                     const float *kp1, const float *kp2, long long n, T *x1, T *x2,
+                                     T *d1, T *d2, long long *n_out) {
     __shared__ int warp_tot[32];
     __shared__ long long running;
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
@@ -1655,7 +1657,8 @@ __global__ void gather_depths_kernel(const float *depth1, int h1, int w1, const 
 // size stacked [F, h, w], pair p = (frame1[p], frame2[p]) with keypoints [in_off[p], in_off[p+1]).  Pass 1: one CTA per
 // pair, stable compaction of the pair's rows INTO ITS OWN INPUT RANGE of the temporary arrays + the kept count; the host
 // reads the n_pairs counts once (it needs the packed offsets anyway: rp_estimate_batch_dev takes them), pass 2 moves
-// every pair's block to its packed position.
+// every pair's block to its packed position.  T: output type, as in gather_depths_kernel.
+template <class T>
 struct GatherBatchArgs {
     int n_pairs, h, w;
     const float *depth;            // [F, h, w]
@@ -1663,11 +1666,12 @@ struct GatherBatchArgs {
     const long long *in_off;       // [n_pairs + 1]
     const long long *out_off;      // [n_pairs + 1] (pass 2)
     const float *kp1, *kp2;        // [N, 2]
-    double *tx1, *tx2, *td1, *td2; // temporaries, capacity N
-    double *x1, *x2, *d1, *d2;     // packed outputs
+    T *tx1, *tx2, *td1, *td2;      // temporaries, capacity N
+    T *x1, *x2, *d1, *d2;          // packed outputs
     int *count;                    // [n_pairs]
 };
-__global__ void gather_depths_batch_kernel(GatherBatchArgs a) {
+template <class T>
+__global__ void gather_depths_batch_kernel(GatherBatchArgs<T> a) {
     __shared__ int warp_tot[32];
     __shared__ int running;
     const int pair = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
@@ -1707,7 +1711,8 @@ __global__ void gather_depths_batch_kernel(GatherBatchArgs a) {
     }
     if (tid == 0) a.count[pair] = running;
 }
-__global__ void gather_depths_pack_kernel(GatherBatchArgs a) {
+template <class T>
+__global__ void gather_depths_pack_kernel(GatherBatchArgs<T> a) {
     const int pair = blockIdx.x;
     const long long i0 = a.in_off[pair], o0 = a.out_off[pair];
     const int n = (int)(a.out_off[pair + 1] - o0);
@@ -1718,6 +1723,22 @@ __global__ void gather_depths_pack_kernel(GatherBatchArgs a) {
     for (int i = threadIdx.x; i < n; i += blockDim.x) {
         a.d1[o0 + i] = a.td1[i0 + i];
         a.d2[o0 + i] = a.td2[i0 + i];
+    }
+}
+
+// float32 inputs (rp_estimate_batch_*_f32): one chunk's x1, x2 [n,2] and d1, d2 [n] widened into the FP64 arrays every
+// kernel downstream reads.  float -> double is exact, so the chunk is bit for bit what the FP64 entry points receive for
+// the same values.  Grid-stride over the 6 n values of the chunk.
+__global__ void widen_inputs_kernel(long long n, const float *x1, const float *x2, const float *d1, const float *d2,
+                                    double *wx1, double *wx2, double *wd1, double *wd2) {
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < 2 * n; i += stride) {
+        wx1[i] = (double)x1[i];
+        wx2[i] = (double)x2[i];
+        if (i < n) {
+            wd1[i] = (double)d1[i];
+            wd2[i] = (double)d2[i];
+        }
     }
 }
 

@@ -123,6 +123,8 @@ def estimate_sharded(estimate_fn, offsets, x1, x2, d1, d2, cams, rank: int, worl
 def estimate_local_shard(ctx, variant, offsets, x1, x2, d1, d2, cams, opt, rank: int, world_size: int, device=None,
                          gather_masks: bool = True):
     """Every rank holds only ITS shard (local offsets and arrays): run it on this rank's GPU (`ctx`: an
-    mdrp_b200._native.Context) and gather on rank 0.  This is what bench.py times at N > 1."""
-    models, stats, masks = ctx.estimate_batch_host(variant, offsets, x1, x2, d1, d2, cams, opt)
+    mdrp_b200._native.Context) and gather on rank 0.  This is what bench.py times at N > 1.  float32 numpy points and
+    depths go through the float32 entry point (half the upload, the same results), everything else through FP64."""
+    from .api import _estimate_host
+    models, stats, masks = _estimate_host(ctx, variant, offsets, x1, x2, d1, d2, cams, opt)
     return gather_results(models, stats, masks, rank, world_size, device=device, gather_masks=gather_masks)

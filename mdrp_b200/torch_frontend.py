@@ -19,35 +19,48 @@ def _ctx_for(t: torch.Tensor) -> nv.Context:
     return api.context(t.device.index or 0)
 
 
-def gather_depths(depth_map1, depth_map2, keypoints1, keypoints2):
+_GATHER_DTYPES = (torch.float64, torch.float32)
+
+
+def _gather_fn(ctx, name, dtype):
+    if dtype not in _GATHER_DTYPES:
+        raise ValueError("dtype must be torch.float64 or torch.float32")
+    return getattr(ctx._lib, name + ("_f32" if dtype == torch.float32 else ""))
+
+
+def gather_depths(depth_map1, depth_map2, keypoints1, keypoints2, dtype=torch.float64):
     """depths at the matched keypoints + removal of rows whose depths are both inf (make_pair.py:97-106),
     on the device.  depth maps: [H,W] float32 CUDA; keypoints: [n,2] float32 CUDA (x, y).
-    Returns (x1, x2, d1, d2) float64 CUDA tensors with the kept rows in order."""
+    Returns (x1, x2, d1, d2) CUDA tensors of `dtype` (float64, or float32: the values unchanged, what `estimate_batch`
+    takes without an FP64 copy) with the kept rows in order."""
     ctx = _ctx_for(depth_map1)
+    fn = _gather_fn(ctx, "rp_gather_depths_dev", dtype)
     dm1 = depth_map1.contiguous().float()
     dm2 = depth_map2.contiguous().float()
     k1 = keypoints1.contiguous().float()
     k2 = keypoints2.contiguous().float()
     n = k1.shape[0]
     dev = dm1.device
-    x1 = torch.empty(n, 2, dtype=torch.float64, device=dev)
-    x2 = torch.empty(n, 2, dtype=torch.float64, device=dev)
-    d1 = torch.empty(n, dtype=torch.float64, device=dev)
-    d2 = torch.empty(n, dtype=torch.float64, device=dev)
+    x1 = torch.empty(n, 2, dtype=dtype, device=dev)
+    x2 = torch.empty(n, 2, dtype=dtype, device=dev)
+    d1 = torch.empty(n, dtype=dtype, device=dev)
+    d2 = torch.empty(n, dtype=dtype, device=dev)
     n_out = C.c_int64(0)
     stream = torch.cuda.current_stream(dev).cuda_stream
-    ctx._call(ctx._lib.rp_gather_depths_dev, ctx._h, dm1.data_ptr(), dm1.shape[0], dm1.shape[1], dm2.data_ptr(),
+    ctx._call(fn, ctx._h, dm1.data_ptr(), dm1.shape[0], dm1.shape[1], dm2.data_ptr(),
               dm2.shape[0], dm2.shape[1], k1.data_ptr(), k2.data_ptr(), n, x1.data_ptr(), x2.data_ptr(),
               d1.data_ptr(), d2.data_ptr(), C.byref(n_out), stream)
     m = n_out.value
     return x1[:m], x2[:m], d1[:m], d2[:m]
 
 
-def gather_depths_batch(depth_maps, frame1, frame2, offsets, keypoints1, keypoints2):
+def gather_depths_batch(depth_maps, frame1, frame2, offsets, keypoints1, keypoints2, dtype=torch.float64):
     """`gather_depths` for a batch of pairs in one call (a video: make_video.py:270-290).  depth_maps: [F,H,W] float32
     CUDA; frame1 / frame2: per-pair frame indices; offsets: [P+1] rows of the packed keypoints [N,2] float32 CUDA.
-    Returns (out_offsets int64 numpy, x1, x2, d1, d2) — the packed float64 CUDA tensors `estimate_batch` takes."""
+    Returns (out_offsets int64 numpy, x1, x2, d1, d2) — the packed CUDA tensors of `dtype` (float64 or float32)
+    `estimate_batch` takes."""
     ctx = _ctx_for(depth_maps)
+    fn = _gather_fn(ctx, "rp_gather_depths_batch_dev", dtype)
     dm = depth_maps.contiguous().float()
     k1, k2 = keypoints1.contiguous().float(), keypoints2.contiguous().float()
     offsets = np.ascontiguousarray(offsets, dtype=np.int64)
@@ -56,12 +69,12 @@ def gather_depths_batch(depth_maps, frame1, frame2, offsets, keypoints1, keypoin
     P, n, dev = len(offsets) - 1, k1.shape[0], dm.device
     if len(f1) != P or len(f2) != P or int(offsets[-1]) - int(offsets[0]) != n:
         raise ValueError("frame1 / frame2 need one entry per pair and offsets must cover the keypoints")
-    x1 = torch.empty(n, 2, dtype=torch.float64, device=dev)
-    x2 = torch.empty(n, 2, dtype=torch.float64, device=dev)
-    d1 = torch.empty(n, dtype=torch.float64, device=dev)
-    d2 = torch.empty(n, dtype=torch.float64, device=dev)
+    x1 = torch.empty(n, 2, dtype=dtype, device=dev)
+    x2 = torch.empty(n, 2, dtype=dtype, device=dev)
+    d1 = torch.empty(n, dtype=dtype, device=dev)
+    d2 = torch.empty(n, dtype=dtype, device=dev)
     out = np.zeros(P + 1, dtype=np.int64)
-    ctx._call(ctx._lib.rp_gather_depths_batch_dev, ctx._h, P, offsets.ctypes.data, dm.data_ptr(), dm.shape[0], dm.shape[1],
+    ctx._call(fn, ctx._h, P, offsets.ctypes.data, dm.data_ptr(), dm.shape[0], dm.shape[1],
               dm.shape[2], f1.ctypes.data, f2.ctypes.data, k1.data_ptr(), k2.data_ptr(), x1.data_ptr(), x2.data_ptr(),
               d1.data_ptr(), d2.data_ptr(), out.ctypes.data, torch.cuda.current_stream(dev).cuda_stream)
     m = int(out[-1])
@@ -71,22 +84,26 @@ def gather_depths_batch(depth_maps, frame1, frame2, offsets, keypoints1, keypoin
 def estimate_batch(variant, offsets, x1, x2, d1, d2, cams, opt: nv.Options):
     """Packed CUDA float64 tensors in (offsets: host int64 array), CUDA tensors out:
     models [P,12] float64, stats [P,5] (int64 view; columns 3,4 are float64 bit patterns — use
-    `stats_to_numpy`), masks [N] uint8."""
+    `stats_to_numpy`), masks [N] uint8.  When x1, x2, d1, d2 are all float32 they are passed as they are to the
+    float32 entry point (no FP64 copy of the batch; the same results as float64 tensors of the same values)."""
     ctx = _ctx_for(x1)
     dev = x1.device
     offsets = np.ascontiguousarray(offsets, dtype=np.int64)
     P, N = len(offsets) - 1, int(offsets[-1])
+    f32 = all(t.dtype == torch.float32 for t in (x1, x2, d1, d2))
     t64 = lambda t: t.contiguous().to(torch.float64)
-    x1, x2, d1, d2 = t64(x1), t64(x2), t64(d1), t64(d2)
+    tin = (lambda t: t.contiguous()) if f32 else t64
+    x1, x2, d1, d2 = tin(x1), tin(x2), tin(d1), tin(d2)
     if x1.shape != (N, 2) or x2.shape != (N, 2) or d1.shape != (N,) or d2.shape != (N,):
         raise ValueError("x1/x2 must be [N,2] and d1/d2 [N] with N = offsets[-1]")
     cams_t = t64(cams) if cams is not None else None
     models = torch.zeros(P, 12, dtype=torch.float64, device=dev)
     stats = torch.zeros(P, 5, dtype=torch.int64, device=dev)
     masks = torch.zeros(max(N, 1), dtype=torch.uint8, device=dev)
-    ctx.estimate_batch_dev(variant, offsets, x1.data_ptr(), x2.data_ptr(), d1.data_ptr(), d2.data_ptr(),
-                           cams_t.data_ptr() if cams_t is not None else None, opt, models.data_ptr(),
-                           stats.data_ptr(), masks.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+    est = ctx.estimate_batch_dev_f32 if f32 else ctx.estimate_batch_dev
+    est(variant, offsets, x1.data_ptr(), x2.data_ptr(), d1.data_ptr(), d2.data_ptr(),
+        cams_t.data_ptr() if cams_t is not None else None, opt, models.data_ptr(),
+        stats.data_ptr(), masks.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
     return models, stats, masks[:N]
 
 
@@ -96,7 +113,8 @@ def stats_to_numpy(stats: torch.Tensor) -> np.ndarray:
 
 def estimate_monodepth_relative_pose(points2D_1, points2D_2, depth_1, depth_2, camera1, camera2, ransac_opt={},
                                      bundle_opt={}, initial_pose=None):
-    """poselib.estimate_monodepth_relative_pose with CUDA tensor inputs; same return objects."""
+    """poselib.estimate_monodepth_relative_pose with CUDA tensor inputs; same return objects.  float32 points and
+    depths take the float32 path of `estimate_batch`."""
     opt = api.make_options(ransac_opt, bundle_opt, focal_variant=False)
     cams = torch.tensor([api.Camera.from_any(camera1).fxfycxcy() + api.Camera.from_any(camera2).fxfycxcy()],
                         dtype=torch.float64, device=points2D_1.device)
