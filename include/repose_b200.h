@@ -156,6 +156,35 @@ RP_API int rp_estimate_batch_dev_f32(rp_ctx *ctx, int variant, int64_t n_pairs, 
                                      const double *cams, const rp_options *opt, rp_model *models,
                                      rp_stats *stats, uint8_t *masks, void *stream);
 
+/* The four estimators with one float32 match quality per correspondence (LightGlue score, RoMa certainty, ...):
+ * quality [offsets[n_pairs]], HOST memory for _host and DEVICE memory for _dev, inserted after d2 in the twin's argument
+ * list.  They order each pair on the device so that PROSAC (opt->progressive_sampling) sees its correspondences from
+ * best to worst, and they are defined by that order:
+ *   - the outputs (models, stats, masks, rp_pair_status) are, as bytes, those of the twin called with every pair's
+ *     correspondences reordered by (quality descending, original index ascending);
+ *   - the ordering key is the float32 quality with NaN taken as -inf and -0 as +0;
+ *   - masks come back in the CALLER's order: masks[o + perm[j]] = (mask of the reordered pair)[o + j].
+ * opt->progressive_sampling is honoured as given (0: uniform sampling on the reordered pairs).  Results depend only on a
+ * pair's data, its quality and opt->seed, never on the batch around it or on the chunking.  A null quality with
+ * n_pairs > 0 is RP_ERR_INVALID; every other check and error code is the twin's.  rp_last_timing slot [14] reports the
+ * ordering (sort, permuting gather, mask scatter). */
+RP_API int rp_estimate_batch_host_quality(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets,
+                                          const double *x1, const double *x2, const double *d1, const double *d2,
+                                          const float *quality, const double *cams, const rp_options *opt,
+                                          rp_model *models, rp_stats *stats, uint8_t *masks);
+RP_API int rp_estimate_batch_dev_quality(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets,
+                                         const double *x1, const double *x2, const double *d1, const double *d2,
+                                         const float *quality, const double *cams, const rp_options *opt,
+                                         rp_model *models, rp_stats *stats, uint8_t *masks, void *stream);
+RP_API int rp_estimate_batch_host_f32_quality(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets,
+                                              const float *x1, const float *x2, const float *d1, const float *d2,
+                                              const float *quality, const double *cams, const rp_options *opt,
+                                              rp_model *models, rp_stats *stats, uint8_t *masks);
+RP_API int rp_estimate_batch_dev_f32_quality(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets,
+                                             const float *x1, const float *x2, const float *d1, const float *d2,
+                                             const float *quality, const double *cams, const rp_options *opt,
+                                             rp_model *models, rp_stats *stats, uint8_t *masks, void *stream);
+
 /* ---- stage entry points (parity tests; all pointers HOST memory) -----------------
  * Each mirrors one exported stage of the reference binary (SURVEY.md §8a). */
 
@@ -166,6 +195,14 @@ RP_API int rp_sample_batch(rp_ctx *ctx, int64_t n, uint64_t seed, int64_t iters,
  * draws from a growing prefix of the (quality-sorted) points for the first max_prosac_iterations-1 samples */
 RP_API int rp_sample_batch_prosac(rp_ctx *ctx, int64_t n, uint64_t seed, int64_t iters, int32_t progressive_sampling,
                                   int64_t max_prosac_iterations, int32_t *samples);
+
+/* The ordering step of the rp_estimate_batch_*_quality entry points on its own (no counterpart in the reference).  Pair p
+ * owns [offsets[p], offsets[p+1]) of quality and perm (offsets non-decreasing, at most 2^24-1 correspondences per pair);
+ * perm[offsets[p] + j] (int32, pair-local) is the index of the pair's j-th correspondence in (quality descending,
+ * index ascending) order, with NaN taken as -inf and -0 as +0.  Pairs of up to RP_ORDER_SMEM_CAP correspondences are
+ * sorted in shared memory, larger ones in global scratch (slower). */
+#define RP_ORDER_SMEM_CAP 12288
+RP_API int rp_order_by_quality(rp_ctx *ctx, int64_t n_pairs, const int64_t *offsets, const float *quality, int32_t *perm);
 
 /* S1-S4: minimal solvers on n_problems independent triplets.  x1h,x2h: [n,3,3] homogeneous
  * (x,y,1) points, d1,d2: [n,3].  models: [n,4], counts: [n] (solutions per problem). */
@@ -245,7 +282,10 @@ RP_API int rp_pair_status(const rp_ctx *ctx, int64_t n_pairs, int32_t *status);
  * [10] D2H, [11] FP32 bound kernel alone, [12] tensor-core count tier alone, [13] widening of float32 inputs to FP64
  * (rp_estimate_batch_*_f32; 0 otherwise).  On the host path the widening runs on the copy stream after the H2D of [9],
  * and for every chunk but the first it overlaps the previous chunk's kernels, so [13] there also counts the time the
- * widening waits for SMs those kernels hold; the device path's [13] is the widening alone.  [14..15] reserved.
+ * widening waits for SMs those kernels hold; the device path's [13] is the widening alone.  [14] ordering of a
+ * rp_estimate_batch_*_quality call: sort, permuting gather (which also widens float32 inputs, so [13] is 0 for these
+ * calls) and mask scatter; 0 for every other call.  On the host path the sort and gather run on the copy stream after
+ * the H2D of [9], so [14] there carries the same caveat as [13].  [15] reserved.
  * counters: [0] minimal models generated, [1] point-scores the FP32 bound kernel resolved (models x correspondences),
  * [2] LM problems, [3] LM iterations, [4] chunks (= launches of each pipeline kernel), [5] minimal models
  * that needed the exact scorer, [6] point-scores the FP32 bound kernel actually evaluated (before abandoning),

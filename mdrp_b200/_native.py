@@ -22,7 +22,10 @@ EXPORTS = [
     "rp_estimate_batch_host", "rp_estimate_batch_dev", "rp_sample_batch", "rp_sample_batch_prosac", "rp_solve_batch",
     "rp_score_batch", "rp_refine_batch", "rp_measure_pipes", "rp_last_timing", "rp_gather_depths_dev", "rp_tc_count_batch", "rp_pair_status", "rp_gather_depths_batch_dev",
     "rp_estimate_batch_host_f32", "rp_estimate_batch_dev_f32", "rp_gather_depths_dev_f32", "rp_gather_depths_batch_dev_f32",
+    "rp_estimate_batch_host_quality", "rp_estimate_batch_dev_quality", "rp_estimate_batch_host_f32_quality",
+    "rp_estimate_batch_dev_f32_quality", "rp_order_by_quality",
 ]
+ORDER_SMEM_CAP = 12288   # RP_ORDER_SMEM_CAP: larger pairs are ordered in global scratch
 
 
 class NativeError(RuntimeError):
@@ -104,6 +107,15 @@ def load():
     L.rp_estimate_batch_host_f32.argtypes = est_args
     L.rp_estimate_batch_dev_f32.restype = C.c_int
     L.rp_estimate_batch_dev_f32.argtypes = est_args + [VP]
+    est_q_args = est_args[:8] + [VP] + est_args[8:]   # quality after d2
+    for name in ("rp_estimate_batch_host_quality", "rp_estimate_batch_host_f32_quality"):
+        getattr(L, name).restype = C.c_int
+        getattr(L, name).argtypes = est_q_args
+    for name in ("rp_estimate_batch_dev_quality", "rp_estimate_batch_dev_f32_quality"):
+        getattr(L, name).restype = C.c_int
+        getattr(L, name).argtypes = est_q_args + [VP]
+    L.rp_order_by_quality.restype = C.c_int
+    L.rp_order_by_quality.argtypes = [VP, C.c_int64, VP, VP, VP]
     L.rp_sample_batch.restype = C.c_int
     L.rp_sample_batch.argtypes = [VP, C.c_int64, C.c_uint64, C.c_int64, VP]
     L.rp_sample_batch_prosac.restype = C.c_int
@@ -155,7 +167,7 @@ def _ptr(a):
 
 
 TIMING_KEYS = ["prepare", "sample", "solve", "score_minimal", "scan", "lo_refine", "lo_score_merge",
-               "final_refine", "device_total", "h2d", "d2h", "bound_kernel", "tc_kernel", "widen", "r14", "r15"]
+               "final_refine", "device_total", "h2d", "d2h", "bound_kernel", "tc_kernel", "widen", "order", "r15"]
 COUNTER_KEYS = ["hypotheses", "point_scores", "lm_problems", "lm_iterations", "chunks", "exact_models",
                 "bound_evaluated", "head_models", "tc_evaluated", "tc_selected", "lm_flops", "c11", "c12", "c13", "c14", "c15"]
 
@@ -228,44 +240,84 @@ class Context:
         bytes out as `estimate_batch_host` on the values converted to float64."""
         return self._estimate_host(self._lib.rp_estimate_batch_host_f32, _f32, variant, offsets, x1, x2, d1, d2, cams, opt)
 
-    def _estimate_host(self, fn, conv, variant, offsets, x1, x2, d1, d2, cams, opt):
+    def estimate_batch_host_quality(self, variant, offsets, x1, x2, d1, d2, cams, opt: Options, quality):
+        """`estimate_batch_host` with one match quality per correspondence (rp_estimate_batch_host[_f32]_quality): every
+        pair is ordered by decreasing float32 quality on the device (ties: original index), masks come back in the
+        caller's order.  float32 points and depths (all four) take the float32 entry point, anything else float64."""
+        quality = _f32(quality)
+        if all(getattr(a, "dtype", None) == np.float32 for a in (x1, x2, d1, d2)):
+            fn, conv = self._lib.rp_estimate_batch_host_f32_quality, _f32
+        else:
+            fn, conv = self._lib.rp_estimate_batch_host_quality, _f64
+        return self._estimate_host(fn, conv, variant, offsets, x1, x2, d1, d2, cams, opt, quality)
+
+    def _estimate_host(self, fn, conv, variant, offsets, x1, x2, d1, d2, cams, opt, quality=None):
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         n_pairs = len(offsets) - 1
         x1, x2, d1, d2 = conv(x1), conv(x2), conv(d1), conv(d2)
         ntot = int(offsets[-1]) if n_pairs >= 0 else 0
         if x1.shape != (ntot, 2) or x2.shape != (ntot, 2) or d1.shape != (ntot,) or d2.shape != (ntot,):
             raise ValueError("x1/x2 must be [N,2] and d1/d2 [N] with N = offsets[-1]")
+        if quality is not None and quality.shape != (ntot,):
+            raise ValueError("quality must be [N] with N = offsets[-1]")
         cams = _f64(cams) if cams is not None else None
         if cams is not None and cams.shape != (n_pairs, 8):
             raise ValueError("cams must be [n_pairs, 8]")
         models = np.zeros(n_pairs, dtype=MODEL_DTYPE)
         stats = np.zeros(n_pairs, dtype=STATS_DTYPE)
         masks = np.zeros(max(ntot, 1), dtype=np.uint8)
+        data = [_ptr(x1), _ptr(x2), _ptr(d1), _ptr(d2)] + ([_ptr(quality)] if quality is not None else [])
         self._call(fn,
-            self._h, int(variant), n_pairs, _ptr(offsets), _ptr(x1), _ptr(x2), _ptr(d1), _ptr(d2),
+            self._h, int(variant), n_pairs, _ptr(offsets), *data,
             _ptr(cams), C.byref(opt), _ptr(models), _ptr(stats), _ptr(masks))
         return models, stats, masks[:ntot]
 
     def estimate_batch_dev(self, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr, opt: Options,
                            models_ptr, stats_ptr, masks_ptr, stream=0):
         """Raw device pointers (e.g. torch tensor .data_ptr()); offsets is a host int64 array."""
-        self._estimate_dev(self._lib.rp_estimate_batch_dev, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr, opt,
+        self._estimate_dev(self._lib.rp_estimate_batch_dev, variant, offsets, [x1_ptr, x2_ptr, d1_ptr, d2_ptr], cams_ptr, opt,
                            models_ptr, stats_ptr, masks_ptr, stream)
 
     def estimate_batch_dev_f32(self, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr, opt: Options,
                                models_ptr, stats_ptr, masks_ptr, stream=0):
         """`estimate_batch_dev` with x1, x2, d1, d2 pointing at float32 device arrays (rp_estimate_batch_dev_f32)."""
-        self._estimate_dev(self._lib.rp_estimate_batch_dev_f32, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr,
+        self._estimate_dev(self._lib.rp_estimate_batch_dev_f32, variant, offsets, [x1_ptr, x2_ptr, d1_ptr, d2_ptr], cams_ptr,
                            opt, models_ptr, stats_ptr, masks_ptr, stream)
 
-    def _estimate_dev(self, fn, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr, opt, models_ptr, stats_ptr,
-                      masks_ptr, stream):
+    def estimate_batch_dev_quality(self, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr, opt: Options,
+                                   models_ptr, stats_ptr, masks_ptr, quality_ptr, stream=0):
+        """`estimate_batch_dev` with a float32 device array of match qualities (rp_estimate_batch_dev_quality)."""
+        self._estimate_dev(self._lib.rp_estimate_batch_dev_quality, variant, offsets,
+                           [x1_ptr, x2_ptr, d1_ptr, d2_ptr, quality_ptr or None], cams_ptr, opt, models_ptr, stats_ptr,
+                           masks_ptr, stream)
+
+    def estimate_batch_dev_f32_quality(self, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr, opt: Options,
+                                       models_ptr, stats_ptr, masks_ptr, quality_ptr, stream=0):
+        """`estimate_batch_dev_f32` with a float32 device array of match qualities (rp_estimate_batch_dev_f32_quality)."""
+        self._estimate_dev(self._lib.rp_estimate_batch_dev_f32_quality, variant, offsets,
+                           [x1_ptr, x2_ptr, d1_ptr, d2_ptr, quality_ptr or None], cams_ptr, opt, models_ptr, stats_ptr,
+                           masks_ptr, stream)
+
+    def _estimate_dev(self, fn, variant, offsets, data, cams_ptr, opt, models_ptr, stats_ptr, masks_ptr, stream):
+        """`data`: the device pointers between offsets and cams (x1, x2, d1, d2 and, for quality calls, quality)."""
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         self._call(fn,
-            self._h, int(variant), len(offsets) - 1, _ptr(offsets), x1_ptr, x2_ptr, d1_ptr, d2_ptr,
+            self._h, int(variant), len(offsets) - 1, _ptr(offsets), *data,
             cams_ptr, C.byref(opt), models_ptr, stats_ptr, masks_ptr, stream or None)
 
     # ---- stage entry points -----------------------------------------------------------------
+    def order(self, offsets, quality):
+        """rp_order_by_quality: per pair, the pair-local indices in (float32 quality descending, index ascending)
+        order (NaN as -inf, -0 as +0); int32 [N]."""
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        quality = _f32(quality)
+        n = int(offsets[-1]) if len(offsets) else 0
+        if len(offsets) < 1 or quality.shape != (n,):
+            raise ValueError("quality must be [N] with N = offsets[-1]")
+        perm = np.zeros(n, dtype=np.int32)
+        self._call(self._lib.rp_order_by_quality, self._h, len(offsets) - 1, _ptr(offsets), _ptr(quality), _ptr(perm))
+        return perm
+
     def sample(self, n, seed, iters, progressive_sampling=False, max_prosac_iterations=100000):
         out = np.zeros((iters, 3), dtype=np.int32)
         if progressive_sampling:

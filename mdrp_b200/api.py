@@ -227,8 +227,25 @@ def _pack_auto(list_x1, list_x2, list_d1, list_d2):
     return _pack(list_x1, list_x2, list_d1, list_d2)
 
 
-def _estimate_host(ctx, variant, offsets, x1, x2, d1, d2, cams, opt):
-    """Packed host arrays through the float32 entry point when they are float32, else the FP64 one."""
+def _pack_quality(quality, offsets):
+    """One match-quality array per pair -> packed float32 [N].  The values are converted to float32 first, so the order
+    the estimator uses is that of the float32 values.  A pair count or length that does not match the points raises
+    ValueError."""
+    n = np.diff(offsets)
+    if len(quality) != len(n):
+        raise ValueError(f"quality needs one array per pair ({len(n)}), got {len(quality)}")
+    qs = [np.asarray(q, dtype=np.float32).reshape(-1) for q in quality]
+    for i, (q, k) in enumerate(zip(qs, n)):
+        if len(q) != k:
+            raise ValueError(f"quality of pair {i} has {len(q)} values for {k} correspondences")
+    return np.concatenate(qs) if qs else np.zeros(0, dtype=np.float32)
+
+
+def _estimate_host(ctx, variant, offsets, x1, x2, d1, d2, cams, opt, quality=None):
+    """Packed host arrays through the float32 entry point when they are float32, else the FP64 one; with a packed
+    `quality` through the quality entry point of that dtype."""
+    if quality is not None:
+        return ctx.estimate_batch_host_quality(variant, offsets, x1, x2, d1, d2, cams, opt, quality)
     if x1.dtype == np.float32 and x2.dtype == np.float32 and d1.dtype == np.float32 and d2.dtype == np.float32:
         return ctx.estimate_batch_host_f32(variant, offsets, x1, x2, d1, d2, cams, opt)
     return ctx.estimate_batch_host(variant, offsets, x1, x2, d1, d2, cams, opt)
@@ -246,22 +263,28 @@ def _geometry(m):
 
 # ---- batched entry points (the unit of GPU work) -----------------------------------------------------
 def estimate_monodepth_relative_pose_batch(points2D_1, points2D_2, depth_1, depth_2, cameras1, cameras2,
-                                           ransac_opt=None, bundle_opt=None, device=0):
+                                           ransac_opt=None, bundle_opt=None, device=0, quality=None):
     """Lists (one entry per image pair) in, list of (MonoDepthTwoViewGeometry, info) out.  When every point and depth
-    array is float32 the batch goes through the float32 entry point (same results, half the upload)."""
+    array is float32 the batch goes through the float32 entry point (same results, half the upload).
+
+    `quality` (optional): one array of match qualities per pair (matcher scores, higher is better).  Each pair is then
+    ordered by decreasing float32 quality on the device (ties: original index; NaN lowest) before the estimator runs,
+    which is the order PROSAC (`progressive_sampling`) expects; the inlier lists come back in the caller's order."""
     offsets, x1, x2, d1, d2 = _pack_auto(points2D_1, points2D_2, depth_1, depth_2)
+    q = _pack_quality(quality, offsets) if quality is not None else None
     cams = np.array([Camera.from_any(a).fxfycxcy() + Camera.from_any(b).fxfycxcy()
                      for a, b in zip(cameras1, cameras2)], dtype=np.float64).reshape(-1, 8)
     opt = make_options(ransac_opt, bundle_opt, focal_variant=False)
     variant = nv.CALIB_SHIFT if opt.estimate_shift else nv.CALIB
-    models, stats, masks = _estimate_host(context(device), variant, offsets, x1, x2, d1, d2, cams, opt)
+    models, stats, masks = _estimate_host(context(device), variant, offsets, x1, x2, d1, d2, cams, opt, q)
     return [(_geometry(models[i]), _info(stats[i], masks[offsets[i]:offsets[i + 1]])) for i in range(len(models))]
 
 
-def _focal_batch(variant, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, bundle_opt, device):
+def _focal_batch(variant, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, bundle_opt, device, quality=None):
     offsets, x1, x2, d1, d2 = _pack_auto(points2D_1, points2D_2, depth_1, depth_2)
+    q = _pack_quality(quality, offsets) if quality is not None else None
     opt = make_options(ransac_opt, bundle_opt, focal_variant=True)
-    models, stats, masks = _estimate_host(context(device), variant, offsets, x1, x2, d1, d2, None, opt)
+    models, stats, masks = _estimate_host(context(device), variant, offsets, x1, x2, d1, d2, None, opt, q)
     out = []
     for i, m in enumerate(models):
         pair = MonoDepthImagePair(_geometry(m), Camera("SIMPLE_PINHOLE", [m["f1"], 0.0, 0.0]),
@@ -271,13 +294,15 @@ def _focal_batch(variant, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, 
 
 
 def estimate_monodepth_shared_focal_relative_pose_batch(points2D_1, points2D_2, depth_1, depth_2,
-                                                        ransac_opt=None, bundle_opt=None, device=0):
-    return _focal_batch(nv.SHARED, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, bundle_opt, device)
+                                                        ransac_opt=None, bundle_opt=None, device=0, quality=None):
+    """`quality`: as in estimate_monodepth_relative_pose_batch."""
+    return _focal_batch(nv.SHARED, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, bundle_opt, device, quality)
 
 
 def estimate_monodepth_varying_focal_relative_pose_batch(points2D_1, points2D_2, depth_1, depth_2,
-                                                         ransac_opt=None, bundle_opt=None, device=0):
-    return _focal_batch(nv.VARYING, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, bundle_opt, device)
+                                                         ransac_opt=None, bundle_opt=None, device=0, quality=None):
+    """`quality`: as in estimate_monodepth_relative_pose_batch."""
+    return _focal_batch(nv.VARYING, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, bundle_opt, device, quality)
 
 
 # ---- the reference's single-pair surface ---------------------------------------------------------------

@@ -9,7 +9,7 @@ OUT = os.path.join(HERE, "librepose_b200.so")
 # (source, extra flags): the LM kernels are built with FMA contraction, everything else without
 SOURCES = [("repose_b200.cu", ["-fmad=false", "-DRP_SOLVE_MIN_BLOCKS=" + os.environ.get("RP_SOLVE_MIN_BLOCKS", "1"),
                                "-DRP_SOLVE2_MIN_BLOCKS=" + os.environ.get("RP_SOLVE2_MIN_BLOCKS", "3")] + os.environ.get("RP_MAIN_EXTRA", "").split()), ("repose_lm.cu", ["-fmad=true", "-DRP_LM_MIN_BLOCKS=" + os.environ.get("RP_LM_MIN_BLOCKS", "3")] + os.environ.get("RP_LM_EXTRA", "").split())]
-HEADERS = ["rp_common.cuh", "rp_types.cuh", "rp_solvers.cuh", "rp_score.cuh", "rp_lm.cuh", "rp_lm_kernel.cuh", "rp_kernels.cuh", "rp_tc.cuh",
+HEADERS = ["rp_common.cuh", "rp_types.cuh", "rp_solvers.cuh", "rp_score.cuh", "rp_lm.cuh", "rp_lm_kernel.cuh", "rp_kernels.cuh", "rp_tc.cuh", "rp_order.cuh",
            "../../include/repose_b200.h"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",

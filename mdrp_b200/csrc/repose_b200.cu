@@ -55,8 +55,12 @@ enum { B_OFFS, B_PAIRS, B_PTS64, B_PTS32, B_BEAR, B_SAMPLES, B_MODELS, B_HYPITER
        // per-pair flags; re-run sub-batches (event-list overflow, early termination that needs more iterations)
        B_PAIRFLAGS, B_SUB_IDX, B_SUB_SRC, B_SUB_DST, B_SUB_X1, B_SUB_X2, B_SUB_D1, B_SUB_D2, B_SUB_CAMS, B_SUB_MODELS,
        B_SUB_STATS, B_SUB_MASK,
-       // float32 inputs, host path: the chunk as uploaded (double-buffered), before it is widened into B_IN_*
-       B_F32_X1, B_F32_X2, B_F32_D1, B_F32_D2, B_F32_X1_B, B_F32_X2_B, B_F32_D1_B, B_F32_D2_B, B_NBUF };
+       // host path of float32 inputs or quality calls: the chunk as uploaded (input type, double-buffered), before it
+       // is widened / gathered into B_IN_*
+       B_STG_X1, B_STG_X2, B_STG_D1, B_STG_D2, B_STG_X1_B, B_STG_X2_B, B_STG_D1_B, B_STG_D2_B,
+       // quality calls (rp_order.cuh): uploaded quality, the chunk's offsets and order, masks in the ordered layout
+       // (double-buffered on the host path), global sort scratch of pairs above RP_ORDER_SMEM_CAP
+       B_QUAL, B_QUAL_B, B_ORDOFFS, B_ORDOFFS_B, B_PERM, B_PERM_B, B_KSORT, B_KSORT_B, B_ORDSCR, B_NBUF };
 
 // device scalars living in B_SCALARS
 struct Scalars {
@@ -68,7 +72,7 @@ struct Scalars {
     unsigned long long tc_evaluated, tc_selected, lm_flops;
 };
 
-constexpr int N_EVENTS = 27;
+constexpr int N_EVENTS = 29;
 
 }  // namespace
 
@@ -702,12 +706,47 @@ size_t bytes_per_pair(int iters, long long avg_points, int ev_cap = EV, size_t i
            (size_t)avg_points * (sizeof(Pt64) + 32 + sizeof(Bear) + 1 + 128 + input_bytes) + 1024;
 }
 
-// widens a float32 chunk into the FP64 input arrays (no-op for an empty chunk)
-int launch_widen(rp_ctx *ctx, long long n, const float *x1, const float *x2, const float *d1, const float *d2, double *wx1,
-                 double *wx2, double *wd1, double *wd2, cudaStream_t st) {
+// widens a float32 chunk into the FP64 input arrays (no-op for an empty chunk); with `perm` (quality calls, float or
+// double inputs) it gathers the chunk into its quality order in the same pass (pairs: [offsets[p] - base, ...))
+template <class In>
+int launch_widen(rp_ctx *ctx, long long n, const In *x1, const In *x2, const In *d1, const In *d2, double *wx1,
+                 double *wx2, double *wd1, double *wd2, cudaStream_t st, const int *perm = nullptr,
+                 const long long *offsets = nullptr, long long base = 0, int n_pairs = 0) {
     if (n <= 0) return RP_OK;
-    const int grid = std::min<long long>(cdiv(2 * n, 256), 16LL * ctx->sms);
-    widen_inputs_kernel<<<grid, 256, 0, st>>>(n, x1, x2, d1, d2, wx1, wx2, wd1, wd2);
+    const int grid = std::min<long long>(cdiv(perm ? n : 2 * n, 256), 16LL * ctx->sms);
+    widen_inputs_kernel<In><<<grid, 256, 0, st>>>(n, x1, x2, d1, d2, perm, offsets, base, n_pairs, wx1, wx2, wd1, wd2);
+    LAUNCHED();
+    return RP_OK;
+}
+
+// quality order of the P pairs of a chunk of n correspondences: `h_offsets` (host) and `d_offsets` (device) are the
+// same P+1 offsets, pair p owning [offsets[p] - base, offsets[p+1] - base) of `quality` and `perm` (no-op for n = 0).
+// The dynamic shared memory is sized to the largest pair up to RP_ORDER_SMEM_CAP; larger pairs use B_ORDSCR.
+int launch_order(rp_ctx *ctx, int P, long long n, const int64_t *h_offsets, const long long *d_offsets, long long base,
+                 const float *quality, int *perm, cudaStream_t st) {
+    if (n <= 0) return RP_OK;
+    long long max_n = 0;
+    for (int p = 0; p < P; ++p) max_n = std::max<long long>(max_n, h_offsets[p + 1] - h_offsets[p]);
+    OrderArgs a;
+    a.offsets = d_offsets; a.base = base; a.quality = quality; a.perm = perm;
+    a.smem_cap = (int)std::min<long long>(max_n, ORDER_SMEM_CAP);
+    a.gkeys = nullptr; a.gidx = nullptr;
+    if (max_n > ORDER_SMEM_CAP) {
+        CK(ctx->buf[B_ORDSCR].reserve(12 * (size_t)n));
+        a.gkeys = ctx->buf[B_ORDSCR].as<unsigned>();
+        a.gidx = (int *)(a.gkeys + 2 * n);
+    }
+    order_by_quality_kernel<<<P, ORDER_THREADS, (size_t)ORDER_SMEM_PER_POINT * a.smem_cap, st>>>(a);
+    LAUNCHED();
+    return RP_OK;
+}
+
+// masks of a chunk in the ordered layout -> the caller's order (no-op for an empty chunk)
+int launch_scatter_masks(rp_ctx *ctx, int P, long long n, const long long *d_offsets, long long base, const int *perm,
+                         const unsigned char *sorted, unsigned char *out, cudaStream_t st) {
+    if (n <= 0) return RP_OK;
+    scatter_masks_kernel<<<(int)std::min<long long>(cdiv(n, 256), 16LL * ctx->sms), 256, 0, st>>>(n, P, d_offsets, base, perm,
+                                                                                                  sorted, out);
     LAUNCHED();
     return RP_OK;
 }
@@ -835,11 +874,19 @@ int rerun_flagged(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO
 // In = double: the FP64 entry points.  In = float: rp_estimate_batch_*_f32 — the host path uploads the float chunk
 // (24 B per correspondence instead of 48) and widens it on the copy stream, the device path widens the caller's
 // chunk on the compute stream; either way every kernel after that reads the same FP64 chunk arrays as with In = double.
+// quality != null: rp_estimate_batch_*_quality — each chunk is sorted pair by pair (order_by_quality_kernel) and gathered
+// into B_IN_* in that order by the permuting widen_inputs_kernel (host path: on the copy stream from In-typed staging;
+// device path: on the compute stream from the caller's arrays).  run_chunk and rerun_flagged then run unchanged on the
+// ordered chunk and write its masks into an ordered-layout buffer, which scatter_masks_kernel writes back in the
+// caller's order.
 template <class In>
 int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const In *x1,
-                  const In *x2, const In *d1, const In *d2, const double *cams, const rp_options *opt_in,
-                  rp_model *models, rp_stats *stats, uint8_t *masks, bool host_io, cudaStream_t st) {
+                  const In *x2, const In *d1, const In *d2, const float *quality, const double *cams,
+                  const rp_options *opt_in, rp_model *models, rp_stats *stats, uint8_t *masks, bool host_io,
+                  cudaStream_t st) {
     constexpr bool f32 = std::is_same<In, float>::value;
+    const bool ordered = quality != nullptr;
+    const bool staged = f32 || ordered;   // host path: In-typed staging, widened / gathered into B_IN_* on the copy stream
     int rc = check_common(ctx, variant, n_pairs, offsets, opt_in);
     if (rc) return rc;
     CK(cudaSetDevice(ctx->device));
@@ -860,16 +907,20 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
     const int iters0 = opt.min_iterations < opt.max_iterations
                            ? (int)std::min<int64_t>(opt.max_iterations, opt.min_iterations + 1)
                            : (int)opt.max_iterations;
-    // float32 inputs: two 24-byte staging sets (host path) or the 48-byte widened copy (device path) per correspondence
-    const size_t bpp = bytes_per_pair(iters0, Ntot / n_pairs + 1, ctx->ev_cap0, f32 ? 48 : 0);
+    // float32 inputs: two 24-byte staging sets (host path) or the 48-byte widened copy (device path) per correspondence.
+    // Quality calls: two staging sets of the inputs, quality, order and ordered-layout mask (host path), or the 48-byte
+    // gathered copy, the order and the ordered-layout mask (device path).
+    size_t in_bytes = f32 ? 48 : 0;
+    if (ordered) in_bytes = host_io ? 2 * (6 * sizeof(In) + 4 + 4 + 1) : 48 + 4 + 1;
+    const size_t bpp = bytes_per_pair(iters0, Ntot / n_pairs + 1, ctx->ev_cap0, in_bytes);
     int64_t chunk = (int64_t)std::max<size_t>(1, ctx->workspace_budget / bpp);
     chunk = std::min<int64_t>(chunk, 32768);
     std::vector<long long> rel;
     DevBuf *B = ctx->buf;
     // Chunk boundaries.  The remainder is split evenly (no tiny last chunk); on the host path a small first
     // chunk goes ahead so that the kernels start early and every later upload hides behind the previous
-    // chunk's kernels.  With U = upload time (+ widening, float32 inputs) and C = kernel time of the whole batch, the exposed time
-    // f U + max(0, (1-f) U - f C) is smallest at f = U / (U + C); U / C is taken from the previous host call on
+    // chunk's kernels.  With U = upload time (+ widening or ordering) and C = kernel time of the whole batch, the exposed
+    // time f U + max(0, (1-f) U - f C) is smallest at f = U / (U + C); U / C is taken from the previous host call on
     // this context (1/8 of the batch before there is one).  Only timing depends on it, never results.
     std::vector<int64_t> bounds(1, 0);
     {
@@ -891,14 +942,17 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
     static const int IN_X1[2] = {B_IN_X1, B_IN_X1_B}, IN_X2[2] = {B_IN_X2, B_IN_X2_B}, IN_D1[2] = {B_IN_D1, B_IN_D1_B},
                      IN_D2[2] = {B_IN_D2, B_IN_D2_B}, IN_CAMS[2] = {B_IN_CAMS, B_IN_CAMS_B}, OUT_M[2] = {B_TMP0, B_TMP0_B},
                      OUT_S[2] = {B_TMP1, B_TMP1_B}, OUT_K[2] = {B_MASK, B_MASK_B};
-    static const int F32_X1[2] = {B_F32_X1, B_F32_X1_B}, F32_X2[2] = {B_F32_X2, B_F32_X2_B}, F32_D1[2] = {B_F32_D1, B_F32_D1_B},
-                     F32_D2[2] = {B_F32_D2, B_F32_D2_B};
+    static const int STG_X1[2] = {B_STG_X1, B_STG_X1_B}, STG_X2[2] = {B_STG_X2, B_STG_X2_B}, STG_D1[2] = {B_STG_D1, B_STG_D1_B},
+                     STG_D2[2] = {B_STG_D2, B_STG_D2_B};
+    static const int QUAL[2] = {B_QUAL, B_QUAL_B}, ORDOFFS[2] = {B_ORDOFFS, B_ORDOFFS_B}, PERM[2] = {B_PERM, B_PERM_B},
+                     KSORT[2] = {B_KSORT, B_KSORT_B};
     cudaStream_t cs = ctx->copy_stream;
     cudaEvent_t *in_ready = &ctx->ev[12], *h2d_begin = &ctx->ev[14], *comp_done = &ctx->ev[16], *d2h_begin = &ctx->ev[18];
-    cudaEvent_t *h2d_end = &ctx->ev[23];  // float32 inputs: end of the upload, start of the widening (host path)
-    cudaEvent_t widen_begin = ctx->ev[25], widen_end = ctx->ev[26];  // float32 inputs, device path
+    cudaEvent_t *h2d_end = &ctx->ev[23];  // staged inputs: end of the upload, start of the widening / ordering (host path)
+    cudaEvent_t widen_begin = ctx->ev[25], widen_end = ctx->ev[26];  // float32 inputs or quality calls, device path
+    cudaEvent_t scatter_begin = ctx->ev[27], scatter_end = ctx->ev[28];  // quality calls: the mask scatter
     cudaEvent_t d2h_end = ctx->ev[11];
-    double widen_per_point0 = 0.0;  // float32 inputs, host path: widening time of chunk 0 per correspondence (ms)
+    double stage_per_point0 = 0.0;  // staged host path: widening / ordering time of chunk 0 per correspondence (ms)
     auto upload = [&](int64_t c) -> int {
         const int64_t p0 = bounds[c], p1 = bounds[c + 1];
         const int P = (int)(p1 - p0), par = (int)(c & 1);
@@ -910,18 +964,36 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
         CK(B[OUT_M[par]].reserve(sizeof(Model) * P)); CK(B[OUT_S[par]].reserve(sizeof(rp_stats) * P));
         CK(B[OUT_K[par]].reserve(nn));
         CK(cudaEventRecord(h2d_begin[par], cs));
-        if constexpr (f32) {
-            CK(B[F32_X1[par]].reserve(8 * nn)); CK(B[F32_X2[par]].reserve(8 * nn));
-            CK(B[F32_D1[par]].reserve(4 * nn)); CK(B[F32_D2[par]].reserve(4 * nn));
-            CK(cudaMemcpyAsync(B[F32_X1[par]].p, x1 + 2 * o0, 8 * (size_t)N, cudaMemcpyHostToDevice, cs));
-            CK(cudaMemcpyAsync(B[F32_X2[par]].p, x2 + 2 * o0, 8 * (size_t)N, cudaMemcpyHostToDevice, cs));
-            CK(cudaMemcpyAsync(B[F32_D1[par]].p, d1 + o0, 4 * (size_t)N, cudaMemcpyHostToDevice, cs));
-            CK(cudaMemcpyAsync(B[F32_D2[par]].p, d2 + o0, 4 * (size_t)N, cudaMemcpyHostToDevice, cs));
+        if (staged) {
+            constexpr size_t E = sizeof(In);
+            CK(B[STG_X1[par]].reserve(2 * E * nn)); CK(B[STG_X2[par]].reserve(2 * E * nn));
+            CK(B[STG_D1[par]].reserve(E * nn)); CK(B[STG_D2[par]].reserve(E * nn));
+            CK(cudaMemcpyAsync(B[STG_X1[par]].p, x1 + 2 * o0, 2 * E * (size_t)N, cudaMemcpyHostToDevice, cs));
+            CK(cudaMemcpyAsync(B[STG_X2[par]].p, x2 + 2 * o0, 2 * E * (size_t)N, cudaMemcpyHostToDevice, cs));
+            CK(cudaMemcpyAsync(B[STG_D1[par]].p, d1 + o0, E * (size_t)N, cudaMemcpyHostToDevice, cs));
+            CK(cudaMemcpyAsync(B[STG_D2[par]].p, d2 + o0, E * (size_t)N, cudaMemcpyHostToDevice, cs));
             if (pose) CK(cudaMemcpyAsync(B[IN_CAMS[par]].p, cams + 8 * p0, 64 * (size_t)P, cudaMemcpyHostToDevice, cs));
+            if (ordered) {
+                CK(B[QUAL[par]].reserve(4 * nn)); CK(B[PERM[par]].reserve(4 * nn)); CK(B[KSORT[par]].reserve(nn));
+                CK(B[ORDOFFS[par]].reserve(8 * ((size_t)P + 1)));
+                CK(cudaMemcpyAsync(B[QUAL[par]].p, quality + o0, 4 * (size_t)N, cudaMemcpyHostToDevice, cs));
+                CK(cudaMemcpyAsync(B[ORDOFFS[par]].p, offsets + p0, 8 * ((size_t)P + 1), cudaMemcpyHostToDevice, cs));
+            }
             CK(cudaEventRecord(h2d_end[par], cs));
-            int rc2 = launch_widen(ctx, N, B[F32_X1[par]].as<float>(), B[F32_X2[par]].as<float>(), B[F32_D1[par]].as<float>(),
-                                   B[F32_D2[par]].as<float>(), B[IN_X1[par]].as<double>(), B[IN_X2[par]].as<double>(),
+            const In *sx1 = B[STG_X1[par]].as<In>(), *sx2 = B[STG_X2[par]].as<In>(), *sd1 = B[STG_D1[par]].as<In>(),
+                     *sd2 = B[STG_D2[par]].as<In>();
+            int rc2 = RP_OK;
+            if (ordered) {
+                const long long *doffs = B[ORDOFFS[par]].as<long long>();
+                rc2 = launch_order(ctx, P, N, offsets + p0, doffs, o0, B[QUAL[par]].as<float>(), B[PERM[par]].as<int>(), cs);
+                if (!rc2)
+                    rc2 = launch_widen(ctx, N, sx1, sx2, sd1, sd2, B[IN_X1[par]].as<double>(), B[IN_X2[par]].as<double>(),
+                                       B[IN_D1[par]].as<double>(), B[IN_D2[par]].as<double>(), cs, B[PERM[par]].as<int>(),
+                                       doffs, o0, P);
+            } else {
+                rc2 = launch_widen(ctx, N, sx1, sx2, sd1, sd2, B[IN_X1[par]].as<double>(), B[IN_X2[par]].as<double>(),
                                    B[IN_D1[par]].as<double>(), B[IN_D2[par]].as<double>(), cs);
+            }
             if (rc2) return rc2;
         } else {
             CK(cudaMemcpyAsync(B[IN_X1[par]].p, x1 + 2 * o0, 16 * (size_t)N, cudaMemcpyHostToDevice, cs));
@@ -945,6 +1017,9 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
         for (int i = 0; i <= P; ++i) rel[i] = offsets[p0 + i] - o0;
         ChunkIO io;
         io.n_pairs = P; io.n_points = N; io.h_offsets_rel = rel.data();
+        // quality calls: where the chunk's order lives and where its masks go in the caller's order
+        const int opar = host_io ? par : 0;
+        unsigned char *masks_caller = nullptr;
         if (host_io) {
             // staging set par^1 was last read by the kernels of chunk c-1 (finished: run_chunk synchronises)
             // and by the D2H of chunk c-1, which is ordered before this upload on the copy stream
@@ -959,23 +1034,43 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
             io.models_out = B[OUT_M[par]].as<Model>(); io.stats_out = B[OUT_S[par]].as<rp_stats>();
             io.masks_out = B[OUT_K[par]].as<unsigned char>();
         } else {
-            if constexpr (f32) {
-                // the chunk widened on the compute stream, ahead of its kernels (B_IN_* are free: run_chunk synchronises)
+            if (staged) {
+                // the chunk widened (float32) or ordered and gathered (quality) on the compute stream, ahead of its
+                // kernels (B_IN_* are free: run_chunk synchronises)
                 const size_t nn = (size_t)std::max<long long>(N, 1);
                 CK(B[B_IN_X1].reserve(16 * nn)); CK(B[B_IN_X2].reserve(16 * nn));
                 CK(B[B_IN_D1].reserve(8 * nn)); CK(B[B_IN_D2].reserve(8 * nn));
+                if (ordered) {
+                    CK(B[PERM[0]].reserve(4 * nn)); CK(B[KSORT[0]].reserve(nn)); CK(B[ORDOFFS[0]].reserve(8 * ((size_t)P + 1)));
+                }
                 CK(cudaEventRecord(widen_begin, st));
-                rc = launch_widen(ctx, N, x1 + 2 * o0, x2 + 2 * o0, d1 + o0, d2 + o0, B[B_IN_X1].as<double>(), B[B_IN_X2].as<double>(),
-                                  B[B_IN_D1].as<double>(), B[B_IN_D2].as<double>(), st);
+                if (ordered) {
+                    const long long *doffs = B[ORDOFFS[0]].as<long long>();
+                    CK(cudaMemcpyAsync(B[ORDOFFS[0]].p, offsets + p0, 8 * ((size_t)P + 1), cudaMemcpyHostToDevice, st));
+                    rc = launch_order(ctx, P, N, offsets + p0, doffs, o0, quality + o0, B[PERM[0]].as<int>(), st);
+                    if (rc) return rc;
+                    rc = launch_widen(ctx, N, x1 + 2 * o0, x2 + 2 * o0, d1 + o0, d2 + o0, B[B_IN_X1].as<double>(),
+                                      B[B_IN_X2].as<double>(), B[B_IN_D1].as<double>(), B[B_IN_D2].as<double>(), st,
+                                      B[PERM[0]].as<int>(), doffs, o0, P);
+                } else {
+                    rc = launch_widen(ctx, N, x1 + 2 * o0, x2 + 2 * o0, d1 + o0, d2 + o0, B[B_IN_X1].as<double>(),
+                                      B[B_IN_X2].as<double>(), B[B_IN_D1].as<double>(), B[B_IN_D2].as<double>(), st);
+                }
                 if (rc) return rc;
                 CK(cudaEventRecord(widen_end, st));
                 io.x1 = B[B_IN_X1].as<double>(); io.x2 = B[B_IN_X2].as<double>();
                 io.d1 = B[B_IN_D1].as<double>(); io.d2 = B[B_IN_D2].as<double>();
             } else {
-                io.x1 = x1 + 2 * o0; io.x2 = x2 + 2 * o0; io.d1 = d1 + o0; io.d2 = d2 + o0;
+                // (In = double here: float32 inputs are always staged)
+                io.x1 = (const double *)(x1 + 2 * o0); io.x2 = (const double *)(x2 + 2 * o0);
+                io.d1 = (const double *)(d1 + o0); io.d2 = (const double *)(d2 + o0);
             }
             io.cams = pose ? cams + 8 * p0 : nullptr;
             io.models_out = (Model *)models + p0; io.stats_out = stats + p0; io.masks_out = masks + o0;
+        }
+        if (ordered) {
+            masks_caller = io.masks_out;
+            io.masks_out = B[KSORT[opar]].as<unsigned char>();
         }
         std::vector<int> flags;
         rc = run_chunk(ctx, variant, opt, io, iters0, ctx->ev_cap0, flags, st);
@@ -983,20 +1078,34 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
         for (int i = 0; i < P; ++i) ctx->pair_status[(size_t)(p0 + i)] = rel[i + 1] - rel[i] < 3 ? RP_PAIR_DEGENERATE : RP_PAIR_OK;
         rc = rerun_flagged(ctx, variant, opt, io, rel, flags, iters0, p0, st);
         if (rc) return rc;
-        if (f32 && !host_io) {
+        if (ordered) {
+            // the re-runs wrote into the ordered-layout masks too: now they go back to the caller's order.  The host waits
+            // for this one small kernel so that its time can be read and the D2H below (copy stream) sees the masks.
+            CK(cudaEventRecord(scatter_begin, st));
+            rc = launch_scatter_masks(ctx, P, N, B[ORDOFFS[opar]].as<long long>(), o0, B[PERM[opar]].as<int>(), io.masks_out,
+                                      masks_caller, st);
+            if (rc) return rc;
+            CK(cudaEventRecord(scatter_end, st));
+            CK(cudaEventSynchronize(scatter_end));
             float ms = 0.f;
-            if (cudaEventElapsedTime(&ms, widen_begin, widen_end) == cudaSuccess) ctx->last_ms[13] += ms;
+            if (cudaEventElapsedTime(&ms, scatter_begin, scatter_end) == cudaSuccess) ctx->last_ms[14] += ms;
+            io.masks_out = masks_caller;
+        }
+        if (staged && !host_io) {
+            float ms = 0.f;
+            if (cudaEventElapsedTime(&ms, widen_begin, widen_end) == cudaSuccess) ctx->last_ms[ordered ? 14 : 13] += ms;
         }
         if (host_io) {
             // run_chunk returned after synchronising the compute stream: results are complete
             float ms = 0.f;
-            if (f32) {
+            if (staged) {
                 if (cudaEventElapsedTime(&ms, h2d_begin[par], h2d_end[par]) == cudaSuccess) ctx->last_ms[9] += ms;
-                // widening of chunks c >= 1 runs while chunk c-1's kernels hold the SMs, so its interval includes waiting
-                // for them; chunk 0's is the widening alone (nothing of this call runs yet) and sizes the next lead chunk
+                // widening / ordering of chunks c >= 1 runs while chunk c-1's kernels hold the SMs, so its interval
+                // includes waiting for them; chunk 0's is that work alone (nothing of this call runs yet) and sizes the
+                // next lead chunk
                 if (cudaEventElapsedTime(&ms, h2d_end[par], in_ready[par]) == cudaSuccess) {
-                    ctx->last_ms[13] += ms;
-                    if (c == 0 && N > 0) widen_per_point0 = ms / (double)N;
+                    ctx->last_ms[ordered ? 14 : 13] += ms;
+                    if (c == 0 && N > 0) stage_per_point0 = ms / (double)N;
                 }
             } else if (cudaEventElapsedTime(&ms, h2d_begin[par], in_ready[par]) == cudaSuccess) {
                 ctx->last_ms[9] += ms;
@@ -1011,7 +1120,7 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
     if (host_io) {
         CK(cudaEventRecord(d2h_end, cs));
         CK(cudaStreamSynchronize(cs));
-        ctx->prev_h2d_ms = ctx->last_ms[9] + widen_per_point0 * (double)Ntot;   // + widening of the batch, 0 with FP64 inputs
+        ctx->prev_h2d_ms = ctx->last_ms[9] + stage_per_point0 * (double)Ntot;   // + widening / ordering of the batch, 0 with FP64 inputs
         ctx->prev_dev_ms = ctx->last_ms[8];
         for (int par = 0; par < 2 && par < n_chunks; ++par) {
             float ms = 0.f;
@@ -1082,7 +1191,9 @@ int rp_create(int device, rp_ctx **out) {
         void *fn = nullptr;
         if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn ||
             qres != cudaDriverEntryPointSuccess ||
-            cudaFuncSetAttribute(tc::tc_count_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES) != cudaSuccess) {
+            cudaFuncSetAttribute(tc::tc_count_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES) != cudaSuccess ||
+            cudaFuncSetAttribute(order_by_quality_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 ORDER_SMEM_PER_POINT * ORDER_SMEM_CAP) != cudaSuccess) {
             g_create_error = "tensor-map entry point / shared-memory opt-in unavailable (driver too old for sm_100a TMA?)";
             rp_destroy(ctx);
             return RP_ERR_CUDA;
@@ -1130,7 +1241,8 @@ int rp_estimate_batch_host(rp_ctx *ctx, int variant, int64_t n_pairs, const int6
     if (!ctx) return RP_ERR_INVALID;
     if (n_pairs > 0 && (!x1 || !x2 || !d1 || !d2 || !models || !stats || !masks))
         return fail(ctx, RP_ERR_INVALID, "null data pointer");
-    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, cams, opt, models, stats, masks, true, ctx->stream);
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, nullptr, cams, opt, models, stats, masks, true,
+                         ctx->stream);
 }
 
 int rp_estimate_batch_dev(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const double *x1,
@@ -1139,7 +1251,7 @@ int rp_estimate_batch_dev(rp_ctx *ctx, int variant, int64_t n_pairs, const int64
     if (!ctx) return RP_ERR_INVALID;
     if (n_pairs > 0 && (!x1 || !x2 || !d1 || !d2 || !models || !stats || !masks))
         return fail(ctx, RP_ERR_INVALID, "null data pointer");
-    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, cams, opt, models, stats, masks, false,
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, nullptr, cams, opt, models, stats, masks, false,
                          stream ? (cudaStream_t)stream : ctx->stream);
 }
 
@@ -1149,7 +1261,8 @@ int rp_estimate_batch_host_f32(rp_ctx *ctx, int variant, int64_t n_pairs, const 
     if (!ctx) return RP_ERR_INVALID;
     if (n_pairs > 0 && (!x1 || !x2 || !d1 || !d2 || !models || !stats || !masks))
         return fail(ctx, RP_ERR_INVALID, "null data pointer");
-    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, cams, opt, models, stats, masks, true, ctx->stream);
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, nullptr, cams, opt, models, stats, masks, true,
+                         ctx->stream);
 }
 
 int rp_estimate_batch_dev_f32(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const float *x1,
@@ -1158,7 +1271,50 @@ int rp_estimate_batch_dev_f32(rp_ctx *ctx, int variant, int64_t n_pairs, const i
     if (!ctx) return RP_ERR_INVALID;
     if (n_pairs > 0 && (!x1 || !x2 || !d1 || !d2 || !models || !stats || !masks))
         return fail(ctx, RP_ERR_INVALID, "null data pointer");
-    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, cams, opt, models, stats, masks, false,
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, nullptr, cams, opt, models, stats, masks, false,
+                         stream ? (cudaStream_t)stream : ctx->stream);
+}
+
+// quality calls: the twins' checks, and a quality array for a non-empty batch
+#define RP_QUALITY_CHECKS()                                                                          \
+    if (!ctx) return RP_ERR_INVALID;                                                                 \
+    if (n_pairs > 0 && (!x1 || !x2 || !d1 || !d2 || !models || !stats || !masks))                     \
+        return fail(ctx, RP_ERR_INVALID, "null data pointer");                                       \
+    if (n_pairs > 0 && !quality) return fail(ctx, RP_ERR_INVALID, "null quality")
+
+int rp_estimate_batch_host_quality(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const double *x1,
+                                   const double *x2, const double *d1, const double *d2, const float *quality,
+                                   const double *cams, const rp_options *opt, rp_model *models, rp_stats *stats,
+                                   uint8_t *masks) {
+    RP_QUALITY_CHECKS();
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, models, stats, masks, true,
+                         ctx->stream);
+}
+
+int rp_estimate_batch_dev_quality(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const double *x1,
+                                  const double *x2, const double *d1, const double *d2, const float *quality,
+                                  const double *cams, const rp_options *opt, rp_model *models, rp_stats *stats,
+                                  uint8_t *masks, void *stream) {
+    RP_QUALITY_CHECKS();
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, models, stats, masks, false,
+                         stream ? (cudaStream_t)stream : ctx->stream);
+}
+
+int rp_estimate_batch_host_f32_quality(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const float *x1,
+                                       const float *x2, const float *d1, const float *d2, const float *quality,
+                                       const double *cams, const rp_options *opt, rp_model *models, rp_stats *stats,
+                                       uint8_t *masks) {
+    RP_QUALITY_CHECKS();
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, models, stats, masks, true,
+                         ctx->stream);
+}
+
+int rp_estimate_batch_dev_f32_quality(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const float *x1,
+                                      const float *x2, const float *d1, const float *d2, const float *quality,
+                                      const double *cams, const rp_options *opt, rp_model *models, rp_stats *stats,
+                                      uint8_t *masks, void *stream) {
+    RP_QUALITY_CHECKS();
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, models, stats, masks, false,
                          stream ? (cudaStream_t)stream : ctx->stream);
 }
 
@@ -1201,6 +1357,30 @@ int rp_sample_batch_prosac(rp_ctx *ctx, int64_t n, uint64_t seed, int64_t iters,
         LAUNCHED();
         CK(cudaMemcpyAsync(samples, B[B_SAMPLES].p, sizeof(int) * 3 * (size_t)iters, cudaMemcpyDeviceToHost, st));
     }
+    CK(cudaStreamSynchronize(st));
+    return RP_OK;
+}
+
+int rp_order_by_quality(rp_ctx *ctx, int64_t n_pairs, const int64_t *offsets, const float *quality, int32_t *perm) {
+    if (!ctx || n_pairs < 0 || n_pairs > INT32_MAX || !offsets) return fail(ctx, RP_ERR_INVALID, "bad argument");
+    for (int64_t p = 0; p < n_pairs; ++p)
+        if (offsets[p + 1] < offsets[p] || offsets[p + 1] - offsets[p] >= (1 << 24))
+            return fail(ctx, RP_ERR_INVALID, "offsets must be non-decreasing, at most 2^24-1 correspondences per pair");
+    const long long N = offsets[n_pairs] - offsets[0];
+    if (N > 0 && (!quality || !perm)) return fail(ctx, RP_ERR_INVALID, "bad argument");
+    if (N == 0) return RP_OK;
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    DevBuf *B = ctx->buf;
+    const int P = (int)n_pairs;
+    CK(B[B_QUAL].reserve(4 * (size_t)N)); CK(B[B_PERM].reserve(4 * (size_t)N));
+    CK(B[B_ORDOFFS].reserve(8 * ((size_t)P + 1)));
+    CK(cudaMemcpyAsync(B[B_QUAL].p, quality + offsets[0], 4 * (size_t)N, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(B[B_ORDOFFS].p, offsets, 8 * ((size_t)P + 1), cudaMemcpyHostToDevice, st));
+    int rc = launch_order(ctx, P, N, offsets, B[B_ORDOFFS].as<long long>(), offsets[0], B[B_QUAL].as<float>(),
+                          B[B_PERM].as<int>(), st);
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(perm + offsets[0], B[B_PERM].p, 4 * (size_t)N, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return RP_OK;
 }

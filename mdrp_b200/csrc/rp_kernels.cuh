@@ -17,6 +17,7 @@
 #include "rp_score.cuh"
 #include "rp_lm_kernel.cuh"
 #include "rp_tc.cuh"
+#include "rp_order.cuh"
 
 namespace rp {
 
@@ -1729,16 +1730,33 @@ __global__ void gather_depths_pack_kernel(GatherBatchArgs<T> a) {
 // float32 inputs (rp_estimate_batch_*_f32): one chunk's x1, x2 [n,2] and d1, d2 [n] widened into the FP64 arrays every
 // kernel downstream reads.  float -> double is exact, so the chunk is bit for bit what the FP64 entry points receive for
 // the same values.  Grid-stride over the 6 n values of the chunk.
-__global__ void widen_inputs_kernel(long long n, const float *x1, const float *x2, const float *d1, const float *d2,
-                                    double *wx1, double *wx2, double *wd1, double *wd2) {
+// With a permutation (rp_estimate_batch_*_quality, In = float or double) the same pass also gathers the chunk into its
+// quality order: correspondence j of the output is correspondence perm[j] of its pair (pair_of over `offsets` - base),
+// so the FP64 arrays hold each pair reordered and every kernel downstream runs unchanged on them.
+template <class In>
+__global__ void widen_inputs_kernel(long long n, const In *x1, const In *x2, const In *d1, const In *d2, const int *perm,
+                                    const long long *offsets, long long base, int n_pairs, double *wx1, double *wx2,
+                                    double *wd1, double *wd2) {
     const long long stride = (long long)gridDim.x * blockDim.x;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < 2 * n; i += stride) {
-        wx1[i] = (double)x1[i];
-        wx2[i] = (double)x2[i];
-        if (i < n) {
-            wd1[i] = (double)d1[i];
-            wd2[i] = (double)d2[i];
+    if (!perm) {
+        for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < 2 * n; i += stride) {
+            wx1[i] = (double)x1[i];
+            wx2[i] = (double)x2[i];
+            if (i < n) {
+                wd1[i] = (double)d1[i];
+                wd2[i] = (double)d2[i];
+            }
         }
+        return;
+    }
+    for (long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += stride) {
+        const long long s = offsets[pair_of(j, offsets, base, n_pairs)] - base + perm[j];
+        wx1[2 * j] = (double)x1[2 * s];
+        wx1[2 * j + 1] = (double)x1[2 * s + 1];
+        wx2[2 * j] = (double)x2[2 * s];
+        wx2[2 * j + 1] = (double)x2[2 * s + 1];
+        wd1[j] = (double)d1[s];
+        wd2[j] = (double)d2[s];
     }
 }
 

@@ -81,11 +81,14 @@ def gather_depths_batch(depth_maps, frame1, frame2, offsets, keypoints1, keypoin
     return out, x1[:m], x2[:m], d1[:m], d2[:m]
 
 
-def estimate_batch(variant, offsets, x1, x2, d1, d2, cams, opt: nv.Options):
+def estimate_batch(variant, offsets, x1, x2, d1, d2, cams, opt: nv.Options, quality=None):
     """Packed CUDA float64 tensors in (offsets: host int64 array), CUDA tensors out:
     models [P,12] float64, stats [P,5] (int64 view; columns 3,4 are float64 bit patterns — use
     `stats_to_numpy`), masks [N] uint8.  When x1, x2, d1, d2 are all float32 they are passed as they are to the
-    float32 entry point (no FP64 copy of the batch; the same results as float64 tensors of the same values)."""
+    float32 entry point (no FP64 copy of the batch; the same results as float64 tensors of the same values).
+    `quality` (optional): CUDA tensor [N] of match qualities, converted to float32 on the device; each pair is then
+    ordered by decreasing quality before the estimator runs (rp_estimate_batch_dev[_f32]_quality), and the masks come
+    back in the caller's order."""
     ctx = _ctx_for(x1)
     dev = x1.device
     offsets = np.ascontiguousarray(offsets, dtype=np.int64)
@@ -97,13 +100,25 @@ def estimate_batch(variant, offsets, x1, x2, d1, d2, cams, opt: nv.Options):
     if x1.shape != (N, 2) or x2.shape != (N, 2) or d1.shape != (N,) or d2.shape != (N,):
         raise ValueError("x1/x2 must be [N,2] and d1/d2 [N] with N = offsets[-1]")
     cams_t = t64(cams) if cams is not None else None
+    if quality is not None:
+        if not quality.is_cuda or quality.device != dev:
+            raise ValueError("quality must be a CUDA tensor on the device of the points")
+        quality = quality.contiguous().to(torch.float32)
+        if quality.shape != (N,):
+            raise ValueError("quality must be [N] with N = offsets[-1]")
     models = torch.zeros(P, 12, dtype=torch.float64, device=dev)
     stats = torch.zeros(P, 5, dtype=torch.int64, device=dev)
     masks = torch.zeros(max(N, 1), dtype=torch.uint8, device=dev)
-    est = ctx.estimate_batch_dev_f32 if f32 else ctx.estimate_batch_dev
-    est(variant, offsets, x1.data_ptr(), x2.data_ptr(), d1.data_ptr(), d2.data_ptr(),
-        cams_t.data_ptr() if cams_t is not None else None, opt, models.data_ptr(),
-        stats.data_ptr(), masks.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+    outs = (models.data_ptr(), stats.data_ptr(), masks.data_ptr())
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    cams_p = cams_t.data_ptr() if cams_t is not None else None
+    if quality is not None:
+        est = ctx.estimate_batch_dev_f32_quality if f32 else ctx.estimate_batch_dev_quality
+        est(variant, offsets, x1.data_ptr(), x2.data_ptr(), d1.data_ptr(), d2.data_ptr(), cams_p, opt, *outs,
+            quality.data_ptr(), stream)
+    else:
+        est = ctx.estimate_batch_dev_f32 if f32 else ctx.estimate_batch_dev
+        est(variant, offsets, x1.data_ptr(), x2.data_ptr(), d1.data_ptr(), d2.data_ptr(), cams_p, opt, *outs, stream)
     return models, stats, masks[:N]
 
 
