@@ -258,6 +258,34 @@ RP_API int rp_gather_depths_batch_dev_f32(rp_ctx *ctx, int64_t n_pairs, const in
                                           const float *kp1, const float *kp2, float *x1, float *x2, float *d1, float *d2,
                                           int64_t *out_offsets, void *stream);
 
+/* The four gathers carrying one float32 match quality per keypoint row (LightGlue score, RoMa certainty, ...), so that the
+ * quality of the rows they keep arrives packed next to them for rp_estimate_batch_dev[_f32]_quality: quality (DEVICE,
+ * one value per input row) inserted after kp2 in the twin's argument list, quality_out (DEVICE, capacity as d1) after d2.
+ * They are defined against their twin:
+ *   - x1, x2, d1, d2 and *n_out / out_offsets are byte for byte the twin's for the same inputs;
+ *   - quality_out is quality[keep], where keep is the twin's keep rule: input order, packed at the same offsets.  Each
+ *     value is copied as its 32-bit pattern (NaN payloads, -0 and infinities unchanged); the keep rule never reads it.
+ * For a non-empty input a null quality or quality_out is RP_ERR_INVALID; every other check and error code is the twin's,
+ * and an empty input returns RP_OK with nothing written.  They synchronise as often as the twin (the batch: twice). */
+RP_API int rp_gather_depths_dev_quality(rp_ctx *ctx, const float *depth1, int h1, int w1, const float *depth2, int h2,
+                                        int w2, const float *kp1, const float *kp2, const float *quality, int64_t n,
+                                        double *x1, double *x2, double *d1, double *d2, float *quality_out,
+                                        int64_t *n_out, void *stream);
+RP_API int rp_gather_depths_dev_f32_quality(rp_ctx *ctx, const float *depth1, int h1, int w1, const float *depth2, int h2,
+                                            int w2, const float *kp1, const float *kp2, const float *quality, int64_t n,
+                                            float *x1, float *x2, float *d1, float *d2, float *quality_out,
+                                            int64_t *n_out, void *stream);
+RP_API int rp_gather_depths_batch_dev_quality(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_offsets,
+                                              const float *depth_maps, int n_frames, int h, int w, const int32_t *frame1,
+                                              const int32_t *frame2, const float *kp1, const float *kp2,
+                                              const float *quality, double *x1, double *x2, double *d1, double *d2,
+                                              float *quality_out, int64_t *out_offsets, void *stream);
+RP_API int rp_gather_depths_batch_dev_f32_quality(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_offsets,
+                                                  const float *depth_maps, int n_frames, int h, int w,
+                                                  const int32_t *frame1, const int32_t *frame2, const float *kp1,
+                                                  const float *kp2, const float *quality, float *x1, float *x2, float *d1,
+                                                  float *d2, float *quality_out, int64_t *out_offsets, void *stream);
+
 /* ---- measurement helpers ---------------------------------------------------------
  * Pipe micro-benchmarks for the roofline denominators SURVEY.md §8d asks for (the driver's
  * MEASURED_PEAKS.json has only HBM and bf16): sustained FP64 and FP32 FMA throughput of

@@ -24,6 +24,8 @@ EXPORTS = [
     "rp_estimate_batch_host_f32", "rp_estimate_batch_dev_f32", "rp_gather_depths_dev_f32", "rp_gather_depths_batch_dev_f32",
     "rp_estimate_batch_host_quality", "rp_estimate_batch_dev_quality", "rp_estimate_batch_host_f32_quality",
     "rp_estimate_batch_dev_f32_quality", "rp_order_by_quality",
+    "rp_gather_depths_dev_quality", "rp_gather_depths_dev_f32_quality", "rp_gather_depths_batch_dev_quality",
+    "rp_gather_depths_batch_dev_f32_quality",
 ]
 ORDER_SMEM_CAP = 12288   # RP_ORDER_SMEM_CAP: larger pairs are ordered in global scratch
 
@@ -138,6 +140,12 @@ def load():
         f.restype = C.c_int
     L.rp_gather_depths_dev_f32.argtypes = L.rp_gather_depths_dev.argtypes
     L.rp_gather_depths_batch_dev_f32.argtypes = L.rp_gather_depths_batch_dev.argtypes
+    # the _quality gathers: the twin's arguments with quality after kp2 and quality_out after d2
+    for twin, kp2, d2 in (("rp_gather_depths_dev", 8, 13), ("rp_gather_depths_batch_dev", 10, 14)):
+        t = getattr(L, twin).argtypes
+        for name in (twin + "_quality", twin + "_f32_quality"):
+            getattr(L, name).restype = C.c_int
+            getattr(L, name).argtypes = t[:kp2 + 1] + [VP] + t[kp2 + 1:d2 + 1] + [VP] + t[d2 + 1:]
     L.rp_measure_pipes.restype = C.c_int
     L.rp_measure_pipes.argtypes = [VP, DP, DP]
     L.rp_pair_status.restype = C.c_int

@@ -60,7 +60,9 @@ enum { B_OFFS, B_PAIRS, B_PTS64, B_PTS32, B_BEAR, B_SAMPLES, B_MODELS, B_HYPITER
        B_STG_X1, B_STG_X2, B_STG_D1, B_STG_D2, B_STG_X1_B, B_STG_X2_B, B_STG_D1_B, B_STG_D2_B,
        // quality calls (rp_order.cuh): uploaded quality, the chunk's offsets and order, masks in the ordered layout
        // (double-buffered on the host path), global sort scratch of pairs above RP_ORDER_SMEM_CAP
-       B_QUAL, B_QUAL_B, B_ORDOFFS, B_ORDOFFS_B, B_PERM, B_PERM_B, B_KSORT, B_KSORT_B, B_ORDSCR, B_NBUF };
+       B_QUAL, B_QUAL_B, B_ORDOFFS, B_ORDOFFS_B, B_PERM, B_PERM_B, B_KSORT, B_KSORT_B, B_ORDSCR,
+       // rp_gather_depths_batch_dev*_quality: the compacted quality between the two passes (4 B per row)
+       B_GATHER_Q, B_NBUF };
 
 // device scalars living in B_SCALARS
 struct Scalars {
@@ -1573,21 +1575,23 @@ int rp_refine_batch(rp_ctx *ctx, int variant, int64_t n_models, rp_model *models
 
 namespace {
 
-// rp_gather_depths_dev[_f32]: T is the output type
+// rp_gather_depths_dev[_f32][_quality]: T is the output type; with_q: the _quality entry points (quality / quality_out)
 template <class T>
 int gather_depths_impl(rp_ctx *ctx, const float *depth1, int h1, int w1, const float *depth2, int h2, int w2,
-                       const float *kp1, const float *kp2, int64_t n, T *x1, T *x2, T *d1, T *d2, int64_t *n_out,
-                       void *stream) {
+                       const float *kp1, const float *kp2, const float *quality, int64_t n, T *x1, T *x2, T *d1, T *d2,
+                       float *quality_out, int64_t *n_out, void *stream, bool with_q) {
     if (!ctx || n < 0 || !n_out || h1 <= 0 || w1 <= 0 || h2 <= 0 || w2 <= 0 ||
         (n > 0 && (!depth1 || !depth2 || !kp1 || !kp2 || !x1 || !x2 || !d1 || !d2)))
         return fail(ctx, RP_ERR_INVALID, "bad argument");
+    if (with_q && n > 0 && (!quality || !quality_out)) return fail(ctx, RP_ERR_INVALID, "null quality / quality_out");
     *n_out = 0;
     if (n == 0) return RP_OK;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
     CK(ctx->buf[B_SCALARS].reserve(sizeof(Scalars)));
     long long *d_n = (long long *)ctx->buf[B_SCALARS].p;
-    gather_depths_kernel<T><<<1, 1024, 0, st>>>(depth1, h1, w1, depth2, h2, w2, kp1, kp2, (long long)n, x1, x2, d1, d2, d_n);
+    gather_depths_kernel<T><<<1, 1024, 0, st>>>(depth1, h1, w1, depth2, h2, w2, kp1, kp2, quality, (long long)n,
+                                                x1, x2, d1, d2, quality_out, d_n);
     LAUNCHED();
     long long h_n = 0;
     CK(cudaMemcpyAsync(&h_n, d_n, sizeof h_n, cudaMemcpyDeviceToHost, st));
@@ -1596,11 +1600,12 @@ int gather_depths_impl(rp_ctx *ctx, const float *depth1, int h1, int w1, const f
     return RP_OK;
 }
 
-// rp_gather_depths_batch_dev[_f32]: T is the output type
+// rp_gather_depths_batch_dev[_f32][_quality]: T is the output type; with_q as above
 template <class T>
 int gather_depths_batch_impl(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_offsets, const float *depth_maps, int n_frames,
                              int h, int w, const int32_t *frame1, const int32_t *frame2, const float *kp1, const float *kp2,
-                             T *x1, T *x2, T *d1, T *d2, int64_t *out_offsets, void *stream) {
+                             const float *quality, T *x1, T *x2, T *d1, T *d2, float *quality_out, int64_t *out_offsets,
+                             void *stream, bool with_q) {
     if (!ctx || n_pairs < 0 || !in_offsets || !out_offsets || h <= 0 || w <= 0 || n_frames <= 0 ||
         (n_pairs > 0 && (!depth_maps || !frame1 || !frame2)))
         return fail(ctx, RP_ERR_INVALID, "bad argument");
@@ -1612,11 +1617,13 @@ int gather_depths_batch_impl(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_off
             return fail(ctx, RP_ERR_INVALID, "offsets must be non-decreasing and frame indices inside [0, n_frames)");
     }
     if (N > 0 && (!kp1 || !kp2 || !x1 || !x2 || !d1 || !d2)) return fail(ctx, RP_ERR_INVALID, "null data pointer");
+    if (with_q && N > 0 && (!quality || !quality_out)) return fail(ctx, RP_ERR_INVALID, "null quality / quality_out");
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
     DevBuf *B = ctx->buf;
     const size_t nn = (size_t)std::max<long long>(N, 1);
     CK(B[B_SUB_X1].reserve(16 * nn)); CK(B[B_SUB_X2].reserve(16 * nn)); CK(B[B_SUB_D1].reserve(8 * nn)); CK(B[B_SUB_D2].reserve(8 * nn));
+    if (with_q) CK(B[B_GATHER_Q].reserve(4 * nn));
     CK(B[B_SUB_SRC].reserve(8 * ((size_t)n_pairs + 1))); CK(B[B_SUB_DST].reserve(8 * ((size_t)n_pairs + 1)));
     CK(B[B_SUB_IDX].reserve(sizeof(int) * 3 * (size_t)n_pairs));
     std::vector<long long> rel((size_t)n_pairs + 1);
@@ -1631,6 +1638,7 @@ int gather_depths_batch_impl(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_off
     g.kp1 = kp1; g.kp2 = kp2;
     g.tx1 = B[B_SUB_X1].as<T>(); g.tx2 = B[B_SUB_X2].as<T>(); g.td1 = B[B_SUB_D1].as<T>(); g.td2 = B[B_SUB_D2].as<T>();
     g.x1 = x1; g.x2 = x2; g.d1 = d1; g.d2 = d2; g.count = d_cnt;
+    g.q_in = quality; g.tq = with_q ? B[B_GATHER_Q].as<float>() : nullptr; g.q_out = quality_out;
     gather_depths_batch_kernel<T><<<(unsigned)n_pairs, 256, 0, st>>>(g);
     LAUNCHED();
     std::vector<int> cnt((size_t)n_pairs);
@@ -1653,28 +1661,60 @@ extern "C" {
 int rp_gather_depths_dev(rp_ctx *ctx, const float *depth1, int h1, int w1, const float *depth2, int h2, int w2,
                          const float *kp1, const float *kp2, int64_t n, double *x1, double *x2, double *d1, double *d2,
                          int64_t *n_out, void *stream) {
-    return gather_depths_impl(ctx, depth1, h1, w1, depth2, h2, w2, kp1, kp2, n, x1, x2, d1, d2, n_out, stream);
+    return gather_depths_impl(ctx, depth1, h1, w1, depth2, h2, w2, kp1, kp2, nullptr, n, x1, x2, d1, d2, nullptr, n_out,
+                              stream, false);
 }
 
 int rp_gather_depths_dev_f32(rp_ctx *ctx, const float *depth1, int h1, int w1, const float *depth2, int h2, int w2,
                              const float *kp1, const float *kp2, int64_t n, float *x1, float *x2, float *d1, float *d2,
                              int64_t *n_out, void *stream) {
-    return gather_depths_impl(ctx, depth1, h1, w1, depth2, h2, w2, kp1, kp2, n, x1, x2, d1, d2, n_out, stream);
+    return gather_depths_impl(ctx, depth1, h1, w1, depth2, h2, w2, kp1, kp2, nullptr, n, x1, x2, d1, d2, nullptr, n_out,
+                              stream, false);
 }
 
 int rp_gather_depths_batch_dev(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_offsets, const float *depth_maps, int n_frames,
                                int h, int w, const int32_t *frame1, const int32_t *frame2, const float *kp1, const float *kp2,
                                double *x1, double *x2, double *d1, double *d2, int64_t *out_offsets, void *stream) {
-    return gather_depths_batch_impl(ctx, n_pairs, in_offsets, depth_maps, n_frames, h, w, frame1, frame2, kp1, kp2, x1, x2, d1,
-                                    d2, out_offsets, stream);
+    return gather_depths_batch_impl(ctx, n_pairs, in_offsets, depth_maps, n_frames, h, w, frame1, frame2, kp1, kp2, nullptr,
+                                    x1, x2, d1, d2, nullptr, out_offsets, stream, false);
 }
 
 int rp_gather_depths_batch_dev_f32(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_offsets, const float *depth_maps,
                                    int n_frames, int h, int w, const int32_t *frame1, const int32_t *frame2, const float *kp1,
                                    const float *kp2, float *x1, float *x2, float *d1, float *d2, int64_t *out_offsets,
                                    void *stream) {
-    return gather_depths_batch_impl(ctx, n_pairs, in_offsets, depth_maps, n_frames, h, w, frame1, frame2, kp1, kp2, x1, x2, d1,
-                                    d2, out_offsets, stream);
+    return gather_depths_batch_impl(ctx, n_pairs, in_offsets, depth_maps, n_frames, h, w, frame1, frame2, kp1, kp2, nullptr,
+                                    x1, x2, d1, d2, nullptr, out_offsets, stream, false);
+}
+
+int rp_gather_depths_dev_quality(rp_ctx *ctx, const float *depth1, int h1, int w1, const float *depth2, int h2, int w2,
+                                 const float *kp1, const float *kp2, const float *quality, int64_t n, double *x1, double *x2,
+                                 double *d1, double *d2, float *quality_out, int64_t *n_out, void *stream) {
+    return gather_depths_impl(ctx, depth1, h1, w1, depth2, h2, w2, kp1, kp2, quality, n, x1, x2, d1, d2, quality_out, n_out,
+                              stream, true);
+}
+
+int rp_gather_depths_dev_f32_quality(rp_ctx *ctx, const float *depth1, int h1, int w1, const float *depth2, int h2, int w2,
+                                     const float *kp1, const float *kp2, const float *quality, int64_t n, float *x1,
+                                     float *x2, float *d1, float *d2, float *quality_out, int64_t *n_out, void *stream) {
+    return gather_depths_impl(ctx, depth1, h1, w1, depth2, h2, w2, kp1, kp2, quality, n, x1, x2, d1, d2, quality_out, n_out,
+                              stream, true);
+}
+
+int rp_gather_depths_batch_dev_quality(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_offsets, const float *depth_maps,
+                                       int n_frames, int h, int w, const int32_t *frame1, const int32_t *frame2,
+                                       const float *kp1, const float *kp2, const float *quality, double *x1, double *x2,
+                                       double *d1, double *d2, float *quality_out, int64_t *out_offsets, void *stream) {
+    return gather_depths_batch_impl(ctx, n_pairs, in_offsets, depth_maps, n_frames, h, w, frame1, frame2, kp1, kp2, quality,
+                                    x1, x2, d1, d2, quality_out, out_offsets, stream, true);
+}
+
+int rp_gather_depths_batch_dev_f32_quality(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_offsets, const float *depth_maps,
+                                           int n_frames, int h, int w, const int32_t *frame1, const int32_t *frame2,
+                                           const float *kp1, const float *kp2, const float *quality, float *x1, float *x2,
+                                           float *d1, float *d2, float *quality_out, int64_t *out_offsets, void *stream) {
+    return gather_depths_batch_impl(ctx, n_pairs, in_offsets, depth_maps, n_frames, h, w, frame1, frame2, kp1, kp2, quality,
+                                    x1, x2, d1, d2, quality_out, out_offsets, stream, true);
 }
 
 int rp_measure_pipes(rp_ctx *ctx, double *fp64_tflops, double *fp32_tflops) {

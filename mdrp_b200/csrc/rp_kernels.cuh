@@ -1613,10 +1613,13 @@ __global__ void fill_int_kernel(int *p, int n, int v) {
 // the lookup, the mask and the stable compaction on the device, straight into the packed layout the
 // estimator takes: T = double for rp_estimate_batch_*, T = float for rp_estimate_batch_*_f32 (the float
 // inputs unchanged).  One block; rows keep their order.
+// q_in / q_out (rp_gather_depths_*_quality; both null otherwise): a kept row's match quality goes to the same output
+// position as its keypoints, copied as a 32-bit pattern (NaN payloads, -0 and infinities unchanged).  The keep rule
+// never reads it.
 template <class T>
 __global__ void gather_depths_kernel(const float *depth1, int h1, int w1, const float *depth2, int h2, int w2,
-                                     const float *kp1, const float *kp2, long long n, T *x1, T *x2,
-                                     T *d1, T *d2, long long *n_out) {
+                                     const float *kp1, const float *kp2, const float *q_in, long long n, T *x1, T *x2,
+                                     T *d1, T *d2, float *q_out, long long *n_out) {
     __shared__ int warp_tot[32];
     __shared__ long long running;
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
@@ -1646,6 +1649,7 @@ __global__ void gather_depths_kernel(const float *depth1, int h1, int w1, const 
             const long long o = running + wbase + __popc(m & ((1u << lane) - 1u));
             x1[2 * o] = ax; x1[2 * o + 1] = ay; x2[2 * o] = bx; x2[2 * o + 1] = by;
             d1[o] = da; d2[o] = db;
+            if (q_out) ((unsigned *)q_out)[o] = ((const unsigned *)q_in)[i];
         }
         __syncthreads();
         if (tid == 0) running += total;
@@ -1658,7 +1662,8 @@ __global__ void gather_depths_kernel(const float *depth1, int h1, int w1, const 
 // size stacked [F, h, w], pair p = (frame1[p], frame2[p]) with keypoints [in_off[p], in_off[p+1]).  Pass 1: one CTA per
 // pair, stable compaction of the pair's rows INTO ITS OWN INPUT RANGE of the temporary arrays + the kept count; the host
 // reads the n_pairs counts once (it needs the packed offsets anyway: rp_estimate_batch_dev takes them), pass 2 moves
-// every pair's block to its packed position.  T: output type, as in gather_depths_kernel.
+// every pair's block to its packed position.  T: output type, as in gather_depths_kernel.  q_in / tq / q_out: the match
+// quality, carried through both passes as in gather_depths_kernel (all three null without one).
 template <class T>
 struct GatherBatchArgs {
     int n_pairs, h, w;
@@ -1670,6 +1675,8 @@ struct GatherBatchArgs {
     T *tx1, *tx2, *td1, *td2;      // temporaries, capacity N
     T *x1, *x2, *d1, *d2;          // packed outputs
     int *count;                    // [n_pairs]
+    const float *q_in;             // [N]
+    float *tq, *q_out;             // temporary (capacity N), packed output
 };
 template <class T>
 __global__ void gather_depths_batch_kernel(GatherBatchArgs<T> a) {
@@ -1705,6 +1712,7 @@ __global__ void gather_depths_batch_kernel(GatherBatchArgs<T> a) {
             const long long o = i0 + running + wbase + __popc(m & ((1u << lane) - 1u));
             a.tx1[2 * o] = ax; a.tx1[2 * o + 1] = ay; a.tx2[2 * o] = bx; a.tx2[2 * o + 1] = by;
             a.td1[o] = da; a.td2[o] = db;
+            if (a.tq) ((unsigned *)a.tq)[o] = ((const unsigned *)a.q_in)[i0 + i];
         }
         __syncthreads();
         if (tid == 0) running += total;
@@ -1725,6 +1733,8 @@ __global__ void gather_depths_pack_kernel(GatherBatchArgs<T> a) {
         a.d1[o0 + i] = a.td1[i0 + i];
         a.d2[o0 + i] = a.td2[i0 + i];
     }
+    if (a.q_out)
+        for (int i = threadIdx.x; i < n; i += blockDim.x) ((unsigned *)a.q_out)[o0 + i] = ((const unsigned *)a.tq)[i0 + i];
 }
 
 // float32 inputs (rp_estimate_batch_*_f32): one chunk's x1, x2 [n,2] and d1, d2 [n] widened into the FP64 arrays every

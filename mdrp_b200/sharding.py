@@ -110,21 +110,25 @@ def gather_results(models, stats, masks, rank: int, world_size: int, device=None
 
 
 def estimate_sharded(estimate_fn, offsets, x1, x2, d1, d2, cams, rank: int, world_size: int, gather: bool = True,
-                     device=None):
+                     device=None, quality=None):
     """Every rank holds (or maps) the whole batch: run `estimate_fn(offsets, x1, x2, d1, d2, cams) -> (models, stats,
-    masks)` on this rank's shard and gather the results on rank 0 in pair order (other ranks get None)."""
+    masks)` on this rank's shard and gather the results on rank 0 in pair order (other ranks get None).  With a
+    `quality` ([N], one match quality per correspondence) the shard's slice of it is passed as a seventh argument."""
     p0, p1, n0, n1, loc = shard_of(offsets, rank, world_size)
-    res = estimate_fn(loc, x1[n0:n1], x2[n0:n1], d1[n0:n1], d2[n0:n1], None if cams is None else cams[p0:p1])
+    args = (loc, x1[n0:n1], x2[n0:n1], d1[n0:n1], d2[n0:n1], None if cams is None else cams[p0:p1])
+    res = estimate_fn(*args) if quality is None else estimate_fn(*args, quality[n0:n1])
     if world_size == 1 or not gather:
         return res
     return gather_results(res[0], res[1], res[2], rank, world_size, device=device)
 
 
 def estimate_local_shard(ctx, variant, offsets, x1, x2, d1, d2, cams, opt, rank: int, world_size: int, device=None,
-                         gather_masks: bool = True):
+                         gather_masks: bool = True, quality=None):
     """Every rank holds only ITS shard (local offsets and arrays): run it on this rank's GPU (`ctx`: an
     mdrp_b200._native.Context) and gather on rank 0.  This is what bench.py times at N > 1.  float32 numpy points and
-    depths go through the float32 entry point (half the upload, the same results), everything else through FP64."""
+    depths go through the float32 entry point (half the upload, the same results), everything else through FP64.
+    `quality` (optional): the shard's match qualities [N], one per correspondence; each pair is then ordered by it
+    (the quality entry point of the same dtype)."""
     from .api import _estimate_host
-    models, stats, masks = _estimate_host(ctx, variant, offsets, x1, x2, d1, d2, cams, opt)
+    models, stats, masks = _estimate_host(ctx, variant, offsets, x1, x2, d1, d2, cams, opt, quality)
     return gather_results(models, stats, masks, rank, world_size, device=device, gather_masks=gather_masks)

@@ -22,19 +22,37 @@ def _ctx_for(t: torch.Tensor) -> nv.Context:
 _GATHER_DTYPES = (torch.float64, torch.float32)
 
 
-def _gather_fn(ctx, name, dtype):
+def _gather_fn(ctx, name, dtype, quality):
     if dtype not in _GATHER_DTYPES:
         raise ValueError("dtype must be torch.float64 or torch.float32")
-    return getattr(ctx._lib, name + ("_f32" if dtype == torch.float32 else ""))
+    return getattr(ctx._lib, name + ("_f32" if dtype == torch.float32 else "") + ("_quality" if quality is not None else ""))
 
 
-def gather_depths(depth_map1, depth_map2, keypoints1, keypoints2, dtype=torch.float64):
+def _quality_buffers(quality, keypoints, n):
+    """For a gather with a match quality: (the quality as contiguous float32 [n], its output tensor [n], and the two
+    pointers the _quality entry point takes after kp2 and after d2, as one-element lists).  Without one: Nones and
+    empty lists, so the twin's argument list is unchanged."""
+    if quality is None:
+        return None, None, [], []
+    if not quality.is_cuda or quality.device != keypoints.device:
+        raise ValueError("quality must be a CUDA tensor on the device of the keypoints")
+    quality = quality.contiguous().to(torch.float32)
+    if quality.shape != (n,):
+        raise ValueError("quality must be [n], one value per keypoint row")
+    q_out = torch.empty(n, dtype=torch.float32, device=keypoints.device)
+    return quality, q_out, [quality.data_ptr()], [q_out.data_ptr()]
+
+
+def gather_depths(depth_map1, depth_map2, keypoints1, keypoints2, dtype=torch.float64, quality=None):
     """depths at the matched keypoints + removal of rows whose depths are both inf (make_pair.py:97-106),
     on the device.  depth maps: [H,W] float32 CUDA; keypoints: [n,2] float32 CUDA (x, y).
     Returns (x1, x2, d1, d2) CUDA tensors of `dtype` (float64, or float32: the values unchanged, what `estimate_batch`
-    takes without an FP64 copy) with the kept rows in order."""
+    takes without an FP64 copy) with the kept rows in order.
+    `quality` (optional): CUDA tensor [n] of match qualities (converted to float32); the kept rows' qualities are then
+    returned as a fifth element, float32 [m], bit for bit and aligned with the other outputs: the `quality` that
+    `estimate_batch` takes for them."""
     ctx = _ctx_for(depth_map1)
-    fn = _gather_fn(ctx, "rp_gather_depths_dev", dtype)
+    fn = _gather_fn(ctx, "rp_gather_depths_dev", dtype, quality)
     dm1 = depth_map1.contiguous().float()
     dm2 = depth_map2.contiguous().float()
     k1 = keypoints1.contiguous().float()
@@ -46,21 +64,23 @@ def gather_depths(depth_map1, depth_map2, keypoints1, keypoints2, dtype=torch.fl
     d1 = torch.empty(n, dtype=dtype, device=dev)
     d2 = torch.empty(n, dtype=dtype, device=dev)
     n_out = C.c_int64(0)
+    q, q_out, q_in_p, q_out_p = _quality_buffers(quality, k1, n)
     stream = torch.cuda.current_stream(dev).cuda_stream
     ctx._call(fn, ctx._h, dm1.data_ptr(), dm1.shape[0], dm1.shape[1], dm2.data_ptr(),
-              dm2.shape[0], dm2.shape[1], k1.data_ptr(), k2.data_ptr(), n, x1.data_ptr(), x2.data_ptr(),
-              d1.data_ptr(), d2.data_ptr(), C.byref(n_out), stream)
+              dm2.shape[0], dm2.shape[1], k1.data_ptr(), k2.data_ptr(), *q_in_p, n, x1.data_ptr(), x2.data_ptr(),
+              d1.data_ptr(), d2.data_ptr(), *q_out_p, C.byref(n_out), stream)
     m = n_out.value
-    return x1[:m], x2[:m], d1[:m], d2[:m]
+    return (x1[:m], x2[:m], d1[:m], d2[:m]) + (() if q_out is None else (q_out[:m],))
 
 
-def gather_depths_batch(depth_maps, frame1, frame2, offsets, keypoints1, keypoints2, dtype=torch.float64):
+def gather_depths_batch(depth_maps, frame1, frame2, offsets, keypoints1, keypoints2, dtype=torch.float64, quality=None):
     """`gather_depths` for a batch of pairs in one call (a video: make_video.py:270-290).  depth_maps: [F,H,W] float32
     CUDA; frame1 / frame2: per-pair frame indices; offsets: [P+1] rows of the packed keypoints [N,2] float32 CUDA.
     Returns (out_offsets int64 numpy, x1, x2, d1, d2) — the packed CUDA tensors of `dtype` (float64 or float32)
-    `estimate_batch` takes."""
+    `estimate_batch` takes.  `quality` (optional): CUDA tensor [N] of match qualities; the packed float32 qualities of
+    the kept rows are then returned as a sixth element, ready for `estimate_batch(..., quality=...)`."""
     ctx = _ctx_for(depth_maps)
-    fn = _gather_fn(ctx, "rp_gather_depths_batch_dev", dtype)
+    fn = _gather_fn(ctx, "rp_gather_depths_batch_dev", dtype, quality)
     dm = depth_maps.contiguous().float()
     k1, k2 = keypoints1.contiguous().float(), keypoints2.contiguous().float()
     offsets = np.ascontiguousarray(offsets, dtype=np.int64)
@@ -74,11 +94,12 @@ def gather_depths_batch(depth_maps, frame1, frame2, offsets, keypoints1, keypoin
     d1 = torch.empty(n, dtype=dtype, device=dev)
     d2 = torch.empty(n, dtype=dtype, device=dev)
     out = np.zeros(P + 1, dtype=np.int64)
+    q, q_out, q_in_p, q_out_p = _quality_buffers(quality, k1, n)
     ctx._call(fn, ctx._h, P, offsets.ctypes.data, dm.data_ptr(), dm.shape[0], dm.shape[1],
-              dm.shape[2], f1.ctypes.data, f2.ctypes.data, k1.data_ptr(), k2.data_ptr(), x1.data_ptr(), x2.data_ptr(),
-              d1.data_ptr(), d2.data_ptr(), out.ctypes.data, torch.cuda.current_stream(dev).cuda_stream)
+              dm.shape[2], f1.ctypes.data, f2.ctypes.data, k1.data_ptr(), k2.data_ptr(), *q_in_p, x1.data_ptr(),
+              x2.data_ptr(), d1.data_ptr(), d2.data_ptr(), *q_out_p, out.ctypes.data, torch.cuda.current_stream(dev).cuda_stream)
     m = int(out[-1])
-    return out, x1[:m], x2[:m], d1[:m], d2[:m]
+    return (out, x1[:m], x2[:m], d1[:m], d2[:m]) + (() if q_out is None else (q_out[:m],))
 
 
 def estimate_batch(variant, offsets, x1, x2, d1, d2, cams, opt: nv.Options, quality=None):
@@ -127,15 +148,16 @@ def stats_to_numpy(stats: torch.Tensor) -> np.ndarray:
 
 
 def estimate_monodepth_relative_pose(points2D_1, points2D_2, depth_1, depth_2, camera1, camera2, ransac_opt={},
-                                     bundle_opt={}, initial_pose=None):
+                                     bundle_opt={}, initial_pose=None, quality=None):
     """poselib.estimate_monodepth_relative_pose with CUDA tensor inputs; same return objects.  float32 points and
-    depths take the float32 path of `estimate_batch`."""
+    depths take the float32 path of `estimate_batch`; `quality` (optional CUDA tensor [n]) is passed on to it."""
     opt = api.make_options(ransac_opt, bundle_opt, focal_variant=False)
     cams = torch.tensor([api.Camera.from_any(camera1).fxfycxcy() + api.Camera.from_any(camera2).fxfycxcy()],
                         dtype=torch.float64, device=points2D_1.device)
     n = points2D_1.shape[0]
     variant = nv.CALIB_SHIFT if opt.estimate_shift else nv.CALIB
-    models, stats, masks = estimate_batch(variant, [0, n], points2D_1, points2D_2, depth_1, depth_2, cams, opt)
+    models, stats, masks = estimate_batch(variant, [0, n], points2D_1, points2D_2, depth_1, depth_2, cams, opt,
+                                         quality=quality)
     m = models[0].cpu().numpy()
     st = stats_to_numpy(stats)[0]
     geom = api.MonoDepthTwoViewGeometry(api.CameraPose(m[:4], m[4:7]), m[7], m[8], m[9])

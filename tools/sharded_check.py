@@ -5,7 +5,11 @@
         tools/sharded_check.py
 
 Every rank builds the same ragged batch, runs its shard through the CUDA estimator (mdrp_b200.sharding over NCCL) and
-rank 0 compares the gathered result with the whole batch run on its own GPU: bytes must be identical."""
+rank 0 compares the gathered result with the whole batch run on its own GPU: bytes must be identical.
+
+--quality: the same batches with one match quality per correspondence and PROSAC on, through both sharded entry points
+(each rank gets its slice of the quality); rank 0 compares with the unsharded estimate_batch_host_quality call."""
+import argparse
 import os
 import sys
 
@@ -19,6 +23,9 @@ from mdrp_b200 import _native as nv, sharding, synth  # noqa: E402
 
 
 def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--quality", action="store_true", help="per-correspondence match quality, PROSAC on")
+    with_q = ap.parse_args().quality
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
@@ -42,18 +49,34 @@ def main():
         o.max_iterations = o.min_iterations = min(c["iters"], 2000)
         o.max_epipolar_error, o.max_reproj_error, o.estimate_shift = 2.0, 16.0, int(c["shift"])
         o.loss_type, o.loss_scale = nv.LOSS["TRUNCATED_CAUCHY"], 1.0
-        fn = lambda of, a, b, e, f, k: ctx.estimate_batch_host(variant, of, a, b, e, f, k, o)  # noqa: E731
-        got = sharding.estimate_sharded(fn, offs, x1, x2, d1, d2, cams, rank, world, device=dev)
-        # the local-shard entry point (each rank holds only its shard)
         p0, p1, n0, n1, loc = sharding.shard_of(offs, rank, world)
-        got2 = sharding.estimate_local_shard(ctx, variant, loc, x1[n0:n1], x2[n0:n1], d1[n0:n1], d2[n0:n1],
-                                             None if cams is None else cams[p0:p1], o, rank, world, device=dev)
+        if with_q:
+            # quality correlated with being an inlier, with ties and a NaN every 101st
+            rng = np.random.default_rng(7)
+            inl = np.concatenate([s.inlier_mask[:n] for s, n in zip(scs, sizes)])
+            q = np.where(inl, rng.uniform(0.3, 1.0, len(inl)), rng.uniform(0.0, 0.7, len(inl))).astype(np.float32)
+            q[::13], q[::101] = 0.5, np.nan
+            o.progressive_sampling = 1
+            fn = lambda of, a, b, e, f, k, qq: ctx.estimate_batch_host_quality(variant, of, a, b, e, f, k, o, qq)  # noqa: E731
+            got = sharding.estimate_sharded(fn, offs, x1, x2, d1, d2, cams, rank, world, device=dev, quality=q)
+            got2 = sharding.estimate_local_shard(ctx, variant, loc, x1[n0:n1], x2[n0:n1], d1[n0:n1], d2[n0:n1],
+                                                 None if cams is None else cams[p0:p1], o, rank, world, device=dev,
+                                                 quality=q[n0:n1])
+            unsharded = lambda: fn(offs, x1, x2, d1, d2, cams, q)  # noqa: E731
+        else:
+            fn = lambda of, a, b, e, f, k: ctx.estimate_batch_host(variant, of, a, b, e, f, k, o)  # noqa: E731
+            got = sharding.estimate_sharded(fn, offs, x1, x2, d1, d2, cams, rank, world, device=dev)
+            # the local-shard entry point (each rank holds only its shard)
+            got2 = sharding.estimate_local_shard(ctx, variant, loc, x1[n0:n1], x2[n0:n1], d1[n0:n1], d2[n0:n1],
+                                                 None if cams is None else cams[p0:p1], o, rank, world, device=dev)
+            unsharded = lambda: fn(offs, x1, x2, d1, d2, cams)  # noqa: E731
         if rank == 0:
-            ref = fn(offs, x1, x2, d1, d2, cams)
+            ref = unsharded()
             for g in (got, got2):
                 same = all(a.tobytes() == b.tobytes() for a, b in zip(g, ref))
                 ok = ok and same
-                print(f"{cfg}: {len(sizes)} pairs over {world} GPUs, sharded == unsharded bytes: {same}", flush=True)
+                print(f"{cfg}{' (quality)' if with_q else ''}: {len(sizes)} pairs over {world} GPUs, sharded == unsharded "
+                      f"bytes: {same}", flush=True)
         else:
             assert got is None and got2 is None
     dist.barrier()
