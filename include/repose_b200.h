@@ -185,6 +185,52 @@ RP_API int rp_estimate_batch_dev_f32_quality(rp_ctx *ctx, int variant, int64_t n
                                              const float *quality, const double *cams, const rp_options *opt,
                                              rp_model *models, rp_stats *stats, uint8_t *masks, void *stream);
 
+/* ---- refinement of caller-supplied models ----------------------------------------
+ * What the estimator does after RANSAC, on start models the caller supplies (the previous frame pair's poses of a
+ * tracker, another method's poses, an estimate to re-refine with other bundle options).  Pair p owns the
+ * correspondences [offsets[p], offsets[p+1]) and starts from init[p]; subset (optional, [offsets[n_pairs]] bytes) selects
+ * S_p = {correspondences with subset != 0}, a null subset means every correspondence.  For every pair the call:
+ *   1. runs the P1/P2 pre-processing over ALL the pair's correspondences, as the estimator does: unprojected (calibrated)
+ *      or normalised (focal variants) points, thr, scale_reproj and the final loss scale (calibrated: 0.5 * thr, the
+ *      user's loss_scale ignored; focal: loss_scale / nscale);
+ *   2. if |S_p| > 3: divides the focal variants' f1, f2 by nscale, runs the final refinement with the bundle fields of
+ *      opt and opt->weight_sampson on S_p only, and multiplies f1, f2 by nscale again;
+ *   3. RP_CALIB refines 7 parameters and holds shift1 / shift2 at their input values; RP_CALIB with opt->estimate_shift,
+ *      or RP_CALIB_SHIFT, refines 9.  The focal variants hold the shifts too; the calibrated variants neither read nor
+ *      change f1 / f2;
+ *   4. a pair that is not refined (|S_p| <= 3, including pairs of fewer than 3 correspondences) returns init[p] byte for
+ *      byte (no nscale round trip) and all-zero bundle stats;
+ *   5. num_inliers / inliers (optional; both are computed when either is non-null): the refined model's get_inliers mask
+ *      at the estimator's thr over all the pair's correspondences (Sampson + cheirality for the calibrated variants,
+ *      Sampson only for the focal ones) and its count; all-zero and 0 for pairs of fewer than 3 correspondences.
+ * A pair's results depend only on its own data, init[p], S_p and opt, never on the batch around it or on the chunking.
+ * The float32 entry points return the FP64 entry points' bytes for the same values.  The calls change neither
+ * rp_pair_status nor rp_last_timing, which keep describing the last estimate call.
+ * Layouts of offsets, x1..d2 and cams are the estimator's; cams is ignored by the focal variants (may be NULL).
+ * offsets and opt are HOST memory; for _host everything else is HOST memory, for _dev DEVICE memory, and _dev returns
+ * after `stream` has finished.  bstats, num_inliers and inliers may be NULL; models may alias init.  Argument checks and
+ * error codes are the estimator's, plus RP_ERR_INVALID for a null init or models with n_pairs > 0. */
+RP_API int rp_refine_pairs_host(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets,
+                                const double *x1, const double *x2, const double *d1, const double *d2,
+                                const double *cams, const rp_options *opt, const rp_model *init,
+                                const uint8_t *subset, rp_model *models, rp_bundle_stats *bstats,
+                                int64_t *num_inliers, uint8_t *inliers);
+RP_API int rp_refine_pairs_dev(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets,
+                               const double *x1, const double *x2, const double *d1, const double *d2,
+                               const double *cams, const rp_options *opt, const rp_model *init,
+                               const uint8_t *subset, rp_model *models, rp_bundle_stats *bstats,
+                               int64_t *num_inliers, uint8_t *inliers, void *stream);
+RP_API int rp_refine_pairs_host_f32(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets,
+                                    const float *x1, const float *x2, const float *d1, const float *d2,
+                                    const double *cams, const rp_options *opt, const rp_model *init,
+                                    const uint8_t *subset, rp_model *models, rp_bundle_stats *bstats,
+                                    int64_t *num_inliers, uint8_t *inliers);
+RP_API int rp_refine_pairs_dev_f32(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets,
+                                   const float *x1, const float *x2, const float *d1, const float *d2,
+                                   const double *cams, const rp_options *opt, const rp_model *init,
+                                   const uint8_t *subset, rp_model *models, rp_bundle_stats *bstats,
+                                   int64_t *num_inliers, uint8_t *inliers, void *stream);
+
 /* ---- stage entry points (parity tests; all pointers HOST memory) -----------------
  * Each mirrors one exported stage of the reference binary (SURVEY.md §8a). */
 

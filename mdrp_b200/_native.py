@@ -26,6 +26,7 @@ EXPORTS = [
     "rp_estimate_batch_dev_f32_quality", "rp_order_by_quality",
     "rp_gather_depths_dev_quality", "rp_gather_depths_dev_f32_quality", "rp_gather_depths_batch_dev_quality",
     "rp_gather_depths_batch_dev_f32_quality",
+    "rp_refine_pairs_host", "rp_refine_pairs_dev", "rp_refine_pairs_host_f32", "rp_refine_pairs_dev_f32",
 ]
 ORDER_SMEM_CAP = 12288   # RP_ORDER_SMEM_CAP: larger pairs are ordered in global scratch
 
@@ -116,6 +117,14 @@ def load():
     for name in ("rp_estimate_batch_dev_quality", "rp_estimate_batch_dev_f32_quality"):
         getattr(L, name).restype = C.c_int
         getattr(L, name).argtypes = est_q_args + [VP]
+    # rp_refine_pairs_*: the estimator's arguments up to opt, then init, subset, models, bstats, num_inliers, inliers
+    refine_args = est_args[:10] + [VP, VP, VP, VP, VP, VP]
+    for name in ("rp_refine_pairs_host", "rp_refine_pairs_host_f32"):
+        getattr(L, name).restype = C.c_int
+        getattr(L, name).argtypes = refine_args
+    for name in ("rp_refine_pairs_dev", "rp_refine_pairs_dev_f32"):
+        getattr(L, name).restype = C.c_int
+        getattr(L, name).argtypes = refine_args + [VP]
     L.rp_order_by_quality.restype = C.c_int
     L.rp_order_by_quality.argtypes = [VP, C.c_int64, VP, VP, VP]
     L.rp_sample_batch.restype = C.c_int
@@ -312,6 +321,61 @@ class Context:
         self._call(fn,
             self._h, int(variant), len(offsets) - 1, _ptr(offsets), *data,
             cams_ptr, C.byref(opt), models_ptr, stats_ptr, masks_ptr, stream or None)
+
+    # ---- refinement of caller-supplied models (rp_refine_pairs_*) --------------------------------
+    def refine_pairs_host(self, variant, offsets, x1, x2, d1, d2, cams, opt: Options, init, subset=None):
+        """The estimator's final refinement from `init` (MODEL_DTYPE [P]) on each pair's `subset` (uint8 [N], None: every
+        correspondence).  Returns (models, bstats, num_inliers int64 [P], inliers uint8 [N]) of the refined models."""
+        return self._refine_host(self._lib.rp_refine_pairs_host, _f64, variant, offsets, x1, x2, d1, d2, cams, opt, init,
+                                 subset)
+
+    def refine_pairs_host_f32(self, variant, offsets, x1, x2, d1, d2, cams, opt: Options, init, subset=None):
+        """`refine_pairs_host` for float32 points and depths (rp_refine_pairs_host_f32): half the upload, the same bytes
+        out as `refine_pairs_host` on the values converted to float64."""
+        return self._refine_host(self._lib.rp_refine_pairs_host_f32, _f32, variant, offsets, x1, x2, d1, d2, cams, opt,
+                                 init, subset)
+
+    def _refine_host(self, fn, conv, variant, offsets, x1, x2, d1, d2, cams, opt, init, subset):
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        n_pairs = len(offsets) - 1
+        x1, x2, d1, d2 = conv(x1), conv(x2), conv(d1), conv(d2)
+        ntot = int(offsets[-1]) if n_pairs >= 0 else 0
+        if x1.shape != (ntot, 2) or x2.shape != (ntot, 2) or d1.shape != (ntot,) or d2.shape != (ntot,):
+            raise ValueError("x1/x2 must be [N,2] and d1/d2 [N] with N = offsets[-1]")
+        init = np.ascontiguousarray(init, dtype=MODEL_DTYPE).reshape(-1)
+        if init.shape != (n_pairs,):
+            raise ValueError("init must hold one model per pair")
+        if subset is not None:
+            subset = np.ascontiguousarray(subset, dtype=np.uint8).reshape(-1)
+            if subset.shape != (ntot,):
+                raise ValueError("subset must be [N] with N = offsets[-1]")
+        cams = _f64(cams) if cams is not None else None
+        if cams is not None and cams.shape != (n_pairs, 8):
+            raise ValueError("cams must be [n_pairs, 8]")
+        models = np.zeros(n_pairs, dtype=MODEL_DTYPE)
+        bstats = np.zeros(n_pairs, dtype=BSTATS_DTYPE)
+        num_inliers = np.zeros(n_pairs, dtype=np.int64)
+        inliers = np.zeros(max(ntot, 1), dtype=np.uint8)
+        self._call(fn, self._h, int(variant), n_pairs, _ptr(offsets), _ptr(x1), _ptr(x2), _ptr(d1), _ptr(d2), _ptr(cams),
+                   C.byref(opt), _ptr(init), _ptr(subset), _ptr(models), _ptr(bstats), _ptr(num_inliers), _ptr(inliers))
+        return models, bstats, num_inliers, inliers[:ntot]
+
+    def refine_pairs_dev(self, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr, opt: Options, init_ptr,
+                         subset_ptr, models_ptr, bstats_ptr, num_inliers_ptr, inliers_ptr, stream=0):
+        """rp_refine_pairs_dev: raw device pointers (subset, bstats, num_inliers, inliers may be None); offsets is a host
+        int64 array."""
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        self._call(self._lib.rp_refine_pairs_dev, self._h, int(variant), len(offsets) - 1, _ptr(offsets), x1_ptr, x2_ptr,
+                   d1_ptr, d2_ptr, cams_ptr, C.byref(opt), init_ptr, subset_ptr or None, models_ptr, bstats_ptr or None,
+                   num_inliers_ptr or None, inliers_ptr or None, stream or None)
+
+    def refine_pairs_dev_f32(self, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr, opt: Options, init_ptr,
+                             subset_ptr, models_ptr, bstats_ptr, num_inliers_ptr, inliers_ptr, stream=0):
+        """`refine_pairs_dev` with x1, x2, d1, d2 pointing at float32 device arrays (rp_refine_pairs_dev_f32)."""
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        self._call(self._lib.rp_refine_pairs_dev_f32, self._h, int(variant), len(offsets) - 1, _ptr(offsets), x1_ptr,
+                   x2_ptr, d1_ptr, d2_ptr, cams_ptr, C.byref(opt), init_ptr, subset_ptr or None, models_ptr,
+                   bstats_ptr or None, num_inliers_ptr or None, inliers_ptr or None, stream or None)
 
     # ---- stage entry points -----------------------------------------------------------------
     def order(self, offsets, quality):

@@ -305,6 +305,131 @@ def estimate_monodepth_varying_focal_relative_pose_batch(points2D_1, points2D_2,
     return _focal_batch(nv.VARYING, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, bundle_opt, device, quality)
 
 
+# ---- refinement of caller-supplied models (rp_refine_pairs_host[_f32]) ----------------------------------------
+def _model_row(geometry, f1=1.0, f2=1.0):
+    """MonoDepthTwoViewGeometry (or a duck-typed one) -> one rp_model: q w-first as the pose stores it, t, scale, shifts,
+    and the two focal lengths (1 for the calibrated variants, which do not read them)."""
+    m = np.zeros((), dtype=nv.MODEL_DTYPE)
+    m["q"] = np.asarray(geometry.pose.q, dtype=np.float64)
+    m["t"] = np.asarray(geometry.pose.t, dtype=np.float64)
+    m["scale"], m["shift1"], m["shift2"] = geometry.scale, geometry.shift1, geometry.shift2
+    m["f1"], m["f2"] = f1, f2
+    return m
+
+
+def _pack_subsets(subsets, offsets):
+    """One boolean / 0-1 array per pair (None for a pair: every correspondence) -> packed uint8 [N]; ValueError on a
+    pair count or length that does not match the points."""
+    n = np.diff(offsets)
+    if len(subsets) != len(n):
+        raise ValueError(f"subsets needs one entry per pair ({len(n)}), got {len(subsets)}")
+    out = []
+    for i, (s, k) in enumerate(zip(subsets, n)):
+        s = np.ones(k, dtype=np.uint8) if s is None else (np.asarray(s).reshape(-1) != 0).astype(np.uint8)
+        if len(s) != k:
+            raise ValueError(f"subset of pair {i} has {len(s)} entries for {k} correspondences")
+        out.append(s)
+    return np.concatenate(out) if out else np.zeros(0, dtype=np.uint8)
+
+
+def _refine_host(variant, points2D_1, points2D_2, depth_1, depth_2, cams, init, ransac_opt, bundle_opt, subsets, device,
+                 focal_variant):
+    """Packed refinement of one model per pair: (models, bstats, num_inliers, inliers, offsets)."""
+    if not (len(points2D_1) == len(points2D_2) == len(depth_1) == len(depth_2) == len(init)):
+        raise ValueError("points, depths and initial models need one entry per pair")
+    offsets, x1, x2, d1, d2 = _pack_auto(points2D_1, points2D_2, depth_1, depth_2)
+    subset = _pack_subsets(subsets, offsets) if subsets is not None else None
+    opt = make_options(ransac_opt, bundle_opt, focal_variant=focal_variant)
+    if variant == nv.CALIB and opt.estimate_shift:
+        variant = nv.CALIB_SHIFT
+    ctx = context(device)
+    fn = ctx.refine_pairs_host_f32 if x1.dtype == np.float32 else ctx.refine_pairs_host
+    init = np.array(init, dtype=nv.MODEL_DTYPE).reshape(-1)
+    return fn(variant, offsets, x1, x2, d1, d2, cams, opt, init, subset) + (offsets,)
+
+
+def _refine_info(bstats_row, num_inliers, mask):
+    n = len(mask)
+    return {"iterations": int(bstats_row["iterations"]), "initial_cost": float(bstats_row["initial_cost"]),
+            "cost": float(bstats_row["cost"]), "lambda": float(bstats_row["lam"]),
+            "invalid_steps": int(bstats_row["invalid_steps"]), "step_norm": float(bstats_row["step_norm"]),
+            "grad_norm": float(bstats_row["grad_norm"]), "num_inliers": int(num_inliers),
+            "inlier_ratio": float(num_inliers) / n if n else 0.0, "inliers": [bool(b) for b in mask]}
+
+
+def refine_monodepth_relative_pose_batch(points2D_1, points2D_2, depth_1, depth_2, cameras1, cameras2,
+                                         initial_geometries, ransac_opt=None, bundle_opt=None, subsets=None, device=0):
+    """The estimator's final refinement (hybrid Sampson + reprojection cost, the bundle options' loss) from caller-supplied
+    start geometries, one per pair, instead of RANSAC's models: a tracker's previous poses, another method's poses, or an
+    estimate to re-refine with other bundle options.  `subsets` (optional): one boolean array per pair selecting the
+    correspondences the refinement uses (None, or a None entry: all of them); a pair with at most 3 selected
+    correspondences keeps its start geometry.  Thresholds and `monodepth_estimate_shift` come from `ransac_opt` as for
+    the estimator.  Returns a list of (MonoDepthTwoViewGeometry, info): info holds BundleStats (iterations, initial_cost,
+    cost, lambda, invalid_steps, step_norm, grad_norm) and num_inliers, inlier_ratio and inliers of the refined model."""
+    if not (len(cameras1) == len(cameras2) == len(points2D_1)):
+        raise ValueError("cameras1 / cameras2 need one camera per pair")
+    cams = np.array([Camera.from_any(a).fxfycxcy() + Camera.from_any(b).fxfycxcy()
+                     for a, b in zip(cameras1, cameras2)], dtype=np.float64).reshape(-1, 8)
+    init = [_model_row(g) for g in initial_geometries]
+    models, bstats, num_inl, inl, offsets = _refine_host(nv.CALIB, points2D_1, points2D_2, depth_1, depth_2, cams, init,
+                                                         ransac_opt, bundle_opt, subsets, device, False)
+    return [(_geometry(models[i]), _refine_info(bstats[i], num_inl[i], inl[offsets[i]:offsets[i + 1]]))
+            for i in range(len(models))]
+
+
+def _refine_focal_batch(variant, points2D_1, points2D_2, depth_1, depth_2, initial_image_pairs, ransac_opt, bundle_opt,
+                        subsets, device):
+    init = [_model_row(p.geometry, Camera.from_any(p.camera1).focal(), Camera.from_any(p.camera2).focal())
+            for p in initial_image_pairs]
+    models, bstats, num_inl, inl, offsets = _refine_host(variant, points2D_1, points2D_2, depth_1, depth_2, None, init,
+                                                         ransac_opt, bundle_opt, subsets, device, True)
+    out = []
+    for i, m in enumerate(models):
+        pair = MonoDepthImagePair(_geometry(m), Camera("SIMPLE_PINHOLE", [m["f1"], 0.0, 0.0]),
+                                  Camera("SIMPLE_PINHOLE", [m["f2"], 0.0, 0.0]))
+        out.append((pair, _refine_info(bstats[i], num_inl[i], inl[offsets[i]:offsets[i + 1]])))
+    return out
+
+
+def refine_monodepth_shared_focal_relative_pose_batch(points2D_1, points2D_2, depth_1, depth_2, initial_image_pairs,
+                                                      ransac_opt=None, bundle_opt=None, subsets=None, device=0):
+    """`refine_monodepth_relative_pose_batch` for the shared-focal estimator: principal-point-centred points, start
+    MonoDepthImagePairs (focal from camera.focal()); returns (MonoDepthImagePair, info) per pair."""
+    return _refine_focal_batch(nv.SHARED, points2D_1, points2D_2, depth_1, depth_2, initial_image_pairs, ransac_opt,
+                               bundle_opt, subsets, device)
+
+
+def refine_monodepth_varying_focal_relative_pose_batch(points2D_1, points2D_2, depth_1, depth_2, initial_image_pairs,
+                                                       ransac_opt=None, bundle_opt=None, subsets=None, device=0):
+    """`refine_monodepth_shared_focal_relative_pose_batch` for the varying-focal estimator."""
+    return _refine_focal_batch(nv.VARYING, points2D_1, points2D_2, depth_1, depth_2, initial_image_pairs, ransac_opt,
+                               bundle_opt, subsets, device)
+
+
+def refine_monodepth_relative_pose(points2D_1, points2D_2, depth_1, depth_2, camera1, camera2, initial_geometry,
+                                   ransac_opt={}, bundle_opt={}, subset=None):
+    """One pair of `refine_monodepth_relative_pose_batch`."""
+    return refine_monodepth_relative_pose_batch([points2D_1], [points2D_2], [depth_1], [depth_2], [camera1], [camera2],
+                                                [initial_geometry], ransac_opt, bundle_opt,
+                                                None if subset is None else [subset])[0]
+
+
+def refine_monodepth_shared_focal_relative_pose(points2D_1, points2D_2, depth_1, depth_2, initial_image_pair,
+                                                ransac_opt={}, bundle_opt={}, subset=None):
+    """One pair of `refine_monodepth_shared_focal_relative_pose_batch`."""
+    return refine_monodepth_shared_focal_relative_pose_batch([points2D_1], [points2D_2], [depth_1], [depth_2],
+                                                             [initial_image_pair], ransac_opt, bundle_opt,
+                                                             None if subset is None else [subset])[0]
+
+
+def refine_monodepth_varying_focal_relative_pose(points2D_1, points2D_2, depth_1, depth_2, initial_image_pair,
+                                                 ransac_opt={}, bundle_opt={}, subset=None):
+    """One pair of `refine_monodepth_varying_focal_relative_pose_batch`."""
+    return refine_monodepth_varying_focal_relative_pose_batch([points2D_1], [points2D_2], [depth_1], [depth_2],
+                                                              [initial_image_pair], ransac_opt, bundle_opt,
+                                                              None if subset is None else [subset])[0]
+
+
 # ---- the reference's single-pair surface ---------------------------------------------------------------
 def estimate_monodepth_relative_pose(points2D_1, points2D_2, depth_1, depth_2, camera1, camera2,
                                      ransac_opt={}, bundle_opt={}, initial_pose=None):

@@ -62,7 +62,9 @@ enum { B_OFFS, B_PAIRS, B_PTS64, B_PTS32, B_BEAR, B_SAMPLES, B_MODELS, B_HYPITER
        // (double-buffered on the host path), global sort scratch of pairs above RP_ORDER_SMEM_CAP
        B_QUAL, B_QUAL_B, B_ORDOFFS, B_ORDOFFS_B, B_PERM, B_PERM_B, B_KSORT, B_KSORT_B, B_ORDSCR,
        // rp_gather_depths_batch_dev*_quality: the compacted quality between the two passes (4 B per row)
-       B_GATHER_Q, B_NBUF };
+       B_GATHER_Q,
+       // rp_refine_pairs_*: start models, subset and inlier counts of a chunk (double-buffered on the host path)
+       B_RF_INIT, B_RF_INIT_B, B_RF_SUB, B_RF_SUB_B, B_RF_NINL, B_RF_NINL_B, B_NBUF };
 
 // device scalars living in B_SCALARS
 struct Scalars {
@@ -1134,6 +1136,254 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
     return RP_OK;
 }
 
+// ---- rp_refine_pairs_*: the estimator's final refinement on caller-supplied start models --------------------------
+struct RefineIO {
+    int n_pairs;
+    long long n_points;
+    const long long *h_offsets_rel;              // host, [n_pairs+1], relative to the chunk
+    const double *x1, *x2, *d1, *d2, *cams;      // device, chunk-local FP64
+    const Model *init;                           // device [n_pairs]
+    const unsigned char *subset;                 // device [n_points] or null (every correspondence)
+    Model *models_out;                           // device [n_pairs] (may alias init)
+    rp_bundle_stats *bstats_out;                 // device [n_pairs] or null
+    long long *num_inliers_out;                  // device [n_pairs] or null
+    unsigned char *inliers_out;                  // device [n_points]; null: no scoring (then num_inliers_out is null)
+};
+
+// One chunk, everything on `st`, no synchronisation: prepare_kernel as run_chunk runs it, refine_import_kernel,
+// the LM launch of run_chunk's step 8 on the work models, the masked score of run_chunk's get_inliers launch on the
+// refined work models, refine_export_kernel (last, because it also turns the score's counts into num_inliers).
+int refine_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const RefineIO &io, cudaStream_t st) {
+    const int P = io.n_pairs;
+    const long long N = io.n_points;
+    const bool pose = variant == RP_CALIB || variant == RP_CALIB_SHIFT;
+    DevBuf *B = ctx->buf;
+    CK(B[B_OFFS].reserve(sizeof(long long) * (P + 1)));
+    CK(B[B_PAIRS].reserve(sizeof(PairParams) * P));
+    CK(B[B_PTS64].reserve(sizeof(Pt64) * std::max<long long>(N, 1)));
+    CK(B[B_PTS32].reserve(sizeof(float4) * std::max<long long>(N, 1)));
+    CK(B[B_PTS32P].reserve(32 * (size_t)((N + P + 4) / 2 + 1)));
+    CK(B[B_BEAR].reserve(sizeof(Bear) * std::max<long long>(N, 1)));
+    CK(B[B_SCALARS].reserve(sizeof(Scalars)));
+    CK(B[B_BEST].reserve(sizeof(Model) * P));
+    CK(B[B_ENABLE].reserve(sizeof(int) * P));
+    CK(B[B_ONES].reserve(sizeof(int) * P));
+    CK(B[B_ONEPFX].reserve(sizeof(int) * (P + 1)));
+    CK(B[B_FINSCORE].reserve(sizeof(double) * P));
+    CK(B[B_FINCNT].reserve(sizeof(int) * P));
+    Scalars *sc = B[B_SCALARS].as<Scalars>();
+    PairParams *pairs = B[B_PAIRS].as<PairParams>();
+    Model *work = B[B_BEST].as<Model>();
+    int *enable = B[B_ENABLE].as<int>();
+    Scalars h_sc;
+    memset(&h_sc, 0, sizeof h_sc);
+    h_sc.n_pairs_scalar = P;
+    CK(cudaMemcpyAsync(sc, &h_sc, sizeof h_sc, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(B[B_OFFS].p, io.h_offsets_rel, sizeof(long long) * (P + 1), cudaMemcpyHostToDevice, st));
+    {
+        PrepareArgs a;
+        a.variant = variant; a.n_pairs = P; a.offsets = B[B_OFFS].as<long long>();
+        a.x1 = io.x1; a.x2 = io.x2; a.cams = io.cams;
+        a.max_epipolar_error = opt.max_epipolar_error; a.max_reproj_error = opt.max_reproj_error;
+        a.loss_scale = opt.loss_scale;
+        a.pts64 = B[B_PTS64].as<Pt64>(); a.pts32 = B[B_PTS32].as<float4>(); a.bear = B[B_BEAR].as<Bear>();
+        a.pairs = pairs; a.pts32p = B[B_PTS32P].as<float>();
+        prepare_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(a);
+        LAUNCHED();
+    }
+    refine_import_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(P, variant, pairs, io.subset, io.init, work, enable,
+                                                                      io.bstats_out);
+    LAUNCHED();
+    {
+        LMArgs la;
+        memset(&la, 0, sizeof la);
+        la.pairs = pairs; la.pts64 = B[B_PTS64].as<Pt64>(); la.d1 = io.d1; la.d2 = io.d2;
+        la.weight_sampson = opt.weight_sampson;
+        la.loss_scale_override = -1.0; la.scale_reproj_override = -1.0;
+        la.prob_list = nullptr; la.n_prob = &sc->n_pairs_scalar; la.prob_per_pair = 1;
+        la.models = work; la.use_final = 1; la.mask = io.subset; la.enable = enable; la.stats = io.bstats_out;
+        la.max_iterations = (int)opt.bundle_max_iterations; la.loss_type = opt.loss_type;
+        la.gradient_tol = opt.gradient_tol; la.step_tol = opt.step_tol; la.initial_lambda = opt.initial_lambda;
+        la.min_lambda = opt.min_lambda; la.max_lambda = opt.max_lambda;
+        int rc = launch_lm(ctx, variant, la, P, st);
+        if (rc) return rc;
+    }
+    if (io.inliers_out) {
+        valid_ones_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, pairs, B[B_ONES].as<int>());
+        LAUNCHED();
+        build_items_kernel<<<1, 1024, 0, st>>>(P, B[B_ONES].as<int>(), B[B_ONEPFX].as<int>(), &sc->n_one_items, nullptr);
+        LAUNCHED();
+        if (N > 0) CK(cudaMemsetAsync(io.inliers_out, 0, (size_t)N, st));
+        ScoreArgs s;
+        memset(&s, 0, sizeof s);
+        s.n_groups = P; s.grp_stride = 1; s.grp_per_pair = 1; s.grp_cnt = B[B_ONES].as<int>();
+        s.item_prefix = B[B_ONEPFX].as<int>(); s.n_items = &sc->n_one_items; s.pairs = pairs; s.models = work;
+        s.pts32 = B[B_PTS32].as<float4>(); s.pts64 = B[B_PTS64].as<Pt64>(); s.bear = B[B_BEAR].as<Bear>();
+        s.score = B[B_FINSCORE].as<double>(); s.count = B[B_FINCNT].as<int>(); s.mask = io.inliers_out;
+        int rc = launch_score(ctx, pose, true, s, st);
+        if (rc) return rc;
+    }
+    refine_export_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, variant, pairs, enable, io.init, work, B[B_FINCNT].as<int>(),
+                                                       io.models_out, io.num_inliers_out);
+    LAUNCHED();
+    return RP_OK;
+}
+
+// Device workspace of a refine chunk.  Per correspondence: pts64 (32 B), pts32 (16), the pair-interleaved FP32 copy
+// (16), bearings (48), and the chunk's I/O: FP64 inputs (48), subset (1), inlier mask (1); the host path double-buffers
+// the I/O and adds the float32 staging (24 B, double-buffered) for float32 inputs.  Per pair: PairParams, the work,
+// start and output models, bundle stats, cams, and a few counters.
+size_t refine_bytes_per_pair(long long avg_points, bool host_io, bool f32) {
+    const size_t io_pt = 48 + 1 + 1 + (host_io && f32 ? 24 : 0);
+    const size_t io_pair = 2 * sizeof(Model) + sizeof(rp_bundle_stats) + 64 + 8;
+    const size_t sets = host_io ? 2 : 1;
+    return (size_t)avg_points * (32 + 16 + 16 + 48 + sets * io_pt) + sizeof(PairParams) + sizeof(Model) + 32 +
+           sets * io_pair + 64;
+}
+
+// rp_refine_pairs_{host,dev}[_f32].  In = float: the float32 inputs are widened into the FP64 chunk arrays first
+// (widen_inputs_kernel without a permutation), so every kernel after that runs on the bytes the FP64 entry points see.
+// Host path: chunk c+1 is uploaded (and widened) on the copy stream into the other staging set while the compute stream
+// runs chunk c; the outputs of chunk c come back on the copy stream.  Neither rp_pair_status nor rp_last_timing changes.
+template <class In>
+int refine_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const In *x1, const In *x2,
+                const In *d1, const In *d2, const double *cams, const rp_options *opt_in, const rp_model *init,
+                const uint8_t *subset, rp_model *models, rp_bundle_stats *bstats, int64_t *num_inliers, uint8_t *inliers,
+                bool host_io, cudaStream_t st) {
+    constexpr bool f32 = std::is_same<In, float>::value;
+    if (!ctx) return RP_ERR_INVALID;
+    if (n_pairs > 0 && (!x1 || !x2 || !d1 || !d2)) return fail(ctx, RP_ERR_INVALID, "null data pointer");
+    if (n_pairs > 0 && (!init || !models)) return fail(ctx, RP_ERR_INVALID, "null init / models");
+    int rc = check_common(ctx, variant, n_pairs, offsets, opt_in);
+    if (rc) return rc;
+    CK(cudaSetDevice(ctx->device));
+    rp_options opt = *opt_in;
+    if (variant == RP_CALIB && opt.estimate_shift) variant = RP_CALIB_SHIFT;
+    const bool pose = variant == RP_CALIB || variant == RP_CALIB_SHIFT;
+    if (pose && !cams && n_pairs > 0) return fail(ctx, RP_ERR_INVALID, "calibrated variants need cams");
+    if (n_pairs == 0) return RP_OK;
+    const bool score = num_inliers || inliers;
+    const long long Ntot = offsets[n_pairs] - offsets[0];
+    int64_t chunk = (int64_t)std::max<size_t>(1, ctx->workspace_budget / refine_bytes_per_pair(Ntot / n_pairs + 1, host_io, f32));
+    chunk = std::min<int64_t>(chunk, 32768);
+    // host path: at least four chunks for batches of 1024 pairs or more, so that three uploads hide behind kernels
+    if (host_io && n_pairs >= 1024) chunk = std::min<int64_t>(chunk, (n_pairs + 3) / 4);
+    const int64_t n_chunks = (n_pairs + chunk - 1) / chunk;
+    std::vector<int64_t> bounds((size_t)n_chunks + 1);
+    for (int64_t i = 0; i <= n_chunks; ++i) bounds[(size_t)i] = (n_pairs * i) / n_chunks;
+    DevBuf *B = ctx->buf;
+    static const int IN_X1[2] = {B_IN_X1, B_IN_X1_B}, IN_X2[2] = {B_IN_X2, B_IN_X2_B}, IN_D1[2] = {B_IN_D1, B_IN_D1_B},
+                     IN_D2[2] = {B_IN_D2, B_IN_D2_B}, IN_CAMS[2] = {B_IN_CAMS, B_IN_CAMS_B}, STG_X1[2] = {B_STG_X1, B_STG_X1_B},
+                     STG_X2[2] = {B_STG_X2, B_STG_X2_B}, STG_D1[2] = {B_STG_D1, B_STG_D1_B}, STG_D2[2] = {B_STG_D2, B_STG_D2_B},
+                     INIT[2] = {B_RF_INIT, B_RF_INIT_B}, SUB[2] = {B_RF_SUB, B_RF_SUB_B}, OUT_M[2] = {B_TMP0, B_TMP0_B},
+                     OUT_S[2] = {B_TMP1, B_TMP1_B}, OUT_K[2] = {B_MASK, B_MASK_B}, OUT_N[2] = {B_RF_NINL, B_RF_NINL_B};
+    cudaStream_t cs = ctx->copy_stream;
+    cudaEvent_t *in_ready = &ctx->ev[12], *comp_done = &ctx->ev[16];
+    auto upload = [&](int64_t c) -> int {
+        const int64_t p0 = bounds[c], p1 = bounds[c + 1];
+        const int P = (int)(p1 - p0), par = (int)(c & 1);
+        const long long o0 = offsets[p0], N = offsets[p1] - o0;
+        const size_t nn = (size_t)std::max<long long>(N, 1);
+        CK(B[IN_X1[par]].reserve(16 * nn)); CK(B[IN_X2[par]].reserve(16 * nn));
+        CK(B[IN_D1[par]].reserve(8 * nn)); CK(B[IN_D2[par]].reserve(8 * nn));
+        CK(B[IN_CAMS[par]].reserve(64 * (size_t)P)); CK(B[INIT[par]].reserve(sizeof(Model) * P));
+        CK(B[OUT_M[par]].reserve(sizeof(Model) * P));
+        if (subset) CK(B[SUB[par]].reserve(nn));
+        if (bstats) CK(B[OUT_S[par]].reserve(sizeof(rp_bundle_stats) * P));
+        if (score) CK(B[OUT_K[par]].reserve(nn));
+        if (num_inliers) CK(B[OUT_N[par]].reserve(sizeof(long long) * P));
+        constexpr size_t E = sizeof(In);
+        void *dx1 = B[IN_X1[par]].p, *dx2 = B[IN_X2[par]].p, *dd1 = B[IN_D1[par]].p, *dd2 = B[IN_D2[par]].p;
+        if (f32) {
+            CK(B[STG_X1[par]].reserve(2 * E * nn)); CK(B[STG_X2[par]].reserve(2 * E * nn));
+            CK(B[STG_D1[par]].reserve(E * nn)); CK(B[STG_D2[par]].reserve(E * nn));
+            dx1 = B[STG_X1[par]].p; dx2 = B[STG_X2[par]].p; dd1 = B[STG_D1[par]].p; dd2 = B[STG_D2[par]].p;
+        }
+        CK(cudaMemcpyAsync(dx1, x1 + 2 * o0, 2 * E * (size_t)N, cudaMemcpyHostToDevice, cs));
+        CK(cudaMemcpyAsync(dx2, x2 + 2 * o0, 2 * E * (size_t)N, cudaMemcpyHostToDevice, cs));
+        CK(cudaMemcpyAsync(dd1, d1 + o0, E * (size_t)N, cudaMemcpyHostToDevice, cs));
+        CK(cudaMemcpyAsync(dd2, d2 + o0, E * (size_t)N, cudaMemcpyHostToDevice, cs));
+        if (pose) CK(cudaMemcpyAsync(B[IN_CAMS[par]].p, cams + 8 * p0, 64 * (size_t)P, cudaMemcpyHostToDevice, cs));
+        CK(cudaMemcpyAsync(B[INIT[par]].p, init + p0, sizeof(Model) * P, cudaMemcpyHostToDevice, cs));
+        if (subset) CK(cudaMemcpyAsync(B[SUB[par]].p, subset + o0, (size_t)N, cudaMemcpyHostToDevice, cs));
+        if (f32) {
+            int rc2 = launch_widen(ctx, N, (const In *)dx1, (const In *)dx2, (const In *)dd1, (const In *)dd2,
+                                   B[IN_X1[par]].as<double>(), B[IN_X2[par]].as<double>(), B[IN_D1[par]].as<double>(),
+                                   B[IN_D2[par]].as<double>(), cs);
+            if (rc2) return rc2;
+        }
+        CK(cudaEventRecord(in_ready[par], cs));
+        return RP_OK;
+    };
+    if (host_io) {
+        rc = upload(0);
+        if (rc) return rc;
+    }
+    std::vector<long long> rel;
+    for (int64_t c = 0; c < n_chunks; ++c) {
+        const int64_t p0 = bounds[c], p1 = bounds[c + 1];
+        const int P = (int)(p1 - p0), par = (int)(c & 1);
+        const long long o0 = offsets[p0], N = offsets[p1] - o0;
+        const size_t nn = (size_t)std::max<long long>(N, 1);
+        rel.resize(P + 1);
+        for (int i = 0; i <= P; ++i) rel[i] = offsets[p0 + i] - o0;
+        RefineIO io;
+        io.n_pairs = P; io.n_points = N; io.h_offsets_rel = rel.data();
+        if (host_io) {
+            CK(cudaStreamWaitEvent(st, in_ready[par], 0));
+            io.x1 = B[IN_X1[par]].as<double>(); io.x2 = B[IN_X2[par]].as<double>();
+            io.d1 = B[IN_D1[par]].as<double>(); io.d2 = B[IN_D2[par]].as<double>();
+            io.cams = pose ? B[IN_CAMS[par]].as<double>() : nullptr;
+            io.init = B[INIT[par]].as<Model>(); io.subset = subset ? B[SUB[par]].as<unsigned char>() : nullptr;
+            io.models_out = B[OUT_M[par]].as<Model>(); io.bstats_out = bstats ? B[OUT_S[par]].as<rp_bundle_stats>() : nullptr;
+            io.num_inliers_out = num_inliers ? B[OUT_N[par]].as<long long>() : nullptr;
+            io.inliers_out = score ? B[OUT_K[par]].as<unsigned char>() : nullptr;
+        } else {
+            if (f32) {
+                // B_IN_* are free: the previous chunk's kernels ran before on this stream
+                CK(B[B_IN_X1].reserve(16 * nn)); CK(B[B_IN_X2].reserve(16 * nn));
+                CK(B[B_IN_D1].reserve(8 * nn)); CK(B[B_IN_D2].reserve(8 * nn));
+                rc = launch_widen(ctx, N, x1 + 2 * o0, x2 + 2 * o0, d1 + o0, d2 + o0, B[B_IN_X1].as<double>(),
+                                  B[B_IN_X2].as<double>(), B[B_IN_D1].as<double>(), B[B_IN_D2].as<double>(), st);
+                if (rc) return rc;
+                io.x1 = B[B_IN_X1].as<double>(); io.x2 = B[B_IN_X2].as<double>();
+                io.d1 = B[B_IN_D1].as<double>(); io.d2 = B[B_IN_D2].as<double>();
+            } else {
+                io.x1 = (const double *)(x1 + 2 * o0); io.x2 = (const double *)(x2 + 2 * o0);
+                io.d1 = (const double *)(d1 + o0); io.d2 = (const double *)(d2 + o0);
+            }
+            io.cams = pose ? cams + 8 * p0 : nullptr;
+            io.init = (const Model *)init + p0; io.subset = subset ? subset + o0 : nullptr;
+            io.models_out = (Model *)models + p0; io.bstats_out = bstats ? bstats + p0 : nullptr;
+            io.num_inliers_out = num_inliers ? (long long *)num_inliers + p0 : nullptr;
+            io.inliers_out = inliers ? inliers + o0 : nullptr;
+            if (score && !inliers) {
+                // num_inliers alone: the mask goes to scratch
+                CK(B[B_MASK].reserve(nn));
+                io.inliers_out = B[B_MASK].as<unsigned char>();
+            }
+        }
+        rc = refine_chunk(ctx, variant, opt, io, st);
+        if (rc) return rc;
+        if (host_io) {
+            CK(cudaEventRecord(comp_done[par], st));
+            if (c + 1 < n_chunks) {
+                // staging set par^1 was last read by chunk c-1's kernels, whose downloads (ordered after them) precede
+                // this upload on the copy stream
+                rc = upload(c + 1);
+                if (rc) return rc;
+            }
+            CK(cudaStreamWaitEvent(cs, comp_done[par], 0));
+            CK(cudaMemcpyAsync(models + p0, io.models_out, sizeof(Model) * P, cudaMemcpyDeviceToHost, cs));
+            if (bstats) CK(cudaMemcpyAsync(bstats + p0, io.bstats_out, sizeof(rp_bundle_stats) * P, cudaMemcpyDeviceToHost, cs));
+            if (num_inliers) CK(cudaMemcpyAsync(num_inliers + p0, io.num_inliers_out, sizeof(long long) * P, cudaMemcpyDeviceToHost, cs));
+            if (inliers && N > 0) CK(cudaMemcpyAsync(inliers + o0, io.inliers_out, (size_t)N, cudaMemcpyDeviceToHost, cs));
+        }
+    }
+    CK(cudaStreamSynchronize(host_io ? cs : st));
+    return RP_OK;
+}
+
 }  // namespace
 
 // ================================================================================================
@@ -1318,6 +1568,38 @@ int rp_estimate_batch_dev_f32_quality(rp_ctx *ctx, int variant, int64_t n_pairs,
     RP_QUALITY_CHECKS();
     return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, models, stats, masks, false,
                          stream ? (cudaStream_t)stream : ctx->stream);
+}
+
+int rp_refine_pairs_host(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const double *x1,
+                         const double *x2, const double *d1, const double *d2, const double *cams, const rp_options *opt,
+                         const rp_model *init, const uint8_t *subset, rp_model *models, rp_bundle_stats *bstats,
+                         int64_t *num_inliers, uint8_t *inliers) {
+    return refine_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, cams, opt, init, subset, models, bstats, num_inliers,
+                       inliers, true, ctx ? ctx->stream : nullptr);
+}
+
+int rp_refine_pairs_dev(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const double *x1,
+                        const double *x2, const double *d1, const double *d2, const double *cams, const rp_options *opt,
+                        const rp_model *init, const uint8_t *subset, rp_model *models, rp_bundle_stats *bstats,
+                        int64_t *num_inliers, uint8_t *inliers, void *stream) {
+    return refine_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, cams, opt, init, subset, models, bstats, num_inliers,
+                       inliers, false, stream ? (cudaStream_t)stream : ctx ? ctx->stream : nullptr);
+}
+
+int rp_refine_pairs_host_f32(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const float *x1,
+                             const float *x2, const float *d1, const float *d2, const double *cams, const rp_options *opt,
+                             const rp_model *init, const uint8_t *subset, rp_model *models, rp_bundle_stats *bstats,
+                             int64_t *num_inliers, uint8_t *inliers) {
+    return refine_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, cams, opt, init, subset, models, bstats, num_inliers,
+                       inliers, true, ctx ? ctx->stream : nullptr);
+}
+
+int rp_refine_pairs_dev_f32(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const float *x1,
+                            const float *x2, const float *d1, const float *d2, const double *cams, const rp_options *opt,
+                            const rp_model *init, const uint8_t *subset, rp_model *models, rp_bundle_stats *bstats,
+                            int64_t *num_inliers, uint8_t *inliers, void *stream) {
+    return refine_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, cams, opt, init, subset, models, bstats, num_inliers,
+                       inliers, false, stream ? (cudaStream_t)stream : ctx ? ctx->stream : nullptr);
 }
 
 int rp_pair_status(const rp_ctx *ctx, int64_t n_pairs, int32_t *status) {

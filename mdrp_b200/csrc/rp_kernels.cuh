@@ -1562,6 +1562,58 @@ __global__ void finalize_kernel(int n_pairs, int variant, const PairParams *pair
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// rp_refine_pairs_*: the final refinement above on caller-supplied start models and subsets.
+// import: warp per pair.  |S_p| = subset bytes != 0 over the pair (all n without a subset), enable = |S_p| > 3 (the
+// estimator's num_inliers > 3); work = init with f1, f2 divided by nscale for the focal variants, for every pair and not
+// only the enabled ones, so that the inlier mask of a pair that is not refined is get_inliers of its start model in the
+// normalised frame, as the estimator's mask is; bundle stats zeroed (the LM skips the pairs it does not refine).
+__global__ void refine_import_kernel(int n_pairs, int variant, const PairParams *pairs, const unsigned char *subset,
+                                     const Model *init, Model *work, int *enable, rp_bundle_stats *bstats) {
+    const int pair = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (pair >= n_pairs) return;
+    const PairParams pp = pairs[pair];
+    int cnt = pp.n;
+    if (subset) {
+        cnt = 0;
+        const unsigned char *s = subset + pp.off;
+        for (int b0 = 0; b0 < pp.n; b0 += 32) cnt += __popc(__ballot_sync(0xffffffffu, b0 + lane < pp.n && s[b0 + lane]));
+    }
+    if (lane != 0) return;
+    Model m = init[pair];
+    if (variant == RP_SHARED || variant == RP_VARYING) {
+        m.f1 /= pp.nscale;
+        m.f2 /= pp.nscale;
+    }
+    work[pair] = m;
+    enable[pair] = cnt > 3;
+    if (bstats) bstats[pair] = rp_bundle_stats{};
+}
+
+// export: thread per pair.  A refined pair's model is the work model with f1, f2 multiplied by nscale (focal variants);
+// any other pair gets init's bytes (no nscale round trip).  With `count` (the masked score of the work models), the
+// pair's inlier count, 0 for pairs of fewer than 3 correspondences, which are not scored.  `out` may alias `init`.
+__global__ void refine_export_kernel(int n_pairs, int variant, const PairParams *pairs, const int *enable,
+                                     const Model *init, const Model *work, const int *count, Model *out,
+                                     long long *num_inliers) {
+    const int pair = blockIdx.x * blockDim.x + threadIdx.x;
+    if (pair >= n_pairs) return;
+    const PairParams pp = pairs[pair];
+    Model m;
+    if (enable[pair]) {
+        m = work[pair];
+        if (variant == RP_SHARED || variant == RP_VARYING) {
+            m.f1 *= pp.nscale;
+            m.f2 *= pp.nscale;
+        }
+    } else {
+        m = init[pair];
+    }
+    out[pair] = m;
+    if (num_inliers) num_inliers[pair] = pp.valid ? count[pair] : 0;
+}
+
 // Re-run sub-batches (estimate_impl): pairs that overflowed their event list or need more iterations are gathered
 // into a compact ragged batch, run again with larger limits, and their results scattered back.  Block per pair.
 struct SubBatchArgs {

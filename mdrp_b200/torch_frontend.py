@@ -143,6 +143,46 @@ def estimate_batch(variant, offsets, x1, x2, d1, d2, cams, opt: nv.Options, qual
     return models, stats, masks[:N]
 
 
+def refine_batch(variant, offsets, x1, x2, d1, d2, cams, init_models, opt: nv.Options, subset=None):
+    """The estimator's final refinement from caller-supplied start models (rp_refine_pairs_dev[_f32]) on CUDA tensors:
+    init_models [P,12] float64 (e.g. the `models` of a previous `estimate_batch` or `refine_batch`), `subset` (optional)
+    [N] CUDA tensor, nonzero = used by the refinement.  Inputs as in `estimate_batch` (float32 passes through, anything
+    else is converted to float64).  Returns (models [P,12] float64, bstats [P,7] (int64 view; columns 1-3, 5, 6 are
+    float64 bit patterns — use `bstats_to_numpy`), num_inliers [P] int64, inliers [N] uint8), all on the device."""
+    ctx = _ctx_for(x1)
+    dev = x1.device
+    offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+    P, N = len(offsets) - 1, int(offsets[-1])
+    f32 = all(t.dtype == torch.float32 for t in (x1, x2, d1, d2))
+    t64 = lambda t: t.contiguous().to(torch.float64)
+    tin = (lambda t: t.contiguous()) if f32 else t64
+    x1, x2, d1, d2 = tin(x1), tin(x2), tin(d1), tin(d2)
+    if x1.shape != (N, 2) or x2.shape != (N, 2) or d1.shape != (N,) or d2.shape != (N,):
+        raise ValueError("x1/x2 must be [N,2] and d1/d2 [N] with N = offsets[-1]")
+    init = t64(init_models)
+    if init.shape != (P, 12) or not init.is_cuda or init.device != dev:
+        raise ValueError("init_models must be a [P,12] CUDA tensor on the device of the points")
+    if subset is not None:
+        if not subset.is_cuda or subset.device != dev or subset.shape != (N,):
+            raise ValueError("subset must be a CUDA tensor [N] on the device of the points")
+        subset = (subset != 0).to(torch.uint8).contiguous()
+    cams_t = t64(cams) if cams is not None else None
+    models = torch.zeros(P, 12, dtype=torch.float64, device=dev)
+    bstats = torch.zeros(P, 7, dtype=torch.int64, device=dev)
+    num_inliers = torch.zeros(P, dtype=torch.int64, device=dev)
+    inliers = torch.zeros(max(N, 1), dtype=torch.uint8, device=dev)
+    fn = ctx.refine_pairs_dev_f32 if f32 else ctx.refine_pairs_dev
+    fn(variant, offsets, x1.data_ptr(), x2.data_ptr(), d1.data_ptr(), d2.data_ptr(),
+       cams_t.data_ptr() if cams_t is not None else None, opt, init.data_ptr(),
+       subset.data_ptr() if subset is not None else None, models.data_ptr(), bstats.data_ptr(), num_inliers.data_ptr(),
+       inliers.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+    return models, bstats, num_inliers, inliers[:N]
+
+
+def bstats_to_numpy(bstats: torch.Tensor) -> np.ndarray:
+    return bstats.cpu().numpy().view(nv.BSTATS_DTYPE).reshape(-1)
+
+
 def stats_to_numpy(stats: torch.Tensor) -> np.ndarray:
     return stats.cpu().numpy().view(nv.STATS_DTYPE).reshape(-1)
 
