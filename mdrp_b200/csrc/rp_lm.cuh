@@ -70,23 +70,39 @@ struct LMParams {
     int loss_type;
 };
 
-// Cost of the Cauchy losses, sum_k t^2 log1p(r_k^2 / t^2), accumulated as t^2 log(prod_k (1 + r_k^2 / t^2)): one FMA per
-// residual instead of a 45-instruction FP64 log1p (the final refinement evaluates three of them per correspondence per
-// pass).  Two running products (the Sampson terms carry weight_sampson), folded into `acc` every 512 factors
-// (TRUNCATED_CAUCHY: factors <= 2, so the product stays below 2^512) or when a product passes 1e150 (CAUCHY).
+// Cost of the Cauchy losses, sum_k t^2 log1p(r_k^2 / t^2), accumulated as t^2 log1p(q) with q = prod_k (1 + r_k^2 / t^2) - 1:
+// one FMA and one add per residual instead of a 45-instruction FP64 log1p (the final refinement evaluates three of them
+// per correspondence per pass).  Carrying q rather than the product itself keeps residuals far below an ulp of 1
+// (near-exact data, r^2 / t^2 down to 1e-20 and less) at full relative accuracy: q <- (1 + q)(1 + x) - 1 = fma(q, x, q + x).
+// Two running values (the Sampson terms carry weight_sampson), folded into `acc` every 512 factors (TRUNCATED_CAUCHY:
+// factors <= 2, so the product stays below 2^512) or when q passes 1e150 (CAUCHY).
+// log1p(q), q >= 0, from log: log(u) with u = 1 + q, plus the first-order correction (q - (u - 1)) / u for the rounding
+// of u (the numerator is exact and at most half an ulp of u, so a rough reciprocal suffices), within a few ulps.  The
+// library log1p, inlined at every fold, would add ~1 800 instructions to each Cauchy kernel, and the final-refinement
+// launch is sensitive to instruction fetch.
+RP_HD double log1p_q(double q) {
+    const double u = 1.0 + q;
+#ifdef __CUDA_ARCH__
+    double r;
+    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(u));
+#else
+    const double r = 1.0 / u;
+#endif
+    return log(u) + (q - (u - 1.0)) * r;
+}
 struct LogProd {
-    double ps, pr, acc;
+    double qs, qr, acc;
     int cnt;
-    RP_HD void init() { ps = 1.0; pr = 1.0; acc = 0.0; cnt = 0; }
-    RP_HD void fold(double ws) { acc += ws * log(ps) + log(pr); ps = 1.0; pr = 1.0; cnt = 0; }
+    RP_HD void init() { qs = 0.0; qr = 0.0; acc = 0.0; cnt = 0; }
+    RP_HD void fold(double ws) { acc += ws * log1p_q(qs) + log1p_q(qr); qs = 0.0; qr = 0.0; cnt = 0; }
     // the accumulated cost, in units of t^2
-    RP_HD double total(double ws) const { return acc + ws * log(ps) + log(pr); }
+    RP_HD double total(double ws) const { return acc + ws * log1p_q(qs) + log1p_q(qr); }
     template <bool SAMPSON>
     RP_HD void add(int type, double x, double ws) {
         if (type == RP_LOSS_TRUNCATED_CAUCHY) x = x > 1.0 ? 1.0 : x;   // (a NaN residual stays NaN, as in loss_eval)
         else if (!(x < 1e100)) { acc += (SAMPSON ? ws : 1.0) * log1p(x); return; }
-        if (SAMPSON) ps = fma_(ps, x, ps); else pr = fma_(pr, x, pr);
-        if (++cnt >= 512 || (type == RP_LOSS_CAUCHY && (ps > 1e150 || pr > 1e150))) fold(ws);
+        if (SAMPSON) qs = fma_(qs, x, qs + x); else qr = fma_(qr, x, qr + x);
+        if (++cnt >= 512 || (type == RP_LOSS_CAUCHY && (qs > 1e150 || qr > 1e150))) fold(ws);
     }
 };
 
