@@ -47,24 +47,39 @@ enum { B_OFFS, B_PAIRS, B_PTS64, B_PTS32, B_BEAR, B_SAMPLES, B_MODELS, B_HYPITER
        B_ITEMPFX, B_SCALARS, B_EVENTS, B_NEVENTS, B_LOMODELS, B_LOOFEV, B_LOCOUNT, B_PROBLIST, B_LOSCORE,
        B_LOCNT, B_LOITEMPFX, B_BEST, B_FINSTART, B_FINSCORE, B_FINCNT, B_ONES, B_ONEPFX, B_ENABLE, B_STATS,
        B_PTS32P, B_UB, B_LB, B_FIRSTCNT, B_FIRSTPFX, B_B0, B_S0, B_SURVLIST, B_SURVCNT, B_SURVPFX, B_WAVECUR, B_WAVECNT,
-       B_MASK, B_IN_X1, B_IN_X2, B_IN_D1, B_IN_D2, B_IN_CAMS, B_TMP0, B_TMP1, B_TMP2,
-       // second staging set (double buffering of the host path)
-       B_MASK_B, B_IN_X1_B, B_IN_X2_B, B_IN_D1_B, B_IN_D2_B, B_IN_CAMS_B, B_TMP0_B, B_TMP1_B,
+       B_TMP2,
        // tensor-core tier: per-point feature rows, per-model outlier counts, survivor lists
        B_FEAT, B_TCOUT, B_TCLIST, B_TCLISTCNT, B_TCLISTPFX, B_PAIRCNT, B_TCPFX, B_TCSPLIT,
        // per-pair flags; re-run sub-batches (event-list overflow, early termination that needs more iterations)
        B_PAIRFLAGS, B_SUB_IDX, B_SUB_SRC, B_SUB_DST, B_SUB_X1, B_SUB_X2, B_SUB_D1, B_SUB_D2, B_SUB_CAMS, B_SUB_MODELS,
        B_SUB_STATS, B_SUB_MASK,
-       // host path of float32 inputs or quality calls: the chunk as uploaded (input type, double-buffered), before it
-       // is widened / gathered into B_IN_*
-       B_STG_X1, B_STG_X2, B_STG_D1, B_STG_D2, B_STG_X1_B, B_STG_X2_B, B_STG_D1_B, B_STG_D2_B,
-       // quality calls (rp_order.cuh): uploaded quality, the chunk's offsets and order, masks in the ordered layout
-       // (double-buffered on the host path), global sort scratch of pairs above RP_ORDER_SMEM_CAP
-       B_QUAL, B_QUAL_B, B_ORDOFFS, B_ORDOFFS_B, B_PERM, B_PERM_B, B_KSORT, B_KSORT_B, B_ORDSCR,
+       // quality calls: global sort scratch of pairs above RP_ORDER_SMEM_CAP
+       B_ORDSCR,
        // rp_gather_depths_batch_dev*_quality: the compacted quality between the two passes (4 B per row)
-       B_GATHER_Q,
-       // rp_refine_pairs_*: start models, subset and inlier counts of a chunk (double-buffered on the host path)
-       B_RF_INIT, B_RF_INIT_B, B_RF_SUB, B_RF_SUB_B, B_RF_NINL, B_RF_NINL_B, B_NBUF };
+       B_GATHER_Q, B_NBUF };
+
+// One double-buffer set of the chunk pipeline (stage_inputs / run_chunks): a chunk's inputs on their way in and its
+// outputs on their way out.  rp_ctx keeps two; on the host path chunk c uses set c & 1, the device path uses set 0 for
+// what it widens or orders, and the stage entry points borrow set 0's buffers as scratch.
+struct StageSet {
+    DevBuf x1, x2, d1, d2, cams;          // the chunk's FP64 inputs
+    DevBuf sx1, sx2, sd1, sd2;            // host path: the chunk as uploaded (input type) when it is widened or ordered
+    DevBuf qual, offs, perm, ksort;       // quality calls: quality, the chunk's offsets and order, masks in the ordered layout
+    DevBuf init, subset;                  // refinement: start models, subset
+    DevBuf models, stats, mask, ninl;     // output staging: models, stats or bundle stats, mask, num_inliers
+    // upload [h2d_begin, h2d_end), widening / ordering [h2d_end, in_ready), kernels done, read-back [d2h_begin, d2h_end)
+    cudaEvent_t h2d_begin = nullptr, h2d_end = nullptr, in_ready = nullptr, done = nullptr, d2h_begin = nullptr,
+                d2h_end = nullptr;
+    void create_events() {
+        for (cudaEvent_t *e : {&h2d_begin, &h2d_end, &in_ready, &done, &d2h_begin, &d2h_end}) cudaEventCreate(e);
+    }
+    void release() {
+        for (DevBuf *b : {&x1, &x2, &d1, &d2, &cams, &sx1, &sx2, &sd1, &sd2, &qual, &offs, &perm, &ksort, &init, &subset,
+                          &models, &stats, &mask, &ninl})
+            b->release();
+        for (cudaEvent_t e : {h2d_begin, h2d_end, in_ready, done, d2h_begin, d2h_end}) cudaEventDestroy(e);
+    }
+};
 
 // device scalars living in B_SCALARS
 struct Scalars {
@@ -76,7 +91,9 @@ struct Scalars {
     unsigned long long tc_evaluated, tc_selected, lm_flops;
 };
 
-constexpr int N_EVENTS = 29;
+// run_chunk: [0..8] stage boundaries, [9] start of the bulk cascade, [10] bound kernel done, [11] tensor-core tier done;
+// [12], [13]: an interval of their own (the mask scatter of quality calls, rp_measure_pipes)
+constexpr int N_EVENTS = 14;
 
 }  // namespace
 
@@ -88,6 +105,7 @@ struct rp_ctx {
     cudaStream_t stream = nullptr;
     cudaStream_t copy_stream = nullptr;  // H2D of chunk c+1 / D2H of chunk c-1 overlap the kernels of chunk c
     DevBuf buf[B_NBUF];
+    StageSet set[2];
     cudaEvent_t ev[N_EVENTS];
     double last_ms[16] = {0};
     double prev_h2d_ms = 0.0, prev_dev_ms = 0.0;  // upload / kernel time of the previous host-path call (lead-chunk sizing)
@@ -268,15 +286,104 @@ __global__ void stage_points_kernel(int n, const double *x1, const double *x2, d
 }
 
 // ---- one chunk of pairs, everything on device ----------------------------------------------------
+// The chunk's FP64 inputs on the device (stage_inputs) and where run_chunk / refine_chunk write its results
 struct ChunkIO {
-    int n_pairs;
-    long long n_points;
-    const long long *h_offsets_rel;  // host, [n_pairs+1], relative to the chunk
-    const double *x1, *x2, *d1, *d2, *cams;  // device, chunk-local
-    Model *models_out;               // device [n_pairs]
-    rp_stats *stats_out;             // device [n_pairs]
-    unsigned char *masks_out;        // device [n_points]
+    int n_pairs = 0;
+    long long n_points = 0;
+    const long long *h_offsets_rel = nullptr;  // host, [n_pairs+1], relative to the chunk
+    const double *x1 = nullptr, *x2 = nullptr, *d1 = nullptr, *d2 = nullptr, *cams = nullptr;  // device, chunk-local
+    const Model *init = nullptr;               // refinement: start models [n_pairs]
+    const unsigned char *subset = nullptr;     // refinement: [n_points] or null (every correspondence)
+    Model *models_out = nullptr;               // [n_pairs] (refinement: may alias init)
+    rp_stats *stats_out = nullptr;             // estimator: [n_pairs]
+    rp_bundle_stats *bstats_out = nullptr;     // refinement: [n_pairs] or null
+    long long *num_inliers_out = nullptr;      // refinement: [n_pairs] or null
+    unsigned char *masks_out = nullptr;        // [n_points]; refinement: null = no scoring (then num_inliers_out is null)
 };
+
+// First step of run_chunk and refine_chunk: the workspace both need, the Scalars (n_pairs_scalar = P) and the chunk's
+// offsets, then prepare_kernel (PairParams, pts64 / pts32 / pts32p / bearings).  `ev_uploaded`, if given, is recorded
+// between the uploads and the launch (run_chunk's slot [0] starts there).
+int prepare_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io, cudaEvent_t ev_uploaded,
+                  cudaStream_t st) {
+    const int P = io.n_pairs;
+    const long long N = io.n_points;
+    DevBuf *B = ctx->buf;
+    CK(B[B_OFFS].reserve(sizeof(long long) * (P + 1)));
+    CK(B[B_PAIRS].reserve(sizeof(PairParams) * P));
+    CK(B[B_PTS64].reserve(sizeof(Pt64) * std::max<long long>(N, 1)));
+    CK(B[B_PTS32].reserve(sizeof(float4) * std::max<long long>(N, 1)));
+    CK(B[B_PTS32P].reserve(32 * (size_t)((N + P + 4) / 2 + 1)));
+    CK(B[B_BEAR].reserve(sizeof(Bear) * std::max<long long>(N, 1)));
+    CK(B[B_SCALARS].reserve(sizeof(Scalars)));
+    Scalars h_sc;
+    memset(&h_sc, 0, sizeof h_sc);
+    h_sc.n_pairs_scalar = P;
+    CK(cudaMemcpyAsync(B[B_SCALARS].p, &h_sc, sizeof h_sc, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(B[B_OFFS].p, io.h_offsets_rel, sizeof(long long) * (P + 1), cudaMemcpyHostToDevice, st));
+    if (ev_uploaded) CK(cudaEventRecord(ev_uploaded, st));
+    PrepareArgs a;
+    a.variant = variant; a.n_pairs = P; a.offsets = B[B_OFFS].as<long long>();
+    a.x1 = io.x1; a.x2 = io.x2; a.cams = io.cams;
+    a.max_epipolar_error = opt.max_epipolar_error; a.max_reproj_error = opt.max_reproj_error;
+    a.loss_scale = opt.loss_scale;
+    a.pts64 = B[B_PTS64].as<Pt64>(); a.pts32 = B[B_PTS32].as<float4>(); a.bear = B[B_BEAR].as<Bear>();
+    a.pairs = B[B_PAIRS].as<PairParams>(); a.pts32p = B[B_PTS32P].as<float>();
+    prepare_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(a);
+    LAUNCHED();
+    return RP_OK;
+}
+
+// The final refinement (run_chunk's step 8, refine_chunk): the caller's bundle options on one model per pair, on the
+// correspondences of `mask` (null: all of them), for the pairs `enable` marks
+LMArgs final_lm_args(rp_ctx *ctx, const rp_options &opt, const ChunkIO &io, Model *models, const unsigned char *mask,
+                     const int *enable) {
+    DevBuf *B = ctx->buf;
+    LMArgs la;
+    memset(&la, 0, sizeof la);
+    la.pairs = B[B_PAIRS].as<PairParams>(); la.pts64 = B[B_PTS64].as<Pt64>(); la.d1 = io.d1; la.d2 = io.d2;
+    la.weight_sampson = opt.weight_sampson;
+    la.loss_scale_override = -1.0; la.scale_reproj_override = -1.0;
+    la.prob_list = nullptr; la.n_prob = &B[B_SCALARS].as<Scalars>()->n_pairs_scalar; la.prob_per_pair = 1;
+    la.models = models; la.use_final = 1; la.mask = mask; la.enable = enable;
+    la.max_iterations = (int)opt.bundle_max_iterations; la.loss_type = opt.loss_type;
+    la.gradient_tol = opt.gradient_tol; la.step_tol = opt.step_tol; la.initial_lambda = opt.initial_lambda;
+    la.min_lambda = opt.min_lambda; la.max_lambda = opt.max_lambda;
+    return la;
+}
+
+// One work item per valid pair (B_ONES, B_ONEPFX, n_one_items): the list pair_score_args scores over.  run_chunk builds
+// it once for the final LO's rescore and its get_inliers.
+int launch_pair_items(rp_ctx *ctx, int P, cudaStream_t st) {
+    DevBuf *B = ctx->buf;
+    valid_ones_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, B[B_PAIRS].as<PairParams>(), B[B_ONES].as<int>());
+    LAUNCHED();
+    build_items_kernel<<<1, 1024, 0, st>>>(P, B[B_ONES].as<int>(), B[B_ONEPFX].as<int>(),
+                                           &B[B_SCALARS].as<Scalars>()->n_one_items, nullptr);
+    LAUNCHED();
+    return RP_OK;
+}
+
+// score_kernel over one model per pair on the launch_pair_items list; score and count per pair go to B_FINSCORE /
+// B_FINCNT, the mask (with the mask variant) to `mask`
+ScoreArgs pair_score_args(rp_ctx *ctx, int P, const Model *models, unsigned char *mask) {
+    DevBuf *B = ctx->buf;
+    ScoreArgs s;
+    memset(&s, 0, sizeof s);
+    s.n_groups = P; s.grp_stride = 1; s.grp_per_pair = 1; s.grp_cnt = B[B_ONES].as<int>();
+    s.item_prefix = B[B_ONEPFX].as<int>(); s.n_items = &B[B_SCALARS].as<Scalars>()->n_one_items;
+    s.pairs = B[B_PAIRS].as<PairParams>(); s.models = models;
+    s.pts32 = B[B_PTS32].as<float4>(); s.pts64 = B[B_PTS64].as<Pt64>(); s.bear = B[B_BEAR].as<Bear>();
+    s.score = B[B_FINSCORE].as<double>(); s.count = B[B_FINCNT].as<int>(); s.mask = mask;
+    return s;
+}
+
+// get_inliers: the inlier mask of `models` (one per pair) over the chunk's correspondences
+int launch_get_inliers(rp_ctx *ctx, bool pose, const ChunkIO &io, const Model *models, unsigned char *mask,
+                       cudaStream_t st) {
+    if (io.n_points > 0) CK(cudaMemsetAsync(mask, 0, (size_t)io.n_points, st));
+    return launch_score(ctx, pose, true, pair_score_args(ctx, io.n_pairs, models, mask), st);
+}
 
 // One pass over a chunk.  `flags` (host, [n_pairs]) receives PAIR_FLAG_* per pair: a flagged pair's outputs are void and
 // the caller runs it again with a larger `ev_cap` / more iterations (estimate_impl).
@@ -290,12 +397,6 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
     const size_t slots = slots_pp * (size_t)P;
 
     DevBuf *B = ctx->buf;
-    CK(B[B_OFFS].reserve(sizeof(long long) * (P + 1)));
-    CK(B[B_PAIRS].reserve(sizeof(PairParams) * P));
-    CK(B[B_PTS64].reserve(sizeof(Pt64) * std::max<long long>(N, 1)));
-    CK(B[B_PTS32].reserve(sizeof(float4) * std::max<long long>(N, 1)));
-    CK(B[B_PTS32P].reserve(32 * (size_t)((N + P + 4) / 2 + 1)));
-    CK(B[B_BEAR].reserve(sizeof(Bear) * std::max<long long>(N, 1)));
     CK(B[B_SAMPLES].reserve(sizeof(int) * 3 * (size_t)P * std::max(iters, 1)));
     CK(B[B_MODELS].reserve(sizeof(Model) * slots));
     CK(B[B_HYPITER].reserve(sizeof(int) * slots));
@@ -303,7 +404,6 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
     CK(B[B_COUNT].reserve(sizeof(int) * slots));
     CK(B[B_SEGCNT].reserve(sizeof(int) * (size_t)P * nseg));
     CK(B[B_ITEMPFX].reserve(sizeof(int) * ((size_t)P * nseg + 1)));
-    CK(B[B_SCALARS].reserve(sizeof(Scalars)));
     CK(B[B_EVENTS].reserve(sizeof(int) * (size_t)P * ev_cap));
     CK(B[B_NEVENTS].reserve(sizeof(int) * P));
     CK(B[B_LOMODELS].reserve(sizeof(Model) * (size_t)P * ev_cap));
@@ -346,6 +446,10 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
         CK(B[B_TCPFX].reserve(sizeof(int) * (P + 1)));
     }
 
+    cudaEvent_t *ev = ctx->ev;
+    // 1. prepare, and the tensor-core tier's feature rows
+    int rc = prepare_chunk(ctx, variant, opt, io, ev[0], st);
+    if (rc) return rc;
     Scalars *sc = B[B_SCALARS].as<Scalars>();
     PairParams *pairs = B[B_PAIRS].as<PairParams>();
     Pt64 *pts64 = B[B_PTS64].as<Pt64>();
@@ -358,29 +462,9 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
     int *count = B[B_COUNT].as<int>();
     int *seg_count = B[B_SEGCNT].as<int>();
     int *item_prefix = B[B_ITEMPFX].as<int>();
-
-    Scalars h_sc;
-    memset(&h_sc, 0, sizeof h_sc);
-    h_sc.n_pairs_scalar = P;
-    CK(cudaMemcpyAsync(sc, &h_sc, sizeof h_sc, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(B[B_OFFS].p, io.h_offsets_rel, sizeof(long long) * (P + 1), cudaMemcpyHostToDevice, st));
-
-    cudaEvent_t *ev = ctx->ev;
-    CK(cudaEventRecord(ev[0], st));
-    // 1. prepare
-    {
-        PrepareArgs a;
-        a.variant = variant; a.n_pairs = P; a.offsets = B[B_OFFS].as<long long>();
-        a.x1 = io.x1; a.x2 = io.x2; a.cams = io.cams;
-        a.max_epipolar_error = opt.max_epipolar_error; a.max_reproj_error = opt.max_reproj_error;
-        a.loss_scale = opt.loss_scale;
-        a.pts64 = pts64; a.pts32 = pts32; a.bear = bear; a.pairs = pairs; a.pts32p = B[B_PTS32P].as<float>();
-        prepare_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(a);
+    if (use_tc && N > 0) {
+        tc::tc_features_kernel<<<cdiv(N, 256), 256, 0, st>>>(N, pts32, B[B_FEAT].as<float4>());
         LAUNCHED();
-        if (use_tc && N > 0) {
-            tc::tc_features_kernel<<<cdiv(N, 256), 256, 0, st>>>(N, pts32, B[B_FEAT].as<float4>());
-            LAUNCHED();
-        }
     }
     CK(cudaEventRecord(ev[1], st));
     // 2. sample
@@ -398,7 +482,7 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
         SolveArgs a;
         a.variant = variant; a.iters = iters; a.nseg = nseg; a.pairs = pairs; a.samples = samples;
         a.pts64 = pts64; a.d1 = io.d1; a.d2 = io.d2; a.models = models; a.hyp_iter = hyp_iter; a.seg_count = seg_count;
-        int rc = launch_solve(ctx, variant, a, P, st);
+        rc = launch_solve(ctx, variant, a, P, st);
         if (rc) return rc;
     }
     CK(cudaEventRecord(ev[3], st));
@@ -412,7 +496,7 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
         sa.n_groups = P * nseg; sa.grp_stride = 4 * SEG; sa.grp_per_pair = nseg; sa.grp_cnt = seg_count;
         sa.item_prefix = item_prefix; sa.n_items = &sc->n_items; sa.models = models; sa.score = score; sa.count = count;
         sa.point_scores = &sc->point_scores;
-        int rc = launch_score(ctx, pose, false, sa, st);
+        rc = launch_score(ctx, pose, false, sa, st);
         if (rc) return rc;
     } else {
         // 4a. the first `head` models of every pair, exactly -> (B0, S0)
@@ -430,7 +514,7 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
         sa.n_groups = P; sa.grp_stride = (int)slots_pp; sa.grp_per_pair = 1; sa.grp_cnt = first_cnt;
         sa.item_prefix = B[B_FIRSTPFX].as<int>(); sa.n_items = &sc->n_first_items; sa.models = models;
         sa.score = score; sa.count = count; sa.point_scores = &sc->point_scores;
-        int rc = launch_score(ctx, pose, false, sa, st);
+        rc = launch_score(ctx, pose, false, sa, st);
         if (rc) return rc;
         pair_bounds_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(P, nseg, first_cnt, score, count,
                                                                        B[B_B0].as<int>(), B[B_S0].as<double>());
@@ -557,8 +641,8 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
                 from = ctx->mid_ends[k];
             }
         }
-        CK(cudaEventRecord(ev[20], st));
-        rc = cascade(from, 0, ctx->tc_two_pass, use_tc ? ev[22] : nullptr, ev[21]);
+        CK(cudaEventRecord(ev[9], st));
+        rc = cascade(from, 0, ctx->tc_two_pass, use_tc ? ev[11] : nullptr, ev[10]);
         if (rc) return rc;
     }
     CK(cudaEventRecord(ev[4], st));
@@ -590,7 +674,7 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
     {
         la.prob_list = B[B_PROBLIST].as<int>(); la.n_prob = &sc->n_prob; la.prob_per_pair = ev_cap;
         la.models = B[B_LOMODELS].as<Model>(); la.use_final = 0;
-        int rc = launch_lm(ctx, variant, la, (long long)P * 8, st);
+        rc = launch_lm(ctx, variant, la, (long long)P * 8, st);
         if (rc) return rc;
     }
     CK(cudaEventRecord(ev[6], st));
@@ -603,7 +687,7 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
         s2.n_groups = P; s2.grp_stride = ev_cap; s2.grp_per_pair = 1; s2.grp_cnt = B[B_LOCOUNT].as<int>();
         s2.item_prefix = B[B_LOITEMPFX].as<int>(); s2.n_items = &sc->n_lo_items; s2.models = B[B_LOMODELS].as<Model>();
         s2.score = B[B_LOSCORE].as<double>(); s2.count = B[B_LOCNT].as<int>(); s2.point_scores = nullptr;
-        int rc = launch_score(ctx, pose, false, s2, st);
+        rc = launch_score(ctx, pose, false, s2, st);
         if (rc) return rc;
         MergeArgs m;
         m.n_pairs = P; m.nseg = nseg; m.iters = iters; m.pairs = pairs; m.events = B[B_EVENTS].as<int>();
@@ -621,15 +705,9 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
         la.models = B[B_FINSTART].as<Model>(); la.use_final = 0;
         rc = launch_lm(ctx, variant, la, P, st);
         if (rc) return rc;
-        valid_ones_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, pairs, B[B_ONES].as<int>());
-        LAUNCHED();
-        build_items_kernel<<<1, 1024, 0, st>>>(P, B[B_ONES].as<int>(), B[B_ONEPFX].as<int>(), &sc->n_one_items, nullptr);
-        LAUNCHED();
-        ScoreArgs s3 = s2;
-        s3.grp_stride = 1; s3.grp_cnt = B[B_ONES].as<int>(); s3.item_prefix = B[B_ONEPFX].as<int>();
-        s3.n_items = &sc->n_one_items; s3.models = B[B_FINSTART].as<Model>();
-        s3.score = B[B_FINSCORE].as<double>(); s3.count = B[B_FINCNT].as<int>();
-        rc = launch_score(ctx, pose, false, s3, st);
+        rc = launch_pair_items(ctx, P, st);
+        if (rc) return rc;
+        rc = launch_score(ctx, pose, false, pair_score_args(ctx, P, B[B_FINSTART].as<Model>(), nullptr), st);
         if (rc) return rc;
         Merge2Args m2;
         m2.n_pairs = P; m2.pairs = pairs; m2.refined = B[B_FINSTART].as<Model>(); m2.ref_score = B[B_FINSCORE].as<double>();
@@ -637,10 +715,7 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
         merge2_kernel<<<cdiv(P, 128), 128, 0, st>>>(m2);
         LAUNCHED();
         // get_inliers of the RANSAC model (this is the mask the reference returns in `info`)
-        CK(cudaMemsetAsync(io.masks_out, 0, (size_t)std::max<long long>(N, 1), st));
-        ScoreArgs s4 = s3;
-        s4.models = B[B_BEST].as<Model>(); s4.mask = io.masks_out;
-        rc = launch_score(ctx, pose, true, s4, st);
+        rc = launch_get_inliers(ctx, pose, io, B[B_BEST].as<Model>(), io.masks_out, st);
         if (rc) return rc;
     }
     CK(cudaEventRecord(ev[7], st));
@@ -648,12 +723,10 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
     {
         enable_final_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, B[B_STATS].as<rp_stats>(), B[B_ENABLE].as<int>());
         LAUNCHED();
-        la.prob_list = nullptr; la.n_prob = &sc->n_pairs_scalar; la.prob_per_pair = 1;
-        la.models = B[B_BEST].as<Model>(); la.use_final = 1; la.mask = io.masks_out; la.enable = B[B_ENABLE].as<int>();
-        la.max_iterations = (int)opt.bundle_max_iterations; la.loss_type = opt.loss_type;
-        la.gradient_tol = opt.gradient_tol; la.step_tol = opt.step_tol; la.initial_lambda = opt.initial_lambda;
-        la.min_lambda = opt.min_lambda; la.max_lambda = opt.max_lambda;
-        int rc = launch_lm(ctx, variant, la, P, st);
+        LMArgs lf = final_lm_args(ctx, opt, io, B[B_BEST].as<Model>(), io.masks_out, B[B_ENABLE].as<int>());
+        lf.lm_iters = &sc->lm_iters;
+        lf.lm_flops = &sc->lm_flops;
+        rc = launch_lm(ctx, variant, lf, P, st);
         if (rc) return rc;
         finalize_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, variant, pairs, B[B_BEST].as<Model>());
         LAUNCHED();
@@ -661,6 +734,7 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
         CK(cudaMemcpyAsync(io.stats_out, B[B_STATS].p, sizeof(rp_stats) * P, cudaMemcpyDeviceToDevice, st));
     }
     CK(cudaEventRecord(ev[8], st));
+    Scalars h_sc;
     CK(cudaMemcpyAsync(&h_sc, sc, sizeof h_sc, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     for (int i = 0; i < 8; ++i) {
@@ -681,10 +755,10 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
     ctx->last_cnt[6] += (int64_t)h_sc.evaluated_ps;
     if (ctx->prune) {
         float msb = 0.f;
-        CK(cudaEventElapsedTime(&msb, use_tc ? ev[22] : ev[20], ev[21]));
+        CK(cudaEventElapsedTime(&msb, use_tc ? ev[11] : ev[9], ev[10]));
         ctx->last_ms[11] += msb;
         if (use_tc) {
-            CK(cudaEventElapsedTime(&msb, ev[20], ev[22]));
+            CK(cudaEventElapsedTime(&msb, ev[9], ev[11]));
             ctx->last_ms[12] += msb;
         }
     }
@@ -755,23 +829,12 @@ int launch_scatter_masks(rp_ctx *ctx, int P, long long n, const long long *d_off
     return RP_OK;
 }
 
-int check_common(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const rp_options *opt) {
-    if (!ctx) return RP_ERR_INVALID;
-    if (variant < 0 || variant > 3) return fail(ctx, RP_ERR_INVALID, "unknown variant");
-    if (n_pairs < 0 || !offsets || !opt) return fail(ctx, RP_ERR_INVALID, "null or negative argument");
-    if (opt->max_iterations < 0 || opt->max_iterations > (1 << 24)) return fail(ctx, RP_ERR_INVALID, "max_iterations out of range");
-    for (int64_t p = 0; p < n_pairs; ++p)
-        if (offsets[p + 1] < offsets[p] || offsets[p + 1] - offsets[p] >= (1 << 24))
-            return fail(ctx, RP_ERR_INVALID, "offsets must be non-decreasing, at most 2^24-1 correspondences per pair");
-    return RP_OK;
-}
-
 // Pairs of a chunk whose first pass was flagged — more trigger events than the list holds, or (early termination) more
 // iterations needed than were generated — are gathered into compact sub-batches and run again on their own with the
 // limits raised (iterations x4 up to max_iterations, event capacity x8), until no flag is left.  Everybody else's
 // results are untouched; what a hard pair costs is bounded by ~1.33x what the reference spends on that pair.  A
 // sub-batch that cannot be run (out of device memory) marks its pairs RP_PAIR_FAILED instead of failing the call.
-int rerun_flagged(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io, const std::vector<long long> &rel,
+int rerun_flagged(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io, const long long *rel,
                   const std::vector<int> &flags0, int iters0, int64_t p0, cudaStream_t st) {
     DevBuf *B = ctx->buf;
     const bool pose = variant == RP_CALIB || variant == RP_CALIB_SHIFT;
@@ -875,14 +938,232 @@ int rerun_flagged(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO
     return RP_OK;
 }
 
-// In = double: the FP64 entry points.  In = float: rp_estimate_batch_*_f32 — the host path uploads the float chunk
-// (24 B per correspondence instead of 48) and widens it on the copy stream, the device path widens the caller's
-// chunk on the compute stream; either way every kernel after that reads the same FP64 chunk arrays as with In = double.
-// quality != null: rp_estimate_batch_*_quality — each chunk is sorted pair by pair (order_by_quality_kernel) and gathered
-// into B_IN_* in that order by the permuting widen_inputs_kernel (host path: on the copy stream from In-typed staging;
-// device path: on the compute stream from the caller's arrays).  run_chunk and rerun_flagged then run unchanged on the
-// ordered chunk and write its masks into an ordered-layout buffer, which scatter_masks_kernel writes back in the
-// caller's order.
+// Checks and set-up shared by estimate_impl and refine_impl (RP_CALIB with estimate_shift runs as RP_CALIB_SHIFT)
+int begin_batch(rp_ctx *ctx, int &variant, int64_t n_pairs, const int64_t *offsets, const double *cams,
+                const rp_options *opt_in, rp_options &opt) {
+    if (!ctx) return RP_ERR_INVALID;
+    if (variant < 0 || variant > 3) return fail(ctx, RP_ERR_INVALID, "unknown variant");
+    if (n_pairs < 0 || !offsets || !opt_in) return fail(ctx, RP_ERR_INVALID, "null or negative argument");
+    if (opt_in->max_iterations < 0 || opt_in->max_iterations > (1 << 24))
+        return fail(ctx, RP_ERR_INVALID, "max_iterations out of range");
+    for (int64_t p = 0; p < n_pairs; ++p)
+        if (offsets[p + 1] < offsets[p] || offsets[p + 1] - offsets[p] >= (1 << 24))
+            return fail(ctx, RP_ERR_INVALID, "offsets must be non-decreasing, at most 2^24-1 correspondences per pair");
+    CK(cudaSetDevice(ctx->device));
+    opt = *opt_in;
+    if (variant == RP_CALIB && opt.estimate_shift) variant = RP_CALIB_SHIFT;
+    if (variant == RP_CALIB_SHIFT) opt.estimate_shift = 1;
+    const bool pose = variant == RP_CALIB || variant == RP_CALIB_SHIFT;
+    if (pose && !cams && n_pairs > 0) return fail(ctx, RP_ERR_INVALID, "calibrated variants need cams");
+    return RP_OK;
+}
+
+// Chunk boundaries of a batch: at most as many pairs per chunk as the workspace budget holds at `bpp` bytes per pair
+// (and 32 768), the remainder split evenly (no tiny last chunk).  On the host path, batches of 1024 pairs or more are
+// split so that uploads hide behind kernels, by one of two policies:
+//   lead = true (the estimator): a small first chunk goes ahead so that the kernels start early and every later upload
+//     hides behind the previous chunk's kernels.  With U = upload time (+ widening or ordering) and C = kernel time of
+//     the whole batch, the exposed time f U + max(0, (1-f) U - f C) is smallest at f = U / (U + C); U / C is taken
+//     from the previous host call on this context (1/8 of the batch before there is one).  RP_NO_LEAD_CHUNK: none.
+//   lead = false (the refinement): at least four chunks, so that three uploads hide behind kernels.
+// Only timing depends on the boundaries, never results.
+std::vector<int64_t> plan_chunks(const rp_ctx *ctx, int64_t n_pairs, size_t bpp, bool host_io, bool lead) {
+    int64_t chunk = (int64_t)std::max<size_t>(1, ctx->workspace_budget / bpp);
+    chunk = std::min<int64_t>(chunk, 32768);
+    int64_t first = 0;
+    if (host_io && n_pairs >= 1024) {
+        if (!lead) {
+            chunk = std::min<int64_t>(chunk, (n_pairs + 3) / 4);
+        } else if (!getenv("RP_NO_LEAD_CHUNK")) {
+            double f = 0.125;
+            if (ctx->prev_h2d_ms > 0.0 && ctx->prev_dev_ms > 0.0) f = ctx->prev_h2d_ms / (ctx->prev_h2d_ms + ctx->prev_dev_ms);
+            f = std::min(1.0 / 3.0, std::max(1.0 / 32.0, f));
+            first = std::min<int64_t>(std::min<int64_t>(n_pairs, chunk), std::max<int64_t>(256, (int64_t)(f * (double)n_pairs)));
+        }
+    }
+    std::vector<int64_t> bounds(1, 0);
+    if (first > 0) bounds.push_back(first);
+    const int64_t rest = n_pairs - first;
+    const int64_t k = (rest + chunk - 1) / chunk;
+    for (int64_t i = 1; i <= k; ++i) bounds.push_back(first + (rest * i) / k);
+    return bounds;
+}
+
+// A batch's inputs as the caller passed them: host memory on the host path, device memory on the device path (offsets
+// are host memory either way)
+template <class In>
+struct BatchIn {
+    const int64_t *offsets;
+    const In *x1, *x2, *d1, *d2;
+    const double *cams;       // null for the focal variants
+    const float *quality;     // quality calls: each chunk is ordered pair by pair
+    const rp_model *init;     // refinement: start models, subset (null: every correspondence)
+    const uint8_t *subset;
+    bool host_io;
+};
+
+// Where the kernels write one output of a chunk, `n` elements from element `at` of the batch: the caller's array on the
+// device path, set buffer `staging` on the host path (read back by the download of run_chunks), null when the caller
+// did not ask for the output
+template <class T>
+cudaError_t chunk_out(bool host_io, DevBuf &staging, T *caller, int64_t at, size_t n, T *&out) {
+    out = caller && !host_io ? caller + at : nullptr;
+    if (!caller || !host_io) return cudaSuccess;
+    const cudaError_t e = staging.reserve(sizeof(T) * n);
+    out = staging.as<T>();
+    return e;
+}
+
+// Puts the inputs of the pairs [p0, p1) where the kernels read them and points io's inputs there.  The kernels read
+// FP64; float32 inputs are widened first, and quality calls sort each pair (order_by_quality_kernel) and gather it in
+// that order with the permuting widen_inputs_kernel.
+//   Host path, on the copy stream into set s: the upload (into the input-type staging when the chunk is widened or
+//   ordered), the widening or ordering, then s.in_ready.
+//   Device path, on the compute stream `st`: FP64 inputs without quality are read where they are; otherwise they are
+//   widened, or ordered, into set s.
+// [s.h2d_begin, s.h2d_end) is the host path's upload (rp_last_timing [9]), [s.h2d_end, s.in_ready) the widening or
+// ordering ([13] / [14]).
+template <class In>
+int stage_inputs(rp_ctx *ctx, const BatchIn<In> &b, int64_t p0, int64_t p1, StageSet &s, cudaStream_t st, ChunkIO &io) {
+    constexpr bool f32 = std::is_same<In, float>::value;
+    const bool ordered = b.quality != nullptr, widen = f32 || ordered;
+    const int P = (int)(p1 - p0);
+    const long long o0 = b.offsets[p0], N = b.offsets[p1] - o0;
+    const size_t nn = (size_t)std::max<long long>(N, 1);
+    // what the kernels or the widening read: the caller's arrays, or on the host path their upload
+    const In *x1 = b.x1 + 2 * o0, *x2 = b.x2 + 2 * o0, *d1 = b.d1 + o0, *d2 = b.d2 + o0;
+    const float *quality = ordered ? b.quality + o0 : nullptr;
+    io.cams = b.cams ? b.cams + 8 * p0 : nullptr;
+    io.init = b.init ? (const Model *)b.init + p0 : nullptr;
+    io.subset = b.subset ? b.subset + o0 : nullptr;
+    if (!b.host_io && !widen) {
+        // (In = double here: float32 inputs are always widened)
+        io.x1 = (const double *)x1; io.x2 = (const double *)x2; io.d1 = (const double *)d1; io.d2 = (const double *)d2;
+        return RP_OK;
+    }
+    const cudaStream_t ws = b.host_io ? ctx->copy_stream : st;
+    CK(s.x1.reserve(16 * nn)); CK(s.x2.reserve(16 * nn));
+    CK(s.d1.reserve(8 * nn)); CK(s.d2.reserve(8 * nn));
+    if (ordered) {
+        CK(s.perm.reserve(4 * nn)); CK(s.ksort.reserve(nn)); CK(s.offs.reserve(8 * ((size_t)P + 1)));
+    }
+    if (b.host_io) {
+        constexpr size_t E = sizeof(In);
+        DevBuf &ux1 = widen ? s.sx1 : s.x1, &ux2 = widen ? s.sx2 : s.x2, &ud1 = widen ? s.sd1 : s.d1,
+               &ud2 = widen ? s.sd2 : s.d2;
+        CK(ux1.reserve(2 * E * nn)); CK(ux2.reserve(2 * E * nn));
+        CK(ud1.reserve(E * nn)); CK(ud2.reserve(E * nn));
+        CK(s.cams.reserve(64 * (size_t)P));
+        CK(cudaEventRecord(s.h2d_begin, ws));
+        CK(cudaMemcpyAsync(ux1.p, x1, 2 * E * (size_t)N, cudaMemcpyHostToDevice, ws));
+        CK(cudaMemcpyAsync(ux2.p, x2, 2 * E * (size_t)N, cudaMemcpyHostToDevice, ws));
+        CK(cudaMemcpyAsync(ud1.p, d1, E * (size_t)N, cudaMemcpyHostToDevice, ws));
+        CK(cudaMemcpyAsync(ud2.p, d2, E * (size_t)N, cudaMemcpyHostToDevice, ws));
+        if (io.cams) {
+            CK(cudaMemcpyAsync(s.cams.p, io.cams, 64 * (size_t)P, cudaMemcpyHostToDevice, ws));
+            io.cams = s.cams.as<double>();
+        }
+        if (ordered) {
+            CK(s.qual.reserve(4 * nn));
+            CK(cudaMemcpyAsync(s.qual.p, quality, 4 * (size_t)N, cudaMemcpyHostToDevice, ws));
+            CK(cudaMemcpyAsync(s.offs.p, b.offsets + p0, 8 * ((size_t)P + 1), cudaMemcpyHostToDevice, ws));
+            quality = s.qual.as<float>();
+        }
+        if (io.init) {
+            CK(s.init.reserve(sizeof(Model) * P));
+            CK(cudaMemcpyAsync(s.init.p, io.init, sizeof(Model) * P, cudaMemcpyHostToDevice, ws));
+            io.init = s.init.as<Model>();
+        }
+        if (io.subset) {
+            CK(s.subset.reserve(nn));
+            CK(cudaMemcpyAsync(s.subset.p, io.subset, (size_t)N, cudaMemcpyHostToDevice, ws));
+            io.subset = s.subset.as<unsigned char>();
+        }
+        x1 = ux1.as<In>(); x2 = ux2.as<In>(); d1 = ud1.as<In>(); d2 = ud2.as<In>();
+    }
+    CK(cudaEventRecord(s.h2d_end, ws));
+    if (ordered) {
+        if (!b.host_io) CK(cudaMemcpyAsync(s.offs.p, b.offsets + p0, 8 * ((size_t)P + 1), cudaMemcpyHostToDevice, ws));
+        int rc = launch_order(ctx, P, N, b.offsets + p0, s.offs.as<long long>(), o0, quality, s.perm.as<int>(), ws);
+        if (rc) return rc;
+    }
+    if (widen) {
+        int rc = launch_widen(ctx, N, x1, x2, d1, d2, s.x1.as<double>(), s.x2.as<double>(), s.d1.as<double>(),
+                              s.d2.as<double>(), ws, ordered ? s.perm.as<int>() : nullptr,
+                              ordered ? s.offs.as<long long>() : nullptr, o0, P);
+        if (rc) return rc;
+    }
+    CK(cudaEventRecord(s.in_ready, ws));
+    io.x1 = s.x1.as<double>(); io.x2 = s.x2.as<double>(); io.d1 = s.d1.as<double>(); io.d2 = s.d2.as<double>();
+    return RP_OK;
+}
+
+// The chunk pipeline of estimate_impl and refine_impl.  For each chunk c, in this order:
+//   host path: make the compute stream wait for chunk c's in_ready; device path: stage_inputs of chunk c on the
+//     compute stream;
+//   work(c, set, io) enqueues chunk c's kernels on the compute stream;
+//   host path: record set.done on the compute stream, make the copy stream wait for it, and download(c, io, copy
+//     stream) reads chunk c's outputs back between set.d2h_begin and set.d2h_end.
+// On the host path the upload of chunk c+1 into the other staging set (stage_inputs on the copy stream) is enqueued
+// next to chunk c's work, so that it overlaps chunk c's kernels, and chunk c's read-back overlaps chunk c+1's kernels.
+// Where depends on what may block the host: with `work_waits` the work returns only after chunk c's kernels have
+// finished (run_chunk synchronises), so the upload goes before it; otherwise it goes after the work, because an upload
+// from pageable host memory waits for the copy stream, and chunk c's kernels must already be enqueued by then.  Either
+// way the copy stream runs upload c+1 before read-back c.  The rule that makes this safe: the copy stream must not
+// write a set before the kernels that last read it have finished.  Chunk c+2's upload into set c & 1 follows chunk c's
+// read-back on the copy stream, which waits for chunk c's `done` event.  At the end the host synchronises the copy
+// stream (host path) or the compute stream (device path).
+template <class In, class Work, class Download>
+int run_chunks(rp_ctx *ctx, const BatchIn<In> &b, const std::vector<int64_t> &bounds, cudaStream_t st, bool work_waits,
+               Work work, Download download) {
+    cudaStream_t cs = ctx->copy_stream;
+    const int64_t n_chunks = (int64_t)bounds.size() - 1;
+    ChunkIO io[2];
+    std::vector<long long> rel;
+    int rc = b.host_io ? stage_inputs(ctx, b, bounds[0], bounds[1], ctx->set[0], st, io[0]) : RP_OK;
+    if (rc) return rc;
+    for (int64_t c = 0; c < n_chunks; ++c) {
+        StageSet &s = ctx->set[b.host_io ? c & 1 : 0];
+        ChunkIO &cur = io[c & 1];
+        auto upload_next = [&]() {
+            return b.host_io && c + 1 < n_chunks
+                       ? stage_inputs(ctx, b, bounds[c + 1], bounds[c + 2], ctx->set[(c + 1) & 1], st, io[(c + 1) & 1])
+                       : RP_OK;
+        };
+        if (work_waits && (rc = upload_next())) return rc;
+        if (b.host_io) {
+            CK(cudaStreamWaitEvent(st, s.in_ready, 0));
+        } else {
+            rc = stage_inputs(ctx, b, bounds[c], bounds[c + 1], s, st, cur);
+            if (rc) return rc;
+        }
+        const int64_t p0 = bounds[c];
+        cur.n_pairs = (int)(bounds[c + 1] - p0);
+        cur.n_points = b.offsets[bounds[c + 1]] - b.offsets[p0];
+        rel.resize((size_t)cur.n_pairs + 1);
+        for (int i = 0; i <= cur.n_pairs; ++i) rel[(size_t)i] = b.offsets[p0 + i] - b.offsets[p0];
+        cur.h_offsets_rel = rel.data();
+        rc = work(c, s, cur);
+        if (rc) return rc;
+        if (!work_waits && (rc = upload_next())) return rc;
+        if (b.host_io) {
+            CK(cudaEventRecord(s.done, st));
+            CK(cudaStreamWaitEvent(cs, s.done, 0));
+            CK(cudaEventRecord(s.d2h_begin, cs));
+            rc = download(c, cur, cs);
+            if (rc) return rc;
+            CK(cudaEventRecord(s.d2h_end, cs));
+        }
+    }
+    CK(cudaStreamSynchronize(b.host_io ? cs : st));
+    return RP_OK;
+}
+
+// rp_estimate_batch_*: run_chunks with run_chunk and rerun_flagged as the work of a chunk.  In = double: the FP64 entry
+// points; In = float: the _f32 ones (24 B per correspondence uploaded instead of 48, then widened); quality != null: the
+// _quality ones, whose chunks run_chunk and rerun_flagged see in the quality order and whose masks they write in that
+// order, which scatter_masks_kernel writes back in the caller's order.  Either way every kernel after stage_inputs
+// reads the same FP64 chunk arrays as the FP64 entry points.
 template <class In>
 int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const In *x1,
                   const In *x2, const In *d1, const In *d2, const float *quality, const double *cams,
@@ -890,15 +1171,11 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
                   cudaStream_t st) {
     constexpr bool f32 = std::is_same<In, float>::value;
     const bool ordered = quality != nullptr;
-    const bool staged = f32 || ordered;   // host path: In-typed staging, widened / gathered into B_IN_* on the copy stream
-    int rc = check_common(ctx, variant, n_pairs, offsets, opt_in);
+    const bool staged = f32 || ordered;   // the chunk is widened or ordered before its kernels
+    rp_options opt;
+    int rc = begin_batch(ctx, variant, n_pairs, offsets, cams, opt_in, opt);
     if (rc) return rc;
-    CK(cudaSetDevice(ctx->device));
-    rp_options opt = *opt_in;
-    if (variant == RP_CALIB && opt.estimate_shift) variant = RP_CALIB_SHIFT;
-    if (variant == RP_CALIB_SHIFT) opt.estimate_shift = 1;
     const bool pose = variant == RP_CALIB || variant == RP_CALIB_SHIFT;
-    if (pose && !cams && n_pairs > 0) return fail(ctx, RP_ERR_INVALID, "calibrated variants need cams");
     memset(ctx->last_ms, 0, sizeof ctx->last_ms);
     memset(ctx->last_cnt, 0, sizeof ctx->last_cnt);
     ctx->pair_status.assign((size_t)n_pairs, RP_PAIR_OK);
@@ -907,7 +1184,7 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
     // Early termination (min_iterations < max_iterations): the reference stops at the first it > min_iterations with
     // it > dynamic_max_iter.  The first pass generates min_iterations + 1 iterations for every pair and the merge
     // kernel replays the stop rule exactly; only the pairs that would have kept going are run again, on their own,
-    // with 4x more iterations (same seed => same prefix), see rerun_flagged below.
+    // with 4x more iterations (same seed => same prefix), see rerun_flagged above.
     const int iters0 = opt.min_iterations < opt.max_iterations
                            ? (int)std::min<int64_t>(opt.max_iterations, opt.min_iterations + 1)
                            : (int)opt.max_iterations;
@@ -916,219 +1193,66 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
     // gathered copy, the order and the ordered-layout mask (device path).
     size_t in_bytes = f32 ? 48 : 0;
     if (ordered) in_bytes = host_io ? 2 * (6 * sizeof(In) + 4 + 4 + 1) : 48 + 4 + 1;
-    const size_t bpp = bytes_per_pair(iters0, Ntot / n_pairs + 1, ctx->ev_cap0, in_bytes);
-    int64_t chunk = (int64_t)std::max<size_t>(1, ctx->workspace_budget / bpp);
-    chunk = std::min<int64_t>(chunk, 32768);
-    std::vector<long long> rel;
-    DevBuf *B = ctx->buf;
-    // Chunk boundaries.  The remainder is split evenly (no tiny last chunk); on the host path a small first
-    // chunk goes ahead so that the kernels start early and every later upload hides behind the previous
-    // chunk's kernels.  With U = upload time (+ widening or ordering) and C = kernel time of the whole batch, the exposed
-    // time f U + max(0, (1-f) U - f C) is smallest at f = U / (U + C); U / C is taken from the previous host call on
-    // this context (1/8 of the batch before there is one).  Only timing depends on it, never results.
-    std::vector<int64_t> bounds(1, 0);
-    {
-        int64_t first = 0;
-        if (host_io && n_pairs >= 1024 && !getenv("RP_NO_LEAD_CHUNK")) {
-            double f = 0.125;
-            if (ctx->prev_h2d_ms > 0.0 && ctx->prev_dev_ms > 0.0) f = ctx->prev_h2d_ms / (ctx->prev_h2d_ms + ctx->prev_dev_ms);
-            f = std::min(1.0 / 3.0, std::max(1.0 / 32.0, f));
-            first = std::min<int64_t>(std::min<int64_t>(n_pairs, chunk), std::max<int64_t>(256, (int64_t)(f * (double)n_pairs)));
-        }
-        if (first > 0) bounds.push_back(first);
-        const int64_t rest = n_pairs - first;
-        const int64_t k = (rest + chunk - 1) / chunk;
-        for (int64_t i = 1; i <= k; ++i) bounds.push_back(first + (rest * i) / k);
-    }
-    const int64_t n_chunks = (int64_t)bounds.size() - 1;
-    // Host path: double-buffered staging.  The copy stream uploads chunk c+1 and downloads chunk c-1
-    // while the compute stream runs the kernels of chunk c (pinned host memory makes this truly async).
-    static const int IN_X1[2] = {B_IN_X1, B_IN_X1_B}, IN_X2[2] = {B_IN_X2, B_IN_X2_B}, IN_D1[2] = {B_IN_D1, B_IN_D1_B},
-                     IN_D2[2] = {B_IN_D2, B_IN_D2_B}, IN_CAMS[2] = {B_IN_CAMS, B_IN_CAMS_B}, OUT_M[2] = {B_TMP0, B_TMP0_B},
-                     OUT_S[2] = {B_TMP1, B_TMP1_B}, OUT_K[2] = {B_MASK, B_MASK_B};
-    static const int STG_X1[2] = {B_STG_X1, B_STG_X1_B}, STG_X2[2] = {B_STG_X2, B_STG_X2_B}, STG_D1[2] = {B_STG_D1, B_STG_D1_B},
-                     STG_D2[2] = {B_STG_D2, B_STG_D2_B};
-    static const int QUAL[2] = {B_QUAL, B_QUAL_B}, ORDOFFS[2] = {B_ORDOFFS, B_ORDOFFS_B}, PERM[2] = {B_PERM, B_PERM_B},
-                     KSORT[2] = {B_KSORT, B_KSORT_B};
-    cudaStream_t cs = ctx->copy_stream;
-    cudaEvent_t *in_ready = &ctx->ev[12], *h2d_begin = &ctx->ev[14], *comp_done = &ctx->ev[16], *d2h_begin = &ctx->ev[18];
-    cudaEvent_t *h2d_end = &ctx->ev[23];  // staged inputs: end of the upload, start of the widening / ordering (host path)
-    cudaEvent_t widen_begin = ctx->ev[25], widen_end = ctx->ev[26];  // float32 inputs or quality calls, device path
-    cudaEvent_t scatter_begin = ctx->ev[27], scatter_end = ctx->ev[28];  // quality calls: the mask scatter
-    cudaEvent_t d2h_end = ctx->ev[11];
-    double stage_per_point0 = 0.0;  // staged host path: widening / ordering time of chunk 0 per correspondence (ms)
-    auto upload = [&](int64_t c) -> int {
-        const int64_t p0 = bounds[c], p1 = bounds[c + 1];
-        const int P = (int)(p1 - p0), par = (int)(c & 1);
-        const long long o0 = offsets[p0], N = offsets[p1] - o0;
-        const size_t nn = (size_t)std::max<long long>(N, 1);
-        CK(B[IN_X1[par]].reserve(16 * nn)); CK(B[IN_X2[par]].reserve(16 * nn));
-        CK(B[IN_D1[par]].reserve(8 * nn)); CK(B[IN_D2[par]].reserve(8 * nn));
-        CK(B[IN_CAMS[par]].reserve(64 * (size_t)P));
-        CK(B[OUT_M[par]].reserve(sizeof(Model) * P)); CK(B[OUT_S[par]].reserve(sizeof(rp_stats) * P));
-        CK(B[OUT_K[par]].reserve(nn));
-        CK(cudaEventRecord(h2d_begin[par], cs));
-        if (staged) {
-            constexpr size_t E = sizeof(In);
-            CK(B[STG_X1[par]].reserve(2 * E * nn)); CK(B[STG_X2[par]].reserve(2 * E * nn));
-            CK(B[STG_D1[par]].reserve(E * nn)); CK(B[STG_D2[par]].reserve(E * nn));
-            CK(cudaMemcpyAsync(B[STG_X1[par]].p, x1 + 2 * o0, 2 * E * (size_t)N, cudaMemcpyHostToDevice, cs));
-            CK(cudaMemcpyAsync(B[STG_X2[par]].p, x2 + 2 * o0, 2 * E * (size_t)N, cudaMemcpyHostToDevice, cs));
-            CK(cudaMemcpyAsync(B[STG_D1[par]].p, d1 + o0, E * (size_t)N, cudaMemcpyHostToDevice, cs));
-            CK(cudaMemcpyAsync(B[STG_D2[par]].p, d2 + o0, E * (size_t)N, cudaMemcpyHostToDevice, cs));
-            if (pose) CK(cudaMemcpyAsync(B[IN_CAMS[par]].p, cams + 8 * p0, 64 * (size_t)P, cudaMemcpyHostToDevice, cs));
-            if (ordered) {
-                CK(B[QUAL[par]].reserve(4 * nn)); CK(B[PERM[par]].reserve(4 * nn)); CK(B[KSORT[par]].reserve(nn));
-                CK(B[ORDOFFS[par]].reserve(8 * ((size_t)P + 1)));
-                CK(cudaMemcpyAsync(B[QUAL[par]].p, quality + o0, 4 * (size_t)N, cudaMemcpyHostToDevice, cs));
-                CK(cudaMemcpyAsync(B[ORDOFFS[par]].p, offsets + p0, 8 * ((size_t)P + 1), cudaMemcpyHostToDevice, cs));
-            }
-            CK(cudaEventRecord(h2d_end[par], cs));
-            const In *sx1 = B[STG_X1[par]].as<In>(), *sx2 = B[STG_X2[par]].as<In>(), *sd1 = B[STG_D1[par]].as<In>(),
-                     *sd2 = B[STG_D2[par]].as<In>();
-            int rc2 = RP_OK;
-            if (ordered) {
-                const long long *doffs = B[ORDOFFS[par]].as<long long>();
-                rc2 = launch_order(ctx, P, N, offsets + p0, doffs, o0, B[QUAL[par]].as<float>(), B[PERM[par]].as<int>(), cs);
-                if (!rc2)
-                    rc2 = launch_widen(ctx, N, sx1, sx2, sd1, sd2, B[IN_X1[par]].as<double>(), B[IN_X2[par]].as<double>(),
-                                       B[IN_D1[par]].as<double>(), B[IN_D2[par]].as<double>(), cs, B[PERM[par]].as<int>(),
-                                       doffs, o0, P);
-            } else {
-                rc2 = launch_widen(ctx, N, sx1, sx2, sd1, sd2, B[IN_X1[par]].as<double>(), B[IN_X2[par]].as<double>(),
-                                   B[IN_D1[par]].as<double>(), B[IN_D2[par]].as<double>(), cs);
-            }
-            if (rc2) return rc2;
-        } else {
-            CK(cudaMemcpyAsync(B[IN_X1[par]].p, x1 + 2 * o0, 16 * (size_t)N, cudaMemcpyHostToDevice, cs));
-            CK(cudaMemcpyAsync(B[IN_X2[par]].p, x2 + 2 * o0, 16 * (size_t)N, cudaMemcpyHostToDevice, cs));
-            CK(cudaMemcpyAsync(B[IN_D1[par]].p, d1 + o0, 8 * (size_t)N, cudaMemcpyHostToDevice, cs));
-            CK(cudaMemcpyAsync(B[IN_D2[par]].p, d2 + o0, 8 * (size_t)N, cudaMemcpyHostToDevice, cs));
-            if (pose) CK(cudaMemcpyAsync(B[IN_CAMS[par]].p, cams + 8 * p0, 64 * (size_t)P, cudaMemcpyHostToDevice, cs));
-        }
-        CK(cudaEventRecord(in_ready[par], cs));
-        return RP_OK;
-    };
-    if (host_io) {
-        rc = upload(0);
-        if (rc) return rc;
-    }
-    for (int64_t c = 0; c < n_chunks; ++c) {
-        const int64_t p0 = bounds[c], p1 = bounds[c + 1];
-        const int P = (int)(p1 - p0), par = (int)(c & 1);
-        const long long o0 = offsets[p0], N = offsets[p1] - o0;
-        rel.resize(P + 1);
-        for (int i = 0; i <= P; ++i) rel[i] = offsets[p0 + i] - o0;
-        ChunkIO io;
-        io.n_pairs = P; io.n_points = N; io.h_offsets_rel = rel.data();
-        // quality calls: where the chunk's order lives and where its masks go in the caller's order
-        const int opar = host_io ? par : 0;
-        unsigned char *masks_caller = nullptr;
-        if (host_io) {
-            // staging set par^1 was last read by the kernels of chunk c-1 (finished: run_chunk synchronises)
-            // and by the D2H of chunk c-1, which is ordered before this upload on the copy stream
-            if (c + 1 < n_chunks) {
-                rc = upload(c + 1);
-                if (rc) return rc;
-            }
-            CK(cudaStreamWaitEvent(st, in_ready[par], 0));
-            io.x1 = B[IN_X1[par]].as<double>(); io.x2 = B[IN_X2[par]].as<double>();
-            io.d1 = B[IN_D1[par]].as<double>(); io.d2 = B[IN_D2[par]].as<double>();
-            io.cams = pose ? B[IN_CAMS[par]].as<double>() : nullptr;
-            io.models_out = B[OUT_M[par]].as<Model>(); io.stats_out = B[OUT_S[par]].as<rp_stats>();
-            io.masks_out = B[OUT_K[par]].as<unsigned char>();
-        } else {
-            if (staged) {
-                // the chunk widened (float32) or ordered and gathered (quality) on the compute stream, ahead of its
-                // kernels (B_IN_* are free: run_chunk synchronises)
-                const size_t nn = (size_t)std::max<long long>(N, 1);
-                CK(B[B_IN_X1].reserve(16 * nn)); CK(B[B_IN_X2].reserve(16 * nn));
-                CK(B[B_IN_D1].reserve(8 * nn)); CK(B[B_IN_D2].reserve(8 * nn));
-                if (ordered) {
-                    CK(B[PERM[0]].reserve(4 * nn)); CK(B[KSORT[0]].reserve(nn)); CK(B[ORDOFFS[0]].reserve(8 * ((size_t)P + 1)));
-                }
-                CK(cudaEventRecord(widen_begin, st));
-                if (ordered) {
-                    const long long *doffs = B[ORDOFFS[0]].as<long long>();
-                    CK(cudaMemcpyAsync(B[ORDOFFS[0]].p, offsets + p0, 8 * ((size_t)P + 1), cudaMemcpyHostToDevice, st));
-                    rc = launch_order(ctx, P, N, offsets + p0, doffs, o0, quality + o0, B[PERM[0]].as<int>(), st);
-                    if (rc) return rc;
-                    rc = launch_widen(ctx, N, x1 + 2 * o0, x2 + 2 * o0, d1 + o0, d2 + o0, B[B_IN_X1].as<double>(),
-                                      B[B_IN_X2].as<double>(), B[B_IN_D1].as<double>(), B[B_IN_D2].as<double>(), st,
-                                      B[PERM[0]].as<int>(), doffs, o0, P);
-                } else {
-                    rc = launch_widen(ctx, N, x1 + 2 * o0, x2 + 2 * o0, d1 + o0, d2 + o0, B[B_IN_X1].as<double>(),
-                                      B[B_IN_X2].as<double>(), B[B_IN_D1].as<double>(), B[B_IN_D2].as<double>(), st);
-                }
-                if (rc) return rc;
-                CK(cudaEventRecord(widen_end, st));
-                io.x1 = B[B_IN_X1].as<double>(); io.x2 = B[B_IN_X2].as<double>();
-                io.d1 = B[B_IN_D1].as<double>(); io.d2 = B[B_IN_D2].as<double>();
-            } else {
-                // (In = double here: float32 inputs are always staged)
-                io.x1 = (const double *)(x1 + 2 * o0); io.x2 = (const double *)(x2 + 2 * o0);
-                io.d1 = (const double *)(d1 + o0); io.d2 = (const double *)(d2 + o0);
-            }
-            io.cams = pose ? cams + 8 * p0 : nullptr;
-            io.models_out = (Model *)models + p0; io.stats_out = stats + p0; io.masks_out = masks + o0;
-        }
-        if (ordered) {
-            masks_caller = io.masks_out;
-            io.masks_out = B[KSORT[opar]].as<unsigned char>();
-        }
+    const std::vector<int64_t> bounds =
+        plan_chunks(ctx, n_pairs, bytes_per_pair(iters0, Ntot / n_pairs + 1, ctx->ev_cap0, in_bytes), host_io, true);
+    const BatchIn<In> b = {offsets, x1, x2, d1, d2, pose ? cams : nullptr, quality, nullptr, nullptr, host_io};
+    double stage_per_point0 = 0.0;  // host path: widening / ordering time of chunk 0 per correspondence (ms)
+    auto work = [&](int64_t c, StageSet &s, ChunkIO &io) -> int {
+        const int64_t p0 = bounds[c];
+        const int P = io.n_pairs;
+        const long long o0 = offsets[p0], N = io.n_points;
+        CK(chunk_out(host_io, s.models, (Model *)models, p0, P, io.models_out));
+        CK(chunk_out(host_io, s.stats, stats, p0, P, io.stats_out));
+        CK(chunk_out(host_io, s.mask, masks, o0, (size_t)std::max<long long>(N, 1), io.masks_out));
+        // quality calls: where the masks go in the caller's order
+        unsigned char *masks_caller = io.masks_out;
+        if (ordered) io.masks_out = s.ksort.as<unsigned char>();
         std::vector<int> flags;
-        rc = run_chunk(ctx, variant, opt, io, iters0, ctx->ev_cap0, flags, st);
-        if (rc) return rc;
+        int rc2 = run_chunk(ctx, variant, opt, io, iters0, ctx->ev_cap0, flags, st);
+        if (rc2) return rc2;
+        const long long *rel = io.h_offsets_rel;
         for (int i = 0; i < P; ++i) ctx->pair_status[(size_t)(p0 + i)] = rel[i + 1] - rel[i] < 3 ? RP_PAIR_DEGENERATE : RP_PAIR_OK;
-        rc = rerun_flagged(ctx, variant, opt, io, rel, flags, iters0, p0, st);
-        if (rc) return rc;
+        rc2 = rerun_flagged(ctx, variant, opt, io, rel, flags, iters0, p0, st);
+        if (rc2) return rc2;
+        float ms = 0.f;
         if (ordered) {
-            // the re-runs wrote into the ordered-layout masks too: now they go back to the caller's order.  The host waits
-            // for this one small kernel so that its time can be read and the D2H below (copy stream) sees the masks.
+            // the re-runs wrote into the ordered-layout masks too: now they go back to the caller's order.  The host
+            // waits for this one small kernel so that its time can be read.
+            cudaEvent_t scatter_begin = ctx->ev[12], scatter_end = ctx->ev[13];
             CK(cudaEventRecord(scatter_begin, st));
-            rc = launch_scatter_masks(ctx, P, N, B[ORDOFFS[opar]].as<long long>(), o0, B[PERM[opar]].as<int>(), io.masks_out,
-                                      masks_caller, st);
-            if (rc) return rc;
+            rc2 = launch_scatter_masks(ctx, P, N, s.offs.as<long long>(), o0, s.perm.as<int>(), io.masks_out, masks_caller, st);
+            if (rc2) return rc2;
             CK(cudaEventRecord(scatter_end, st));
             CK(cudaEventSynchronize(scatter_end));
-            float ms = 0.f;
             if (cudaEventElapsedTime(&ms, scatter_begin, scatter_end) == cudaSuccess) ctx->last_ms[14] += ms;
             io.masks_out = masks_caller;
         }
-        if (staged && !host_io) {
-            float ms = 0.f;
-            if (cudaEventElapsedTime(&ms, widen_begin, widen_end) == cudaSuccess) ctx->last_ms[ordered ? 14 : 13] += ms;
+        // (run_chunk returned after synchronising the compute stream, which waited for s.in_ready)
+        if (host_io && cudaEventElapsedTime(&ms, s.h2d_begin, s.h2d_end) == cudaSuccess) ctx->last_ms[9] += ms;
+        if (staged && cudaEventElapsedTime(&ms, s.h2d_end, s.in_ready) == cudaSuccess) {
+            // on the host path the widening / ordering of chunks c >= 1 runs while chunk c-1's kernels hold the SMs, so
+            // its interval includes waiting for them; chunk 0's is that work alone (nothing of this call runs yet) and
+            // sizes the next lead chunk
+            ctx->last_ms[ordered ? 14 : 13] += ms;
+            if (c == 0 && N > 0) stage_per_point0 = ms / (double)N;
         }
-        if (host_io) {
-            // run_chunk returned after synchronising the compute stream: results are complete
-            float ms = 0.f;
-            if (staged) {
-                if (cudaEventElapsedTime(&ms, h2d_begin[par], h2d_end[par]) == cudaSuccess) ctx->last_ms[9] += ms;
-                // widening / ordering of chunks c >= 1 runs while chunk c-1's kernels hold the SMs, so its interval
-                // includes waiting for them; chunk 0's is that work alone (nothing of this call runs yet) and sizes the
-                // next lead chunk
-                if (cudaEventElapsedTime(&ms, h2d_end[par], in_ready[par]) == cudaSuccess) {
-                    ctx->last_ms[ordered ? 14 : 13] += ms;
-                    if (c == 0 && N > 0) stage_per_point0 = ms / (double)N;
-                }
-            } else if (cudaEventElapsedTime(&ms, h2d_begin[par], in_ready[par]) == cudaSuccess) {
-                ctx->last_ms[9] += ms;
-            }
-            CK(cudaEventRecord(d2h_begin[par], cs));
-            CK(cudaMemcpyAsync(models + p0, io.models_out, sizeof(Model) * P, cudaMemcpyDeviceToHost, cs));
-            CK(cudaMemcpyAsync(stats + p0, io.stats_out, sizeof(rp_stats) * P, cudaMemcpyDeviceToHost, cs));
-            if (N > 0) CK(cudaMemcpyAsync(masks + o0, io.masks_out, (size_t)N, cudaMemcpyDeviceToHost, cs));
-            CK(cudaEventRecord(comp_done[par], cs));
-        }
-    }
+        return RP_OK;
+    };
+    auto download = [&](int64_t c, const ChunkIO &io, cudaStream_t cs) -> int {
+        const int64_t p0 = bounds[c];
+        CK(cudaMemcpyAsync(models + p0, io.models_out, sizeof(Model) * io.n_pairs, cudaMemcpyDeviceToHost, cs));
+        CK(cudaMemcpyAsync(stats + p0, io.stats_out, sizeof(rp_stats) * io.n_pairs, cudaMemcpyDeviceToHost, cs));
+        if (io.n_points > 0) CK(cudaMemcpyAsync(masks + offsets[p0], io.masks_out, (size_t)io.n_points, cudaMemcpyDeviceToHost, cs));
+        return RP_OK;
+    };
+    rc = run_chunks(ctx, b, bounds, st, true, work, download);
+    if (rc) return rc;
     if (host_io) {
-        CK(cudaEventRecord(d2h_end, cs));
-        CK(cudaStreamSynchronize(cs));
         ctx->prev_h2d_ms = ctx->last_ms[9] + stage_per_point0 * (double)Ntot;   // + widening / ordering of the batch, 0 with FP64 inputs
         ctx->prev_dev_ms = ctx->last_ms[8];
-        for (int par = 0; par < 2 && par < n_chunks; ++par) {
+        for (int par = 0; par < 2 && par + 1 < (int)bounds.size(); ++par) {
             float ms = 0.f;
-            if (cudaEventElapsedTime(&ms, d2h_begin[par], comp_done[par]) == cudaSuccess) ctx->last_ms[10] += ms;
+            if (cudaEventElapsedTime(&ms, ctx->set[par].d2h_begin, ctx->set[par].d2h_end) == cudaSuccess) ctx->last_ms[10] += ms;
         }
     }
     for (int32_t v : ctx->pair_status)
@@ -1137,90 +1261,36 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
 }
 
 // ---- rp_refine_pairs_*: the estimator's final refinement on caller-supplied start models --------------------------
-struct RefineIO {
-    int n_pairs;
-    long long n_points;
-    const long long *h_offsets_rel;              // host, [n_pairs+1], relative to the chunk
-    const double *x1, *x2, *d1, *d2, *cams;      // device, chunk-local FP64
-    const Model *init;                           // device [n_pairs]
-    const unsigned char *subset;                 // device [n_points] or null (every correspondence)
-    Model *models_out;                           // device [n_pairs] (may alias init)
-    rp_bundle_stats *bstats_out;                 // device [n_pairs] or null
-    long long *num_inliers_out;                  // device [n_pairs] or null
-    unsigned char *inliers_out;                  // device [n_points]; null: no scoring (then num_inliers_out is null)
-};
-
-// One chunk, everything on `st`, no synchronisation: prepare_kernel as run_chunk runs it, refine_import_kernel,
-// the LM launch of run_chunk's step 8 on the work models, the masked score of run_chunk's get_inliers launch on the
-// refined work models, refine_export_kernel (last, because it also turns the score's counts into num_inliers).
-int refine_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const RefineIO &io, cudaStream_t st) {
+// One chunk, everything on `st`, no synchronisation: prepare_chunk, refine_import_kernel, the final refinement
+// (final_lm_args) on the work models, the one-item-per-pair list and get_inliers on the refined work models,
+// refine_export_kernel (last, because it also turns get_inliers' counts into num_inliers).  These are run_chunk's
+// launches on the same inputs, which is why the refinement returns the estimator's bytes.
+int refine_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io, cudaStream_t st) {
     const int P = io.n_pairs;
-    const long long N = io.n_points;
     const bool pose = variant == RP_CALIB || variant == RP_CALIB_SHIFT;
     DevBuf *B = ctx->buf;
-    CK(B[B_OFFS].reserve(sizeof(long long) * (P + 1)));
-    CK(B[B_PAIRS].reserve(sizeof(PairParams) * P));
-    CK(B[B_PTS64].reserve(sizeof(Pt64) * std::max<long long>(N, 1)));
-    CK(B[B_PTS32].reserve(sizeof(float4) * std::max<long long>(N, 1)));
-    CK(B[B_PTS32P].reserve(32 * (size_t)((N + P + 4) / 2 + 1)));
-    CK(B[B_BEAR].reserve(sizeof(Bear) * std::max<long long>(N, 1)));
-    CK(B[B_SCALARS].reserve(sizeof(Scalars)));
     CK(B[B_BEST].reserve(sizeof(Model) * P));
     CK(B[B_ENABLE].reserve(sizeof(int) * P));
     CK(B[B_ONES].reserve(sizeof(int) * P));
     CK(B[B_ONEPFX].reserve(sizeof(int) * (P + 1)));
     CK(B[B_FINSCORE].reserve(sizeof(double) * P));
     CK(B[B_FINCNT].reserve(sizeof(int) * P));
-    Scalars *sc = B[B_SCALARS].as<Scalars>();
+    int rc = prepare_chunk(ctx, variant, opt, io, nullptr, st);
+    if (rc) return rc;
     PairParams *pairs = B[B_PAIRS].as<PairParams>();
     Model *work = B[B_BEST].as<Model>();
     int *enable = B[B_ENABLE].as<int>();
-    Scalars h_sc;
-    memset(&h_sc, 0, sizeof h_sc);
-    h_sc.n_pairs_scalar = P;
-    CK(cudaMemcpyAsync(sc, &h_sc, sizeof h_sc, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(B[B_OFFS].p, io.h_offsets_rel, sizeof(long long) * (P + 1), cudaMemcpyHostToDevice, st));
-    {
-        PrepareArgs a;
-        a.variant = variant; a.n_pairs = P; a.offsets = B[B_OFFS].as<long long>();
-        a.x1 = io.x1; a.x2 = io.x2; a.cams = io.cams;
-        a.max_epipolar_error = opt.max_epipolar_error; a.max_reproj_error = opt.max_reproj_error;
-        a.loss_scale = opt.loss_scale;
-        a.pts64 = B[B_PTS64].as<Pt64>(); a.pts32 = B[B_PTS32].as<float4>(); a.bear = B[B_BEAR].as<Bear>();
-        a.pairs = pairs; a.pts32p = B[B_PTS32P].as<float>();
-        prepare_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(a);
-        LAUNCHED();
-    }
     refine_import_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(P, variant, pairs, io.subset, io.init, work, enable,
                                                                       io.bstats_out);
     LAUNCHED();
-    {
-        LMArgs la;
-        memset(&la, 0, sizeof la);
-        la.pairs = pairs; la.pts64 = B[B_PTS64].as<Pt64>(); la.d1 = io.d1; la.d2 = io.d2;
-        la.weight_sampson = opt.weight_sampson;
-        la.loss_scale_override = -1.0; la.scale_reproj_override = -1.0;
-        la.prob_list = nullptr; la.n_prob = &sc->n_pairs_scalar; la.prob_per_pair = 1;
-        la.models = work; la.use_final = 1; la.mask = io.subset; la.enable = enable; la.stats = io.bstats_out;
-        la.max_iterations = (int)opt.bundle_max_iterations; la.loss_type = opt.loss_type;
-        la.gradient_tol = opt.gradient_tol; la.step_tol = opt.step_tol; la.initial_lambda = opt.initial_lambda;
-        la.min_lambda = opt.min_lambda; la.max_lambda = opt.max_lambda;
-        int rc = launch_lm(ctx, variant, la, P, st);
+    LMArgs la = final_lm_args(ctx, opt, io, work, io.subset, enable);
+    la.stats = io.bstats_out;
+    rc = launch_lm(ctx, variant, la, P, st);
+    if (rc) return rc;
+    if (io.masks_out) {
+        rc = launch_pair_items(ctx, P, st);
         if (rc) return rc;
-    }
-    if (io.inliers_out) {
-        valid_ones_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, pairs, B[B_ONES].as<int>());
-        LAUNCHED();
-        build_items_kernel<<<1, 1024, 0, st>>>(P, B[B_ONES].as<int>(), B[B_ONEPFX].as<int>(), &sc->n_one_items, nullptr);
-        LAUNCHED();
-        if (N > 0) CK(cudaMemsetAsync(io.inliers_out, 0, (size_t)N, st));
-        ScoreArgs s;
-        memset(&s, 0, sizeof s);
-        s.n_groups = P; s.grp_stride = 1; s.grp_per_pair = 1; s.grp_cnt = B[B_ONES].as<int>();
-        s.item_prefix = B[B_ONEPFX].as<int>(); s.n_items = &sc->n_one_items; s.pairs = pairs; s.models = work;
-        s.pts32 = B[B_PTS32].as<float4>(); s.pts64 = B[B_PTS64].as<Pt64>(); s.bear = B[B_BEAR].as<Bear>();
-        s.score = B[B_FINSCORE].as<double>(); s.count = B[B_FINCNT].as<int>(); s.mask = io.inliers_out;
-        int rc = launch_score(ctx, pose, true, s, st);
+        rc = launch_get_inliers(ctx, pose, io, work, io.masks_out, st);
         if (rc) return rc;
     }
     refine_export_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, variant, pairs, enable, io.init, work, B[B_FINCNT].as<int>(),
@@ -1241,10 +1311,9 @@ size_t refine_bytes_per_pair(long long avg_points, bool host_io, bool f32) {
            sets * io_pair + 64;
 }
 
-// rp_refine_pairs_{host,dev}[_f32].  In = float: the float32 inputs are widened into the FP64 chunk arrays first
-// (widen_inputs_kernel without a permutation), so every kernel after that runs on the bytes the FP64 entry points see.
-// Host path: chunk c+1 is uploaded (and widened) on the copy stream into the other staging set while the compute stream
-// runs chunk c; the outputs of chunk c come back on the copy stream.  Neither rp_pair_status nor rp_last_timing changes.
+// rp_refine_pairs_{host,dev}[_f32]: run_chunks with refine_chunk as the work of a chunk.  In = float: the float32
+// inputs are widened into the FP64 chunk arrays first, so every kernel after that runs on the bytes the FP64 entry
+// points see.  Neither rp_pair_status nor rp_last_timing changes.
 template <class In>
 int refine_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const In *x1, const In *x2,
                 const In *d1, const In *d2, const double *cams, const rp_options *opt_in, const rp_model *init,
@@ -1254,134 +1323,40 @@ int refine_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offset
     if (!ctx) return RP_ERR_INVALID;
     if (n_pairs > 0 && (!x1 || !x2 || !d1 || !d2)) return fail(ctx, RP_ERR_INVALID, "null data pointer");
     if (n_pairs > 0 && (!init || !models)) return fail(ctx, RP_ERR_INVALID, "null init / models");
-    int rc = check_common(ctx, variant, n_pairs, offsets, opt_in);
+    rp_options opt;
+    int rc = begin_batch(ctx, variant, n_pairs, offsets, cams, opt_in, opt);
     if (rc) return rc;
-    CK(cudaSetDevice(ctx->device));
-    rp_options opt = *opt_in;
-    if (variant == RP_CALIB && opt.estimate_shift) variant = RP_CALIB_SHIFT;
     const bool pose = variant == RP_CALIB || variant == RP_CALIB_SHIFT;
-    if (pose && !cams && n_pairs > 0) return fail(ctx, RP_ERR_INVALID, "calibrated variants need cams");
     if (n_pairs == 0) return RP_OK;
-    const bool score = num_inliers || inliers;
     const long long Ntot = offsets[n_pairs] - offsets[0];
-    int64_t chunk = (int64_t)std::max<size_t>(1, ctx->workspace_budget / refine_bytes_per_pair(Ntot / n_pairs + 1, host_io, f32));
-    chunk = std::min<int64_t>(chunk, 32768);
-    // host path: at least four chunks for batches of 1024 pairs or more, so that three uploads hide behind kernels
-    if (host_io && n_pairs >= 1024) chunk = std::min<int64_t>(chunk, (n_pairs + 3) / 4);
-    const int64_t n_chunks = (n_pairs + chunk - 1) / chunk;
-    std::vector<int64_t> bounds((size_t)n_chunks + 1);
-    for (int64_t i = 0; i <= n_chunks; ++i) bounds[(size_t)i] = (n_pairs * i) / n_chunks;
-    DevBuf *B = ctx->buf;
-    static const int IN_X1[2] = {B_IN_X1, B_IN_X1_B}, IN_X2[2] = {B_IN_X2, B_IN_X2_B}, IN_D1[2] = {B_IN_D1, B_IN_D1_B},
-                     IN_D2[2] = {B_IN_D2, B_IN_D2_B}, IN_CAMS[2] = {B_IN_CAMS, B_IN_CAMS_B}, STG_X1[2] = {B_STG_X1, B_STG_X1_B},
-                     STG_X2[2] = {B_STG_X2, B_STG_X2_B}, STG_D1[2] = {B_STG_D1, B_STG_D1_B}, STG_D2[2] = {B_STG_D2, B_STG_D2_B},
-                     INIT[2] = {B_RF_INIT, B_RF_INIT_B}, SUB[2] = {B_RF_SUB, B_RF_SUB_B}, OUT_M[2] = {B_TMP0, B_TMP0_B},
-                     OUT_S[2] = {B_TMP1, B_TMP1_B}, OUT_K[2] = {B_MASK, B_MASK_B}, OUT_N[2] = {B_RF_NINL, B_RF_NINL_B};
-    cudaStream_t cs = ctx->copy_stream;
-    cudaEvent_t *in_ready = &ctx->ev[12], *comp_done = &ctx->ev[16];
-    auto upload = [&](int64_t c) -> int {
-        const int64_t p0 = bounds[c], p1 = bounds[c + 1];
-        const int P = (int)(p1 - p0), par = (int)(c & 1);
-        const long long o0 = offsets[p0], N = offsets[p1] - o0;
-        const size_t nn = (size_t)std::max<long long>(N, 1);
-        CK(B[IN_X1[par]].reserve(16 * nn)); CK(B[IN_X2[par]].reserve(16 * nn));
-        CK(B[IN_D1[par]].reserve(8 * nn)); CK(B[IN_D2[par]].reserve(8 * nn));
-        CK(B[IN_CAMS[par]].reserve(64 * (size_t)P)); CK(B[INIT[par]].reserve(sizeof(Model) * P));
-        CK(B[OUT_M[par]].reserve(sizeof(Model) * P));
-        if (subset) CK(B[SUB[par]].reserve(nn));
-        if (bstats) CK(B[OUT_S[par]].reserve(sizeof(rp_bundle_stats) * P));
-        if (score) CK(B[OUT_K[par]].reserve(nn));
-        if (num_inliers) CK(B[OUT_N[par]].reserve(sizeof(long long) * P));
-        constexpr size_t E = sizeof(In);
-        void *dx1 = B[IN_X1[par]].p, *dx2 = B[IN_X2[par]].p, *dd1 = B[IN_D1[par]].p, *dd2 = B[IN_D2[par]].p;
-        if (f32) {
-            CK(B[STG_X1[par]].reserve(2 * E * nn)); CK(B[STG_X2[par]].reserve(2 * E * nn));
-            CK(B[STG_D1[par]].reserve(E * nn)); CK(B[STG_D2[par]].reserve(E * nn));
-            dx1 = B[STG_X1[par]].p; dx2 = B[STG_X2[par]].p; dd1 = B[STG_D1[par]].p; dd2 = B[STG_D2[par]].p;
+    const std::vector<int64_t> bounds =
+        plan_chunks(ctx, n_pairs, refine_bytes_per_pair(Ntot / n_pairs + 1, host_io, f32), host_io, false);
+    const BatchIn<In> b = {offsets, x1, x2, d1, d2, pose ? cams : nullptr, nullptr, init, subset, host_io};
+    auto work = [&](int64_t c, StageSet &s, ChunkIO &io) -> int {
+        const int64_t p0 = bounds[c];
+        const int P = io.n_pairs;
+        const size_t nn = (size_t)std::max<long long>(io.n_points, 1);
+        CK(chunk_out(host_io, s.models, (Model *)models, p0, P, io.models_out));
+        CK(chunk_out(host_io, s.stats, bstats, p0, P, io.bstats_out));
+        CK(chunk_out(host_io, s.ninl, (long long *)num_inliers, p0, P, io.num_inliers_out));
+        CK(chunk_out(host_io, s.mask, inliers, offsets[p0], nn, io.masks_out));
+        if (num_inliers && !inliers) {
+            // num_inliers alone: the mask goes to scratch
+            CK(s.mask.reserve(nn));
+            io.masks_out = s.mask.as<unsigned char>();
         }
-        CK(cudaMemcpyAsync(dx1, x1 + 2 * o0, 2 * E * (size_t)N, cudaMemcpyHostToDevice, cs));
-        CK(cudaMemcpyAsync(dx2, x2 + 2 * o0, 2 * E * (size_t)N, cudaMemcpyHostToDevice, cs));
-        CK(cudaMemcpyAsync(dd1, d1 + o0, E * (size_t)N, cudaMemcpyHostToDevice, cs));
-        CK(cudaMemcpyAsync(dd2, d2 + o0, E * (size_t)N, cudaMemcpyHostToDevice, cs));
-        if (pose) CK(cudaMemcpyAsync(B[IN_CAMS[par]].p, cams + 8 * p0, 64 * (size_t)P, cudaMemcpyHostToDevice, cs));
-        CK(cudaMemcpyAsync(B[INIT[par]].p, init + p0, sizeof(Model) * P, cudaMemcpyHostToDevice, cs));
-        if (subset) CK(cudaMemcpyAsync(B[SUB[par]].p, subset + o0, (size_t)N, cudaMemcpyHostToDevice, cs));
-        if (f32) {
-            int rc2 = launch_widen(ctx, N, (const In *)dx1, (const In *)dx2, (const In *)dd1, (const In *)dd2,
-                                   B[IN_X1[par]].as<double>(), B[IN_X2[par]].as<double>(), B[IN_D1[par]].as<double>(),
-                                   B[IN_D2[par]].as<double>(), cs);
-            if (rc2) return rc2;
-        }
-        CK(cudaEventRecord(in_ready[par], cs));
+        return refine_chunk(ctx, variant, opt, io, st);
+    };
+    auto download = [&](int64_t c, const ChunkIO &io, cudaStream_t cs) -> int {
+        const int64_t p0 = bounds[c];
+        const int P = io.n_pairs;
+        CK(cudaMemcpyAsync(models + p0, io.models_out, sizeof(Model) * P, cudaMemcpyDeviceToHost, cs));
+        if (bstats) CK(cudaMemcpyAsync(bstats + p0, io.bstats_out, sizeof(rp_bundle_stats) * P, cudaMemcpyDeviceToHost, cs));
+        if (num_inliers) CK(cudaMemcpyAsync(num_inliers + p0, io.num_inliers_out, sizeof(long long) * P, cudaMemcpyDeviceToHost, cs));
+        if (inliers && io.n_points > 0) CK(cudaMemcpyAsync(inliers + offsets[p0], io.masks_out, (size_t)io.n_points, cudaMemcpyDeviceToHost, cs));
         return RP_OK;
     };
-    if (host_io) {
-        rc = upload(0);
-        if (rc) return rc;
-    }
-    std::vector<long long> rel;
-    for (int64_t c = 0; c < n_chunks; ++c) {
-        const int64_t p0 = bounds[c], p1 = bounds[c + 1];
-        const int P = (int)(p1 - p0), par = (int)(c & 1);
-        const long long o0 = offsets[p0], N = offsets[p1] - o0;
-        const size_t nn = (size_t)std::max<long long>(N, 1);
-        rel.resize(P + 1);
-        for (int i = 0; i <= P; ++i) rel[i] = offsets[p0 + i] - o0;
-        RefineIO io;
-        io.n_pairs = P; io.n_points = N; io.h_offsets_rel = rel.data();
-        if (host_io) {
-            CK(cudaStreamWaitEvent(st, in_ready[par], 0));
-            io.x1 = B[IN_X1[par]].as<double>(); io.x2 = B[IN_X2[par]].as<double>();
-            io.d1 = B[IN_D1[par]].as<double>(); io.d2 = B[IN_D2[par]].as<double>();
-            io.cams = pose ? B[IN_CAMS[par]].as<double>() : nullptr;
-            io.init = B[INIT[par]].as<Model>(); io.subset = subset ? B[SUB[par]].as<unsigned char>() : nullptr;
-            io.models_out = B[OUT_M[par]].as<Model>(); io.bstats_out = bstats ? B[OUT_S[par]].as<rp_bundle_stats>() : nullptr;
-            io.num_inliers_out = num_inliers ? B[OUT_N[par]].as<long long>() : nullptr;
-            io.inliers_out = score ? B[OUT_K[par]].as<unsigned char>() : nullptr;
-        } else {
-            if (f32) {
-                // B_IN_* are free: the previous chunk's kernels ran before on this stream
-                CK(B[B_IN_X1].reserve(16 * nn)); CK(B[B_IN_X2].reserve(16 * nn));
-                CK(B[B_IN_D1].reserve(8 * nn)); CK(B[B_IN_D2].reserve(8 * nn));
-                rc = launch_widen(ctx, N, x1 + 2 * o0, x2 + 2 * o0, d1 + o0, d2 + o0, B[B_IN_X1].as<double>(),
-                                  B[B_IN_X2].as<double>(), B[B_IN_D1].as<double>(), B[B_IN_D2].as<double>(), st);
-                if (rc) return rc;
-                io.x1 = B[B_IN_X1].as<double>(); io.x2 = B[B_IN_X2].as<double>();
-                io.d1 = B[B_IN_D1].as<double>(); io.d2 = B[B_IN_D2].as<double>();
-            } else {
-                io.x1 = (const double *)(x1 + 2 * o0); io.x2 = (const double *)(x2 + 2 * o0);
-                io.d1 = (const double *)(d1 + o0); io.d2 = (const double *)(d2 + o0);
-            }
-            io.cams = pose ? cams + 8 * p0 : nullptr;
-            io.init = (const Model *)init + p0; io.subset = subset ? subset + o0 : nullptr;
-            io.models_out = (Model *)models + p0; io.bstats_out = bstats ? bstats + p0 : nullptr;
-            io.num_inliers_out = num_inliers ? (long long *)num_inliers + p0 : nullptr;
-            io.inliers_out = inliers ? inliers + o0 : nullptr;
-            if (score && !inliers) {
-                // num_inliers alone: the mask goes to scratch
-                CK(B[B_MASK].reserve(nn));
-                io.inliers_out = B[B_MASK].as<unsigned char>();
-            }
-        }
-        rc = refine_chunk(ctx, variant, opt, io, st);
-        if (rc) return rc;
-        if (host_io) {
-            CK(cudaEventRecord(comp_done[par], st));
-            if (c + 1 < n_chunks) {
-                // staging set par^1 was last read by chunk c-1's kernels, whose downloads (ordered after them) precede
-                // this upload on the copy stream
-                rc = upload(c + 1);
-                if (rc) return rc;
-            }
-            CK(cudaStreamWaitEvent(cs, comp_done[par], 0));
-            CK(cudaMemcpyAsync(models + p0, io.models_out, sizeof(Model) * P, cudaMemcpyDeviceToHost, cs));
-            if (bstats) CK(cudaMemcpyAsync(bstats + p0, io.bstats_out, sizeof(rp_bundle_stats) * P, cudaMemcpyDeviceToHost, cs));
-            if (num_inliers) CK(cudaMemcpyAsync(num_inliers + p0, io.num_inliers_out, sizeof(long long) * P, cudaMemcpyDeviceToHost, cs));
-            if (inliers && N > 0) CK(cudaMemcpyAsync(inliers + o0, io.inliers_out, (size_t)N, cudaMemcpyDeviceToHost, cs));
-        }
-    }
-    CK(cudaStreamSynchronize(host_io ? cs : st));
-    return RP_OK;
+    return run_chunks(ctx, b, bounds, st, false, work, download);
 }
 
 }  // namespace
@@ -1417,6 +1392,7 @@ int rp_create(int device, rp_ctx **out) {
         return RP_ERR_CUDA;
     }
     for (auto &ev : ctx->ev) cudaEventCreate(&ev);
+    for (auto &s : ctx->set) s.create_events();
     if (const char *np = getenv("RP_NO_PRUNE")) ctx->prune = !(np[0] == '1');
     if (const char *nw = getenv("RP_NO_WAVES")) ctx->waves = !(nw[0] == '1');
     if (const char *lw = getenv("RP_LM_WARP")) ctx->lm_warp = atoi(lw) & 0x1f;
@@ -1467,6 +1443,7 @@ void rp_destroy(rp_ctx *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
     for (auto &b : ctx->buf) b.release();
+    for (auto &s : ctx->set) s.release();
     for (auto &ev : ctx->ev) cudaEventDestroy(ev);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
@@ -1655,16 +1632,16 @@ int rp_order_by_quality(rp_ctx *ctx, int64_t n_pairs, const int64_t *offsets, co
     if (N == 0) return RP_OK;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    DevBuf *B = ctx->buf;
+    StageSet &s0 = ctx->set[0];  // the chunk pipeline's set 0, free between calls
     const int P = (int)n_pairs;
-    CK(B[B_QUAL].reserve(4 * (size_t)N)); CK(B[B_PERM].reserve(4 * (size_t)N));
-    CK(B[B_ORDOFFS].reserve(8 * ((size_t)P + 1)));
-    CK(cudaMemcpyAsync(B[B_QUAL].p, quality + offsets[0], 4 * (size_t)N, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(B[B_ORDOFFS].p, offsets, 8 * ((size_t)P + 1), cudaMemcpyHostToDevice, st));
-    int rc = launch_order(ctx, P, N, offsets, B[B_ORDOFFS].as<long long>(), offsets[0], B[B_QUAL].as<float>(),
-                          B[B_PERM].as<int>(), st);
+    CK(s0.qual.reserve(4 * (size_t)N)); CK(s0.perm.reserve(4 * (size_t)N));
+    CK(s0.offs.reserve(8 * ((size_t)P + 1)));
+    CK(cudaMemcpyAsync(s0.qual.p, quality + offsets[0], 4 * (size_t)N, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(s0.offs.p, offsets, 8 * ((size_t)P + 1), cudaMemcpyHostToDevice, st));
+    int rc = launch_order(ctx, P, N, offsets, s0.offs.as<long long>(), offsets[0], s0.qual.as<float>(),
+                          s0.perm.as<int>(), st);
     if (rc) return rc;
-    CK(cudaMemcpyAsync(perm + offsets[0], B[B_PERM].p, 4 * (size_t)N, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(perm + offsets[0], s0.perm.p, 4 * (size_t)N, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return RP_OK;
 }
@@ -1677,16 +1654,17 @@ int rp_solve_batch(rp_ctx *ctx, int variant, int64_t n, const double *x1h, const
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     DevBuf *B = ctx->buf;
-    CK(B[B_IN_X1].reserve(72 * (size_t)n)); CK(B[B_IN_X2].reserve(72 * (size_t)n));
-    CK(B[B_IN_D1].reserve(24 * (size_t)n)); CK(B[B_IN_D2].reserve(24 * (size_t)n));
+    StageSet &s0 = ctx->set[0];  // the chunk pipeline's set 0, free between calls
+    CK(s0.x1.reserve(72 * (size_t)n)); CK(s0.x2.reserve(72 * (size_t)n));
+    CK(s0.d1.reserve(24 * (size_t)n)); CK(s0.d2.reserve(24 * (size_t)n));
     CK(B[B_MODELS].reserve(sizeof(Model) * 4 * (size_t)n)); CK(B[B_COUNT].reserve(sizeof(int) * (size_t)n));
-    CK(cudaMemcpyAsync(B[B_IN_X1].p, x1h, 72 * (size_t)n, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(B[B_IN_X2].p, x2h, 72 * (size_t)n, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(B[B_IN_D1].p, d1, 24 * (size_t)n, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(B[B_IN_D2].p, d2, 24 * (size_t)n, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(s0.x1.p, x1h, 72 * (size_t)n, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(s0.x2.p, x2h, 72 * (size_t)n, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(s0.d1.p, d1, 24 * (size_t)n, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(s0.d2.p, d2, 24 * (size_t)n, cudaMemcpyHostToDevice, st));
     CK(cudaMemsetAsync(B[B_MODELS].p, 0, sizeof(Model) * 4 * (size_t)n, st));
-    solve_problems_kernel<<<cdiv(n, 128), 128, 0, st>>>(variant, n, B[B_IN_X1].as<double>(), B[B_IN_X2].as<double>(),
-                                                       B[B_IN_D1].as<double>(), B[B_IN_D2].as<double>(),
+    solve_problems_kernel<<<cdiv(n, 128), 128, 0, st>>>(variant, n, s0.x1.as<double>(), s0.x2.as<double>(),
+                                                       s0.d1.as<double>(), s0.d2.as<double>(),
                                                        B[B_MODELS].as<Model>(), B[B_COUNT].as<int>());
     LAUNCHED();
     CK(cudaMemcpyAsync(models, B[B_MODELS].p, sizeof(Model) * 4 * (size_t)n, cudaMemcpyDeviceToHost, st));
@@ -1697,13 +1675,14 @@ int rp_solve_batch(rp_ctx *ctx, int variant, int64_t n, const double *x1h, const
 
 static int stage_pair(rp_ctx *ctx, int64_t n_points, const double *x1, const double *x2, double sq_thr, cudaStream_t st) {
     DevBuf *B = ctx->buf;
+    StageSet &s0 = ctx->set[0];  // the chunk pipeline's set 0, free between calls
     const size_t nn = (size_t)std::max<int64_t>(n_points, 1);
     CK(B[B_PAIRS].reserve(sizeof(PairParams)));
     CK(B[B_PTS64].reserve(sizeof(Pt64) * nn)); CK(B[B_PTS32].reserve(sizeof(float4) * nn)); CK(B[B_BEAR].reserve(sizeof(Bear) * nn));
-    CK(B[B_IN_X1].reserve(16 * nn)); CK(B[B_IN_X2].reserve(16 * nn));
-    CK(cudaMemcpyAsync(B[B_IN_X1].p, x1, 16 * (size_t)n_points, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(B[B_IN_X2].p, x2, 16 * (size_t)n_points, cudaMemcpyHostToDevice, st));
-    stage_points_kernel<<<1, 32, 0, st>>>((int)n_points, B[B_IN_X1].as<double>(), B[B_IN_X2].as<double>(), sq_thr,
+    CK(s0.x1.reserve(16 * nn)); CK(s0.x2.reserve(16 * nn));
+    CK(cudaMemcpyAsync(s0.x1.p, x1, 16 * (size_t)n_points, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(s0.x2.p, x2, 16 * (size_t)n_points, cudaMemcpyHostToDevice, st));
+    stage_points_kernel<<<1, 32, 0, st>>>((int)n_points, s0.x1.as<double>(), s0.x2.as<double>(), sq_thr,
                                          B[B_PTS64].as<Pt64>(), B[B_PTS32].as<float4>(), B[B_BEAR].as<Bear>(),
                                          B[B_PAIRS].as<PairParams>());
     LAUNCHED();
@@ -1720,6 +1699,7 @@ int rp_score_batch(rp_ctx *ctx, int variant, int64_t n_models, const rp_model *m
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     DevBuf *B = ctx->buf;
+    StageSet &s0 = ctx->set[0];  // the chunk pipeline's set 0, free between calls
     const bool pose = variant == RP_CALIB || variant == RP_CALIB_SHIFT;
     int rc = stage_pair(ctx, n_points, x1, x2, sq_threshold, st);
     if (rc) return rc;
@@ -1748,19 +1728,19 @@ int rp_score_batch(rp_ctx *ctx, int variant, int64_t n_models, const rp_model *m
     for (int64_t i = 0; i < n_models; ++i) counts[i] = h_cnt[(size_t)i];
     if (masks && n_points > 0) {
         // I1 get_inliers: one launch per model with the mask variant of the same kernel
-        CK(B[B_MASK].reserve((size_t)n_points)); CK(B[B_TMP0].reserve(sizeof(double))); CK(B[B_TMP1].reserve(sizeof(int)));
+        CK(s0.mask.reserve((size_t)n_points)); CK(s0.models.reserve(sizeof(double))); CK(s0.stats.reserve(sizeof(int)));
         const int one = 1;
         CK(cudaMemcpyAsync(B[B_SEGCNT].p, &one, sizeof(int), cudaMemcpyHostToDevice, st));
         build_items_kernel<<<1, 1024, 0, st>>>(1, B[B_SEGCNT].as<int>(), B[B_ITEMPFX].as<int>(), &sc->n_items, nullptr);
         LAUNCHED();
         for (int64_t i = 0; i < n_models; ++i) {
-            CK(cudaMemsetAsync(B[B_MASK].p, 0, (size_t)n_points, st));
+            CK(cudaMemsetAsync(s0.mask.p, 0, (size_t)n_points, st));
             ScoreArgs m = a;
-            m.models = B[B_MODELS].as<Model>() + i; m.score = B[B_TMP0].as<double>(); m.count = B[B_TMP1].as<int>();
-            m.mask = B[B_MASK].as<unsigned char>();
+            m.models = B[B_MODELS].as<Model>() + i; m.score = s0.models.as<double>(); m.count = s0.stats.as<int>();
+            m.mask = s0.mask.as<unsigned char>();
             rc = launch_score(ctx, pose, true, m, st);
             if (rc) return rc;
-            CK(cudaMemcpyAsync(masks + i * n_points, B[B_MASK].p, (size_t)n_points, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(masks + i * n_points, s0.mask.p, (size_t)n_points, cudaMemcpyDeviceToHost, st));
         }
         CK(cudaStreamSynchronize(st));
     }
@@ -1818,15 +1798,16 @@ int rp_refine_batch(rp_ctx *ctx, int variant, int64_t n_models, rp_model *models
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     DevBuf *B = ctx->buf;
+    StageSet &s0 = ctx->set[0];  // the chunk pipeline's set 0, free between calls
     int rc = stage_pair(ctx, n_points, x1, x2, 1.0, st);
     if (rc) return rc;
     const size_t nn = (size_t)std::max<int64_t>(n_points, 1);
-    CK(B[B_IN_D1].reserve(8 * nn)); CK(B[B_IN_D2].reserve(8 * nn)); CK(B[B_MASK].reserve(nn));
+    CK(s0.d1.reserve(8 * nn)); CK(s0.d2.reserve(8 * nn)); CK(s0.mask.reserve(nn));
     CK(B[B_MODELS].reserve(sizeof(Model) * (size_t)n_models)); CK(B[B_SCALARS].reserve(sizeof(Scalars)));
     CK(B[B_TMP2].reserve(sizeof(rp_bundle_stats) * (size_t)n_models));
-    CK(cudaMemcpyAsync(B[B_IN_D1].p, d1, 8 * (size_t)n_points, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(B[B_IN_D2].p, d2, 8 * (size_t)n_points, cudaMemcpyHostToDevice, st));
-    if (mask) CK(cudaMemcpyAsync(B[B_MASK].p, mask, (size_t)n_points, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(s0.d1.p, d1, 8 * (size_t)n_points, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(s0.d2.p, d2, 8 * (size_t)n_points, cudaMemcpyHostToDevice, st));
+    if (mask) CK(cudaMemcpyAsync(s0.mask.p, mask, (size_t)n_points, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(B[B_MODELS].p, models, sizeof(Model) * (size_t)n_models, cudaMemcpyHostToDevice, st));
     Scalars h;
     memset(&h, 0, sizeof h);
@@ -1837,8 +1818,8 @@ int rp_refine_batch(rp_ctx *ctx, int variant, int64_t n_models, rp_model *models
     memset(&la, 0, sizeof la);
     la.prob_list = nullptr; la.n_prob = &sc->n_prob; la.prob_per_pair = 1 << 30;  // every problem -> pair 0
     la.pairs = B[B_PAIRS].as<PairParams>(); la.pts64 = B[B_PTS64].as<Pt64>();
-    la.d1 = B[B_IN_D1].as<double>(); la.d2 = B[B_IN_D2].as<double>();
-    la.mask = mask ? B[B_MASK].as<unsigned char>() : nullptr; la.enable = nullptr;
+    la.d1 = s0.d1.as<double>(); la.d2 = s0.d2.as<double>();
+    la.mask = mask ? s0.mask.as<unsigned char>() : nullptr; la.enable = nullptr;
     la.models = B[B_MODELS].as<Model>(); la.use_final = 1;
     la.max_iterations = (int)opt->max_iterations; la.loss_type = opt->loss_type;
     la.weight_sampson = weight_sampson; la.gradient_tol = opt->gradient_tol; la.step_tol = opt->step_tol;
@@ -2003,16 +1984,16 @@ int rp_measure_pipes(rp_ctx *ctx, double *fp64_tflops, double *fp32_tflops) {
     if (!ctx) return RP_ERR_INVALID;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    DevBuf *B = ctx->buf;
+    StageSet &s0 = ctx->set[0];  // the chunk pipeline's set 0, free between calls
     const int blocks = ctx->sms * 8, threads = 256, iters = 1 << 13;
-    CK(B[B_TMP0].reserve(sizeof(double) * (size_t)blocks * threads));
+    CK(s0.models.reserve(sizeof(double) * (size_t)blocks * threads));
     cudaEvent_t e0 = ctx->ev[9], e1 = ctx->ev[10];
     for (int pass = 0; pass < 2; ++pass) {
         double best = 0.0;
         for (int rep = 0; rep < 4; ++rep) {
             CK(cudaEventRecord(e0, st));
-            if (pass == 0) fp64_pipe_kernel<<<blocks, threads, 0, st>>>(B[B_TMP0].as<double>(), iters);
-            else fp32_pipe_kernel<<<blocks, threads, 0, st>>>(B[B_TMP0].as<float>(), iters);
+            if (pass == 0) fp64_pipe_kernel<<<blocks, threads, 0, st>>>(s0.models.as<double>(), iters);
+            else fp32_pipe_kernel<<<blocks, threads, 0, st>>>(s0.models.as<float>(), iters);
             LAUNCHED();
             CK(cudaEventRecord(e1, st));
             CK(cudaStreamSynchronize(st));
