@@ -21,9 +21,16 @@ namespace {
 
 std::string g_create_error;
 
+inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b); }
+
+// A device buffer that grows on demand and is freed with its owner
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { release(); }
     cudaError_t reserve(size_t bytes) {
         if (bytes <= cap) return cudaSuccess;
         if (p) cudaFree(p);
@@ -43,20 +50,130 @@ struct DevBuf {
     T *as() const { return (T *)p; }
 };
 
-enum { B_OFFS, B_PAIRS, B_PTS64, B_PTS32, B_BEAR, B_SAMPLES, B_MODELS, B_HYPITER, B_SCORE, B_COUNT, B_SEGCNT,
-       B_ITEMPFX, B_SCALARS, B_EVENTS, B_NEVENTS, B_LOMODELS, B_LOOFEV, B_LOCOUNT, B_PROBLIST, B_LOSCORE,
-       B_LOCNT, B_LOITEMPFX, B_BEST, B_FINSTART, B_FINSCORE, B_FINCNT, B_ONES, B_ONEPFX, B_ENABLE, B_STATS,
-       B_PTS32P, B_UB, B_LB, B_FIRSTCNT, B_FIRSTPFX, B_B0, B_S0, B_SURVLIST, B_SURVCNT, B_SURVPFX, B_WAVECUR, B_WAVECNT,
-       B_TMP2,
-       // tensor-core tier: per-point feature rows, per-model outlier counts, survivor lists
-       B_FEAT, B_TCOUT, B_TCLIST, B_TCLISTCNT, B_TCLISTPFX, B_PAIRCNT, B_TCPFX, B_TCSPLIT,
-       // per-pair flags; re-run sub-batches (event-list overflow, early termination that needs more iterations)
-       B_PAIRFLAGS, B_SUB_IDX, B_SUB_SRC, B_SUB_DST, B_SUB_X1, B_SUB_X2, B_SUB_D1, B_SUB_D2, B_SUB_CAMS, B_SUB_MODELS,
-       B_SUB_STATS, B_SUB_MASK,
-       // quality calls: global sort scratch of pairs above RP_ORDER_SMEM_CAP
-       B_ORDSCR,
-       // rp_gather_depths_batch_dev*_quality: the compacted quality between the two passes (4 B per row)
-       B_GATHER_Q, B_NBUF };
+// Reserves each (buffer, bytes) in turn; stops at the first failure
+cudaError_t reserve_all(std::initializer_list<std::pair<DevBuf *, size_t>> bufs) {
+    for (const auto &b : bufs)
+        if (const cudaError_t e = b.first->reserve(b.second)) return e;
+    return cudaSuccess;
+}
+
+// device scalars living in PointBufs::scalars
+struct Scalars {
+    int n_items, n_lo_items, n_one_items, n_prob, n_pairs_scalar, any_flag, reserved0, n_first_items;
+    int n_surv_items, bound_work, lm_work, score_work;  // *_work: counters the persistent kernels draw work from
+    unsigned long long point_scores, lm_iters, n_survivors, evaluated_ps;
+    long long n_hyp;
+    int n_tc_items, n_tcsel_items;
+    unsigned long long tc_evaluated, tc_selected, lm_flops;
+};
+
+// ---- the work arrays of a chunk, by the stage that owns them ---------------------------------------------------
+// Each group's reserve states its sizes for a chunk of P pairs, N correspondences, nseg segments (slots = P nseg 4 SEG
+// model slots) and ev_cap events.  bytes_per_pair and refine_bytes_per_pair below are the chunk planner's estimate of
+// the same per pair.  Between calls the stage entry points borrow these buffers as scratch.
+
+// points and pairs: prepare_kernel's output and the device scalars
+struct PointBufs {
+    DevBuf offs, pairs, pts64, pts32, pts32p, bear, scalars;
+    cudaError_t reserve(int P, long long N) {
+        const size_t n = (size_t)std::max<long long>(N, 1);
+        return reserve_all({{&offs, sizeof(long long) * (P + 1)}, {&pairs, sizeof(PairParams) * P}, {&pts64, sizeof(Pt64) * n},
+                            {&pts32, sizeof(float4) * n}, {&pts32p, 32 * (size_t)((N + P + 4) / 2 + 1)}, {&bear, sizeof(Bear) * n},
+                            {&scalars, sizeof(Scalars)}});
+    }
+};
+// hypotheses: samples, minimal models and their exact scores, per-segment counts and work-item prefix
+struct HypBufs {
+    DevBuf samples, models, hyp_iter, score, count, seg_count, item_prefix;
+    cudaError_t reserve(int P, int iters, int nseg) {
+        const size_t slots = (size_t)P * nseg * 4 * SEG;
+        return reserve_all({{&samples, sizeof(int) * 3 * (size_t)P * std::max(iters, 1)}, {&models, sizeof(Model) * slots},
+                            {&hyp_iter, sizeof(int) * slots}, {&score, sizeof(double) * slots}, {&count, sizeof(int) * slots},
+                            {&seg_count, sizeof(int) * (size_t)P * nseg}, {&item_prefix, sizeof(int) * ((size_t)P * nseg + 1)}});
+    }
+};
+// LO: the trigger events, the LO problems and their scores, the re-run flags
+struct LoBufs {
+    DevBuf events, n_events, lo_models, lo_of_event, lo_count, prob_list, lo_score, lo_cnt, lo_item_prefix, pair_flags;
+    cudaError_t reserve(int P, int ev_cap) {
+        const size_t e = (size_t)P * ev_cap;
+        return reserve_all({{&events, sizeof(int) * e}, {&n_events, sizeof(int) * P}, {&lo_models, sizeof(Model) * e},
+                            {&lo_of_event, sizeof(int) * e}, {&lo_count, sizeof(int) * P}, {&prob_list, sizeof(int) * e},
+                            {&lo_score, sizeof(double) * e}, {&pair_flags, sizeof(int) * P}, {&lo_cnt, sizeof(int) * e},
+                            {&lo_item_prefix, sizeof(int) * (P + 1)}});
+    }
+};
+// per-pair results: the best model, the final LO's start and rescore, the one-item-per-pair list, the final
+// refinement's enable flags, the stats (the merge's final_start and stats only with `merge`: the refinement has no merge)
+struct ResultBufs {
+    DevBuf best, final_start, final_score, final_count, ones, one_prefix, enable, stats;
+    cudaError_t reserve(int P, bool merge) {
+        if (merge) {
+            if (const cudaError_t e = reserve_all({{&final_start, sizeof(Model) * P}, {&stats, sizeof(rp_stats) * P}})) return e;
+        }
+        return reserve_all({{&best, sizeof(Model) * P}, {&final_score, sizeof(double) * P}, {&final_count, sizeof(int) * P},
+                            {&ones, sizeof(int) * P}, {&one_prefix, sizeof(int) * (P + 1)}, {&enable, sizeof(int) * P}});
+    }
+};
+// prune and waves (with the FP32 bound kernel): bounds per slot, the head's bar (B0, S0), survivor lists and waves
+struct PruneBufs {
+    DevBuf ub, lb, first_cnt, first_prefix, B0, S0, surv_list, surv_cnt, surv_prefix, wave_cursor, wave_cnt;
+    cudaError_t reserve(int P, int nseg) {
+        const size_t slots = (size_t)P * nseg * 4 * SEG;
+        return reserve_all({{&ub, sizeof(int) * slots}, {&lb, sizeof(float) * slots}, {&surv_list, sizeof(int) * slots},
+                            {&first_cnt, sizeof(int) * P}, {&first_prefix, sizeof(int) * (P + 1)}, {&B0, sizeof(int) * P},
+                            {&S0, sizeof(double) * P}, {&surv_cnt, sizeof(int) * P}, {&wave_cursor, sizeof(int) * P},
+                            {&wave_cnt, sizeof(int) * P}, {&surv_prefix, sizeof(int) * (P + 1)}});
+    }
+};
+// tensor-core tier: per-correspondence feature rows, per-model certain-outlier counts, the lists it passes on
+struct TcBufs {
+    DevBuf feat, out, list, list_cnt, list_prefix, pair_cnt, prefix, split;
+    cudaError_t reserve(int P, long long N, int nseg) {
+        const size_t slots = (size_t)P * nseg * 4 * SEG;
+        return reserve_all({{&feat, 128 * (size_t)std::max<long long>(N, 1) + 128 * tc::NT}, {&out, sizeof(int) * slots},
+                            {&list, sizeof(int) * slots}, {&list_cnt, sizeof(int) * P}, {&list_prefix, sizeof(int) * (P + 1)},
+                            {&pair_cnt, sizeof(int) * P}, {&split, sizeof(int) * P}, {&prefix, sizeof(int) * (P + 1)}});
+    }
+};
+// re-run sub-batch of S pairs and n correspondences (rerun_flagged): pair index and offsets, the gathered inputs, the
+// sub-batch's outputs.  The batch depth gather borrows idx, src, dst and x1 … d2.
+struct SubBufs {
+    DevBuf idx, src, dst, x1, x2, d1, d2, cams, models, stats, mask;
+    cudaError_t reserve(int S, size_t n) {
+        return reserve_all({{&idx, sizeof(int) * S}, {&src, 8 * (size_t)S}, {&dst, 8 * ((size_t)S + 1)}, {&x1, 16 * n},
+                            {&x2, 16 * n}, {&d1, 8 * n}, {&d2, 8 * n}, {&cams, 64 * (size_t)S}, {&models, sizeof(Model) * S},
+                            {&stats, sizeof(rp_stats) * S}, {&mask, n}});
+    }
+};
+// the remaining scratch
+struct ScratchBufs {
+    DevBuf order;     // quality calls: global sort scratch of pairs above RP_ORDER_SMEM_CAP
+    DevBuf gather_q;  // rp_gather_depths_batch_dev*_quality: the compacted quality between the two passes (4 B per row)
+    DevBuf tmp2;      // rp_refine_batch: bundle stats
+};
+
+// Device bytes per pair of an estimator chunk (the chunk planner's estimate; the reserves above are the exact sizes)
+size_t bytes_per_pair(int iters, long long avg_points, int ev_cap = EV, size_t input_bytes = 0) {
+    const int nseg = std::max(1, cdiv(iters, SEG));
+    const size_t slots_pp = (size_t)nseg * 4 * SEG;
+    // per slot: model, hyp_iter, score, count, ub, lb, survivor list, tensor-core count + list; per correspondence:
+    // FP64 / FP32 / interleaved copies, bearings, mask, 128-byte feature row, `input_bytes` of input staging
+    return slots_pp * (sizeof(Model) + 4 + 8 + 4 + 12 + 8) + (size_t)iters * 12 + (size_t)ev_cap * (sizeof(Model) + 24) +
+           (size_t)avg_points * (sizeof(Pt64) + 32 + sizeof(Bear) + 1 + 128 + input_bytes) + 1024;
+}
+
+// Device workspace of a refine chunk.  Per correspondence: pts64 (32 B), pts32 (16), the pair-interleaved FP32 copy
+// (16), bearings (48), and the chunk's I/O: FP64 inputs (48), subset (1), inlier mask (1); the host path double-buffers
+// the I/O and adds the float32 staging (24 B, double-buffered) for float32 inputs.  Per pair: PairParams, the work,
+// start and output models, bundle stats, cams, and a few counters.
+size_t refine_bytes_per_pair(long long avg_points, bool host_io, bool f32) {
+    const size_t io_pt = 48 + 1 + 1 + (host_io && f32 ? 24 : 0);
+    const size_t io_pair = 2 * sizeof(Model) + sizeof(rp_bundle_stats) + 64 + 8;
+    const size_t sets = host_io ? 2 : 1;
+    return (size_t)avg_points * (32 + 16 + 16 + 48 + sets * io_pt) + sizeof(PairParams) + sizeof(Model) + 32 +
+           sets * io_pair + 64;
+}
 
 // One double-buffer set of the chunk pipeline (stage_inputs / run_chunks): a chunk's inputs on their way in and its
 // outputs on their way out.  rp_ctx keeps two; on the host path chunk c uses set c & 1, the device path uses set 0 for
@@ -73,23 +190,15 @@ struct StageSet {
     void create_events() {
         for (cudaEvent_t *e : {&h2d_begin, &h2d_end, &in_ready, &done, &d2h_begin, &d2h_end}) cudaEventCreate(e);
     }
-    void release() {
-        for (DevBuf *b : {&x1, &x2, &d1, &d2, &cams, &sx1, &sx2, &sd1, &sd2, &qual, &offs, &perm, &ksort, &init, &subset,
-                          &models, &stats, &mask, &ninl})
-            b->release();
+    void destroy_events() {
         for (cudaEvent_t e : {h2d_begin, h2d_end, in_ready, done, d2h_begin, d2h_end}) cudaEventDestroy(e);
     }
 };
 
-// device scalars living in B_SCALARS
-struct Scalars {
-    int n_items, n_lo_items, n_one_items, n_prob, n_pairs_scalar, any_flag, reserved0, n_first_items;
-    int n_surv_items, bound_work, lm_work, score_work;  // *_work: counters the persistent kernels draw work from
-    unsigned long long point_scores, lm_iters, n_survivors, evaluated_ps;
-    long long n_hyp;
-    int n_tc_items, n_tcsel_items;
-    unsigned long long tc_evaluated, tc_selected, lm_flops;
-};
+// The minimal-model scoring: the exact head is HB models per pair; with the tensor-core tier a short head of
+// HEAD_SMALL models is followed by one mid stage over positions [HEAD_SMALL, MID_END) of the pair's first segment
+// (profiles/r02_head_sweep.txt, r02_mid_stage_sweep.txt)
+constexpr int HEAD_SMALL = 32, MID_END = 256;
 
 // run_chunk: [0..8] stage boundaries, [9] start of the bulk cascade, [10] bound kernel done, [11] tensor-core tier done;
 // [12], [13]: an interval of their own (the mask scatter of quality calls, rp_measure_pipes)
@@ -104,7 +213,14 @@ struct rp_ctx {
     int64_t launches = 0;
     cudaStream_t stream = nullptr;
     cudaStream_t copy_stream = nullptr;  // H2D of chunk c+1 / D2H of chunk c-1 overlap the kernels of chunk c
-    DevBuf buf[B_NBUF];
+    PointBufs pt;
+    HypBufs hyp;
+    LoBufs lo;
+    ResultBufs res;
+    PruneBufs prn;
+    TcBufs tcb;
+    SubBufs sub;
+    ScratchBufs scratch;
     StageSet set[2];
     cudaEvent_t ev[N_EVENTS];
     double last_ms[16] = {0};
@@ -113,20 +229,17 @@ struct rp_ctx {
     size_t workspace_budget = (size_t)80 << 30;  // HBM is 180 GB: big chunks amortise kernel tails and launches (10 000 pairs x 10 000
                                                  // iterations = one 71 GB chunk; measured 32 -> 80 GB: +3 %); capped at half of the free memory
     bool prune = true;  // hypothesis-level pruning (RP_NO_PRUNE=1 scores every minimal model exactly)
-    int head = HB;      // models per pair scored exactly before the bound kernel (RP_HEAD=32|64|96|128; measured: 128 best on cfg2/cfg4, 64 marginally better on the 1000-iteration configs)
     bool waves = true;  // survivors of the prune scored in waves (RP_NO_WAVES=1: all at once)
-    int lm_warp = 0xf;  // bit v: the LO refinements of variant v run one warp per LM problem (lm_warp_kernel) instead of one block
-                        // (RP_LM_WARP=mask; 0 = the block-per-problem kernel everywhere)
-    int head_small = 32;  // with the tensor-core tier: models per pair scored exactly up front (RP_HEAD_SMALL) ...
-    int mid_end = 256;    // ... and end of the mid stage that replaces the rest of the head (RP_MID_END; 0: no mid stage, head = RP_HEAD)
-    int mid_ends[4] = {256, 0, 0, 0}, n_mid = 1;   // RP_MID_END=a,b,..: several mid stages
+    bool lm_warp = true;  // the LO refinements run one warp per LM problem (lm_warp_kernel) instead of one block
+                          // (RP_LM_WARP=0: the block-per-problem kernel everywhere)
+    bool mid = true;    // with the tensor-core tier: short head + mid stage (RP_MID_END=0: the HB-model exact head)
     bool tc = true;     // tensor-core count tier in front of the FP32 bound kernel (RP_NO_TC=1: off)
-    int tc_two_pass = -115;    // that tier in two passes: < 0: the first pass covers -tc_two_pass % of the pair's abandonment threshold
-                               // (RP_TC_ADAPT_PCT); RP_TC_SPLIT=1..15: a fixed share in sixteenths; RP_TC_ONE_PASS=1: one pass over everything
+    bool tc_two_pass = true;  // that tier in two passes, split per pair by tc_split (RP_TC_ONE_PASS=1: one pass over everything)
+    bool solve_generic = false;  // RP_SOLVE_GENERIC: the thread-per-iteration solve kernel for every variant (the
+                                 // two-phase kernels must give bit-identical models)
     void *encode_tiled = nullptr;  // cuTensorMapEncodeTiled (driver entry point, resolved at rp_create)
     int ev_cap0 = EV;   // event-list capacity of the first pass (RP_EV_CAP: small values exercise the re-run path)
     std::vector<int32_t> pair_status;  // per pair of the last rp_estimate_batch_* call (rp_pair_status)
-    int occ_score[4] = {0}, occ_lm[4] = {0};
 };
 
 namespace {
@@ -148,8 +261,6 @@ namespace {
         ctx->launches++;                                                                             \
         CK(cudaGetLastError());                                                                      \
     } while (0)
-
-inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b); }
 
 int fail(rp_ctx *ctx, int code, const char *msg) {
     if (ctx) ctx->err = msg;
@@ -191,7 +302,7 @@ int occupancy_grid(rp_ctx *ctx, K kernel, int threads) {
 int launch_score(rp_ctx *ctx, bool pose, bool mask, const ScoreArgs &args, cudaStream_t st) {
     int grid;
     ScoreArgs a = args;
-    a.work_counter = &ctx->buf[B_SCALARS].as<Scalars>()->score_work;
+    a.work_counter = &ctx->pt.scalars.as<Scalars>()->score_work;
     CK(cudaMemsetAsync(a.work_counter, 0, sizeof(int), st));
     if (pose) {
         if (mask) { grid = occupancy_grid(ctx, score_kernel<true, true>, SCORE_THREADS); score_kernel<true, true><<<grid, SCORE_THREADS, 0, st>>>(a); }
@@ -212,40 +323,16 @@ int launch_bound(rp_ctx *ctx, bool pose, const BoundArgs &a, cudaStream_t st) {
     return RP_OK;
 }
 
-int launch_lm(rp_ctx *ctx, int variant, const LMArgs &a, long long expected_problems, cudaStream_t st) {
+// (counted by hand: launch_lm_kernel launches the one LM kernel it selects)
+int launch_lm(rp_ctx *ctx, int variant, const LMArgs &a, cudaStream_t st) {
     ctx->launches++;
-    (void)expected_problems;
     // problems differ in cost (1..max_iterations LM iterations): blocks draw them from a counter
     LMArgs la = a;
-    la.work_counter = &ctx->buf[B_SCALARS].as<Scalars>()->lm_work;
-    la.warp_kernel = (ctx->lm_warp >> variant) & 1;
-    la.warp_single = (ctx->lm_warp >> 4) & 1;
+    la.work_counter = &ctx->pt.scalars.as<Scalars>()->lm_work;
+    la.warp_kernel = ctx->lm_warp ? 1 : 0;
+    la.warp_single = 0;   // the final LO (one problem per pair, no problem list) stays on the block kernel
     CK(cudaMemsetAsync(la.work_counter, 0, sizeof(int), st));
     CK((cudaError_t)launch_lm_kernel(ctx->sms, variant, la, st));
-    return RP_OK;
-}
-
-int launch_solve(rp_ctx *ctx, int variant, const SolveArgs &a, int n_pairs, cudaStream_t st) {
-    dim3 grid(a.nseg, n_pairs);
-    // RP_SOLVE_GENERIC=1: the thread-per-iteration kernel for every variant (the two-phase kernels must give
-    // bit-identical models)
-    const bool generic = getenv("RP_SOLVE_GENERIC") != nullptr;
-    switch (variant) {
-    case RP_CALIB:
-        if (generic) solve_kernel<RP_CALIB><<<grid, SOLVE_THREADS, 0, st>>>(a);
-        else solve2_kernel<P3PCand><<<grid, SOLVE_THREADS, 0, st>>>(a);
-        break;
-    case RP_CALIB_SHIFT:
-        if (generic) solve_kernel<RP_CALIB_SHIFT><<<grid, SOLVE_THREADS, 0, st>>>(a);
-        else solve2_kernel<ShiftCand><<<grid, SOLVE_THREADS, 0, st>>>(a);
-        break;
-    case RP_SHARED:
-        if (generic) solve_kernel<RP_SHARED><<<grid, SOLVE_THREADS, 0, st>>>(a);
-        else solve2_kernel<FocalCand><<<grid, SOLVE_THREADS, 0, st>>>(a);
-        break;
-    default: solve_kernel<RP_VARYING><<<grid, SOLVE_THREADS, 0, st>>>(a); break;
-    }
-    LAUNCHED();
     return RP_OK;
 }
 
@@ -307,28 +394,21 @@ struct ChunkIO {
 int prepare_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io, cudaEvent_t ev_uploaded,
                   cudaStream_t st) {
     const int P = io.n_pairs;
-    const long long N = io.n_points;
-    DevBuf *B = ctx->buf;
-    CK(B[B_OFFS].reserve(sizeof(long long) * (P + 1)));
-    CK(B[B_PAIRS].reserve(sizeof(PairParams) * P));
-    CK(B[B_PTS64].reserve(sizeof(Pt64) * std::max<long long>(N, 1)));
-    CK(B[B_PTS32].reserve(sizeof(float4) * std::max<long long>(N, 1)));
-    CK(B[B_PTS32P].reserve(32 * (size_t)((N + P + 4) / 2 + 1)));
-    CK(B[B_BEAR].reserve(sizeof(Bear) * std::max<long long>(N, 1)));
-    CK(B[B_SCALARS].reserve(sizeof(Scalars)));
+    PointBufs &B = ctx->pt;
+    CK(B.reserve(P, io.n_points));
     Scalars h_sc;
     memset(&h_sc, 0, sizeof h_sc);
     h_sc.n_pairs_scalar = P;
-    CK(cudaMemcpyAsync(B[B_SCALARS].p, &h_sc, sizeof h_sc, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(B[B_OFFS].p, io.h_offsets_rel, sizeof(long long) * (P + 1), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(B.scalars.p, &h_sc, sizeof h_sc, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(B.offs.p, io.h_offsets_rel, sizeof(long long) * (P + 1), cudaMemcpyHostToDevice, st));
     if (ev_uploaded) CK(cudaEventRecord(ev_uploaded, st));
     PrepareArgs a;
-    a.variant = variant; a.n_pairs = P; a.offsets = B[B_OFFS].as<long long>();
+    a.variant = variant; a.n_pairs = P; a.offsets = B.offs.as<long long>();
     a.x1 = io.x1; a.x2 = io.x2; a.cams = io.cams;
     a.max_epipolar_error = opt.max_epipolar_error; a.max_reproj_error = opt.max_reproj_error;
     a.loss_scale = opt.loss_scale;
-    a.pts64 = B[B_PTS64].as<Pt64>(); a.pts32 = B[B_PTS32].as<float4>(); a.bear = B[B_BEAR].as<Bear>();
-    a.pairs = B[B_PAIRS].as<PairParams>(); a.pts32p = B[B_PTS32P].as<float>();
+    a.pts64 = B.pts64.as<Pt64>(); a.pts32 = B.pts32.as<float4>(); a.bear = B.bear.as<Bear>();
+    a.pairs = B.pairs.as<PairParams>(); a.pts32p = B.pts32p.as<float>();
     prepare_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(a);
     LAUNCHED();
     return RP_OK;
@@ -338,13 +418,13 @@ int prepare_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO
 // correspondences of `mask` (null: all of them), for the pairs `enable` marks
 LMArgs final_lm_args(rp_ctx *ctx, const rp_options &opt, const ChunkIO &io, Model *models, const unsigned char *mask,
                      const int *enable) {
-    DevBuf *B = ctx->buf;
+    const PointBufs &B = ctx->pt;
     LMArgs la;
     memset(&la, 0, sizeof la);
-    la.pairs = B[B_PAIRS].as<PairParams>(); la.pts64 = B[B_PTS64].as<Pt64>(); la.d1 = io.d1; la.d2 = io.d2;
+    la.pairs = B.pairs.as<PairParams>(); la.pts64 = B.pts64.as<Pt64>(); la.d1 = io.d1; la.d2 = io.d2;
     la.weight_sampson = opt.weight_sampson;
     la.loss_scale_override = -1.0; la.scale_reproj_override = -1.0;
-    la.prob_list = nullptr; la.n_prob = &B[B_SCALARS].as<Scalars>()->n_pairs_scalar; la.prob_per_pair = 1;
+    la.prob_list = nullptr; la.n_prob = &B.scalars.as<Scalars>()->n_pairs_scalar; la.prob_per_pair = 1;
     la.models = models; la.use_final = 1; la.mask = mask; la.enable = enable;
     la.max_iterations = (int)opt.bundle_max_iterations; la.loss_type = opt.loss_type;
     la.gradient_tol = opt.gradient_tol; la.step_tol = opt.step_tol; la.initial_lambda = opt.initial_lambda;
@@ -352,29 +432,36 @@ LMArgs final_lm_args(rp_ctx *ctx, const rp_options &opt, const ChunkIO &io, Mode
     return la;
 }
 
-// One work item per valid pair (B_ONES, B_ONEPFX, n_one_items): the list pair_score_args scores over.  run_chunk builds
+// One work item per valid pair (ones, one_prefix, n_one_items): the list pair_score_args scores over.  run_chunk builds
 // it once for the final LO's rescore and its get_inliers.
 int launch_pair_items(rp_ctx *ctx, int P, cudaStream_t st) {
-    DevBuf *B = ctx->buf;
-    valid_ones_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, B[B_PAIRS].as<PairParams>(), B[B_ONES].as<int>());
+    const ResultBufs &R = ctx->res;
+    valid_ones_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, ctx->pt.pairs.as<PairParams>(), R.ones.as<int>());
     LAUNCHED();
-    build_items_kernel<<<1, 1024, 0, st>>>(P, B[B_ONES].as<int>(), B[B_ONEPFX].as<int>(),
-                                           &B[B_SCALARS].as<Scalars>()->n_one_items, nullptr);
+    build_items_kernel<<<1, 1024, 0, st>>>(P, R.ones.as<int>(), R.one_prefix.as<int>(),
+                                           &ctx->pt.scalars.as<Scalars>()->n_one_items, nullptr);
     LAUNCHED();
     return RP_OK;
 }
 
-// score_kernel over one model per pair on the launch_pair_items list; score and count per pair go to B_FINSCORE /
-// B_FINCNT, the mask (with the mask variant) to `mask`
-ScoreArgs pair_score_args(rp_ctx *ctx, int P, const Model *models, unsigned char *mask) {
-    DevBuf *B = ctx->buf;
+// score_kernel's view of the chunk's pairs and correspondences; the caller fills in the models and the work items
+ScoreArgs chunk_score_args(const rp_ctx *ctx) {
     ScoreArgs s;
     memset(&s, 0, sizeof s);
-    s.n_groups = P; s.grp_stride = 1; s.grp_per_pair = 1; s.grp_cnt = B[B_ONES].as<int>();
-    s.item_prefix = B[B_ONEPFX].as<int>(); s.n_items = &B[B_SCALARS].as<Scalars>()->n_one_items;
-    s.pairs = B[B_PAIRS].as<PairParams>(); s.models = models;
-    s.pts32 = B[B_PTS32].as<float4>(); s.pts64 = B[B_PTS64].as<Pt64>(); s.bear = B[B_BEAR].as<Bear>();
-    s.score = B[B_FINSCORE].as<double>(); s.count = B[B_FINCNT].as<int>(); s.mask = mask;
+    s.pairs = ctx->pt.pairs.as<PairParams>();
+    s.pts32 = ctx->pt.pts32.as<float4>(); s.pts64 = ctx->pt.pts64.as<Pt64>(); s.bear = ctx->pt.bear.as<Bear>();
+    return s;
+}
+
+// score_kernel over one model per pair on the launch_pair_items list; score and count per pair go to final_score /
+// final_count, the mask (with the mask variant) to `mask`
+ScoreArgs pair_score_args(rp_ctx *ctx, int P, const Model *models, unsigned char *mask) {
+    const ResultBufs &R = ctx->res;
+    ScoreArgs s = chunk_score_args(ctx);
+    s.n_groups = P; s.grp_stride = 1; s.grp_per_pair = 1; s.grp_cnt = R.ones.as<int>();
+    s.item_prefix = R.one_prefix.as<int>(); s.n_items = &ctx->pt.scalars.as<Scalars>()->n_one_items;
+    s.models = models;
+    s.score = R.final_score.as<double>(); s.count = R.final_count.as<int>(); s.mask = mask;
     return s;
 }
 
@@ -385,358 +472,370 @@ int launch_get_inliers(rp_ctx *ctx, bool pose, const ChunkIO &io, const Model *m
     return launch_score(ctx, pose, true, pair_score_args(ctx, io.n_pairs, models, mask), st);
 }
 
-// One pass over a chunk.  `flags` (host, [n_pairs]) receives PAIR_FLAG_* per pair: a flagged pair's outputs are void and
-// the caller runs it again with a larger `ev_cap` / more iterations (estimate_impl).
-int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io, int iters, int ev_cap,
-              std::vector<int> &flags, cudaStream_t st) {
-    const int P = io.n_pairs;
-    const long long N = io.n_points;
-    const bool pose = variant == RP_CALIB || variant == RP_CALIB_SHIFT;
-    const int nseg = std::max(1, cdiv(iters, SEG));
-    const size_t slots_pp = (size_t)nseg * 4 * SEG;
-    const size_t slots = slots_pp * (size_t)P;
+// What the stages of one run_chunk call share, filled once after the reserves (rerun_flagged's nested run_chunk fills
+// its own)
+struct Chunk {
+    const rp_options *opt;
+    const ChunkIO *io;
+    int variant, P, iters, nseg, ev_cap;
+    bool pose, use_tc, mid;  // use_tc: the tensor-core tier (it needs the prune); mid: short head + mid stage (with that tier)
+    int head;                // with the prune: models per pair scored exactly up front
+    long long N;
+    size_t slots_pp;
+    cudaStream_t st;
+    // the device arrays the stages share
+    Scalars *sc;
+    PairParams *pairs;
+    Pt64 *pts64;
+    float4 *pts32;
+    Model *models;
+    double *score;
+    int *hyp_iter, *count, *seg_count, *item_prefix;
+};
 
-    DevBuf *B = ctx->buf;
-    CK(B[B_SAMPLES].reserve(sizeof(int) * 3 * (size_t)P * std::max(iters, 1)));
-    CK(B[B_MODELS].reserve(sizeof(Model) * slots));
-    CK(B[B_HYPITER].reserve(sizeof(int) * slots));
-    CK(B[B_SCORE].reserve(sizeof(double) * slots));
-    CK(B[B_COUNT].reserve(sizeof(int) * slots));
-    CK(B[B_SEGCNT].reserve(sizeof(int) * (size_t)P * nseg));
-    CK(B[B_ITEMPFX].reserve(sizeof(int) * ((size_t)P * nseg + 1)));
-    CK(B[B_EVENTS].reserve(sizeof(int) * (size_t)P * ev_cap));
-    CK(B[B_NEVENTS].reserve(sizeof(int) * P));
-    CK(B[B_LOMODELS].reserve(sizeof(Model) * (size_t)P * ev_cap));
-    CK(B[B_LOOFEV].reserve(sizeof(int) * (size_t)P * ev_cap));
-    CK(B[B_LOCOUNT].reserve(sizeof(int) * P));
-    CK(B[B_PROBLIST].reserve(sizeof(int) * (size_t)P * ev_cap));
-    CK(B[B_LOSCORE].reserve(sizeof(double) * (size_t)P * ev_cap));
-    CK(B[B_PAIRFLAGS].reserve(sizeof(int) * P));
-    CK(B[B_LOCNT].reserve(sizeof(int) * (size_t)P * ev_cap));
-    CK(B[B_LOITEMPFX].reserve(sizeof(int) * (P + 1)));
-    CK(B[B_BEST].reserve(sizeof(Model) * P));
-    CK(B[B_FINSTART].reserve(sizeof(Model) * P));
-    CK(B[B_FINSCORE].reserve(sizeof(double) * P));
-    CK(B[B_FINCNT].reserve(sizeof(int) * P));
-    CK(B[B_ONES].reserve(sizeof(int) * P));
-    CK(B[B_ONEPFX].reserve(sizeof(int) * (P + 1)));
-    CK(B[B_ENABLE].reserve(sizeof(int) * P));
-    CK(B[B_STATS].reserve(sizeof(rp_stats) * P));
-    if (ctx->prune) {
-        CK(B[B_UB].reserve(sizeof(int) * slots));
-        CK(B[B_LB].reserve(sizeof(float) * slots));
-        CK(B[B_SURVLIST].reserve(sizeof(int) * slots));
-        CK(B[B_FIRSTCNT].reserve(sizeof(int) * P));
-        CK(B[B_FIRSTPFX].reserve(sizeof(int) * (P + 1)));
-        CK(B[B_B0].reserve(sizeof(int) * P));
-        CK(B[B_S0].reserve(sizeof(double) * P));
-        CK(B[B_SURVCNT].reserve(sizeof(int) * P));
-        CK(B[B_WAVECUR].reserve(sizeof(int) * P)); CK(B[B_WAVECNT].reserve(sizeof(int) * P));
-        CK(B[B_SURVPFX].reserve(sizeof(int) * (P + 1)));
-    }
-    const bool use_tc = ctx->prune && ctx->tc;
-    if (use_tc) {
-        CK(B[B_FEAT].reserve(128 * (size_t)std::max<long long>(N, 1) + 128 * tc::NT));
-        CK(B[B_TCOUT].reserve(sizeof(int) * slots));
-        CK(B[B_TCLIST].reserve(sizeof(int) * slots));
-        CK(B[B_TCLISTCNT].reserve(sizeof(int) * P));
-        CK(B[B_TCLISTPFX].reserve(sizeof(int) * (P + 1)));
-        CK(B[B_PAIRCNT].reserve(sizeof(int) * P));
-        CK(B[B_TCSPLIT].reserve(sizeof(int) * P));
-        CK(B[B_TCPFX].reserve(sizeof(int) * (P + 1)));
-    }
+Chunk chunk_of(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io, int iters, int ev_cap,
+               cudaStream_t st) {
+    Chunk c;
+    c.opt = &opt; c.io = &io; c.variant = variant; c.pose = variant == RP_CALIB || variant == RP_CALIB_SHIFT;
+    c.use_tc = ctx->prune && ctx->tc; c.mid = c.use_tc && ctx->mid; c.head = c.mid ? HEAD_SMALL : HB;
+    c.P = io.n_pairs; c.N = io.n_points; c.iters = iters; c.nseg = std::max(1, cdiv(iters, SEG)); c.ev_cap = ev_cap;
+    c.slots_pp = (size_t)c.nseg * 4 * SEG; c.st = st;
+    c.sc = ctx->pt.scalars.as<Scalars>(); c.pairs = ctx->pt.pairs.as<PairParams>(); c.pts64 = ctx->pt.pts64.as<Pt64>();
+    c.pts32 = ctx->pt.pts32.as<float4>();
+    c.models = ctx->hyp.models.as<Model>(); c.hyp_iter = ctx->hyp.hyp_iter.as<int>(); c.score = ctx->hyp.score.as<double>();
+    c.count = ctx->hyp.count.as<int>(); c.seg_count = ctx->hyp.seg_count.as<int>();
+    c.item_prefix = ctx->hyp.item_prefix.as<int>();
+    return c;
+}
 
-    cudaEvent_t *ev = ctx->ev;
-    // 1. prepare, and the tensor-core tier's feature rows
-    int rc = prepare_chunk(ctx, variant, opt, io, ev[0], st);
-    if (rc) return rc;
-    Scalars *sc = B[B_SCALARS].as<Scalars>();
-    PairParams *pairs = B[B_PAIRS].as<PairParams>();
-    Pt64 *pts64 = B[B_PTS64].as<Pt64>();
-    float4 *pts32 = B[B_PTS32].as<float4>();
-    Bear *bear = B[B_BEAR].as<Bear>();
-    int *samples = B[B_SAMPLES].as<int>();
-    Model *models = B[B_MODELS].as<Model>();
-    int *hyp_iter = B[B_HYPITER].as<int>();
-    double *score = B[B_SCORE].as<double>();
-    int *count = B[B_COUNT].as<int>();
-    int *seg_count = B[B_SEGCNT].as<int>();
-    int *item_prefix = B[B_ITEMPFX].as<int>();
-    if (use_tc && N > 0) {
-        tc::tc_features_kernel<<<cdiv(N, 256), 256, 0, st>>>(N, pts32, B[B_FEAT].as<float4>());
-        LAUNCHED();
-    }
-    CK(cudaEventRecord(ev[1], st));
-    // 2. sample
-    if (iters > 0) {
-        if (opt.progressive_sampling)
-            sample_prosac_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(
-                P, iters, pairs, opt.seed, (unsigned long long)std::max<int64_t>(opt.max_prosac_iterations, 0), samples);
-        else
-            sample_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(P, iters, pairs, opt.seed, samples);
-        LAUNCHED();
-    }
-    CK(cudaEventRecord(ev[2], st));
-    // 3. solve
-    {
-        SolveArgs a;
-        a.variant = variant; a.iters = iters; a.nseg = nseg; a.pairs = pairs; a.samples = samples;
-        a.pts64 = pts64; a.d1 = io.d1; a.d2 = io.d2; a.models = models; a.hyp_iter = hyp_iter; a.seg_count = seg_count;
-        rc = launch_solve(ctx, variant, a, P, st);
-        if (rc) return rc;
-    }
-    CK(cudaEventRecord(ev[3], st));
-    // 4. score the minimal models
-    ScoreArgs sa;
-    sa.pairs = pairs; sa.pts32 = pts32; sa.pts64 = pts64; sa.bear = bear; sa.mask = nullptr;
-    sa.slot_list = nullptr; sa.list_stride = 0;
-    build_items_kernel<<<1, 1024, 0, st>>>(P * nseg, seg_count, item_prefix, &sc->n_items, &sc->n_hyp);
+// 2. sample
+int sample_stage(rp_ctx *ctx, const Chunk &c) {
+    if (c.iters <= 0) return RP_OK;
+    const rp_options &opt = *c.opt;
+    int *samples = ctx->hyp.samples.as<int>();
+    if (opt.progressive_sampling)
+        sample_prosac_kernel<<<cdiv((long long)c.P * 32, 256), 256, 0, c.st>>>(
+            c.P, c.iters, c.pairs, opt.seed, (unsigned long long)std::max<int64_t>(opt.max_prosac_iterations, 0), samples);
+    else
+        sample_kernel<<<cdiv((long long)c.P * 32, 256), 256, 0, c.st>>>(c.P, c.iters, c.pairs, opt.seed, samples);
     LAUNCHED();
+    return RP_OK;
+}
+
+// 3. solve: the two-phase kernel of the variant, or with RP_SOLVE_GENERIC the thread-per-iteration kernel (the one
+// RP_VARYING always runs)
+int solve_stage(rp_ctx *ctx, const Chunk &c) {
+    SolveArgs a;
+    a.variant = c.variant; a.iters = c.iters; a.nseg = c.nseg; a.pairs = c.pairs; a.samples = ctx->hyp.samples.as<int>();
+    a.pts64 = c.pts64; a.d1 = c.io->d1; a.d2 = c.io->d2; a.models = c.models; a.hyp_iter = c.hyp_iter; a.seg_count = c.seg_count;
+    const dim3 grid(c.nseg, c.P);
+    const bool generic = ctx->solve_generic;
+    cudaStream_t st = c.st;
+    switch (c.variant) {
+    case RP_CALIB:
+        if (generic) solve_kernel<RP_CALIB><<<grid, SOLVE_THREADS, 0, st>>>(a);
+        else solve2_kernel<P3PCand><<<grid, SOLVE_THREADS, 0, st>>>(a);
+        break;
+    case RP_CALIB_SHIFT:
+        if (generic) solve_kernel<RP_CALIB_SHIFT><<<grid, SOLVE_THREADS, 0, st>>>(a);
+        else solve2_kernel<ShiftCand><<<grid, SOLVE_THREADS, 0, st>>>(a);
+        break;
+    case RP_SHARED:
+        if (generic) solve_kernel<RP_SHARED><<<grid, SOLVE_THREADS, 0, st>>>(a);
+        else solve2_kernel<FocalCand><<<grid, SOLVE_THREADS, 0, st>>>(a);
+        break;
+    default: solve_kernel<RP_VARYING><<<grid, SOLVE_THREADS, 0, st>>>(a); break;
+    }
+    LAUNCHED();
+    return RP_OK;
+}
+
+// The tensor-core tier over the models at positions [start, limit) of the first segment (limit > 0) or [start, end) of
+// the pair (limit = 0): pass 0 counts every model of the range against the first part of its pair's correspondences
+// (with `two_pass`; all of them otherwise) and tc_select_kernel drops what already has enough certain outliers; pass 1
+// counts the remaining correspondences for the models that are left and tc_select_list_kernel decides again.  The
+// models it passes on are the per-pair lists (list, list_cnt, list_prefix, n_tcsel_items) of the bound kernel.
+// `ev_tc`, if given, is recorded when the tier is done.
+int tc_tier(rp_ctx *ctx, const Chunk &c, int start, int limit, bool two_pass, cudaEvent_t ev_tc) {
+    const int P = c.P;
+    cudaStream_t st = c.st;
+    Scalars *sc = c.sc;
+    const TcBufs &T = ctx->tcb;
+    const PruneBufs &W = ctx->prn;
+    range_count_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, c.nseg, c.seg_count, start, limit, T.pair_cnt.as<int>());
+    LAUNCHED();
+    build_items_kernel<<<1, 1024, 0, st>>>(P, T.pair_cnt.as<int>(), T.prefix.as<int>(), &sc->n_tc_items, nullptr, tc::TILE_MODELS);
+    LAUNCHED();
+    tc::TcArgs ta;
+    memset(&ta, 0, sizeof ta);
+    ta.n_pairs = P; ta.nseg = c.nseg; ta.pairs = c.pairs; ta.seg_count = c.seg_count; ta.item_prefix = T.prefix.as<int>();
+    ta.n_items = &sc->n_tc_items; ta.models = c.models; ta.out = T.out.as<int>(); ta.pose = c.pose ? 1 : 0;
+    ta.evaluated = &sc->tc_evaluated; ta.first = start;
+    ta.two_pass = two_pass ? 1 : 0; ta.pass = 0; ta.split = T.split.as<int>();
+    if (two_pass) {
+        tc::tc_split_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, c.pairs, W.B0.as<int>(), W.S0.as<double>(), T.split.as<int>());
+        LAUNCHED();
+    }
+    int rc = launch_tc(ctx, ta, T.feat.as<float4>(), c.N, st);
+    if (rc) return rc;
+    TcSelectArgs sel;
+    sel.n_pairs = P; sel.nseg = c.nseg; sel.head = start; sel.limit = limit; sel.pairs = c.pairs; sel.seg_count = c.seg_count;
+    sel.out = T.out.as<int>(); sel.B0 = W.B0.as<int>(); sel.S0 = W.S0.as<double>(); sel.ub = W.ub.as<int>();
+    sel.lb = W.lb.as<float>(); sel.list = T.list.as<int>(); sel.list_cnt = T.list_cnt.as<int>();
+    sel.n_selected = two_pass ? nullptr : &sc->tc_selected;
+    tc_select_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(sel);
+    LAUNCHED();
+    if (two_pass) {
+        build_items_kernel<<<1, 1024, 0, st>>>(P, T.list_cnt.as<int>(), T.prefix.as<int>(), &sc->n_tc_items, nullptr, tc::TILE_MODELS);
+        LAUNCHED();
+        ta.pass = 1; ta.first = 0; ta.list = T.list.as<int>(); ta.list_cnt = T.list_cnt.as<int>(); ta.list_stride = (int)c.slots_pp;
+        rc = launch_tc(ctx, ta, T.feat.as<float4>(), c.N, st);
+        if (rc) return rc;
+        sel.n_selected = &sc->tc_selected;
+        tc_select_list_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(sel);
+        LAUNCHED();
+    }
+    if (ev_tc) CK(cudaEventRecord(ev_tc, st));
+    build_items_kernel<<<1, 1024, 0, st>>>(P, T.list_cnt.as<int>(), T.list_prefix.as<int>(), &sc->n_tcsel_items, nullptr);
+    LAUNCHED();
+    return RP_OK;
+}
+
+// The survivors of the prune scored exactly, all at once (RP_NO_WAVES=1: the check that the waves change nothing).
+// `fold`: a later stage follows, so these exact results are folded into (B0, S0).
+int score_survivors_at_once(rp_ctx *ctx, const Chunk &c, ScoreArgs sv, WaveArgs wa, bool fold) {
+    build_items_kernel<<<1, 1024, 0, c.st>>>(c.P, wa.surv_cnt, ctx->prn.surv_prefix.as<int>(), &c.sc->n_surv_items, nullptr);
+    LAUNCHED();
+    sv.grp_cnt = wa.surv_cnt;
+    int rc = launch_score(ctx, c.pose, false, sv, c.st);
+    if (rc) return rc;
+    if (fold) {
+        CK(cudaMemsetAsync(wa.cursor, 0, sizeof(int) * c.P, c.st));
+        CK(cudaMemcpyAsync(wa.wave_cnt, wa.surv_cnt, sizeof(int) * c.P, cudaMemcpyDeviceToDevice, c.st));
+        wa.wave_size = 0; wa.first = 0; wa.n_exact = nullptr;
+        wave_select_kernel<<<cdiv((long long)c.P * 32, 256), 256, 0, c.st>>>(wa);
+        LAUNCHED();
+    }
+    return RP_OK;
+}
+
+// The survivors of the prune scored exactly in waves of growing size, each raising the bar for the next
+// (wave_select_kernel).  `fold`: a later stage follows, so the last wave's exact results are folded into (B0, S0).
+int score_survivors_in_waves(rp_ctx *ctx, const Chunk &c, ScoreArgs sv, WaveArgs wa, bool fold) {
+    CK(cudaMemsetAsync(wa.cursor, 0, sizeof(int) * c.P, c.st));
+    static const int WAVES[] = {8, 16, 32, 64, 0x7fffffff};
+    for (int k = 0; k < 5; ++k) {
+        wa.wave_size = WAVES[k]; wa.first = k == 0;
+        wave_select_kernel<<<cdiv((long long)c.P * 32, 256), 256, 0, c.st>>>(wa);
+        LAUNCHED();
+        build_items_kernel<<<1, 1024, 0, c.st>>>(c.P, wa.wave_cnt, ctx->prn.surv_prefix.as<int>(), &c.sc->n_surv_items, nullptr);
+        LAUNCHED();
+        sv.grp_cnt = wa.wave_cnt;
+        int rc = launch_score(ctx, c.pose, false, sv, c.st);
+        if (rc) return rc;
+    }
+    if (fold) {
+        wa.wave_size = 0; wa.first = 0; wa.n_exact = nullptr;
+        wave_select_kernel<<<cdiv((long long)c.P * 32, 256), 256, 0, c.st>>>(wa);
+        LAUNCHED();
+    }
+    return RP_OK;
+}
+
+// 4b / 4c for the models at positions [start, limit) of the first segment (limit > 0: the mid stage) or [start, end) of
+// the pair (limit = 0: the bulk): tensor-core tier (with the tier on), FP32 bound kernel over what that tier could not
+// drop, prune, exact scoring of the survivors.  (B0, S0) are raised in place.  `ev_bound`, if given, is recorded when
+// the bound kernel is done.
+int cascade(rp_ctx *ctx, const Chunk &c, int start, int limit, bool two_pass, cudaEvent_t ev_tc, cudaEvent_t ev_bound) {
+    const int P = c.P;
+    const int stride = (int)c.slots_pp;
+    cudaStream_t st = c.st;
+    Scalars *sc = c.sc;
+    const PruneBufs &W = ctx->prn;
+    const TcBufs &T = ctx->tcb;
+    BoundArgs ba;
+    ba.n_groups = P * c.nseg; ba.grp_stride = 4 * SEG; ba.grp_per_pair = c.nseg; ba.grp_cnt = c.seg_count;
+    ba.item_prefix = c.item_prefix; ba.n_items = &sc->n_items; ba.pairs = c.pairs; ba.models = c.models;
+    ba.pts32p = ctx->pt.pts32p.as<ulonglong2>();
+    ba.ub = W.ub.as<int>(); ba.lb = W.lb.as<float>(); ba.point_scores = &sc->point_scores;
+    ba.B0 = W.B0.as<int>(); ba.S0 = W.S0.as<double>();
+    ba.evaluated = &sc->evaluated_ps;
+    ba.work_counter = &sc->bound_work; ba.head = start;
+    ba.slot_list = nullptr; ba.list_stride = 0;
+    int rc;
+    if (c.use_tc) {
+        if ((rc = tc_tier(ctx, c, start, limit, two_pass, ev_tc))) return rc;
+        ba.n_groups = P; ba.grp_stride = stride; ba.grp_per_pair = 1; ba.grp_cnt = T.list_cnt.as<int>();
+        ba.item_prefix = T.list_prefix.as<int>(); ba.n_items = &sc->n_tcsel_items;
+        ba.slot_list = T.list.as<int>(); ba.list_stride = stride;
+    }
+    if ((rc = launch_bound(ctx, c.pose, ba, st))) return rc;
+    if (ev_bound) CK(cudaEventRecord(ev_bound, st));
+    // prune, then score the survivors exactly
+    PruneArgs pa;
+    pa.n_pairs = P; pa.nseg = c.nseg; pa.seg_count = c.seg_count; pa.ub = ba.ub; pa.lb = ba.lb;
+    pa.B0 = ba.B0; pa.S0 = ba.S0; pa.score = c.score; pa.count = c.count; pa.head = start; pa.limit = limit;
+    pa.surv_list = W.surv_list.as<int>(); pa.surv_cnt = W.surv_cnt.as<int>();
+    pa.n_survivors = ctx->waves ? nullptr : &sc->n_survivors;
+    prune_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(pa);
+    LAUNCHED();
+    ScoreArgs sv = chunk_score_args(ctx);
+    sv.n_groups = P; sv.grp_stride = stride; sv.grp_per_pair = 1; sv.models = c.models; sv.score = c.score; sv.count = c.count;
+    sv.item_prefix = W.surv_prefix.as<int>(); sv.n_items = &sc->n_surv_items;
+    sv.slot_list = pa.surv_list; sv.list_stride = stride;
+    WaveArgs wa;
+    wa.n_pairs = P; wa.slots_pp = c.slots_pp; wa.surv_list = pa.surv_list; wa.surv_cnt = pa.surv_cnt;
+    wa.cursor = W.wave_cursor.as<int>(); wa.wave_cnt = W.wave_cnt.as<int>(); wa.ub = ba.ub; wa.lb = ba.lb;
+    wa.B = W.B0.as<int>(); wa.S = W.S0.as<double>(); wa.score = c.score; wa.count = c.count;
+    wa.n_exact = &sc->n_survivors;
+    return ctx->waves ? score_survivors_in_waves(ctx, c, sv, wa, limit != 0)
+                      : score_survivors_at_once(ctx, c, sv, wa, limit != 0);
+}
+
+// 4. score the minimal models: all of them exactly (RP_NO_PRUNE=1), or the first c.head models of every pair exactly
+// -> (B0, S0), then with the mid stage the models at positions [HEAD_SMALL, MID_END) of the pair's first segment
+// through the same cascade as the bulk (one tensor-core pass, FP32 bound, prune, exact waves) against the short head's
+// bar, which leaves (B0, S0) = the exact best of everything before MID_END for the bulk at a fraction of the cost of
+// scoring a long head exactly; then the bulk.  ev[9] starts the bulk, ev[10] marks its bound kernel done, ev[11] its
+// tensor-core tier.
+int score_minimal(rp_ctx *ctx, const Chunk &c) {
+    const int P = c.P;
+    cudaStream_t st = c.st;
+    Scalars *sc = c.sc;
+    build_items_kernel<<<1, 1024, 0, st>>>(P * c.nseg, c.seg_count, c.item_prefix, &sc->n_items, &sc->n_hyp);
+    LAUNCHED();
+    ScoreArgs sa = chunk_score_args(ctx);
+    sa.models = c.models; sa.score = c.score; sa.count = c.count; sa.point_scores = &sc->point_scores;
     if (!ctx->prune) {
-        sa.n_groups = P * nseg; sa.grp_stride = 4 * SEG; sa.grp_per_pair = nseg; sa.grp_cnt = seg_count;
-        sa.item_prefix = item_prefix; sa.n_items = &sc->n_items; sa.models = models; sa.score = score; sa.count = count;
-        sa.point_scores = &sc->point_scores;
-        rc = launch_score(ctx, pose, false, sa, st);
-        if (rc) return rc;
-    } else {
-        // 4a. the first `head` models of every pair, exactly -> (B0, S0)
-        // With the tensor-core tier a short head (ctx->head_small) is followed by a MID stage: the models at positions
-        // [head_small, mid_end) of the pair's first segment go through the same cascade as the bulk (one tensor-core
-        // pass, FP32 bound, prune, exact waves) against the short head's bar, which leaves (B0, S0) = the exact best of
-        // everything before mid_end for the bulk at a fraction of the cost of scoring a long head exactly.
-        const bool mid = use_tc && ctx->mid_end > ctx->head_small && ctx->mid_end > 0;
-        const int head = mid ? ctx->head_small : ctx->head;
-        int *first_cnt = B[B_FIRSTCNT].as<int>();
-        first_count_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, nseg, seg_count, first_cnt, head);
-        LAUNCHED();
-        build_items_kernel<<<1, 1024, 0, st>>>(P, first_cnt, B[B_FIRSTPFX].as<int>(), &sc->n_first_items, nullptr);
-        LAUNCHED();
-        sa.n_groups = P; sa.grp_stride = (int)slots_pp; sa.grp_per_pair = 1; sa.grp_cnt = first_cnt;
-        sa.item_prefix = B[B_FIRSTPFX].as<int>(); sa.n_items = &sc->n_first_items; sa.models = models;
-        sa.score = score; sa.count = count; sa.point_scores = &sc->point_scores;
-        rc = launch_score(ctx, pose, false, sa, st);
-        if (rc) return rc;
-        pair_bounds_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(P, nseg, first_cnt, score, count,
-                                                                       B[B_B0].as<int>(), B[B_S0].as<double>());
-        LAUNCHED();
-        // 4b/4c for the models at positions [start, limit) of the first segment (limit > 0) or [start, end) of the pair
-        // (limit = 0): tensor-core tier (certain-outlier counts, rp_tc.cuh), FP32 bound kernel over what that tier could
-        // not drop, prune, exact scoring of the survivors in bar-raising waves.  (B0, S0) are raised in place.
-        auto cascade = [&](int start, int limit, int two_pass, cudaEvent_t ev_tc, cudaEvent_t ev_bound) -> int {
-            BoundArgs ba;
-            ba.n_groups = P * nseg; ba.grp_stride = 4 * SEG; ba.grp_per_pair = nseg; ba.grp_cnt = seg_count;
-            ba.item_prefix = item_prefix; ba.n_items = &sc->n_items; ba.pairs = pairs; ba.models = models; ba.pts32p = B[B_PTS32P].as<ulonglong2>();
-            ba.ub = B[B_UB].as<int>(); ba.lb = B[B_LB].as<float>(); ba.point_scores = &sc->point_scores;
-            ba.B0 = B[B_B0].as<int>(); ba.S0 = B[B_S0].as<double>();
-            ba.evaluated = &sc->evaluated_ps;
-            ba.work_counter = &sc->bound_work; ba.head = start;
-            ba.slot_list = nullptr; ba.list_stride = 0;
-            if (use_tc) {
-                range_count_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, nseg, seg_count, start, limit, B[B_PAIRCNT].as<int>());
-                LAUNCHED();
-                build_items_kernel<<<1, 1024, 0, st>>>(P, B[B_PAIRCNT].as<int>(), B[B_TCPFX].as<int>(), &sc->n_tc_items, nullptr, tc::TILE_MODELS);
-                LAUNCHED();
-                // pass 0: every model of the range against the first part of its pair's correspondences (or all of them)
-                tc::TcArgs ta;
-                memset(&ta, 0, sizeof ta);
-                ta.n_pairs = P; ta.nseg = nseg; ta.pairs = pairs; ta.seg_count = seg_count; ta.item_prefix = B[B_TCPFX].as<int>();
-                ta.n_items = &sc->n_tc_items; ta.models = models; ta.out = B[B_TCOUT].as<int>(); ta.pose = pose ? 1 : 0;
-                ta.evaluated = &sc->tc_evaluated; ta.first = start;
-                ta.two_pass = two_pass; ta.pass = 0; ta.split = B[B_TCSPLIT].as<int>();
-                if (two_pass) {
-                    tc::tc_split_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, pairs, ba.B0, ba.S0, two_pass, B[B_TCSPLIT].as<int>());
-                    LAUNCHED();
-                }
-                int rc = launch_tc(ctx, ta, B[B_FEAT].as<float4>(), N, st);
-                if (rc) return rc;
-                TcSelectArgs sel;
-                sel.n_pairs = P; sel.nseg = nseg; sel.head = start; sel.limit = limit; sel.pairs = pairs; sel.seg_count = seg_count;
-                sel.out = B[B_TCOUT].as<int>(); sel.B0 = ba.B0; sel.S0 = ba.S0; sel.ub = ba.ub; sel.lb = ba.lb;
-                sel.list = B[B_TCLIST].as<int>(); sel.list_cnt = B[B_TCLISTCNT].as<int>();
-                sel.n_selected = two_pass ? nullptr : &sc->tc_selected;
-                tc_select_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(sel);
-                LAUNCHED();
-                if (two_pass) {
-                    // pass 1: the remaining correspondences, only for the models that are not yet certain to be pruned
-                    build_items_kernel<<<1, 1024, 0, st>>>(P, B[B_TCLISTCNT].as<int>(), B[B_TCPFX].as<int>(), &sc->n_tc_items, nullptr, tc::TILE_MODELS);
-                    LAUNCHED();
-                    ta.pass = 1; ta.first = 0; ta.list = B[B_TCLIST].as<int>(); ta.list_cnt = B[B_TCLISTCNT].as<int>(); ta.list_stride = (int)slots_pp;
-                    rc = launch_tc(ctx, ta, B[B_FEAT].as<float4>(), N, st);
-                    if (rc) return rc;
-                    sel.n_selected = &sc->tc_selected;
-                    tc_select_list_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(sel);
-                    LAUNCHED();
-                }
-                if (ev_tc) CK(cudaEventRecord(ev_tc, st));
-                build_items_kernel<<<1, 1024, 0, st>>>(P, B[B_TCLISTCNT].as<int>(), B[B_TCLISTPFX].as<int>(), &sc->n_tcsel_items, nullptr);
-                LAUNCHED();
-                ba.n_groups = P; ba.grp_stride = (int)slots_pp; ba.grp_per_pair = 1; ba.grp_cnt = B[B_TCLISTCNT].as<int>();
-                ba.item_prefix = B[B_TCLISTPFX].as<int>(); ba.n_items = &sc->n_tcsel_items;
-                ba.slot_list = B[B_TCLIST].as<int>(); ba.list_stride = (int)slots_pp;
-            }
-            int rc = launch_bound(ctx, pose, ba, st);
-            if (rc) return rc;
-            if (ev_bound) CK(cudaEventRecord(ev_bound, st));
-            // prune, then score the survivors exactly
-            PruneArgs pa;
-            pa.n_pairs = P; pa.nseg = nseg; pa.seg_count = seg_count; pa.ub = ba.ub; pa.lb = ba.lb;
-            pa.B0 = B[B_B0].as<int>(); pa.S0 = B[B_S0].as<double>(); pa.score = score; pa.count = count; pa.head = start; pa.limit = limit;
-            pa.surv_list = B[B_SURVLIST].as<int>(); pa.surv_cnt = B[B_SURVCNT].as<int>();
-            pa.n_survivors = ctx->waves ? nullptr : &sc->n_survivors;
-            prune_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(pa);
-            LAUNCHED();
-            ScoreArgs sv = sa;
-            sv.item_prefix = B[B_SURVPFX].as<int>(); sv.n_items = &sc->n_surv_items;
-            sv.slot_list = pa.surv_list; sv.list_stride = (int)slots_pp; sv.point_scores = nullptr;
-            WaveArgs wa;
-            wa.n_pairs = P; wa.slots_pp = slots_pp; wa.surv_list = pa.surv_list; wa.surv_cnt = pa.surv_cnt;
-            wa.cursor = B[B_WAVECUR].as<int>(); wa.wave_cnt = B[B_WAVECNT].as<int>(); wa.ub = ba.ub; wa.lb = ba.lb;
-            wa.B = B[B_B0].as<int>(); wa.S = B[B_S0].as<double>(); wa.score = score; wa.count = count;
-            wa.n_exact = &sc->n_survivors;
-            if (!ctx->waves) {
-                // all survivors at once (RP_NO_WAVES=1: the check that the waves below change nothing)
-                build_items_kernel<<<1, 1024, 0, st>>>(P, pa.surv_cnt, B[B_SURVPFX].as<int>(), &sc->n_surv_items, nullptr);
-                LAUNCHED();
-                sv.grp_cnt = pa.surv_cnt;
-                rc = launch_score(ctx, pose, false, sv, st);
-                if (rc) return rc;
-                if (limit) {
-                    // a later stage follows: fold these exact results into (B0, S0)
-                    CK(cudaMemsetAsync(wa.cursor, 0, sizeof(int) * P, st));
-                    CK(cudaMemcpyAsync(wa.wave_cnt, pa.surv_cnt, sizeof(int) * P, cudaMemcpyDeviceToDevice, st));
-                    wa.wave_size = 0; wa.first = 0; wa.n_exact = nullptr;
-                    wave_select_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(wa);
-                    LAUNCHED();
-                }
-            } else {
-                // survivors in waves of growing size, each raising the bar for the next (wave_select_kernel)
-                CK(cudaMemsetAsync(wa.cursor, 0, sizeof(int) * P, st));
-                static const int WAVES[] = {8, 16, 32, 64, 0x7fffffff};
-                for (int k = 0; k < 5; ++k) {
-                    wa.wave_size = WAVES[k]; wa.first = k == 0;
-                    wave_select_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(wa);
-                    LAUNCHED();
-                    build_items_kernel<<<1, 1024, 0, st>>>(P, wa.wave_cnt, B[B_SURVPFX].as<int>(), &sc->n_surv_items, nullptr);
-                    LAUNCHED();
-                    sv.grp_cnt = wa.wave_cnt;
-                    rc = launch_score(ctx, pose, false, sv, st);
-                    if (rc) return rc;
-                }
-                if (limit) {
-                    // a later stage follows: fold the last wave's exact results into (B0, S0)
-                    wa.wave_size = 0; wa.first = 0; wa.n_exact = nullptr;
-                    wave_select_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(wa);
-                    LAUNCHED();
-                }
-            }
-            return RP_OK;
-        };
-        int from = head;
-        if (mid) {
-            // (RP_MID_END=a,b,..: several mid stages, each against the bar the previous one left)
-            for (int k = 0; k < ctx->n_mid; ++k) {
-                if (ctx->mid_ends[k] <= from) continue;
-                rc = cascade(from, ctx->mid_ends[k], 0, nullptr, nullptr);
-                if (rc) return rc;
-                from = ctx->mid_ends[k];
-            }
-        }
-        CK(cudaEventRecord(ev[9], st));
-        rc = cascade(from, 0, ctx->tc_two_pass, use_tc ? ev[11] : nullptr, ev[10]);
-        if (rc) return rc;
+        sa.n_groups = P * c.nseg; sa.grp_stride = 4 * SEG; sa.grp_per_pair = c.nseg; sa.grp_cnt = c.seg_count;
+        sa.item_prefix = c.item_prefix; sa.n_items = &sc->n_items;
+        return launch_score(ctx, c.pose, false, sa, st);
     }
-    CK(cudaEventRecord(ev[4], st));
-    // 5. scan + LO problem list
-    {
-        ScanArgs a;
-        a.n_pairs = P; a.nseg = nseg; a.seg_count = seg_count; a.score = score; a.count = count;
-        a.events = B[B_EVENTS].as<int>(); a.n_events = B[B_NEVENTS].as<int>(); a.ev_cap = ev_cap;
-        a.pair_flags = B[B_PAIRFLAGS].as<int>(); a.any_flag = &sc->any_flag;
-        scan_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(a);
-        LAUNCHED();
-        LoPrepArgs l;
-        l.n_pairs = P; l.nseg = nseg; l.events = a.events; l.n_events = a.n_events; l.hyp_iter = hyp_iter; l.ev_cap = ev_cap;
-        l.models = models; l.lo_models = B[B_LOMODELS].as<Model>(); l.lo_of_event = B[B_LOOFEV].as<int>();
-        l.lo_count = B[B_LOCOUNT].as<int>(); l.prob_list = B[B_PROBLIST].as<int>(); l.n_prob = &sc->n_prob;
-        lo_prepare_kernel<<<cdiv(P, 128), 128, 0, st>>>(l);
-        LAUNCHED();
-    }
-    CK(cudaEventRecord(ev[5], st));
-    // 6. LO refinement of every trigger (independent problems)
+    // 4a. the exact head
+    const PruneBufs &W = ctx->prn;
+    int *first_cnt = W.first_cnt.as<int>();
+    first_count_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, c.nseg, c.seg_count, first_cnt, c.head);
+    LAUNCHED();
+    build_items_kernel<<<1, 1024, 0, st>>>(P, first_cnt, W.first_prefix.as<int>(), &sc->n_first_items, nullptr);
+    LAUNCHED();
+    sa.n_groups = P; sa.grp_stride = (int)c.slots_pp; sa.grp_per_pair = 1; sa.grp_cnt = first_cnt;
+    sa.item_prefix = W.first_prefix.as<int>(); sa.n_items = &sc->n_first_items;
+    int rc = launch_score(ctx, c.pose, false, sa, st);
+    if (rc) return rc;
+    pair_bounds_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(P, c.nseg, first_cnt, c.score, c.count,
+                                                                   W.B0.as<int>(), W.S0.as<double>());
+    LAUNCHED();
+    // 4b. the mid stage, 4c. the bulk
+    if (c.mid && (rc = cascade(ctx, c, HEAD_SMALL, MID_END, false, nullptr, nullptr))) return rc;
+    CK(cudaEventRecord(ctx->ev[9], st));
+    return cascade(ctx, c, c.mid ? MID_END : c.head, 0, ctx->tc_two_pass, c.use_tc ? ctx->ev[11] : nullptr, ctx->ev[10]);
+}
+
+// 5. scan for the trigger events, and the LO problem list
+int scan_stage(rp_ctx *ctx, const Chunk &c) {
+    const LoBufs &L = ctx->lo;
+    ScanArgs a;
+    a.n_pairs = c.P; a.nseg = c.nseg; a.seg_count = c.seg_count; a.score = c.score; a.count = c.count;
+    a.events = L.events.as<int>(); a.n_events = L.n_events.as<int>(); a.ev_cap = c.ev_cap;
+    a.pair_flags = L.pair_flags.as<int>(); a.any_flag = &c.sc->any_flag;
+    scan_kernel<<<cdiv((long long)c.P * 32, 256), 256, 0, c.st>>>(a);
+    LAUNCHED();
+    LoPrepArgs l;
+    l.n_pairs = c.P; l.nseg = c.nseg; l.events = a.events; l.n_events = a.n_events; l.hyp_iter = c.hyp_iter; l.ev_cap = c.ev_cap;
+    l.models = c.models; l.lo_models = L.lo_models.as<Model>(); l.lo_of_event = L.lo_of_event.as<int>();
+    l.lo_count = L.lo_count.as<int>(); l.prob_list = L.prob_list.as<int>(); l.n_prob = &c.sc->n_prob;
+    lo_prepare_kernel<<<cdiv(c.P, 128), 128, 0, c.st>>>(l);
+    LAUNCHED();
+    return RP_OK;
+}
+
+// The LM settings of the LO refinements (the trigger LOs and the final LO)
+LMArgs lo_lm_args(const Chunk &c) {
     LMArgs la;
     memset(&la, 0, sizeof la);
-    la.pairs = pairs; la.pts64 = pts64; la.d1 = io.d1; la.d2 = io.d2;
-    la.weight_sampson = opt.weight_sampson; la.gradient_tol = 1e-10; la.step_tol = 1e-8;
+    la.pairs = c.pairs; la.pts64 = c.pts64; la.d1 = c.io->d1; la.d2 = c.io->d2;
+    la.weight_sampson = c.opt->weight_sampson; la.gradient_tol = 1e-10; la.step_tol = 1e-8;
     la.initial_lambda = 1e-3; la.min_lambda = 1e-10; la.max_lambda = 1e10;
     la.loss_scale_override = -1.0; la.scale_reproj_override = -1.0;
-    la.lm_iters = &sc->lm_iters;
-    la.lm_flops = &sc->lm_flops;
-    {
-        la.prob_list = B[B_PROBLIST].as<int>(); la.n_prob = &sc->n_prob; la.prob_per_pair = ev_cap;
-        la.models = B[B_LOMODELS].as<Model>(); la.use_final = 0;
-        rc = launch_lm(ctx, variant, la, (long long)P * 8, st);
-        if (rc) return rc;
-    }
-    CK(cudaEventRecord(ev[6], st));
-    // 7. score LO results, merge
-    {
-        build_items_kernel<<<1, 1024, 0, st>>>(P, B[B_LOCOUNT].as<int>(), B[B_LOITEMPFX].as<int>(), &sc->n_lo_items, nullptr);
-        LAUNCHED();
-        ScoreArgs s2 = sa;
-        s2.slot_list = nullptr; s2.list_stride = 0;
-        s2.n_groups = P; s2.grp_stride = ev_cap; s2.grp_per_pair = 1; s2.grp_cnt = B[B_LOCOUNT].as<int>();
-        s2.item_prefix = B[B_LOITEMPFX].as<int>(); s2.n_items = &sc->n_lo_items; s2.models = B[B_LOMODELS].as<Model>();
-        s2.score = B[B_LOSCORE].as<double>(); s2.count = B[B_LOCNT].as<int>(); s2.point_scores = nullptr;
-        rc = launch_score(ctx, pose, false, s2, st);
-        if (rc) return rc;
-        MergeArgs m;
-        m.n_pairs = P; m.nseg = nseg; m.iters = iters; m.pairs = pairs; m.events = B[B_EVENTS].as<int>();
-        m.min_iterations = opt.min_iterations; m.max_iterations = opt.max_iterations;
-        m.dyn_num_trials_mult = opt.dyn_num_trials_mult; m.log_prob_missing = log(1.0 - opt.success_prob);
-        m.hyp_iter = hyp_iter; m.ev_cap = ev_cap; m.pair_flags = B[B_PAIRFLAGS].as<int>(); m.any_flag = &sc->any_flag;
-        m.n_events = B[B_NEVENTS].as<int>(); m.lo_of_event = B[B_LOOFEV].as<int>(); m.score = score; m.count = count;
-        m.models = models; m.lo_score = B[B_LOSCORE].as<double>(); m.lo_count_inl = B[B_LOCNT].as<int>();
-        m.lo_models = B[B_LOMODELS].as<Model>(); m.lo_count = B[B_LOCOUNT].as<int>();
-        m.best = B[B_BEST].as<Model>(); m.stats = B[B_STATS].as<rp_stats>(); m.final_start = B[B_FINSTART].as<Model>();
-        merge_kernel<<<cdiv(P, 128), 128, 0, st>>>(m);
-        LAUNCHED();
-        // final LO from the best model, rescore, accept when strictly better
-        la.prob_list = nullptr; la.n_prob = &sc->n_pairs_scalar; la.prob_per_pair = 1;
-        la.models = B[B_FINSTART].as<Model>(); la.use_final = 0;
-        rc = launch_lm(ctx, variant, la, P, st);
-        if (rc) return rc;
-        rc = launch_pair_items(ctx, P, st);
-        if (rc) return rc;
-        rc = launch_score(ctx, pose, false, pair_score_args(ctx, P, B[B_FINSTART].as<Model>(), nullptr), st);
-        if (rc) return rc;
-        Merge2Args m2;
-        m2.n_pairs = P; m2.pairs = pairs; m2.refined = B[B_FINSTART].as<Model>(); m2.ref_score = B[B_FINSCORE].as<double>();
-        m2.ref_count = B[B_FINCNT].as<int>(); m2.best = B[B_BEST].as<Model>(); m2.stats = B[B_STATS].as<rp_stats>();
-        merge2_kernel<<<cdiv(P, 128), 128, 0, st>>>(m2);
-        LAUNCHED();
-        // get_inliers of the RANSAC model (this is the mask the reference returns in `info`)
-        rc = launch_get_inliers(ctx, pose, io, B[B_BEST].as<Model>(), io.masks_out, st);
-        if (rc) return rc;
-    }
-    CK(cudaEventRecord(ev[7], st));
-    // 8. final refinement on the inliers with the user's bundle options (if num_inliers > 3)
-    {
-        enable_final_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, B[B_STATS].as<rp_stats>(), B[B_ENABLE].as<int>());
-        LAUNCHED();
-        LMArgs lf = final_lm_args(ctx, opt, io, B[B_BEST].as<Model>(), io.masks_out, B[B_ENABLE].as<int>());
-        lf.lm_iters = &sc->lm_iters;
-        lf.lm_flops = &sc->lm_flops;
-        rc = launch_lm(ctx, variant, lf, P, st);
-        if (rc) return rc;
-        finalize_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, variant, pairs, B[B_BEST].as<Model>());
-        LAUNCHED();
-        CK(cudaMemcpyAsync(io.models_out, B[B_BEST].p, sizeof(Model) * P, cudaMemcpyDeviceToDevice, st));
-        CK(cudaMemcpyAsync(io.stats_out, B[B_STATS].p, sizeof(rp_stats) * P, cudaMemcpyDeviceToDevice, st));
-    }
-    CK(cudaEventRecord(ev[8], st));
+    la.lm_iters = &c.sc->lm_iters;
+    la.lm_flops = &c.sc->lm_flops;
+    return la;
+}
+
+// 6. LO refinement of every trigger (independent problems)
+int lo_stage(rp_ctx *ctx, const Chunk &c) {
+    LMArgs la = lo_lm_args(c);
+    la.prob_list = ctx->lo.prob_list.as<int>(); la.n_prob = &c.sc->n_prob; la.prob_per_pair = c.ev_cap;
+    la.models = ctx->lo.lo_models.as<Model>();
+    return launch_lm(ctx, c.variant, la, c.st);
+}
+
+// 7. score the LO results and merge them into the pair's record; the final LO from the best model, its rescore
+// (accepted when strictly better); get_inliers of the RANSAC model (the mask the reference returns in `info`)
+int merge_stage(rp_ctx *ctx, const Chunk &c) {
+    const int P = c.P;
+    cudaStream_t st = c.st;
+    Scalars *sc = c.sc;
+    const LoBufs &L = ctx->lo;
+    const ResultBufs &R = ctx->res;
+    build_items_kernel<<<1, 1024, 0, st>>>(P, L.lo_count.as<int>(), L.lo_item_prefix.as<int>(), &sc->n_lo_items, nullptr);
+    LAUNCHED();
+    ScoreArgs s = chunk_score_args(ctx);
+    s.n_groups = P; s.grp_stride = c.ev_cap; s.grp_per_pair = 1; s.grp_cnt = L.lo_count.as<int>();
+    s.item_prefix = L.lo_item_prefix.as<int>(); s.n_items = &sc->n_lo_items; s.models = L.lo_models.as<Model>();
+    s.score = L.lo_score.as<double>(); s.count = L.lo_cnt.as<int>();
+    int rc = launch_score(ctx, c.pose, false, s, st);
+    if (rc) return rc;
+    const rp_options &opt = *c.opt;
+    MergeArgs m;
+    m.n_pairs = P; m.nseg = c.nseg; m.iters = c.iters; m.pairs = c.pairs; m.events = L.events.as<int>();
+    m.min_iterations = opt.min_iterations; m.max_iterations = opt.max_iterations;
+    m.dyn_num_trials_mult = opt.dyn_num_trials_mult; m.log_prob_missing = log(1.0 - opt.success_prob);
+    m.hyp_iter = c.hyp_iter; m.ev_cap = c.ev_cap; m.pair_flags = L.pair_flags.as<int>(); m.any_flag = &sc->any_flag;
+    m.n_events = L.n_events.as<int>(); m.lo_of_event = L.lo_of_event.as<int>(); m.score = c.score; m.count = c.count;
+    m.models = c.models; m.lo_score = L.lo_score.as<double>(); m.lo_count_inl = L.lo_cnt.as<int>();
+    m.lo_models = L.lo_models.as<Model>(); m.lo_count = L.lo_count.as<int>();
+    m.best = R.best.as<Model>(); m.stats = R.stats.as<rp_stats>(); m.final_start = R.final_start.as<Model>();
+    merge_kernel<<<cdiv(P, 128), 128, 0, st>>>(m);
+    LAUNCHED();
+    // final LO from the best model, rescore, accept when strictly better
+    LMArgs la = lo_lm_args(c);
+    la.prob_list = nullptr; la.n_prob = &sc->n_pairs_scalar; la.prob_per_pair = 1;
+    la.models = R.final_start.as<Model>();
+    if ((rc = launch_lm(ctx, c.variant, la, st))) return rc;
+    if ((rc = launch_pair_items(ctx, P, st))) return rc;
+    if ((rc = launch_score(ctx, c.pose, false, pair_score_args(ctx, P, R.final_start.as<Model>(), nullptr), st))) return rc;
+    Merge2Args m2;
+    m2.n_pairs = P; m2.pairs = c.pairs; m2.refined = R.final_start.as<Model>(); m2.ref_score = R.final_score.as<double>();
+    m2.ref_count = R.final_count.as<int>(); m2.best = R.best.as<Model>(); m2.stats = R.stats.as<rp_stats>();
+    merge2_kernel<<<cdiv(P, 128), 128, 0, st>>>(m2);
+    LAUNCHED();
+    return launch_get_inliers(ctx, c.pose, *c.io, R.best.as<Model>(), c.io->masks_out, st);
+}
+
+// 8. final refinement on the inliers with the user's bundle options (if num_inliers > 3); the chunk's models and stats out
+int final_stage(rp_ctx *ctx, const Chunk &c) {
+    const ResultBufs &R = ctx->res;
+    enable_final_kernel<<<cdiv(c.P, 256), 256, 0, c.st>>>(c.P, R.stats.as<rp_stats>(), R.enable.as<int>());
+    LAUNCHED();
+    LMArgs lf = final_lm_args(ctx, *c.opt, *c.io, R.best.as<Model>(), c.io->masks_out, R.enable.as<int>());
+    lf.lm_iters = &c.sc->lm_iters;
+    lf.lm_flops = &c.sc->lm_flops;
+    int rc = launch_lm(ctx, c.variant, lf, c.st);
+    if (rc) return rc;
+    finalize_kernel<<<cdiv(c.P, 256), 256, 0, c.st>>>(c.P, c.variant, c.pairs, R.best.as<Model>());
+    LAUNCHED();
+    CK(cudaMemcpyAsync(c.io->models_out, R.best.p, sizeof(Model) * c.P, cudaMemcpyDeviceToDevice, c.st));
+    CK(cudaMemcpyAsync(c.io->stats_out, R.stats.p, sizeof(rp_stats) * c.P, cudaMemcpyDeviceToDevice, c.st));
+    return RP_OK;
+}
+
+// Waits for the chunk's kernels, adds its stage times (rp_last_timing) and counters, and returns its pairs' flags
+int read_back(rp_ctx *ctx, const Chunk &c, std::vector<int> &flags) {
+    cudaEvent_t *ev = ctx->ev;
     Scalars h_sc;
-    CK(cudaMemcpyAsync(&h_sc, sc, sizeof h_sc, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
+    CK(cudaMemcpyAsync(&h_sc, c.sc, sizeof h_sc, cudaMemcpyDeviceToHost, c.st));
+    CK(cudaStreamSynchronize(c.st));
     for (int i = 0; i < 8; ++i) {
         float ms = 0.f;
         CK(cudaEventElapsedTime(&ms, ev[i], ev[i + 1]));
@@ -749,15 +848,15 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
     }
     ctx->last_cnt[0] += h_sc.n_hyp;
     ctx->last_cnt[1] += (int64_t)h_sc.point_scores;
-    ctx->last_cnt[2] += h_sc.n_prob + P;
+    ctx->last_cnt[2] += h_sc.n_prob + c.P;
     ctx->last_cnt[3] += (int64_t)h_sc.lm_iters;
     ctx->last_cnt[4] += 1;
     ctx->last_cnt[6] += (int64_t)h_sc.evaluated_ps;
     if (ctx->prune) {
         float msb = 0.f;
-        CK(cudaEventElapsedTime(&msb, use_tc ? ev[11] : ev[9], ev[10]));
+        CK(cudaEventElapsedTime(&msb, c.use_tc ? ev[11] : ev[9], ev[10]));
         ctx->last_ms[11] += msb;
-        if (use_tc) {
+        if (c.use_tc) {
             CK(cudaEventElapsedTime(&msb, ev[9], ev[11]));
             ctx->last_ms[12] += msb;
         }
@@ -765,23 +864,53 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
     ctx->last_cnt[8] += (int64_t)h_sc.tc_evaluated;
     ctx->last_cnt[9] += (int64_t)h_sc.tc_selected;
     ctx->last_cnt[10] += (int64_t)h_sc.lm_flops;
-    ctx->last_cnt[5] += ctx->prune ? (int64_t)h_sc.n_survivors + std::min<int64_t>(h_sc.n_hyp, (int64_t)P * ((ctx->tc && ctx->mid_end > ctx->head_small) ? ctx->head_small : ctx->head)) : h_sc.n_hyp;
-    ctx->last_cnt[7] = ctx->head;
-    flags.assign((size_t)P, 0);
+    // models through the exact kernel: the survivors and the exact head
+    ctx->last_cnt[5] += ctx->prune ? (int64_t)h_sc.n_survivors + std::min<int64_t>(h_sc.n_hyp, (int64_t)c.P * c.head) : h_sc.n_hyp;
+    ctx->last_cnt[7] = HB;
+    flags.assign((size_t)c.P, 0);
     if (h_sc.any_flag) {
-        CK(cudaMemcpyAsync(flags.data(), B[B_PAIRFLAGS].p, sizeof(int) * (size_t)P, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
+        CK(cudaMemcpyAsync(flags.data(), ctx->lo.pair_flags.p, sizeof(int) * (size_t)c.P, cudaMemcpyDeviceToHost, c.st));
+        CK(cudaStreamSynchronize(c.st));
     }
     return RP_OK;
 }
 
-size_t bytes_per_pair(int iters, long long avg_points, int ev_cap = EV, size_t input_bytes = 0) {
+// One pass over a chunk.  `flags` (host, [n_pairs]) receives PAIR_FLAG_* per pair: a flagged pair's outputs are void and
+// the caller runs it again with a larger `ev_cap` / more iterations (estimate_impl).
+int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io, int iters, int ev_cap,
+              std::vector<int> &flags, cudaStream_t st) {
+    const int P = io.n_pairs;
     const int nseg = std::max(1, cdiv(iters, SEG));
-    const size_t slots_pp = (size_t)nseg * 4 * SEG;
-    // per slot: model, hyp_iter, score, count, ub, lb, survivor list, tensor-core count + list; per correspondence:
-    // FP64 / FP32 / interleaved copies, bearings, mask, 128-byte feature row, `input_bytes` of input staging
-    return slots_pp * (sizeof(Model) + 4 + 8 + 4 + 12 + 8) + (size_t)iters * 12 + (size_t)ev_cap * (sizeof(Model) + 24) +
-           (size_t)avg_points * (sizeof(Pt64) + 32 + sizeof(Bear) + 1 + 128 + input_bytes) + 1024;
+    CK(ctx->hyp.reserve(P, iters, nseg));
+    CK(ctx->lo.reserve(P, ev_cap));
+    CK(ctx->res.reserve(P, true));
+    if (ctx->prune) CK(ctx->prn.reserve(P, nseg));
+    if (ctx->prune && ctx->tc) CK(ctx->tcb.reserve(P, io.n_points, nseg));
+    cudaEvent_t *ev = ctx->ev;
+    // 1. prepare, and the tensor-core tier's feature rows
+    int rc = prepare_chunk(ctx, variant, opt, io, ev[0], st);
+    if (rc) return rc;
+    const Chunk c = chunk_of(ctx, variant, opt, io, iters, ev_cap, st);
+    if (c.use_tc && c.N > 0) {
+        tc::tc_features_kernel<<<cdiv(c.N, 256), 256, 0, st>>>(c.N, c.pts32, ctx->tcb.feat.as<float4>());
+        LAUNCHED();
+    }
+    CK(cudaEventRecord(ev[1], st));
+    if ((rc = sample_stage(ctx, c))) return rc;
+    CK(cudaEventRecord(ev[2], st));
+    if ((rc = solve_stage(ctx, c))) return rc;
+    CK(cudaEventRecord(ev[3], st));
+    if ((rc = score_minimal(ctx, c))) return rc;
+    CK(cudaEventRecord(ev[4], st));
+    if ((rc = scan_stage(ctx, c))) return rc;
+    CK(cudaEventRecord(ev[5], st));
+    if ((rc = lo_stage(ctx, c))) return rc;
+    CK(cudaEventRecord(ev[6], st));
+    if ((rc = merge_stage(ctx, c))) return rc;
+    CK(cudaEventRecord(ev[7], st));
+    if ((rc = final_stage(ctx, c))) return rc;
+    CK(cudaEventRecord(ev[8], st));
+    return read_back(ctx, c, flags);
 }
 
 // widens a float32 chunk into the FP64 input arrays (no-op for an empty chunk); with `perm` (quality calls, float or
@@ -799,7 +928,7 @@ int launch_widen(rp_ctx *ctx, long long n, const In *x1, const In *x2, const In 
 
 // quality order of the P pairs of a chunk of n correspondences: `h_offsets` (host) and `d_offsets` (device) are the
 // same P+1 offsets, pair p owning [offsets[p] - base, offsets[p+1] - base) of `quality` and `perm` (no-op for n = 0).
-// The dynamic shared memory is sized to the largest pair up to RP_ORDER_SMEM_CAP; larger pairs use B_ORDSCR.
+// The dynamic shared memory is sized to the largest pair up to RP_ORDER_SMEM_CAP; larger pairs use the global sort scratch.
 int launch_order(rp_ctx *ctx, int P, long long n, const int64_t *h_offsets, const long long *d_offsets, long long base,
                  const float *quality, int *perm, cudaStream_t st) {
     if (n <= 0) return RP_OK;
@@ -810,8 +939,8 @@ int launch_order(rp_ctx *ctx, int P, long long n, const int64_t *h_offsets, cons
     a.smem_cap = (int)std::min<long long>(max_n, ORDER_SMEM_CAP);
     a.gkeys = nullptr; a.gidx = nullptr;
     if (max_n > ORDER_SMEM_CAP) {
-        CK(ctx->buf[B_ORDSCR].reserve(12 * (size_t)n));
-        a.gkeys = ctx->buf[B_ORDSCR].as<unsigned>();
+        CK(ctx->scratch.order.reserve(12 * (size_t)n));
+        a.gkeys = ctx->scratch.order.as<unsigned>();
         a.gidx = (int *)(a.gkeys + 2 * n);
     }
     order_by_quality_kernel<<<P, ORDER_THREADS, (size_t)ORDER_SMEM_PER_POINT * a.smem_cap, st>>>(a);
@@ -836,7 +965,6 @@ int launch_scatter_masks(rp_ctx *ctx, int P, long long n, const long long *d_off
 // sub-batch that cannot be run (out of device memory) marks its pairs RP_PAIR_FAILED instead of failing the call.
 int rerun_flagged(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io, const long long *rel,
                   const std::vector<int> &flags0, int iters0, int64_t p0, cudaStream_t st) {
-    DevBuf *B = ctx->buf;
     const bool pose = variant == RP_CALIB || variant == RP_CALIB_SHIFT;
     std::vector<int> todo;
     for (int i = 0; i < io.n_pairs; ++i)
@@ -882,36 +1010,31 @@ int rerun_flagged(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO
             int rc = RP_OK;
             std::vector<int> flags;
             do {  // single pass; `break` = this sub-batch failed
-                cudaError_t e = cudaSuccess;
-                (void)e;
-                if ((e = B[B_SUB_IDX].reserve(sizeof(int) * S)) || (e = B[B_SUB_SRC].reserve(8 * (size_t)S)) ||
-                    (e = B[B_SUB_DST].reserve(8 * ((size_t)S + 1))) || (e = B[B_SUB_X1].reserve(16 * nn)) ||
-                    (e = B[B_SUB_X2].reserve(16 * nn)) || (e = B[B_SUB_D1].reserve(8 * nn)) || (e = B[B_SUB_D2].reserve(8 * nn)) ||
-                    (e = B[B_SUB_CAMS].reserve(64 * (size_t)S)) || (e = B[B_SUB_MODELS].reserve(sizeof(Model) * S)) ||
-                    (e = B[B_SUB_STATS].reserve(sizeof(rp_stats) * S)) || (e = B[B_SUB_MASK].reserve(nn))) {
+                SubBufs &B = ctx->sub;
+                if (B.reserve(S, nn)) {
                     rc = RP_ERR_CUDA;
                     break;
                 }
-                CK(cudaMemcpyAsync(B[B_SUB_IDX].p, idx.data(), sizeof(int) * S, cudaMemcpyHostToDevice, st));
-                CK(cudaMemcpyAsync(B[B_SUB_SRC].p, src.data(), 8 * (size_t)S, cudaMemcpyHostToDevice, st));
-                CK(cudaMemcpyAsync(B[B_SUB_DST].p, dst.data(), 8 * ((size_t)S + 1), cudaMemcpyHostToDevice, st));
+                CK(cudaMemcpyAsync(B.idx.p, idx.data(), sizeof(int) * S, cudaMemcpyHostToDevice, st));
+                CK(cudaMemcpyAsync(B.src.p, src.data(), 8 * (size_t)S, cudaMemcpyHostToDevice, st));
+                CK(cudaMemcpyAsync(B.dst.p, dst.data(), 8 * ((size_t)S + 1), cudaMemcpyHostToDevice, st));
                 SubBatchArgs g;
-                g.n_sub = S; g.pair_idx = B[B_SUB_IDX].as<int>(); g.src_off = B[B_SUB_SRC].as<long long>();
-                g.dst_off = B[B_SUB_DST].as<long long>();
+                g.n_sub = S; g.pair_idx = B.idx.as<int>(); g.src_off = B.src.as<long long>();
+                g.dst_off = B.dst.as<long long>();
                 g.x1 = io.x1; g.x2 = io.x2; g.d1 = io.d1; g.d2 = io.d2; g.cams = pose ? io.cams : nullptr;
-                g.sx1 = B[B_SUB_X1].as<double>(); g.sx2 = B[B_SUB_X2].as<double>(); g.sd1 = B[B_SUB_D1].as<double>();
-                g.sd2 = B[B_SUB_D2].as<double>(); g.scams = B[B_SUB_CAMS].as<double>();
+                g.sx1 = B.x1.as<double>(); g.sx2 = B.x2.as<double>(); g.sd1 = B.d1.as<double>();
+                g.sd2 = B.d2.as<double>(); g.scams = B.cams.as<double>();
                 g.models = io.models_out; g.stats = io.stats_out; g.masks = io.masks_out;
-                g.smodels = B[B_SUB_MODELS].as<Model>(); g.sstats = B[B_SUB_STATS].as<rp_stats>();
-                g.smasks = B[B_SUB_MASK].as<unsigned char>();
+                g.smodels = B.models.as<Model>(); g.sstats = B.stats.as<rp_stats>();
+                g.smasks = B.mask.as<unsigned char>();
                 gather_pairs_kernel<<<S, 256, 0, st>>>(g);
                 LAUNCHED();
                 CK(cudaStreamSynchronize(st));  // idx / src / dst are stack-lifetime host buffers
                 ChunkIO sub;
                 sub.n_pairs = S; sub.n_points = npts; sub.h_offsets_rel = dst.data();
                 sub.x1 = g.sx1; sub.x2 = g.sx2; sub.d1 = g.sd1; sub.d2 = g.sd2; sub.cams = pose ? g.scams : nullptr;
-                sub.models_out = B[B_SUB_MODELS].as<Model>(); sub.stats_out = B[B_SUB_STATS].as<rp_stats>();
-                sub.masks_out = B[B_SUB_MASK].as<unsigned char>();
+                sub.models_out = B.models.as<Model>(); sub.stats_out = B.stats.as<rp_stats>();
+                sub.masks_out = B.mask.as<unsigned char>();
                 rc = run_chunk(ctx, variant, opt, sub, iters, ev_cap, flags, st);
                 if (rc) break;
                 scatter_pairs_kernel<<<S, 256, 0, st>>>(g);
@@ -964,7 +1087,7 @@ int begin_batch(rp_ctx *ctx, int &variant, int64_t n_pairs, const int64_t *offse
 //   lead = true (the estimator): a small first chunk goes ahead so that the kernels start early and every later upload
 //     hides behind the previous chunk's kernels.  With U = upload time (+ widening or ordering) and C = kernel time of
 //     the whole batch, the exposed time f U + max(0, (1-f) U - f C) is smallest at f = U / (U + C); U / C is taken
-//     from the previous host call on this context (1/8 of the batch before there is one).  RP_NO_LEAD_CHUNK: none.
+//     from the previous host call on this context (1/8 of the batch before there is one).
 //   lead = false (the refinement): at least four chunks, so that three uploads hide behind kernels.
 // Only timing depends on the boundaries, never results.
 std::vector<int64_t> plan_chunks(const rp_ctx *ctx, int64_t n_pairs, size_t bpp, bool host_io, bool lead) {
@@ -974,7 +1097,7 @@ std::vector<int64_t> plan_chunks(const rp_ctx *ctx, int64_t n_pairs, size_t bpp,
     if (host_io && n_pairs >= 1024) {
         if (!lead) {
             chunk = std::min<int64_t>(chunk, (n_pairs + 3) / 4);
-        } else if (!getenv("RP_NO_LEAD_CHUNK")) {
+        } else {
             double f = 0.125;
             if (ctx->prev_h2d_ms > 0.0 && ctx->prev_dev_ms > 0.0) f = ctx->prev_h2d_ms / (ctx->prev_h2d_ms + ctx->prev_dev_ms);
             f = std::min(1.0 / 3.0, std::max(1.0 / 32.0, f));
@@ -1268,24 +1391,18 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
 int refine_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io, cudaStream_t st) {
     const int P = io.n_pairs;
     const bool pose = variant == RP_CALIB || variant == RP_CALIB_SHIFT;
-    DevBuf *B = ctx->buf;
-    CK(B[B_BEST].reserve(sizeof(Model) * P));
-    CK(B[B_ENABLE].reserve(sizeof(int) * P));
-    CK(B[B_ONES].reserve(sizeof(int) * P));
-    CK(B[B_ONEPFX].reserve(sizeof(int) * (P + 1)));
-    CK(B[B_FINSCORE].reserve(sizeof(double) * P));
-    CK(B[B_FINCNT].reserve(sizeof(int) * P));
+    CK(ctx->res.reserve(P, false));
     int rc = prepare_chunk(ctx, variant, opt, io, nullptr, st);
     if (rc) return rc;
-    PairParams *pairs = B[B_PAIRS].as<PairParams>();
-    Model *work = B[B_BEST].as<Model>();
-    int *enable = B[B_ENABLE].as<int>();
+    PairParams *pairs = ctx->pt.pairs.as<PairParams>();
+    Model *work = ctx->res.best.as<Model>();
+    int *enable = ctx->res.enable.as<int>();
     refine_import_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(P, variant, pairs, io.subset, io.init, work, enable,
                                                                       io.bstats_out);
     LAUNCHED();
     LMArgs la = final_lm_args(ctx, opt, io, work, io.subset, enable);
     la.stats = io.bstats_out;
-    rc = launch_lm(ctx, variant, la, P, st);
+    rc = launch_lm(ctx, variant, la, st);
     if (rc) return rc;
     if (io.masks_out) {
         rc = launch_pair_items(ctx, P, st);
@@ -1293,22 +1410,10 @@ int refine_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO 
         rc = launch_get_inliers(ctx, pose, io, work, io.masks_out, st);
         if (rc) return rc;
     }
-    refine_export_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, variant, pairs, enable, io.init, work, B[B_FINCNT].as<int>(),
+    refine_export_kernel<<<cdiv(P, 256), 256, 0, st>>>(P, variant, pairs, enable, io.init, work, ctx->res.final_count.as<int>(),
                                                        io.models_out, io.num_inliers_out);
     LAUNCHED();
     return RP_OK;
-}
-
-// Device workspace of a refine chunk.  Per correspondence: pts64 (32 B), pts32 (16), the pair-interleaved FP32 copy
-// (16), bearings (48), and the chunk's I/O: FP64 inputs (48), subset (1), inlier mask (1); the host path double-buffers
-// the I/O and adds the float32 staging (24 B, double-buffered) for float32 inputs.  Per pair: PairParams, the work,
-// start and output models, bundle stats, cams, and a few counters.
-size_t refine_bytes_per_pair(long long avg_points, bool host_io, bool f32) {
-    const size_t io_pt = 48 + 1 + 1 + (host_io && f32 ? 24 : 0);
-    const size_t io_pair = 2 * sizeof(Model) + sizeof(rp_bundle_stats) + 64 + 8;
-    const size_t sets = host_io ? 2 : 1;
-    return (size_t)avg_points * (32 + 16 + 16 + 48 + sets * io_pt) + sizeof(PairParams) + sizeof(Model) + 32 +
-           sets * io_pair + 64;
 }
 
 // rp_refine_pairs_{host,dev}[_f32]: run_chunks with refine_chunk as the work of a chunk.  In = float: the float32
@@ -1395,24 +1500,11 @@ int rp_create(int device, rp_ctx **out) {
     for (auto &s : ctx->set) s.create_events();
     if (const char *np = getenv("RP_NO_PRUNE")) ctx->prune = !(np[0] == '1');
     if (const char *nw = getenv("RP_NO_WAVES")) ctx->waves = !(nw[0] == '1');
-    if (const char *lw = getenv("RP_LM_WARP")) ctx->lm_warp = atoi(lw) & 0x1f;
-    if (const char *hs = getenv("RP_HEAD_SMALL")) { const int v = atoi(hs); if (v >= 0 && v <= 256 && v % 32 == 0) ctx->head_small = v; }
-    if (const char *me = getenv("RP_MID_END")) {
-        int n = 0, vals[4] = {0, 0, 0, 0};
-        bool ok = true;
-        for (const char *p = me; *p && n < 4;) {
-            const int v = atoi(p);
-            if (v < 0 || v > SEG || v % 32 != 0 || (n && v <= vals[n - 1])) ok = false;
-            vals[n++] = v;
-            while (*p && *p != ',') ++p;
-            if (*p == ',') ++p;
-        }
-        if (ok && n) { ctx->n_mid = n; for (int k = 0; k < 4; ++k) ctx->mid_ends[k] = vals[k]; ctx->mid_end = vals[n - 1]; }
-    }
+    if (const char *lw = getenv("RP_LM_WARP")) ctx->lm_warp = atoi(lw) != 0;
+    if (const char *me = getenv("RP_MID_END")) ctx->mid = atoi(me) != 0;
     if (const char *nt = getenv("RP_NO_TC")) ctx->tc = !(nt[0] == '1');
-    if (const char *sp = getenv("RP_TC_SPLIT")) { const int v = atoi(sp); if (v >= 1 && v <= 15) ctx->tc_two_pass = v; }
-    if (const char *ap = getenv("RP_TC_ADAPT_PCT")) { const int v = atoi(ap); if (v >= 50 && v <= 200) ctx->tc_two_pass = -v; }
-    if (const char *op = getenv("RP_TC_ONE_PASS")) { if (op[0] == '1') ctx->tc_two_pass = 0; }
+    if (const char *op = getenv("RP_TC_ONE_PASS")) { if (op[0] == '1') ctx->tc_two_pass = false; }
+    ctx->solve_generic = getenv("RP_SOLVE_GENERIC") != nullptr;
     if (const char *ec = getenv("RP_EV_CAP")) { const int v = atoi(ec); if (v >= 1 && v <= EV) ctx->ev_cap0 = v; }
     {
         cudaDriverEntryPointQueryResult qres;
@@ -1428,7 +1520,6 @@ int rp_create(int device, rp_ctx **out) {
         }
         ctx->encode_tiled = fn;
     }
-    if (const char *hd = getenv("RP_HEAD")) { const int v = atoi(hd); if (v == 32 || v == 64 || v == 96 || v == 128) ctx->head = v; }
     if (const char *gb = getenv("RP_WORKSPACE_GB")) {
         const double v = atof(gb);
         if (v > 0.01) ctx->workspace_budget = (size_t)(v * (double)((size_t)1 << 30));
@@ -1442,12 +1533,11 @@ int rp_create(int device, rp_ctx **out) {
 void rp_destroy(rp_ctx *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
-    for (auto &b : ctx->buf) b.release();
-    for (auto &s : ctx->set) s.release();
+    for (auto &s : ctx->set) s.destroy_events();
     for (auto &ev : ctx->ev) cudaEventDestroy(ev);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
-    delete ctx;
+    delete ctx;   // frees the workspace
 }
 
 const char *rp_last_error(const rp_ctx *ctx) { return ctx ? ctx->err.c_str() : g_create_error.c_str(); }
@@ -1602,21 +1692,20 @@ int rp_sample_batch_prosac(rp_ctx *ctx, int64_t n, uint64_t seed, int64_t iters,
     if (!ctx || !samples || n < 3 || iters < 0 || max_prosac_iterations < 0) return fail(ctx, RP_ERR_INVALID, "bad argument");
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    DevBuf *B = ctx->buf;
-    CK(B[B_PAIRS].reserve(sizeof(PairParams)));
-    CK(B[B_SAMPLES].reserve(sizeof(int) * 3 * (size_t)std::max<int64_t>(iters, 1)));
+    CK(ctx->pt.pairs.reserve(sizeof(PairParams)));
+    CK(ctx->hyp.samples.reserve(sizeof(int) * 3 * (size_t)std::max<int64_t>(iters, 1)));
     PairParams pp;
     memset(&pp, 0, sizeof pp);
     pp.n = (int)n; pp.valid = 1;
-    CK(cudaMemcpyAsync(B[B_PAIRS].p, &pp, sizeof pp, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ctx->pt.pairs.p, &pp, sizeof pp, cudaMemcpyHostToDevice, st));
     if (iters > 0) {
         if (progressive_sampling)
-            sample_prosac_kernel<<<1, 32, 0, st>>>(1, (int)iters, B[B_PAIRS].as<PairParams>(), seed,
-                                                   (unsigned long long)max_prosac_iterations, B[B_SAMPLES].as<int>());
+            sample_prosac_kernel<<<1, 32, 0, st>>>(1, (int)iters, ctx->pt.pairs.as<PairParams>(), seed,
+                                                   (unsigned long long)max_prosac_iterations, ctx->hyp.samples.as<int>());
         else
-            sample_kernel<<<1, 32, 0, st>>>(1, (int)iters, B[B_PAIRS].as<PairParams>(), seed, B[B_SAMPLES].as<int>());
+            sample_kernel<<<1, 32, 0, st>>>(1, (int)iters, ctx->pt.pairs.as<PairParams>(), seed, ctx->hyp.samples.as<int>());
         LAUNCHED();
-        CK(cudaMemcpyAsync(samples, B[B_SAMPLES].p, sizeof(int) * 3 * (size_t)iters, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(samples, ctx->hyp.samples.p, sizeof(int) * 3 * (size_t)iters, cudaMemcpyDeviceToHost, st));
     }
     CK(cudaStreamSynchronize(st));
     return RP_OK;
@@ -1653,38 +1742,36 @@ int rp_solve_batch(rp_ctx *ctx, int variant, int64_t n, const double *x1h, const
     if (n == 0) return RP_OK;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    DevBuf *B = ctx->buf;
     StageSet &s0 = ctx->set[0];  // the chunk pipeline's set 0, free between calls
     CK(s0.x1.reserve(72 * (size_t)n)); CK(s0.x2.reserve(72 * (size_t)n));
     CK(s0.d1.reserve(24 * (size_t)n)); CK(s0.d2.reserve(24 * (size_t)n));
-    CK(B[B_MODELS].reserve(sizeof(Model) * 4 * (size_t)n)); CK(B[B_COUNT].reserve(sizeof(int) * (size_t)n));
+    CK(ctx->hyp.models.reserve(sizeof(Model) * 4 * (size_t)n)); CK(ctx->hyp.count.reserve(sizeof(int) * (size_t)n));
     CK(cudaMemcpyAsync(s0.x1.p, x1h, 72 * (size_t)n, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(s0.x2.p, x2h, 72 * (size_t)n, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(s0.d1.p, d1, 24 * (size_t)n, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(s0.d2.p, d2, 24 * (size_t)n, cudaMemcpyHostToDevice, st));
-    CK(cudaMemsetAsync(B[B_MODELS].p, 0, sizeof(Model) * 4 * (size_t)n, st));
+    CK(cudaMemsetAsync(ctx->hyp.models.p, 0, sizeof(Model) * 4 * (size_t)n, st));
     solve_problems_kernel<<<cdiv(n, 128), 128, 0, st>>>(variant, n, s0.x1.as<double>(), s0.x2.as<double>(),
                                                        s0.d1.as<double>(), s0.d2.as<double>(),
-                                                       B[B_MODELS].as<Model>(), B[B_COUNT].as<int>());
+                                                       ctx->hyp.models.as<Model>(), ctx->hyp.count.as<int>());
     LAUNCHED();
-    CK(cudaMemcpyAsync(models, B[B_MODELS].p, sizeof(Model) * 4 * (size_t)n, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(counts, B[B_COUNT].p, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(models, ctx->hyp.models.p, sizeof(Model) * 4 * (size_t)n, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(counts, ctx->hyp.count.p, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return RP_OK;
 }
 
 static int stage_pair(rp_ctx *ctx, int64_t n_points, const double *x1, const double *x2, double sq_thr, cudaStream_t st) {
-    DevBuf *B = ctx->buf;
     StageSet &s0 = ctx->set[0];  // the chunk pipeline's set 0, free between calls
     const size_t nn = (size_t)std::max<int64_t>(n_points, 1);
-    CK(B[B_PAIRS].reserve(sizeof(PairParams)));
-    CK(B[B_PTS64].reserve(sizeof(Pt64) * nn)); CK(B[B_PTS32].reserve(sizeof(float4) * nn)); CK(B[B_BEAR].reserve(sizeof(Bear) * nn));
+    CK(ctx->pt.pairs.reserve(sizeof(PairParams)));
+    CK(ctx->pt.pts64.reserve(sizeof(Pt64) * nn)); CK(ctx->pt.pts32.reserve(sizeof(float4) * nn)); CK(ctx->pt.bear.reserve(sizeof(Bear) * nn));
     CK(s0.x1.reserve(16 * nn)); CK(s0.x2.reserve(16 * nn));
     CK(cudaMemcpyAsync(s0.x1.p, x1, 16 * (size_t)n_points, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(s0.x2.p, x2, 16 * (size_t)n_points, cudaMemcpyHostToDevice, st));
     stage_points_kernel<<<1, 32, 0, st>>>((int)n_points, s0.x1.as<double>(), s0.x2.as<double>(), sq_thr,
-                                         B[B_PTS64].as<Pt64>(), B[B_PTS32].as<float4>(), B[B_BEAR].as<Bear>(),
-                                         B[B_PAIRS].as<PairParams>());
+                                         ctx->pt.pts64.as<Pt64>(), ctx->pt.pts32.as<float4>(), ctx->pt.bear.as<Bear>(),
+                                         ctx->pt.pairs.as<PairParams>());
     LAUNCHED();
     return RP_OK;
 }
@@ -1698,45 +1785,44 @@ int rp_score_batch(rp_ctx *ctx, int variant, int64_t n_models, const rp_model *m
     if (n_models == 0) return RP_OK;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    DevBuf *B = ctx->buf;
     StageSet &s0 = ctx->set[0];  // the chunk pipeline's set 0, free between calls
     const bool pose = variant == RP_CALIB || variant == RP_CALIB_SHIFT;
     int rc = stage_pair(ctx, n_points, x1, x2, sq_threshold, st);
     if (rc) return rc;
-    CK(B[B_MODELS].reserve(sizeof(Model) * (size_t)n_models));
-    CK(B[B_SCORE].reserve(sizeof(double) * (size_t)n_models)); CK(B[B_COUNT].reserve(sizeof(int) * (size_t)n_models));
-    CK(B[B_SEGCNT].reserve(sizeof(int) * 2)); CK(B[B_ITEMPFX].reserve(sizeof(int) * 4)); CK(B[B_SCALARS].reserve(sizeof(Scalars)));
-    Scalars *sc = B[B_SCALARS].as<Scalars>();
+    CK(ctx->hyp.models.reserve(sizeof(Model) * (size_t)n_models));
+    CK(ctx->hyp.score.reserve(sizeof(double) * (size_t)n_models)); CK(ctx->hyp.count.reserve(sizeof(int) * (size_t)n_models));
+    CK(ctx->hyp.seg_count.reserve(sizeof(int) * 2)); CK(ctx->hyp.item_prefix.reserve(sizeof(int) * 4)); CK(ctx->pt.scalars.reserve(sizeof(Scalars)));
+    Scalars *sc = ctx->pt.scalars.as<Scalars>();
     CK(cudaMemsetAsync(sc, 0, sizeof(Scalars), st));
-    CK(cudaMemcpyAsync(B[B_MODELS].p, models, sizeof(Model) * (size_t)n_models, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ctx->hyp.models.p, models, sizeof(Model) * (size_t)n_models, cudaMemcpyHostToDevice, st));
     const int cnt = (int)n_models;
-    CK(cudaMemcpyAsync(B[B_SEGCNT].p, &cnt, sizeof(int), cudaMemcpyHostToDevice, st));
-    build_items_kernel<<<1, 1024, 0, st>>>(1, B[B_SEGCNT].as<int>(), B[B_ITEMPFX].as<int>(), &sc->n_items, nullptr);
+    CK(cudaMemcpyAsync(ctx->hyp.seg_count.p, &cnt, sizeof(int), cudaMemcpyHostToDevice, st));
+    build_items_kernel<<<1, 1024, 0, st>>>(1, ctx->hyp.seg_count.as<int>(), ctx->hyp.item_prefix.as<int>(), &sc->n_items, nullptr);
     LAUNCHED();
     ScoreArgs a;
-    a.n_groups = 1; a.grp_stride = 0; a.grp_per_pair = 1; a.grp_cnt = B[B_SEGCNT].as<int>();
-    a.item_prefix = B[B_ITEMPFX].as<int>(); a.n_items = &sc->n_items; a.pairs = B[B_PAIRS].as<PairParams>();
-    a.models = B[B_MODELS].as<Model>(); a.pts32 = B[B_PTS32].as<float4>(); a.pts64 = B[B_PTS64].as<Pt64>();
-    a.bear = B[B_BEAR].as<Bear>(); a.score = B[B_SCORE].as<double>(); a.count = B[B_COUNT].as<int>();
+    a.n_groups = 1; a.grp_stride = 0; a.grp_per_pair = 1; a.grp_cnt = ctx->hyp.seg_count.as<int>();
+    a.item_prefix = ctx->hyp.item_prefix.as<int>(); a.n_items = &sc->n_items; a.pairs = ctx->pt.pairs.as<PairParams>();
+    a.models = ctx->hyp.models.as<Model>(); a.pts32 = ctx->pt.pts32.as<float4>(); a.pts64 = ctx->pt.pts64.as<Pt64>();
+    a.bear = ctx->pt.bear.as<Bear>(); a.score = ctx->hyp.score.as<double>(); a.count = ctx->hyp.count.as<int>();
     a.mask = nullptr; a.point_scores = nullptr; a.slot_list = nullptr; a.list_stride = 0;
     rc = launch_score(ctx, pose, false, a, st);
     if (rc) return rc;
     std::vector<int> h_cnt((size_t)n_models);
-    CK(cudaMemcpyAsync(scores, B[B_SCORE].p, sizeof(double) * (size_t)n_models, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(h_cnt.data(), B[B_COUNT].p, sizeof(int) * (size_t)n_models, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(scores, ctx->hyp.score.p, sizeof(double) * (size_t)n_models, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(h_cnt.data(), ctx->hyp.count.p, sizeof(int) * (size_t)n_models, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     for (int64_t i = 0; i < n_models; ++i) counts[i] = h_cnt[(size_t)i];
     if (masks && n_points > 0) {
         // I1 get_inliers: one launch per model with the mask variant of the same kernel
         CK(s0.mask.reserve((size_t)n_points)); CK(s0.models.reserve(sizeof(double))); CK(s0.stats.reserve(sizeof(int)));
         const int one = 1;
-        CK(cudaMemcpyAsync(B[B_SEGCNT].p, &one, sizeof(int), cudaMemcpyHostToDevice, st));
-        build_items_kernel<<<1, 1024, 0, st>>>(1, B[B_SEGCNT].as<int>(), B[B_ITEMPFX].as<int>(), &sc->n_items, nullptr);
+        CK(cudaMemcpyAsync(ctx->hyp.seg_count.p, &one, sizeof(int), cudaMemcpyHostToDevice, st));
+        build_items_kernel<<<1, 1024, 0, st>>>(1, ctx->hyp.seg_count.as<int>(), ctx->hyp.item_prefix.as<int>(), &sc->n_items, nullptr);
         LAUNCHED();
         for (int64_t i = 0; i < n_models; ++i) {
             CK(cudaMemsetAsync(s0.mask.p, 0, (size_t)n_points, st));
             ScoreArgs m = a;
-            m.models = B[B_MODELS].as<Model>() + i; m.score = s0.models.as<double>(); m.count = s0.stats.as<int>();
+            m.models = ctx->hyp.models.as<Model>() + i; m.score = s0.models.as<double>(); m.count = s0.stats.as<int>();
             m.mask = s0.mask.as<unsigned char>();
             rc = launch_score(ctx, pose, true, m, st);
             if (rc) return rc;
@@ -1755,34 +1841,33 @@ int rp_tc_count_batch(rp_ctx *ctx, int variant, int64_t n_models, const rp_model
     if (n_models == 0) return RP_OK;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    DevBuf *B = ctx->buf;
     const bool pose = variant == RP_CALIB || variant == RP_CALIB_SHIFT;
     int rc = stage_pair(ctx, n_points, x1, x2, sq_threshold, st);
     if (rc) return rc;
     const size_t nn = (size_t)std::max<int64_t>(n_points, 1);
-    CK(B[B_FEAT].reserve(128 * nn + 128 * tc::NT));
-    CK(B[B_MODELS].reserve(sizeof(Model) * 4 * SEG)); CK(B[B_TCOUT].reserve(sizeof(int) * 4 * SEG));
-    CK(B[B_SEGCNT].reserve(sizeof(int) * 2)); CK(B[B_TCPFX].reserve(sizeof(int) * 4)); CK(B[B_SCALARS].reserve(sizeof(Scalars)));
-    Scalars *sc = B[B_SCALARS].as<Scalars>();
+    CK(ctx->tcb.feat.reserve(128 * nn + 128 * tc::NT));
+    CK(ctx->hyp.models.reserve(sizeof(Model) * 4 * SEG)); CK(ctx->tcb.out.reserve(sizeof(int) * 4 * SEG));
+    CK(ctx->hyp.seg_count.reserve(sizeof(int) * 2)); CK(ctx->tcb.prefix.reserve(sizeof(int) * 4)); CK(ctx->pt.scalars.reserve(sizeof(Scalars)));
+    Scalars *sc = ctx->pt.scalars.as<Scalars>();
     CK(cudaMemsetAsync(sc, 0, sizeof(Scalars), st));
-    CK(cudaMemcpyAsync(B[B_MODELS].p, models, sizeof(Model) * (size_t)n_models, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ctx->hyp.models.p, models, sizeof(Model) * (size_t)n_models, cudaMemcpyHostToDevice, st));
     const int cnt = (int)n_models;
-    CK(cudaMemcpyAsync(B[B_SEGCNT].p, &cnt, sizeof(int), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ctx->hyp.seg_count.p, &cnt, sizeof(int), cudaMemcpyHostToDevice, st));
     if (n_points > 0) {
-        tc::tc_features_kernel<<<cdiv(n_points, 256), 256, 0, st>>>(n_points, B[B_PTS32].as<float4>(), B[B_FEAT].as<float4>());
+        tc::tc_features_kernel<<<cdiv(n_points, 256), 256, 0, st>>>(n_points, ctx->pt.pts32.as<float4>(), ctx->tcb.feat.as<float4>());
         LAUNCHED();
     }
-    build_items_kernel<<<1, 1024, 0, st>>>(1, B[B_SEGCNT].as<int>(), B[B_TCPFX].as<int>(), &sc->n_tc_items, nullptr, tc::TILE_MODELS);
+    build_items_kernel<<<1, 1024, 0, st>>>(1, ctx->hyp.seg_count.as<int>(), ctx->tcb.prefix.as<int>(), &sc->n_tc_items, nullptr, tc::TILE_MODELS);
     LAUNCHED();
     tc::TcArgs ta;
     memset(&ta, 0, sizeof ta);
-    ta.n_pairs = 1; ta.nseg = 1; ta.pairs = B[B_PAIRS].as<PairParams>(); ta.seg_count = B[B_SEGCNT].as<int>();
-    ta.item_prefix = B[B_TCPFX].as<int>(); ta.n_items = &sc->n_tc_items; ta.models = B[B_MODELS].as<Model>();
-    ta.out = B[B_TCOUT].as<int>(); ta.pose = pose ? 1 : 0;
-    rc = launch_tc(ctx, ta, B[B_FEAT].as<float4>(), n_points, st);
+    ta.n_pairs = 1; ta.nseg = 1; ta.pairs = ctx->pt.pairs.as<PairParams>(); ta.seg_count = ctx->hyp.seg_count.as<int>();
+    ta.item_prefix = ctx->tcb.prefix.as<int>(); ta.n_items = &sc->n_tc_items; ta.models = ctx->hyp.models.as<Model>();
+    ta.out = ctx->tcb.out.as<int>(); ta.pose = pose ? 1 : 0;
+    rc = launch_tc(ctx, ta, ctx->tcb.feat.as<float4>(), n_points, st);
     if (rc) return rc;
     std::vector<int> h((size_t)n_models);
-    CK(cudaMemcpyAsync(h.data(), B[B_TCOUT].p, sizeof(int) * (size_t)n_models, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(h.data(), ctx->tcb.out.p, sizeof(int) * (size_t)n_models, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     for (int64_t i = 0; i < n_models; ++i) certain_outliers[i] = h[(size_t)i];
     return RP_OK;
@@ -1797,39 +1882,38 @@ int rp_refine_batch(rp_ctx *ctx, int variant, int64_t n_models, rp_model *models
     if (n_models == 0) return RP_OK;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    DevBuf *B = ctx->buf;
     StageSet &s0 = ctx->set[0];  // the chunk pipeline's set 0, free between calls
     int rc = stage_pair(ctx, n_points, x1, x2, 1.0, st);
     if (rc) return rc;
     const size_t nn = (size_t)std::max<int64_t>(n_points, 1);
     CK(s0.d1.reserve(8 * nn)); CK(s0.d2.reserve(8 * nn)); CK(s0.mask.reserve(nn));
-    CK(B[B_MODELS].reserve(sizeof(Model) * (size_t)n_models)); CK(B[B_SCALARS].reserve(sizeof(Scalars)));
-    CK(B[B_TMP2].reserve(sizeof(rp_bundle_stats) * (size_t)n_models));
+    CK(ctx->hyp.models.reserve(sizeof(Model) * (size_t)n_models)); CK(ctx->pt.scalars.reserve(sizeof(Scalars)));
+    CK(ctx->scratch.tmp2.reserve(sizeof(rp_bundle_stats) * (size_t)n_models));
     CK(cudaMemcpyAsync(s0.d1.p, d1, 8 * (size_t)n_points, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(s0.d2.p, d2, 8 * (size_t)n_points, cudaMemcpyHostToDevice, st));
     if (mask) CK(cudaMemcpyAsync(s0.mask.p, mask, (size_t)n_points, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(B[B_MODELS].p, models, sizeof(Model) * (size_t)n_models, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ctx->hyp.models.p, models, sizeof(Model) * (size_t)n_models, cudaMemcpyHostToDevice, st));
     Scalars h;
     memset(&h, 0, sizeof h);
     h.n_prob = (int)n_models;
-    Scalars *sc = B[B_SCALARS].as<Scalars>();
+    Scalars *sc = ctx->pt.scalars.as<Scalars>();
     CK(cudaMemcpyAsync(sc, &h, sizeof h, cudaMemcpyHostToDevice, st));
     LMArgs la;
     memset(&la, 0, sizeof la);
     la.prob_list = nullptr; la.n_prob = &sc->n_prob; la.prob_per_pair = 1 << 30;  // every problem -> pair 0
-    la.pairs = B[B_PAIRS].as<PairParams>(); la.pts64 = B[B_PTS64].as<Pt64>();
+    la.pairs = ctx->pt.pairs.as<PairParams>(); la.pts64 = ctx->pt.pts64.as<Pt64>();
     la.d1 = s0.d1.as<double>(); la.d2 = s0.d2.as<double>();
     la.mask = mask ? s0.mask.as<unsigned char>() : nullptr; la.enable = nullptr;
-    la.models = B[B_MODELS].as<Model>(); la.use_final = 1;
+    la.models = ctx->hyp.models.as<Model>(); la.use_final = 1;
     la.max_iterations = (int)opt->max_iterations; la.loss_type = opt->loss_type;
     la.weight_sampson = weight_sampson; la.gradient_tol = opt->gradient_tol; la.step_tol = opt->step_tol;
     la.initial_lambda = opt->initial_lambda; la.min_lambda = opt->min_lambda; la.max_lambda = opt->max_lambda;
     la.loss_scale_override = opt->loss_scale; la.scale_reproj_override = scale_reproj;
-    la.stats = B[B_TMP2].as<rp_bundle_stats>(); la.lm_iters = nullptr;
-    rc = launch_lm(ctx, variant, la, n_models, st);
+    la.stats = ctx->scratch.tmp2.as<rp_bundle_stats>(); la.lm_iters = nullptr;
+    rc = launch_lm(ctx, variant, la, st);
     if (rc) return rc;
-    CK(cudaMemcpyAsync(models, B[B_MODELS].p, sizeof(Model) * (size_t)n_models, cudaMemcpyDeviceToHost, st));
-    if (stats) CK(cudaMemcpyAsync(stats, B[B_TMP2].p, sizeof(rp_bundle_stats) * (size_t)n_models, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(models, ctx->hyp.models.p, sizeof(Model) * (size_t)n_models, cudaMemcpyDeviceToHost, st));
+    if (stats) CK(cudaMemcpyAsync(stats, ctx->scratch.tmp2.p, sizeof(rp_bundle_stats) * (size_t)n_models, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return RP_OK;
 }
@@ -1851,8 +1935,8 @@ int gather_depths_impl(rp_ctx *ctx, const float *depth1, int h1, int w1, const f
     if (n == 0) return RP_OK;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-    CK(ctx->buf[B_SCALARS].reserve(sizeof(Scalars)));
-    long long *d_n = (long long *)ctx->buf[B_SCALARS].p;
+    CK(ctx->pt.scalars.reserve(sizeof(Scalars)));
+    long long *d_n = (long long *)ctx->pt.scalars.p;
     gather_depths_kernel<T><<<1, 1024, 0, st>>>(depth1, h1, w1, depth2, h2, w2, kp1, kp2, quality, (long long)n,
                                                 x1, x2, d1, d2, quality_out, d_n);
     LAUNCHED();
@@ -1883,25 +1967,24 @@ int gather_depths_batch_impl(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_off
     if (with_q && N > 0 && (!quality || !quality_out)) return fail(ctx, RP_ERR_INVALID, "null quality / quality_out");
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-    DevBuf *B = ctx->buf;
     const size_t nn = (size_t)std::max<long long>(N, 1);
-    CK(B[B_SUB_X1].reserve(16 * nn)); CK(B[B_SUB_X2].reserve(16 * nn)); CK(B[B_SUB_D1].reserve(8 * nn)); CK(B[B_SUB_D2].reserve(8 * nn));
-    if (with_q) CK(B[B_GATHER_Q].reserve(4 * nn));
-    CK(B[B_SUB_SRC].reserve(8 * ((size_t)n_pairs + 1))); CK(B[B_SUB_DST].reserve(8 * ((size_t)n_pairs + 1)));
-    CK(B[B_SUB_IDX].reserve(sizeof(int) * 3 * (size_t)n_pairs));
+    CK(ctx->sub.x1.reserve(16 * nn)); CK(ctx->sub.x2.reserve(16 * nn)); CK(ctx->sub.d1.reserve(8 * nn)); CK(ctx->sub.d2.reserve(8 * nn));
+    if (with_q) CK(ctx->scratch.gather_q.reserve(4 * nn));
+    CK(ctx->sub.src.reserve(8 * ((size_t)n_pairs + 1))); CK(ctx->sub.dst.reserve(8 * ((size_t)n_pairs + 1)));
+    CK(ctx->sub.idx.reserve(sizeof(int) * 3 * (size_t)n_pairs));
     std::vector<long long> rel((size_t)n_pairs + 1);
     for (int64_t p = 0; p <= n_pairs; ++p) rel[(size_t)p] = in_offsets[p] - in_offsets[0];
-    int *d_f1 = B[B_SUB_IDX].as<int>(), *d_f2 = d_f1 + n_pairs, *d_cnt = d_f2 + n_pairs;
-    CK(cudaMemcpyAsync(B[B_SUB_SRC].p, rel.data(), 8 * ((size_t)n_pairs + 1), cudaMemcpyHostToDevice, st));
+    int *d_f1 = ctx->sub.idx.as<int>(), *d_f2 = d_f1 + n_pairs, *d_cnt = d_f2 + n_pairs;
+    CK(cudaMemcpyAsync(ctx->sub.src.p, rel.data(), 8 * ((size_t)n_pairs + 1), cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(d_f1, frame1, sizeof(int) * (size_t)n_pairs, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(d_f2, frame2, sizeof(int) * (size_t)n_pairs, cudaMemcpyHostToDevice, st));
     GatherBatchArgs<T> g;
     g.n_pairs = (int)n_pairs; g.h = h; g.w = w; g.depth = depth_maps; g.frame1 = d_f1; g.frame2 = d_f2;
-    g.in_off = B[B_SUB_SRC].as<long long>(); g.out_off = B[B_SUB_DST].as<long long>();
+    g.in_off = ctx->sub.src.as<long long>(); g.out_off = ctx->sub.dst.as<long long>();
     g.kp1 = kp1; g.kp2 = kp2;
-    g.tx1 = B[B_SUB_X1].as<T>(); g.tx2 = B[B_SUB_X2].as<T>(); g.td1 = B[B_SUB_D1].as<T>(); g.td2 = B[B_SUB_D2].as<T>();
+    g.tx1 = ctx->sub.x1.as<T>(); g.tx2 = ctx->sub.x2.as<T>(); g.td1 = ctx->sub.d1.as<T>(); g.td2 = ctx->sub.d2.as<T>();
     g.x1 = x1; g.x2 = x2; g.d1 = d1; g.d2 = d2; g.count = d_cnt;
-    g.q_in = quality; g.tq = with_q ? B[B_GATHER_Q].as<float>() : nullptr; g.q_out = quality_out;
+    g.q_in = quality; g.tq = with_q ? ctx->scratch.gather_q.as<float>() : nullptr; g.q_out = quality_out;
     gather_depths_batch_kernel<T><<<(unsigned)n_pairs, 256, 0, st>>>(g);
     LAUNCHED();
     std::vector<int> cnt((size_t)n_pairs);
@@ -1910,7 +1993,7 @@ int gather_depths_batch_impl(rp_ctx *ctx, int64_t n_pairs, const int64_t *in_off
     std::vector<long long> out((size_t)n_pairs + 1, 0);
     for (int64_t p = 0; p < n_pairs; ++p) out[(size_t)p + 1] = out[(size_t)p] + cnt[(size_t)p];
     for (int64_t p = 0; p <= n_pairs; ++p) out_offsets[p] = out[(size_t)p];
-    CK(cudaMemcpyAsync(B[B_SUB_DST].p, out.data(), 8 * ((size_t)n_pairs + 1), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ctx->sub.dst.p, out.data(), 8 * ((size_t)n_pairs + 1), cudaMemcpyHostToDevice, st));
     gather_depths_pack_kernel<T><<<(unsigned)n_pairs, 256, 0, st>>>(g);
     LAUNCHED();
     CK(cudaStreamSynchronize(st));   // `out` is a stack-lifetime host buffer

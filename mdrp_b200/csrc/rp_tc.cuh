@@ -277,27 +277,24 @@ RP_HD int need_outliers(int n, double sq_thr, int B0, double S0) {
     return need_d > 2.0e9 ? 0x7fffffff : (need_d < 1.0 ? 1 : (int)need_d);
 }
 
-// First correspondence of pass 1 (a multiple of the point tile; n itself = no second pass).  `sixteenths` > 0: a fixed
-// share of the pair.  Otherwise adaptive: a hopeless model collects ~0.97 certain outliers per correspondence, so it can be
-// dropped after need / 0.95 of them; pairs whose threshold sits beyond 85 % of their correspondences (many outliers, a
-// weak head) are not worth a second pass.  Any choice gives the same results — only the amount of work changes.
-RP_HD int tc_split(int n, int sixteenths, int need, int pct = 105) {
-    if (n < 4 * 64) return n;
-    long long s;
-    if (sixteenths > 0) s = (long long)n * sixteenths / 16;
-    else if (need > n) return n;
-    else s = (long long)need * pct / 100 + 1;
-    s = (s + 63) / 64 * 64;
+// First correspondence of pass 1 (a multiple of the point tile; n itself = no second pass), adaptive: a hopeless model
+// collects ~0.97 certain outliers per correspondence, so it can be dropped after need / 0.95 of them; the split sits at
+// 115 % of `need` (profiles/r02_tc_adapt_sweep.txt: 105 / 115 / 125 % and a fixed half, r02_tc_split_sweep.txt: fixed
+// shares); pairs whose threshold sits beyond 85 % of their correspondences (many outliers, a weak head) are not worth a
+// second pass.  Any choice gives the same results — only the amount of work changes.
+RP_HD int tc_split(int n, int need) {
+    if (n < 4 * 64 || need > n) return n;
+    const long long s = ((long long)need * 115 / 100 + 1 + 63) / 64 * 64;
     return s >= (long long)n * 85 / 100 ? n : (int)s;
 }
 
 // Per pair, once per chunk: the split of the two passes (the kernel's three warp roles only read it; evaluating
 // need_outliers' FP64 division per work item inside them cost 2-4 ms per 10 000 pairs).
-__global__ void tc_split_kernel(int n_pairs, const PairParams *pairs, const int *B0, const double *S0, int two_pass, int *split) {
+__global__ void tc_split_kernel(int n_pairs, const PairParams *pairs, const int *B0, const double *S0, int *split) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= n_pairs) return;
     const PairParams pp = pairs[p];
-    split[p] = two_pass > 0 ? tc_split(pp.n, two_pass, 0) : tc_split(pp.n, 0, need_outliers(pp.n, pp.sq_thr, B0[p], S0[p]), -two_pass);
+    split[p] = tc_split(pp.n, need_outliers(pp.n, pp.sq_thr, B0[p], S0[p]));
 }
 
 // ---- the kernel -------------------------------------------------------------------------------------------------

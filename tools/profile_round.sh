@@ -23,5 +23,4 @@ cap lm lm_warp_kernel 0
 cap score_survivors score_kernel 1
 cap solve solve2_kernel 0
 bash tools/all_configs_bench.sh > gpurun_out/${TAG}_all_configs.txt 2>&1
-# bash tools/head_sweep.sh > gpurun_out/${TAG}_head_sweep.txt 2>&1
 ls -la gpurun_out | head -40
