@@ -185,6 +185,45 @@ RP_API int rp_estimate_batch_dev_f32_quality(rp_ctx *ctx, int variant, int64_t n
                                              const float *quality, const double *cams, const rp_options *opt,
                                              rp_model *models, rp_stats *stats, uint8_t *masks, void *stream);
 
+/* ---- estimation from a prior ----------------------------------------------------
+ * The estimator with one prior model per pair (a tracker's previous pose, another method's estimate): the _quality
+ * twin's arguments with quality NULLABLE (NULL: the plain twin), plus init [n_pairs] inserted after opt, HOST memory for
+ * _host and DEVICE memory for _dev, in the layout and frame of the models the estimator returns (focal variants: f1, f2
+ * in pixels).  For each pair, RANSAC runs as the twin's except that before its first iteration the prior is scored
+ * (MSAC, as a minimal model is) and, as a minimal model that beats every earlier one, locally optimised by the in-loop LO;
+ * the best model, stats.model_score / num_inliers / inlier_ratio and the dynamic iteration limit are updated exactly as
+ * after an in-loop LO, and stats.refinements counts that LO.  Then come the sampled iterations (stats.iterations counts
+ * only those), the final LO, the final refinement and the mask, unchanged.  So:
+ *   - stats.model_score <= min(score(prior), score(LO(prior))): the result is never worse than the locally optimised
+ *     prior, and RANSAC still samples, so a wrong prior is recovered from;
+ *   - opt->max_iterations = 0 returns the LO of the prior, then the final LO and the final refinement (refinements 2);
+ *   - a prior with a non-finite field the variant reads (q, t, scale, shift1, shift2; f1, f2 for the focal variants)
+ *     means "no prior" for that pair: NaN rows leave pairs without a prior, and such a pair's bytes are the twin's;
+ *   - pairs of fewer than 3 correspondences keep the degenerate result (identity, iterations 0).
+ * The calibrated variants use q, t, scale, shift1, shift2 as given (RP_CALIB holds the shifts, as its LO does); the
+ * focal variants divide f1, f2 by the pair's normalisation scale, as the estimator's own frame is.  Results depend only
+ * on a pair's data, its prior, its quality and opt, never on the batch around it or on the chunking; the float32 entry
+ * points return the FP64 bytes.  A null init with n_pairs > 0 is RP_ERR_INVALID; every other check and error code is
+ * the twin's, and so is rp_pair_status.  rp_last_timing slot [15] reports the prior stage. */
+RP_API int rp_estimate_batch_host_init(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets,
+                                       const double *x1, const double *x2, const double *d1, const double *d2,
+                                       const float *quality, const double *cams, const rp_options *opt,
+                                       const rp_model *init, rp_model *models, rp_stats *stats, uint8_t *masks);
+RP_API int rp_estimate_batch_dev_init(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets,
+                                      const double *x1, const double *x2, const double *d1, const double *d2,
+                                      const float *quality, const double *cams, const rp_options *opt,
+                                      const rp_model *init, rp_model *models, rp_stats *stats, uint8_t *masks,
+                                      void *stream);
+RP_API int rp_estimate_batch_host_f32_init(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets,
+                                           const float *x1, const float *x2, const float *d1, const float *d2,
+                                           const float *quality, const double *cams, const rp_options *opt,
+                                           const rp_model *init, rp_model *models, rp_stats *stats, uint8_t *masks);
+RP_API int rp_estimate_batch_dev_f32_init(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets,
+                                          const float *x1, const float *x2, const float *d1, const float *d2,
+                                          const float *quality, const double *cams, const rp_options *opt,
+                                          const rp_model *init, rp_model *models, rp_stats *stats, uint8_t *masks,
+                                          void *stream);
+
 /* ---- refinement of caller-supplied models ----------------------------------------
  * What the estimator does after RANSAC, on start models the caller supplies (the previous frame pair's poses of a
  * tracker, another method's poses, an estimate to re-refine with other bundle options).  Pair p owns the
@@ -359,7 +398,8 @@ RP_API int rp_pair_status(const rp_ctx *ctx, int64_t n_pairs, int32_t *status);
  * widening waits for SMs those kernels hold; the device path's [13] is the widening alone.  [14] ordering of a
  * rp_estimate_batch_*_quality call: sort, permuting gather (which also widens float32 inputs, so [13] is 0 for these
  * calls) and mask scatter; 0 for every other call.  On the host path the sort and gather run on the copy stream after
- * the H2D of [9], so [14] there carries the same caveat as [13].  [15] reserved.
+ * the H2D of [9], so [14] there carries the same caveat as [13].  [15] the prior stage of a rp_estimate_batch_*_init call
+ * (import and exact scoring of the priors; its LO runs with the others in [5]), 0 for every other call.
  * counters: [0] minimal models generated, [1] point-scores the FP32 bound kernel resolved (models x correspondences),
  * [2] LM problems, [3] LM iterations, [4] chunks (= launches of each pipeline kernel), [5] minimal models
  * that needed the exact scorer, [6] point-scores the FP32 bound kernel actually evaluated (before abandoning),

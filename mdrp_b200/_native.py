@@ -27,6 +27,8 @@ EXPORTS = [
     "rp_gather_depths_dev_quality", "rp_gather_depths_dev_f32_quality", "rp_gather_depths_batch_dev_quality",
     "rp_gather_depths_batch_dev_f32_quality",
     "rp_refine_pairs_host", "rp_refine_pairs_dev", "rp_refine_pairs_host_f32", "rp_refine_pairs_dev_f32",
+    "rp_estimate_batch_host_init", "rp_estimate_batch_dev_init", "rp_estimate_batch_host_f32_init",
+    "rp_estimate_batch_dev_f32_init",
 ]
 ORDER_SMEM_CAP = 12288   # RP_ORDER_SMEM_CAP: larger pairs are ordered in global scratch
 
@@ -117,6 +119,14 @@ def load():
     for name in ("rp_estimate_batch_dev_quality", "rp_estimate_batch_dev_f32_quality"):
         getattr(L, name).restype = C.c_int
         getattr(L, name).argtypes = est_q_args + [VP]
+    # rp_estimate_batch_*_init: the quality twin's arguments (quality nullable) with init after opt
+    est_init_args = est_q_args[:11] + [VP] + est_q_args[11:]
+    for name in ("rp_estimate_batch_host_init", "rp_estimate_batch_host_f32_init"):
+        getattr(L, name).restype = C.c_int
+        getattr(L, name).argtypes = est_init_args
+    for name in ("rp_estimate_batch_dev_init", "rp_estimate_batch_dev_f32_init"):
+        getattr(L, name).restype = C.c_int
+        getattr(L, name).argtypes = est_init_args + [VP]
     # rp_refine_pairs_*: the estimator's arguments up to opt, then init, subset, models, bstats, num_inliers, inliers
     refine_args = est_args[:10] + [VP, VP, VP, VP, VP, VP]
     for name in ("rp_refine_pairs_host", "rp_refine_pairs_host_f32"):
@@ -268,7 +278,22 @@ class Context:
             fn, conv = self._lib.rp_estimate_batch_host_quality, _f64
         return self._estimate_host(fn, conv, variant, offsets, x1, x2, d1, d2, cams, opt, quality)
 
-    def _estimate_host(self, fn, conv, variant, offsets, x1, x2, d1, d2, cams, opt, quality=None):
+    def estimate_batch_host_init(self, variant, offsets, x1, x2, d1, d2, cams, opt: Options, init, quality=None):
+        """`estimate_batch_host` from one prior per pair (rp_estimate_batch_host[_f32]_init): `init` (MODEL_DTYPE [P], a
+        NaN row leaves its pair without a prior) is scored and locally optimised before RANSAC's first iteration.
+        `quality` (optional) as in `estimate_batch_host_quality`; float32 points and depths (all four) take the float32
+        entry point, anything else float64."""
+        init = np.ascontiguousarray(init, dtype=MODEL_DTYPE).reshape(-1)
+        if init.shape != (len(offsets) - 1,):
+            raise ValueError("init must hold one model per pair")
+        quality = _f32(quality) if quality is not None else None
+        if all(getattr(a, "dtype", None) == np.float32 for a in (x1, x2, d1, d2)):
+            fn, conv = self._lib.rp_estimate_batch_host_f32_init, _f32
+        else:
+            fn, conv = self._lib.rp_estimate_batch_host_init, _f64
+        return self._estimate_host(fn, conv, variant, offsets, x1, x2, d1, d2, cams, opt, quality, init)
+
+    def _estimate_host(self, fn, conv, variant, offsets, x1, x2, d1, d2, cams, opt, quality=None, init=None):
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         n_pairs = len(offsets) - 1
         x1, x2, d1, d2 = conv(x1), conv(x2), conv(d1), conv(d2)
@@ -283,10 +308,11 @@ class Context:
         models = np.zeros(n_pairs, dtype=MODEL_DTYPE)
         stats = np.zeros(n_pairs, dtype=STATS_DTYPE)
         masks = np.zeros(max(ntot, 1), dtype=np.uint8)
-        data = [_ptr(x1), _ptr(x2), _ptr(d1), _ptr(d2)] + ([_ptr(quality)] if quality is not None else [])
+        data = [_ptr(x1), _ptr(x2), _ptr(d1), _ptr(d2)] + ([_ptr(quality)] if quality is not None or init is not None else [])
+        prior = [_ptr(init)] if init is not None else []
         self._call(fn,
             self._h, int(variant), n_pairs, _ptr(offsets), *data,
-            _ptr(cams), C.byref(opt), _ptr(models), _ptr(stats), _ptr(masks))
+            _ptr(cams), C.byref(opt), *prior, _ptr(models), _ptr(stats), _ptr(masks))
         return models, stats, masks[:ntot]
 
     def estimate_batch_dev(self, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr, opt: Options,
@@ -315,12 +341,30 @@ class Context:
                            [x1_ptr, x2_ptr, d1_ptr, d2_ptr, quality_ptr or None], cams_ptr, opt, models_ptr, stats_ptr,
                            masks_ptr, stream)
 
-    def _estimate_dev(self, fn, variant, offsets, data, cams_ptr, opt, models_ptr, stats_ptr, masks_ptr, stream):
-        """`data`: the device pointers between offsets and cams (x1, x2, d1, d2 and, for quality calls, quality)."""
+    def estimate_batch_dev_init(self, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr, opt: Options, init_ptr,
+                                models_ptr, stats_ptr, masks_ptr, quality_ptr=None, stream=0):
+        """`estimate_batch_dev` from one prior per pair (rp_estimate_batch_dev_init): `init_ptr` points at [P] rp_model
+        in device memory (NaN rows: no prior); `quality_ptr` (optional) at float32 match qualities."""
+        self._estimate_dev(self._lib.rp_estimate_batch_dev_init, variant, offsets,
+                           [x1_ptr, x2_ptr, d1_ptr, d2_ptr, quality_ptr or None], cams_ptr, opt, models_ptr, stats_ptr,
+                           masks_ptr, stream, init_ptr)
+
+    def estimate_batch_dev_f32_init(self, variant, offsets, x1_ptr, x2_ptr, d1_ptr, d2_ptr, cams_ptr, opt: Options,
+                                    init_ptr, models_ptr, stats_ptr, masks_ptr, quality_ptr=None, stream=0):
+        """`estimate_batch_dev_init` with x1, x2, d1, d2 pointing at float32 device arrays (rp_estimate_batch_dev_f32_init)."""
+        self._estimate_dev(self._lib.rp_estimate_batch_dev_f32_init, variant, offsets,
+                           [x1_ptr, x2_ptr, d1_ptr, d2_ptr, quality_ptr or None], cams_ptr, opt, models_ptr, stats_ptr,
+                           masks_ptr, stream, init_ptr)
+
+    def _estimate_dev(self, fn, variant, offsets, data, cams_ptr, opt, models_ptr, stats_ptr, masks_ptr, stream,
+                      init_ptr=None):
+        """`data`: the device pointers between offsets and cams (x1, x2, d1, d2 and, for quality and prior calls,
+        quality); `init_ptr`: the priors of the _init calls."""
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        prior = [init_ptr] if init_ptr is not None else []
         self._call(fn,
             self._h, int(variant), len(offsets) - 1, _ptr(offsets), *data,
-            cams_ptr, C.byref(opt), models_ptr, stats_ptr, masks_ptr, stream or None)
+            cams_ptr, C.byref(opt), *prior, models_ptr, stats_ptr, masks_ptr, stream or None)
 
     # ---- refinement of caller-supplied models (rp_refine_pairs_*) --------------------------------
     def refine_pairs_host(self, variant, offsets, x1, x2, d1, d2, cams, opt: Options, init, subset=None):

@@ -241,9 +241,24 @@ def _pack_quality(quality, offsets):
     return np.concatenate(qs) if qs else np.zeros(0, dtype=np.float32)
 
 
-def _estimate_host(ctx, variant, offsets, x1, x2, d1, d2, cams, opt, quality=None):
+def _pack_priors(rows, n_pairs):
+    """One rp_model row per pair (None for a pair: no prior) -> MODEL_DTYPE [n_pairs] with NaN rows for the Nones; a
+    pair count that does not match the points raises ValueError."""
+    if len(rows) != n_pairs:
+        raise ValueError(f"initial models need one entry per pair ({n_pairs}), got {len(rows)}")
+    out = np.zeros(n_pairs, dtype=nv.MODEL_DTYPE)
+    out.view(np.float64).reshape(n_pairs, 12)[:] = np.nan
+    for i, r in enumerate(rows):
+        if r is not None:
+            out[i] = r
+    return out
+
+
+def _estimate_host(ctx, variant, offsets, x1, x2, d1, d2, cams, opt, quality=None, init=None):
     """Packed host arrays through the float32 entry point when they are float32, else the FP64 one; with a packed
-    `quality` through the quality entry point of that dtype."""
+    `quality` through the quality entry point of that dtype; with packed priors `init` through the _init entry point."""
+    if init is not None:
+        return ctx.estimate_batch_host_init(variant, offsets, x1, x2, d1, d2, cams, opt, init, quality)
     if quality is not None:
         return ctx.estimate_batch_host_quality(variant, offsets, x1, x2, d1, d2, cams, opt, quality)
     if x1.dtype == np.float32 and x2.dtype == np.float32 and d1.dtype == np.float32 and d2.dtype == np.float32:
@@ -263,28 +278,41 @@ def _geometry(m):
 
 # ---- batched entry points (the unit of GPU work) -----------------------------------------------------
 def estimate_monodepth_relative_pose_batch(points2D_1, points2D_2, depth_1, depth_2, cameras1, cameras2,
-                                           ransac_opt=None, bundle_opt=None, device=0, quality=None):
+                                           ransac_opt=None, bundle_opt=None, device=0, quality=None,
+                                           initial_geometries=None):
     """Lists (one entry per image pair) in, list of (MonoDepthTwoViewGeometry, info) out.  When every point and depth
     array is float32 the batch goes through the float32 entry point (same results, half the upload).
 
     `quality` (optional): one array of match qualities per pair (matcher scores, higher is better).  Each pair is then
     ordered by decreasing float32 quality on the device (ties: original index; NaN lowest) before the estimator runs,
-    which is the order PROSAC (`progressive_sampling`) expects; the inlier lists come back in the caller's order."""
+    which is the order PROSAC (`progressive_sampling`) expects; the inlier lists come back in the caller's order.
+
+    `initial_geometries` (optional): one MonoDepthTwoViewGeometry per pair (None: no prior for that pair), e.g. a
+    tracker's previous pose.  RANSAC scores and locally optimises it before its first iteration, so the result is never
+    worse than the locally optimised prior, and then samples as usual, so a wrong prior is recovered from;
+    `info["iterations"]` counts only the sampled iterations and `info["refinements"]` includes the prior's LO."""
     offsets, x1, x2, d1, d2 = _pack_auto(points2D_1, points2D_2, depth_1, depth_2)
     q = _pack_quality(quality, offsets) if quality is not None else None
+    init = (_pack_priors([None if g is None else _model_row(g) for g in initial_geometries], len(offsets) - 1)
+            if initial_geometries is not None else None)
     cams = np.array([Camera.from_any(a).fxfycxcy() + Camera.from_any(b).fxfycxcy()
                      for a, b in zip(cameras1, cameras2)], dtype=np.float64).reshape(-1, 8)
     opt = make_options(ransac_opt, bundle_opt, focal_variant=False)
     variant = nv.CALIB_SHIFT if opt.estimate_shift else nv.CALIB
-    models, stats, masks = _estimate_host(context(device), variant, offsets, x1, x2, d1, d2, cams, opt, q)
+    models, stats, masks = _estimate_host(context(device), variant, offsets, x1, x2, d1, d2, cams, opt, q, init)
     return [(_geometry(models[i]), _info(stats[i], masks[offsets[i]:offsets[i + 1]])) for i in range(len(models))]
 
 
-def _focal_batch(variant, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, bundle_opt, device, quality=None):
+def _focal_batch(variant, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, bundle_opt, device, quality=None,
+                 initial_image_pairs=None):
     offsets, x1, x2, d1, d2 = _pack_auto(points2D_1, points2D_2, depth_1, depth_2)
     q = _pack_quality(quality, offsets) if quality is not None else None
+    init = (_pack_priors([None if p is None else _model_row(p.geometry, Camera.from_any(p.camera1).focal(),
+                                                            Camera.from_any(p.camera2).focal())
+                          for p in initial_image_pairs], len(offsets) - 1)
+            if initial_image_pairs is not None else None)
     opt = make_options(ransac_opt, bundle_opt, focal_variant=True)
-    models, stats, masks = _estimate_host(context(device), variant, offsets, x1, x2, d1, d2, None, opt, q)
+    models, stats, masks = _estimate_host(context(device), variant, offsets, x1, x2, d1, d2, None, opt, q, init)
     out = []
     for i, m in enumerate(models):
         pair = MonoDepthImagePair(_geometry(m), Camera("SIMPLE_PINHOLE", [m["f1"], 0.0, 0.0]),
@@ -294,15 +322,20 @@ def _focal_batch(variant, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, 
 
 
 def estimate_monodepth_shared_focal_relative_pose_batch(points2D_1, points2D_2, depth_1, depth_2,
-                                                        ransac_opt=None, bundle_opt=None, device=0, quality=None):
-    """`quality`: as in estimate_monodepth_relative_pose_batch."""
-    return _focal_batch(nv.SHARED, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, bundle_opt, device, quality)
+                                                        ransac_opt=None, bundle_opt=None, device=0, quality=None,
+                                                        initial_image_pairs=None):
+    """`quality`: as in estimate_monodepth_relative_pose_batch.  `initial_image_pairs` (optional): one MonoDepthImagePair
+    per pair (None: no prior), used as `initial_geometries` there; its cameras' focal lengths are the prior's."""
+    return _focal_batch(nv.SHARED, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, bundle_opt, device, quality,
+                        initial_image_pairs)
 
 
 def estimate_monodepth_varying_focal_relative_pose_batch(points2D_1, points2D_2, depth_1, depth_2,
-                                                         ransac_opt=None, bundle_opt=None, device=0, quality=None):
-    """`quality`: as in estimate_monodepth_relative_pose_batch."""
-    return _focal_batch(nv.VARYING, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, bundle_opt, device, quality)
+                                                         ransac_opt=None, bundle_opt=None, device=0, quality=None,
+                                                         initial_image_pairs=None):
+    """`quality`, `initial_image_pairs`: as in estimate_monodepth_shared_focal_relative_pose_batch."""
+    return _focal_batch(nv.VARYING, points2D_1, points2D_2, depth_1, depth_2, ransac_opt, bundle_opt, device, quality,
+                        initial_image_pairs)
 
 
 # ---- refinement of caller-supplied models (rp_refine_pairs_host[_f32]) ----------------------------------------

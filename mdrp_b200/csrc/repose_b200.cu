@@ -139,13 +139,24 @@ struct TcBufs {
 // re-run sub-batch of S pairs and n correspondences (rerun_flagged): pair index and offsets, the gathered inputs, the
 // sub-batch's outputs.  The batch depth gather borrows idx, src, dst and x1 … d2.
 struct SubBufs {
-    DevBuf idx, src, dst, x1, x2, d1, d2, cams, models, stats, mask;
-    cudaError_t reserve(int S, size_t n) {
+    DevBuf idx, src, dst, x1, x2, d1, d2, cams, models, stats, mask, init;
+    cudaError_t reserve(int S, size_t n, bool prior) {
+        if (prior) {
+            if (const cudaError_t e = init.reserve(sizeof(Model) * S)) return e;
+        }
         return reserve_all({{&idx, sizeof(int) * S}, {&src, 8 * (size_t)S}, {&dst, 8 * ((size_t)S + 1)}, {&x1, 16 * n},
                             {&x2, 16 * n}, {&d1, 8 * n}, {&d2, 8 * n}, {&cams, 64 * (size_t)S}, {&models, sizeof(Model) * S},
                             {&stats, sizeof(rp_stats) * S}, {&mask, n}});
     }
 };
+// priors (estimator calls with init): the prior of each pair in the normalised frame and its exact count and score
+struct PriorBufs {
+    DevBuf model, count, score;
+    cudaError_t reserve(int P) {
+        return reserve_all({{&model, sizeof(Model) * P}, {&count, sizeof(int) * P}, {&score, sizeof(double) * P}});
+    }
+};
+constexpr size_t PRIOR_BYTES_PER_PAIR = sizeof(Model) + sizeof(int) + sizeof(double);
 // the remaining scratch
 struct ScratchBufs {
     DevBuf order;     // quality calls: global sort scratch of pairs above RP_ORDER_SMEM_CAP
@@ -153,14 +164,15 @@ struct ScratchBufs {
     DevBuf tmp2;      // rp_refine_batch: bundle stats
 };
 
-// Device bytes per pair of an estimator chunk (the chunk planner's estimate; the reserves above are the exact sizes)
-size_t bytes_per_pair(int iters, long long avg_points, int ev_cap = EV, size_t input_bytes = 0) {
+// Device bytes per pair of an estimator chunk (the chunk planner's estimate; the reserves above are the exact sizes);
+// `pair_bytes`: per-pair extras (PRIOR_BYTES_PER_PAIR with priors)
+size_t bytes_per_pair(int iters, long long avg_points, int ev_cap = EV, size_t input_bytes = 0, size_t pair_bytes = 0) {
     const int nseg = std::max(1, cdiv(iters, SEG));
     const size_t slots_pp = (size_t)nseg * 4 * SEG;
     // per slot: model, hyp_iter, score, count, ub, lb, survivor list, tensor-core count + list; per correspondence:
     // FP64 / FP32 / interleaved copies, bearings, mask, 128-byte feature row, `input_bytes` of input staging
     return slots_pp * (sizeof(Model) + 4 + 8 + 4 + 12 + 8) + (size_t)iters * 12 + (size_t)ev_cap * (sizeof(Model) + 24) +
-           (size_t)avg_points * (sizeof(Pt64) + 32 + sizeof(Bear) + 1 + 128 + input_bytes) + 1024;
+           (size_t)avg_points * (sizeof(Pt64) + 32 + sizeof(Bear) + 1 + 128 + input_bytes) + 1024 + pair_bytes;
 }
 
 // Device workspace of a refine chunk.  Per correspondence: pts64 (32 B), pts32 (16), the pair-interleaved FP32 copy
@@ -201,8 +213,9 @@ struct StageSet {
 constexpr int HEAD_SMALL = 32, MID_END = 256;
 
 // run_chunk: [0..8] stage boundaries, [9] start of the bulk cascade, [10] bound kernel done, [11] tensor-core tier done;
-// [12], [13]: an interval of their own (the mask scatter of quality calls, rp_measure_pipes)
-constexpr int N_EVENTS = 14;
+// [12], [13]: an interval of their own (the mask scatter of quality calls, rp_measure_pipes); [14] start of the prior
+// stage (calls with priors: it ends at [1])
+constexpr int N_EVENTS = 15;
 
 }  // namespace
 
@@ -220,6 +233,7 @@ struct rp_ctx {
     PruneBufs prn;
     TcBufs tcb;
     SubBufs sub;
+    PriorBufs pri;
     ScratchBufs scratch;
     StageSet set[2];
     cudaEvent_t ev[N_EVENTS];
@@ -379,7 +393,7 @@ struct ChunkIO {
     long long n_points = 0;
     const long long *h_offsets_rel = nullptr;  // host, [n_pairs+1], relative to the chunk
     const double *x1 = nullptr, *x2 = nullptr, *d1 = nullptr, *d2 = nullptr, *cams = nullptr;  // device, chunk-local
-    const Model *init = nullptr;               // refinement: start models [n_pairs]
+    const Model *init = nullptr;               // refinement: start models; estimator: priors (null: none) [n_pairs]
     const unsigned char *subset = nullptr;     // refinement: [n_points] or null (every correspondence)
     Model *models_out = nullptr;               // [n_pairs] (refinement: may alias init)
     rp_stats *stats_out = nullptr;             // estimator: [n_pairs]
@@ -491,6 +505,10 @@ struct Chunk {
     Model *models;
     double *score;
     int *hyp_iter, *count, *seg_count, *item_prefix;
+    // with priors (io->init): the normalised priors and their exact counts and scores; null otherwise
+    Model *prior;
+    int *prior_cnt;
+    double *prior_score;
 };
 
 Chunk chunk_of(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io, int iters, int ev_cap,
@@ -505,7 +523,26 @@ Chunk chunk_of(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &i
     c.models = ctx->hyp.models.as<Model>(); c.hyp_iter = ctx->hyp.hyp_iter.as<int>(); c.score = ctx->hyp.score.as<double>();
     c.count = ctx->hyp.count.as<int>(); c.seg_count = ctx->hyp.seg_count.as<int>();
     c.item_prefix = ctx->hyp.item_prefix.as<int>();
+    const bool pri = io.init != nullptr;
+    c.prior = pri ? ctx->pri.model.as<Model>() : nullptr;
+    c.prior_cnt = pri ? ctx->pri.count.as<int>() : nullptr;
+    c.prior_score = pri ? ctx->pri.score.as<double>() : nullptr;
     return c;
+}
+
+// 1b. the prior stage (calls with priors): the priors into the normalised frame, and one exact score per pair with a
+// usable prior (count, score of the prior: scan_kernel's starting point, the seed of the cascade's bars, the merge's
+// first event)
+int prior_stage(rp_ctx *ctx, const Chunk &c) {
+    prior_import_kernel<<<cdiv(c.P, 256), 256, 0, c.st>>>(c.P, c.variant, c.pairs, c.io->init, c.prior,
+                                                          ctx->res.ones.as<int>(), c.prior_cnt, c.prior_score);
+    LAUNCHED();
+    build_items_kernel<<<1, 1024, 0, c.st>>>(c.P, ctx->res.ones.as<int>(), ctx->res.one_prefix.as<int>(),
+                                             &c.sc->n_one_items, nullptr);
+    LAUNCHED();
+    ScoreArgs s = pair_score_args(ctx, c.P, c.prior, nullptr);
+    s.score = c.prior_score; s.count = c.prior_cnt;
+    return launch_score(ctx, c.pose, false, s, c.st);
 }
 
 // 2. sample
@@ -723,7 +760,8 @@ int score_minimal(rp_ctx *ctx, const Chunk &c) {
     int rc = launch_score(ctx, c.pose, false, sa, st);
     if (rc) return rc;
     pair_bounds_kernel<<<cdiv((long long)P * 32, 256), 256, 0, st>>>(P, c.nseg, first_cnt, c.score, c.count,
-                                                                   W.B0.as<int>(), W.S0.as<double>());
+                                                                   W.B0.as<int>(), W.S0.as<double>(), c.prior_cnt,
+                                                                   c.prior_score);
     LAUNCHED();
     // 4b. the mid stage, 4c. the bulk
     if (c.mid && (rc = cascade(ctx, c, HEAD_SMALL, MID_END, false, nullptr, nullptr))) return rc;
@@ -738,12 +776,13 @@ int scan_stage(rp_ctx *ctx, const Chunk &c) {
     a.n_pairs = c.P; a.nseg = c.nseg; a.seg_count = c.seg_count; a.score = c.score; a.count = c.count;
     a.events = L.events.as<int>(); a.n_events = L.n_events.as<int>(); a.ev_cap = c.ev_cap;
     a.pair_flags = L.pair_flags.as<int>(); a.any_flag = &c.sc->any_flag;
+    a.prior_cnt = c.prior_cnt; a.prior_score = c.prior_score;
     scan_kernel<<<cdiv((long long)c.P * 32, 256), 256, 0, c.st>>>(a);
     LAUNCHED();
     LoPrepArgs l;
     l.n_pairs = c.P; l.nseg = c.nseg; l.events = a.events; l.n_events = a.n_events; l.hyp_iter = c.hyp_iter; l.ev_cap = c.ev_cap;
     l.models = c.models; l.lo_models = L.lo_models.as<Model>(); l.lo_of_event = L.lo_of_event.as<int>();
-    l.lo_count = L.lo_count.as<int>(); l.prob_list = L.prob_list.as<int>(); l.n_prob = &c.sc->n_prob;
+    l.lo_count = L.lo_count.as<int>(); l.prob_list = L.prob_list.as<int>(); l.n_prob = &c.sc->n_prob; l.prior = c.prior;
     lo_prepare_kernel<<<cdiv(c.P, 128), 128, 0, c.st>>>(l);
     LAUNCHED();
     return RP_OK;
@@ -796,6 +835,7 @@ int merge_stage(rp_ctx *ctx, const Chunk &c) {
     m.models = c.models; m.lo_score = L.lo_score.as<double>(); m.lo_count_inl = L.lo_cnt.as<int>();
     m.lo_models = L.lo_models.as<Model>(); m.lo_count = L.lo_count.as<int>();
     m.best = R.best.as<Model>(); m.stats = R.stats.as<rp_stats>(); m.final_start = R.final_start.as<Model>();
+    m.prior = c.prior; m.prior_score = c.prior_score; m.prior_cnt = c.prior_cnt;
     merge_kernel<<<cdiv(P, 128), 128, 0, st>>>(m);
     LAUNCHED();
     // final LO from the best model, rescore, accept when strictly better
@@ -836,10 +876,16 @@ int read_back(rp_ctx *ctx, const Chunk &c, std::vector<int> &flags) {
     Scalars h_sc;
     CK(cudaMemcpyAsync(&h_sc, c.sc, sizeof h_sc, cudaMemcpyDeviceToHost, c.st));
     CK(cudaStreamSynchronize(c.st));
+    const bool pri = c.prior != nullptr;
     for (int i = 0; i < 8; ++i) {
         float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, ev[i], ev[i + 1]));
+        CK(cudaEventElapsedTime(&ms, ev[i], i == 0 && pri ? ev[14] : ev[i + 1]));
         ctx->last_ms[i] += ms;
+    }
+    if (pri) {
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, ev[14], ev[1]));
+        ctx->last_ms[15] += ms;
     }
     {
         float ms = 0.f;
@@ -886,6 +932,7 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
     CK(ctx->res.reserve(P, true));
     if (ctx->prune) CK(ctx->prn.reserve(P, nseg));
     if (ctx->prune && ctx->tc) CK(ctx->tcb.reserve(P, io.n_points, nseg));
+    if (io.init) CK(ctx->pri.reserve(P));
     cudaEvent_t *ev = ctx->ev;
     // 1. prepare, and the tensor-core tier's feature rows
     int rc = prepare_chunk(ctx, variant, opt, io, ev[0], st);
@@ -894,6 +941,10 @@ int run_chunk(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO &io
     if (c.use_tc && c.N > 0) {
         tc::tc_features_kernel<<<cdiv(c.N, 256), 256, 0, st>>>(c.N, c.pts32, ctx->tcb.feat.as<float4>());
         LAUNCHED();
+    }
+    if (c.prior) {
+        CK(cudaEventRecord(ev[14], st));
+        if ((rc = prior_stage(ctx, c))) return rc;
     }
     CK(cudaEventRecord(ev[1], st));
     if ((rc = sample_stage(ctx, c))) return rc;
@@ -992,7 +1043,7 @@ int rerun_flagged(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO
             long long npts = 0;
             while (end < todo.size()) {
                 const long long n = rel[(size_t)todo[end] + 1] - rel[(size_t)todo[end]];
-                const size_t b = bytes_per_pair(iters, n, ev_cap);
+                const size_t b = bytes_per_pair(iters, n, ev_cap, 0, io.init ? PRIOR_BYTES_PER_PAIR : 0);
                 if (end > pos && bytes + b > ctx->workspace_budget) break;
                 bytes += b;
                 npts += n;
@@ -1011,7 +1062,7 @@ int rerun_flagged(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO
             std::vector<int> flags;
             do {  // single pass; `break` = this sub-batch failed
                 SubBufs &B = ctx->sub;
-                if (B.reserve(S, nn)) {
+                if (B.reserve(S, nn, io.init != nullptr)) {
                     rc = RP_ERR_CUDA;
                     break;
                 }
@@ -1027,6 +1078,7 @@ int rerun_flagged(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO
                 g.models = io.models_out; g.stats = io.stats_out; g.masks = io.masks_out;
                 g.smodels = B.models.as<Model>(); g.sstats = B.stats.as<rp_stats>();
                 g.smasks = B.mask.as<unsigned char>();
+                g.init = io.init; g.sinit = io.init ? B.init.as<Model>() : nullptr;
                 gather_pairs_kernel<<<S, 256, 0, st>>>(g);
                 LAUNCHED();
                 CK(cudaStreamSynchronize(st));  // idx / src / dst are stack-lifetime host buffers
@@ -1035,6 +1087,7 @@ int rerun_flagged(rp_ctx *ctx, int variant, const rp_options &opt, const ChunkIO
                 sub.x1 = g.sx1; sub.x2 = g.sx2; sub.d1 = g.sd1; sub.d2 = g.sd2; sub.cams = pose ? g.scams : nullptr;
                 sub.models_out = B.models.as<Model>(); sub.stats_out = B.stats.as<rp_stats>();
                 sub.masks_out = B.mask.as<unsigned char>();
+                sub.init = g.sinit;
                 rc = run_chunk(ctx, variant, opt, sub, iters, ev_cap, flags, st);
                 if (rc) break;
                 scatter_pairs_kernel<<<S, 256, 0, st>>>(g);
@@ -1286,12 +1339,13 @@ int run_chunks(rp_ctx *ctx, const BatchIn<In> &b, const std::vector<int64_t> &bo
 // points; In = float: the _f32 ones (24 B per correspondence uploaded instead of 48, then widened); quality != null: the
 // _quality ones, whose chunks run_chunk and rerun_flagged see in the quality order and whose masks they write in that
 // order, which scatter_masks_kernel writes back in the caller's order.  Either way every kernel after stage_inputs
-// reads the same FP64 chunk arrays as the FP64 entry points.
+// reads the same FP64 chunk arrays as the FP64 entry points.  init != null: the _init ones, one prior per pair (host
+// memory on the host path, uploaded with the chunk's inputs; device memory on the device path).
 template <class In>
 int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const In *x1,
                   const In *x2, const In *d1, const In *d2, const float *quality, const double *cams,
-                  const rp_options *opt_in, rp_model *models, rp_stats *stats, uint8_t *masks, bool host_io,
-                  cudaStream_t st) {
+                  const rp_options *opt_in, const rp_model *init, rp_model *models, rp_stats *stats, uint8_t *masks,
+                  bool host_io, cudaStream_t st) {
     constexpr bool f32 = std::is_same<In, float>::value;
     const bool ordered = quality != nullptr;
     const bool staged = f32 || ordered;   // the chunk is widened or ordered before its kernels
@@ -1316,9 +1370,10 @@ int estimate_impl(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offs
     // gathered copy, the order and the ordered-layout mask (device path).
     size_t in_bytes = f32 ? 48 : 0;
     if (ordered) in_bytes = host_io ? 2 * (6 * sizeof(In) + 4 + 4 + 1) : 48 + 4 + 1;
-    const std::vector<int64_t> bounds =
-        plan_chunks(ctx, n_pairs, bytes_per_pair(iters0, Ntot / n_pairs + 1, ctx->ev_cap0, in_bytes), host_io, true);
-    const BatchIn<In> b = {offsets, x1, x2, d1, d2, pose ? cams : nullptr, quality, nullptr, nullptr, host_io};
+    const std::vector<int64_t> bounds = plan_chunks(
+        ctx, n_pairs, bytes_per_pair(iters0, Ntot / n_pairs + 1, ctx->ev_cap0, in_bytes, init ? PRIOR_BYTES_PER_PAIR : 0),
+        host_io, true);
+    const BatchIn<In> b = {offsets, x1, x2, d1, d2, pose ? cams : nullptr, quality, init, nullptr, host_io};
     double stage_per_point0 = 0.0;  // host path: widening / ordering time of chunk 0 per correspondence (ms)
     auto work = [&](int64_t c, StageSet &s, ChunkIO &io) -> int {
         const int64_t p0 = bounds[c];
@@ -1560,7 +1615,7 @@ int rp_estimate_batch_host(rp_ctx *ctx, int variant, int64_t n_pairs, const int6
     if (!ctx) return RP_ERR_INVALID;
     if (n_pairs > 0 && (!x1 || !x2 || !d1 || !d2 || !models || !stats || !masks))
         return fail(ctx, RP_ERR_INVALID, "null data pointer");
-    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, nullptr, cams, opt, models, stats, masks, true,
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, nullptr, cams, opt, nullptr, models, stats, masks, true,
                          ctx->stream);
 }
 
@@ -1570,7 +1625,7 @@ int rp_estimate_batch_dev(rp_ctx *ctx, int variant, int64_t n_pairs, const int64
     if (!ctx) return RP_ERR_INVALID;
     if (n_pairs > 0 && (!x1 || !x2 || !d1 || !d2 || !models || !stats || !masks))
         return fail(ctx, RP_ERR_INVALID, "null data pointer");
-    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, nullptr, cams, opt, models, stats, masks, false,
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, nullptr, cams, opt, nullptr, models, stats, masks, false,
                          stream ? (cudaStream_t)stream : ctx->stream);
 }
 
@@ -1580,7 +1635,7 @@ int rp_estimate_batch_host_f32(rp_ctx *ctx, int variant, int64_t n_pairs, const 
     if (!ctx) return RP_ERR_INVALID;
     if (n_pairs > 0 && (!x1 || !x2 || !d1 || !d2 || !models || !stats || !masks))
         return fail(ctx, RP_ERR_INVALID, "null data pointer");
-    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, nullptr, cams, opt, models, stats, masks, true,
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, nullptr, cams, opt, nullptr, models, stats, masks, true,
                          ctx->stream);
 }
 
@@ -1590,7 +1645,7 @@ int rp_estimate_batch_dev_f32(rp_ctx *ctx, int variant, int64_t n_pairs, const i
     if (!ctx) return RP_ERR_INVALID;
     if (n_pairs > 0 && (!x1 || !x2 || !d1 || !d2 || !models || !stats || !masks))
         return fail(ctx, RP_ERR_INVALID, "null data pointer");
-    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, nullptr, cams, opt, models, stats, masks, false,
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, nullptr, cams, opt, nullptr, models, stats, masks, false,
                          stream ? (cudaStream_t)stream : ctx->stream);
 }
 
@@ -1606,7 +1661,7 @@ int rp_estimate_batch_host_quality(rp_ctx *ctx, int variant, int64_t n_pairs, co
                                    const double *cams, const rp_options *opt, rp_model *models, rp_stats *stats,
                                    uint8_t *masks) {
     RP_QUALITY_CHECKS();
-    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, models, stats, masks, true,
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, nullptr, models, stats, masks, true,
                          ctx->stream);
 }
 
@@ -1615,7 +1670,7 @@ int rp_estimate_batch_dev_quality(rp_ctx *ctx, int variant, int64_t n_pairs, con
                                   const double *cams, const rp_options *opt, rp_model *models, rp_stats *stats,
                                   uint8_t *masks, void *stream) {
     RP_QUALITY_CHECKS();
-    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, models, stats, masks, false,
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, nullptr, models, stats, masks, false,
                          stream ? (cudaStream_t)stream : ctx->stream);
 }
 
@@ -1624,7 +1679,7 @@ int rp_estimate_batch_host_f32_quality(rp_ctx *ctx, int variant, int64_t n_pairs
                                        const double *cams, const rp_options *opt, rp_model *models, rp_stats *stats,
                                        uint8_t *masks) {
     RP_QUALITY_CHECKS();
-    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, models, stats, masks, true,
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, nullptr, models, stats, masks, true,
                          ctx->stream);
 }
 
@@ -1633,8 +1688,51 @@ int rp_estimate_batch_dev_f32_quality(rp_ctx *ctx, int variant, int64_t n_pairs,
                                       const double *cams, const rp_options *opt, rp_model *models, rp_stats *stats,
                                       uint8_t *masks, void *stream) {
     RP_QUALITY_CHECKS();
-    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, models, stats, masks, false,
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, nullptr, models, stats, masks, false,
                          stream ? (cudaStream_t)stream : ctx->stream);
+}
+
+// prior calls: the _quality twins' checks with quality nullable, and an init array for a non-empty batch
+#define RP_INIT_CHECKS()                                                                             \
+    if (!ctx) return RP_ERR_INVALID;                                                                 \
+    if (n_pairs > 0 && (!x1 || !x2 || !d1 || !d2 || !models || !stats || !masks))                     \
+        return fail(ctx, RP_ERR_INVALID, "null data pointer");                                       \
+    if (n_pairs > 0 && !init) return fail(ctx, RP_ERR_INVALID, "null init")
+
+int rp_estimate_batch_host_init(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const double *x1,
+                                const double *x2, const double *d1, const double *d2, const float *quality,
+                                const double *cams, const rp_options *opt, const rp_model *init, rp_model *models,
+                                rp_stats *stats, uint8_t *masks) {
+    RP_INIT_CHECKS();
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, init, models, stats, masks,
+                         true, ctx->stream);
+}
+
+int rp_estimate_batch_dev_init(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const double *x1,
+                               const double *x2, const double *d1, const double *d2, const float *quality,
+                               const double *cams, const rp_options *opt, const rp_model *init, rp_model *models,
+                               rp_stats *stats, uint8_t *masks, void *stream) {
+    RP_INIT_CHECKS();
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, init, models, stats, masks,
+                         false, stream ? (cudaStream_t)stream : ctx->stream);
+}
+
+int rp_estimate_batch_host_f32_init(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const float *x1,
+                                    const float *x2, const float *d1, const float *d2, const float *quality,
+                                    const double *cams, const rp_options *opt, const rp_model *init, rp_model *models,
+                                    rp_stats *stats, uint8_t *masks) {
+    RP_INIT_CHECKS();
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, init, models, stats, masks,
+                         true, ctx->stream);
+}
+
+int rp_estimate_batch_dev_f32_init(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const float *x1,
+                                   const float *x2, const float *d1, const float *d2, const float *quality,
+                                   const double *cams, const rp_options *opt, const rp_model *init, rp_model *models,
+                                   rp_stats *stats, uint8_t *masks, void *stream) {
+    RP_INIT_CHECKS();
+    return estimate_impl(ctx, variant, n_pairs, offsets, x1, x2, d1, d2, quality, cams, opt, init, models, stats, masks,
+                         false, stream ? (cudaStream_t)stream : ctx->stream);
 }
 
 int rp_refine_pairs_host(rp_ctx *ctx, int variant, int64_t n_pairs, const int64_t *offsets, const double *x1,

@@ -1170,16 +1170,18 @@ __global__ void tc_select_list_kernel(TcSelectArgs a) {
     }
 }
 
-// B0 / S0 of a pair: max count and min score over its first `first_cnt` (<= HB) models, scored exactly
+// B0 / S0 of a pair: max count and min score over its first `first_cnt` (<= HB) models, scored exactly, and over the
+// prior (prior_cnt / prior_score, optional), which precedes every minimal model
 __global__ void pair_bounds_kernel(int n_pairs, int nseg, const int *first_cnt, const double *score, const int *count,
-                                   int *B0, double *S0) {
+                                   int *B0, double *S0, const int *prior_cnt = nullptr,
+                                   const double *prior_score = nullptr) {
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (warp >= n_pairs) return;
     const size_t slot0 = (size_t)warp * nseg * (4 * SEG);
     const int cnt = first_cnt[warp];
-    int b = 0;
-    double s = DBL_MAX;
+    int b = prior_cnt ? prior_cnt[warp] : 0;
+    double s = prior_score ? fmin(DBL_MAX, prior_score[warp]) : DBL_MAX;
     for (int h = lane; h < cnt; h += 32) {
         b = max(b, count[slot0 + h]);
         const double v = score[slot0 + h];
@@ -1327,7 +1329,9 @@ __global__ void wave_select_kernel(WaveArgs a) {
 // scan: the part of score_models() so@0x22ebc0 that does not depend on LO results.  A minimal
 // model "triggers" when it has more inliers than every earlier minimal model or a lower MSAC
 // score than every earlier one (running max / running min, strict).  One warp per pair walks the
-// pair's slots in order and emits the triggering slots.
+// pair's slots in order and emits the triggering slots.  With a prior, the running best starts from the prior's
+// (count, score) and the prior, when it triggers, is event 0 with slot PRIOR_SLOT.
+constexpr int PRIOR_SLOT = -1;
 constexpr int PAIR_FLAG_OVERFLOW = 1;   // more trigger events than the list holds: outputs of the pair are void
 constexpr int PAIR_FLAG_NEED_MORE = 2;  // early termination: neither stopped nor at max_iterations within the generated iterations
 
@@ -1341,6 +1345,8 @@ struct ScanArgs {
     int ev_cap;       // capacity of a pair's event list (EV; larger when an overflowing pair is re-run)
     int *pair_flags;  // [n_pairs] PAIR_FLAG_OVERFLOW is set for a pair with more triggers than ev_cap
     int *any_flag;    // scalar: some pair was flagged
+    const int *prior_cnt;       // [n_pairs] or null: the prior's exact count and score (0, DBL_MAX: no prior)
+    const double *prior_score;
 };
 
 __global__ void scan_kernel(ScanArgs a) {
@@ -1350,6 +1356,18 @@ __global__ void scan_kernel(ScanArgs a) {
     long long best_cnt = 0;  // best_minimal_inlier_count starts at 0
     double best_score = DBL_MAX;
     int nev = 0;
+    if (a.prior_cnt) {
+        // score_models on {prior} before the first iteration: the same strict test against (0, DBL_MAX)
+        const long long c = a.prior_cnt[warp];
+        double s = a.prior_score[warp];
+        if (s != s) s = DBL_MAX;
+        if (c > best_cnt || s < best_score) {
+            if (lane == 0) a.events[(size_t)warp * a.ev_cap] = PRIOR_SLOT;
+            nev = 1;
+            best_cnt = c;
+            best_score = s;
+        }
+    }
     for (int seg = 0; seg < a.nseg; ++seg) {
         const int e = warp * a.nseg + seg;
         const int cnt = a.seg_count[e];
@@ -1404,6 +1422,7 @@ struct LoPrepArgs {
     int *lo_count;      // [n_pairs]
     int *prob_list;     // compact list of lo_models indices
     int *n_prob;
+    const Model *prior; // [n_pairs] or null: the model of a PRIOR_SLOT event
 };
 
 __global__ void lo_prepare_kernel(LoPrepArgs a) {
@@ -1413,12 +1432,14 @@ __global__ void lo_prepare_kernel(LoPrepArgs a) {
     const int nev = a.n_events[pair];
     const size_t eb = (size_t)pair * a.ev_cap;
     int nlo = 0;
+    // the prior is iteration -1, alone in it
+    auto iter_of = [&](int ev) { return ev == PRIOR_SLOT ? -1 : a.hyp_iter[pslot + ev]; };
     for (int i = 0; i < nev; ++i) {
         const int ev = a.events[eb + i];
-        const int it = a.hyp_iter[pslot + ev];
-        const bool last = (i + 1 == nev) || a.hyp_iter[pslot + a.events[eb + i + 1]] != it;
+        const int it = iter_of(ev);
+        const bool last = (i + 1 == nev) || iter_of(a.events[eb + i + 1]) != it;
         if (last) {
-            a.lo_models[eb + nlo] = a.models[pslot + ev];
+            a.lo_models[eb + nlo] = ev == PRIOR_SLOT ? a.prior[pair] : a.models[pslot + ev];
             a.lo_of_event[eb + i] = nlo;
             ++nlo;
         } else {
@@ -1456,6 +1477,9 @@ struct MergeArgs {
     Model *final_start;      // [n_pairs] copy of best (start of the final LO)
     int *pair_flags;         // [n_pairs] |= PAIR_FLAG_NEED_MORE when a pair neither stopped nor reached max_iterations
     int *any_flag;
+    const Model *prior;      // [n_pairs] or null: model, score and count of a PRIOR_SLOT event
+    const double *prior_score;
+    const int *prior_cnt;
 };
 
 __global__ void merge_kernel(MergeArgs a) {
@@ -1477,15 +1501,16 @@ __global__ void merge_kernel(MergeArgs a) {
         long long stop_it = -1, it_prev = -1;
         for (int i = 0; i < nev; ++i) {
             const int ev = a.events[eb + i];
-            const long long it_e = a.hyp_iter[pslot + ev];
+            const bool prior = ev == PRIOR_SLOT;   // before iteration 0: never a stopping point
+            const long long it_e = prior ? -1 : a.hyp_iter[pslot + ev];
             const long long cand = max(max(a.min_iterations + 1, (long long)floor(dyn_max_iter) + 1), it_prev + 1);
             if (cand <= it_e) { stop_it = cand; break; }
             it_prev = it_e;
-            const double s = a.score[pslot + ev];
+            const double s = prior ? a.prior_score[pair] : a.score[pslot + ev];
             if (s < st.model_score) {
                 st.model_score = s;
-                best = a.models[pslot + ev];
-                st.num_inliers = a.count[pslot + ev];
+                best = prior ? a.prior[pair] : a.models[pslot + ev];
+                st.num_inliers = prior ? a.prior_cnt[pair] : a.count[pslot + ev];
             }
             const int lo = a.lo_of_event[eb + i];
             if (lo >= 0) {
@@ -1591,6 +1616,30 @@ __global__ void refine_import_kernel(int n_pairs, int variant, const PairParams 
     if (bstats) bstats[pair] = rp_bundle_stats{};
 }
 
+// Estimator with priors: the prior of every pair in the normalised frame (focal variants: f1, f2 divided by nscale, as
+// refine_import_kernel does) and one scoring item for each valid pair whose prior is usable, that is, finite in every
+// field the variant reads (the calibrated variants do not read f1, f2).  (count, score) start at (0, DBL_MAX), which
+// is what a pair without a usable prior keeps: such a prior never triggers.  Thread per pair.
+__global__ void prior_import_kernel(int n_pairs, int variant, const PairParams *pairs, const Model *init, Model *work,
+                                    int *ones, int *count, double *score) {
+    const int pair = blockIdx.x * blockDim.x + threadIdx.x;
+    if (pair >= n_pairs) return;
+    const PairParams pp = pairs[pair];
+    Model m = init[pair];
+    const bool focal = variant == RP_SHARED || variant == RP_VARYING;
+    bool usable = isfinite(m.q.w) && isfinite(m.q.x) && isfinite(m.q.y) && isfinite(m.q.z) && isfinite(m.t.x) &&
+                  isfinite(m.t.y) && isfinite(m.t.z) && isfinite(m.scale) && isfinite(m.shift1) && isfinite(m.shift2);
+    if (focal) {
+        usable = usable && isfinite(m.f1) && isfinite(m.f2);
+        m.f1 /= pp.nscale;
+        m.f2 /= pp.nscale;
+    }
+    work[pair] = m;
+    ones[pair] = pp.valid && usable ? 1 : 0;
+    count[pair] = 0;
+    score[pair] = DBL_MAX;
+}
+
 // export: thread per pair.  A refined pair's model is the work model with f1, f2 multiplied by nscale (focal variants);
 // any other pair gets init's bytes (no nscale round trip).  With `count` (the masked score of the work models), the
 // pair's inlier count, 0 for pairs of fewer than 3 correspondences, which are not scored.  `out` may alias `init`.
@@ -1625,6 +1674,7 @@ struct SubBatchArgs {
     double *sx1, *sx2, *sd1, *sd2, *scams;    // compact inputs
     Model *models; rp_stats *stats; unsigned char *masks;        // chunk outputs
     const Model *smodels; const rp_stats *sstats; const unsigned char *smasks;   // compact outputs
+    const Model *init; Model *sinit;          // priors of the chunk (may be null) and of the compact batch
 };
 __global__ void gather_pairs_kernel(SubBatchArgs a) {
     const int j = blockIdx.x;
@@ -1640,6 +1690,7 @@ __global__ void gather_pairs_kernel(SubBatchArgs a) {
         a.sd2[d0 + i] = a.d2[so + i];
     }
     if (a.cams && threadIdx.x < 8) a.scams[8 * (size_t)j + threadIdx.x] = a.cams[8 * (size_t)a.pair_idx[j] + threadIdx.x];
+    if (a.init && threadIdx.x == 0) a.sinit[j] = a.init[a.pair_idx[j]];
 }
 __global__ void scatter_pairs_kernel(SubBatchArgs a) {
     const int j = blockIdx.x;

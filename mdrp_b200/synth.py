@@ -156,3 +156,23 @@ def make_batch(config: str, n_pairs: int, seed: int = 0, n: int | None = None):
     cams = None if focal else np.tile(np.array([f1, f1, PP[0], PP[1], f2, f2, PP[0], PP[1]]), (P, 1))
     return dict(offsets=np.arange(P + 1, dtype=np.int64) * n, x1=x1n.reshape(-1, 2), x2=x2n.reshape(-1, 2),
                 d1=d1.reshape(-1), d2=d2.reshape(-1), cams=cams, R=R, t=t, inliers=~outl.reshape(-1))
+
+
+def quat_from_rotmat(R):
+    """w-first unit quaternion of a rotation matrix (w >= 0)."""
+    R = np.asarray(R, dtype=np.float64)
+    w = np.sqrt(max(0.0, 1.0 + R[0, 0] + R[1, 1] + R[2, 2])) / 2.0
+    x = np.copysign(np.sqrt(max(0.0, 1.0 + R[0, 0] - R[1, 1] - R[2, 2])) / 2.0, R[2, 1] - R[1, 2])
+    y = np.copysign(np.sqrt(max(0.0, 1.0 - R[0, 0] + R[1, 1] - R[2, 2])) / 2.0, R[0, 2] - R[2, 0])
+    z = np.copysign(np.sqrt(max(0.0, 1.0 - R[0, 0] - R[1, 1] + R[2, 2])) / 2.0, R[1, 0] - R[0, 1])
+    q = np.array([w, x, y, z])
+    return q / np.linalg.norm(q)
+
+
+def gt_model(sc: Scene, rot_noise_deg: float = 0.0, seed: int = 0) -> np.ndarray:
+    """The scene's ground truth as a 12-vector model row (q, t, scale, shift1, shift2, f1, f2; f in pixels), with the
+    rotation turned by `rot_noise_deg` about a random axis and t turned by as much (a tracker-like prior)."""
+    rng = np.random.default_rng(seed)
+    dR = rodrigues(rng.normal(size=3), np.deg2rad(rot_noise_deg))
+    t = rodrigues(rng.normal(size=3), np.deg2rad(rot_noise_deg)) @ sc.t
+    return np.r_[quat_from_rotmat(dR @ sc.R), t, sc.scale, sc.shift1, sc.shift2, sc.f1, sc.f2]

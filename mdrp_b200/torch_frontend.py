@@ -102,14 +102,17 @@ def gather_depths_batch(depth_maps, frame1, frame2, offsets, keypoints1, keypoin
     return (out, x1[:m], x2[:m], d1[:m], d2[:m]) + (() if q_out is None else (q_out[:m],))
 
 
-def estimate_batch(variant, offsets, x1, x2, d1, d2, cams, opt: nv.Options, quality=None):
+def estimate_batch(variant, offsets, x1, x2, d1, d2, cams, opt: nv.Options, quality=None, init_models=None):
     """Packed CUDA float64 tensors in (offsets: host int64 array), CUDA tensors out:
     models [P,12] float64, stats [P,5] (int64 view; columns 3,4 are float64 bit patterns — use
     `stats_to_numpy`), masks [N] uint8.  When x1, x2, d1, d2 are all float32 they are passed as they are to the
     float32 entry point (no FP64 copy of the batch; the same results as float64 tensors of the same values).
     `quality` (optional): CUDA tensor [N] of match qualities, converted to float32 on the device; each pair is then
     ordered by decreasing quality before the estimator runs (rp_estimate_batch_dev[_f32]_quality), and the masks come
-    back in the caller's order."""
+    back in the caller's order.
+    `init_models` (optional): CUDA float64 tensor [P,12] of priors (e.g. the previous frame pair's `models`), a NaN row
+    for a pair without one; RANSAC scores and locally optimises each prior before its first iteration
+    (rp_estimate_batch_dev[_f32]_init)."""
     ctx = _ctx_for(x1)
     dev = x1.device
     offsets = np.ascontiguousarray(offsets, dtype=np.int64)
@@ -127,13 +130,23 @@ def estimate_batch(variant, offsets, x1, x2, d1, d2, cams, opt: nv.Options, qual
         quality = quality.contiguous().to(torch.float32)
         if quality.shape != (N,):
             raise ValueError("quality must be [N] with N = offsets[-1]")
+    if init_models is not None:
+        if not init_models.is_cuda or init_models.device != dev or init_models.dtype != torch.float64:
+            raise ValueError("init_models must be a CUDA float64 tensor on the device of the points")
+        init_models = init_models.contiguous()
+        if init_models.shape != (P, 12):
+            raise ValueError("init_models must be [n_pairs, 12]")
     models = torch.zeros(P, 12, dtype=torch.float64, device=dev)
     stats = torch.zeros(P, 5, dtype=torch.int64, device=dev)
     masks = torch.zeros(max(N, 1), dtype=torch.uint8, device=dev)
     outs = (models.data_ptr(), stats.data_ptr(), masks.data_ptr())
     stream = torch.cuda.current_stream(dev).cuda_stream
     cams_p = cams_t.data_ptr() if cams_t is not None else None
-    if quality is not None:
+    if init_models is not None:
+        est = ctx.estimate_batch_dev_f32_init if f32 else ctx.estimate_batch_dev_init
+        est(variant, offsets, x1.data_ptr(), x2.data_ptr(), d1.data_ptr(), d2.data_ptr(), cams_p, opt,
+            init_models.data_ptr(), *outs, quality.data_ptr() if quality is not None else None, stream)
+    elif quality is not None:
         est = ctx.estimate_batch_dev_f32_quality if f32 else ctx.estimate_batch_dev_quality
         est(variant, offsets, x1.data_ptr(), x2.data_ptr(), d1.data_ptr(), d2.data_ptr(), cams_p, opt, *outs,
             quality.data_ptr(), stream)
